@@ -2,7 +2,7 @@
 """Benchmark of the RecNet hot path on B200: train samples/s for decoder + local reconstructor (fwd + bwd + clip +
 Adam), MSVD shape, batch 100 per GPU, bf16 tensor-core GEMMs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--recon local|global|none]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--recon local|global|none] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1).  Prints ONE JSON line on rank 0 (contract in the task statement):
   value      device-timed throughput with inputs resident in HBM (CUDA-graph replay of the whole step)
@@ -44,7 +44,13 @@ def parse():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--cpu-iters", type=int, default=8)
     ap.add_argument("--no-extras", action="store_true", help="skip the fp32 record and the other-config workloads (N = 1 only anyway)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (losses, updated parameters and their gradients) "
+                         "as DIR/<name>.npy in float32; a tensor of more than 2^19 elements as the same seeded sample of positions every run")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def peaks():
@@ -111,7 +117,7 @@ def cpu_model_name():
 def run_reference(args, rank):
     if rank != 0:
         return
-    iters = max(1, min(args.steps, 12))
+    iters = args.steps
     sps, sec = cpu_oracle_samples_per_s(args.recon, iters, warmup=min(args.warmup, 1) or 1)
     cores = os.cpu_count() or 1
     sample = f"{iters} timed iterations of fwd+bwd+clip+Adam at batch {SHAPE['B']}, L=31, fp32, {cores} torch threads ({cpu_model_name()})"
@@ -326,7 +332,7 @@ def extra_records(args, dev, lib, T, synthetic_batch, pk):
     """fp32 build of the headline step + BASELINE configs 1 (decoder only), 2 (global reconstructor), 4 (greedy, batch 1024) and
     5 (MSR-VTT-shaped stress: 40 frames x 3584-d, 2-layer LSTM decoder, local reconstructor with R = 3584), batch 100 on this GPU."""
     C = T.C
-    steps, warm = max(10, min(args.steps, 20)), 3
+    steps, warm = args.steps, 3
     out = {}
 
     def train_record(shp, recon, precision, dec_layers=1, with_e2e=False):
@@ -412,6 +418,28 @@ def extra_records(args, dev, lib, T, synthetic_batch, pk):
     return out
 
 
+DUMP_SAMPLE = 1 << 19        # positions kept of a larger tensor: the headline step's dump stays near 30 MB (limit 64 MB)
+
+
+def dump_outputs(out_dir, tensors):
+    """Write each tensor as <out_dir>/<name>.npy in float32.  A tensor of more than DUMP_SAMPLE elements is reduced to DUMP_SAMPLE
+    flat positions drawn from a fixed seed, the same positions in every run, so that two builds can be compared output for output."""
+    import numpy as np
+    arrays = {}
+    for name, t in tensors.items():
+        a = t.detach().float().cpu()
+        if a.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            a = a.reshape(-1)[idx]
+        arrays[name] = a.numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the 64 MB limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def dbg(rank, msg):
     if os.environ.get("RECNET_BENCH_VERBOSE"):
         print(f"[bench rank {rank} {time.strftime('%H:%M:%S')}] {msg}", file=sys.stderr, flush=True)
@@ -476,11 +504,13 @@ def main():
     targets_d = torch.empty_like(targets_h, device=dev)
     feats_d.copy_(feats_h); targets_d.copy_(targets_h)
     loss_d = torch.zeros((), device=dev)
+    last = {}                                   # decoder / reconstructor loss tensors of the latest step (or capture)
 
     def make_step(fd, td):
         def _step():
             reducer.start_iteration()
-            loss, _, _ = T.train_step(dec, rec, fd, td, n_steps=L, reducer=reducer if world > 1 or dp_self else None)
+            loss, last["dec_loss"], last["rec_loss"] = T.train_step(dec, rec, fd, td, n_steps=L,
+                                                                    reducer=reducer if world > 1 or dp_self else None)
             loss_d.copy_(loss.detach())
         return _step
 
@@ -540,6 +570,21 @@ def main():
             graph = None
             torch.cuda.synchronize()
     dbg(rank, f"graph captured: {graph is not None}")
+
+    def step_outputs():
+        """The step's results as its caller sees them: losses, parameters, and the gradients its backward left in p.grad."""
+        outs = {"loss": loss_d, "dec_loss": last["dec_loss"]}
+        if last["rec_loss"] is not None:
+            outs["rec_loss"] = last["rec_loss"]
+        for prefix, d in (("decoder", dec), ("reconstructor", rec)):
+            for k, p in (d["model"].named_parameters() if d else ()):
+                outs[f"{prefix}.{k}"] = p
+                if p.grad is not None:
+                    outs[f"{prefix}.{k}.grad"] = p.grad
+        return outs
+    # each capture creates new loss and p.grad tensors (zero_grad(set_to_none=True)): keep the ones the replayed graph writes
+    # before the e2e leg's capture below replaces them
+    graph_outputs = step_outputs() if args.dump_outputs and graph is not None else None
     # e2e leg, single GPU: a second capture of the same step over a second pair of static input buffers (same memory pool), so
     # that step i+1's batch can be copied from pinned host memory STRAIGHT into its graph's inputs while step i runs
     # (no device-to-device hop through a staging buffer: 34 MB less L2 / HBM traffic per step).
@@ -598,6 +643,8 @@ def main():
     total_ms = timed(run, args.steps)
     clocks = sampler.stop() if sampler else None
     dbg(rank, f"timed region done: {total_ms:.2f} ms")
+    if args.dump_outputs and rank == 0:          # before the e2e leg below steps the same model further
+        dump_outputs(args.dump_outputs, graph_outputs if graph is not None else step_outputs())
 
     # ---- e2e: host buffers -> H2D -> step -> D2H loss, every step, inside the timed region ------------------------
     # Software pipeline: step i+1's batch is copied from pinned host memory into a staging buffer on a copy stream

@@ -24,7 +24,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
-from tests.golden.make_golden import CASES, OUT, REF, import_reference, make_inputs      # noqa: E402
+from tests.golden.make_golden import CASES, OUT, REF, import_reference, make_inputs, save_golden      # noqa: E402
 from tests.philox_ref import SITE_EMB, SITE_GLOBAL_MP, SITE_LOCAL_X, SITE_LOGITS, dropout_scales      # noqa: E402
 
 SEEDS = {"dec": 0xDEC0, "local": 0x10CA, "global": 0x610B}     # models.py: _init_rng seeds; offset is 1 in the first training forward
@@ -102,7 +102,7 @@ def train_case(name, c, ref_train):
             out[f"grad_{kind}.dec." + k] = p.grad.numpy().copy()
         for k, p in rec["model"].named_parameters():
             out[f"grad_{kind}.{kind}." + k] = p.grad.numpy().copy()
-    np.savez_compressed(os.path.join(OUT, name + "_train.npz"), **out)
+    save_golden(name, "_train", out)
     print(name + "_train", "dec_loss", float(out["dec_loss"]), "global", float(out["global_loss"]), "local", float(out["local_loss"]))
 
 

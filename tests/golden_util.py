@@ -12,16 +12,25 @@ GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 def golden_cases():
     """Eval-mode fixtures of make_golden.py (the train-mode / beam fixtures of make_golden_train.py have their own loaders below)."""
     names = sorted(os.path.splitext(os.path.basename(p))[0] for p in glob.glob(os.path.join(GOLDEN_DIR, "*.npz")))
-    return [n for n in names if not n.endswith("_train") and not n.endswith("_beam")]
+    return [n for n in names if not n.endswith(("_train", "_beam", "_inputs"))]
+
+
+def _arrays(name, suffix=""):
+    """<name><suffix>.npz, plus <name>_inputs.npz where the case keeps its shared inputs apart (make_golden.save_golden)."""
+    z = dict(np.load(os.path.join(GOLDEN_DIR, name + suffix + ".npz")))
+    shared = os.path.join(GOLDEN_DIR, name + "_inputs.npz")
+    if os.path.exists(shared):
+        z.update(np.load(shared))
+    return z
 
 
 def load_golden(name, dtype=torch.float64):
-    z = np.load(os.path.join(GOLDEN_DIR, name + ".npz"))
+    z = _arrays(name)
     meta = ast.literal_eval(str(z["meta"]))
 
     def group(prefix):
         out = {}
-        for k in z.files:
+        for k in z:
             if k.startswith(prefix):
                 t = torch.from_numpy(z[k])
                 out[k[len(prefix):]] = t.to(dtype) if t.is_floating_point() else t
@@ -43,12 +52,12 @@ def load_golden(name, dtype=torch.float64):
 
 def load_golden_train(name, dtype=torch.float64):
     """<name>_train.npz: the reference in TRAIN mode with the Philox masks of tests/philox_ref.py injected (make_golden_train.py)."""
-    z = np.load(os.path.join(GOLDEN_DIR, name + "_train.npz"))
+    z = _arrays(name, "_train")
     meta = ast.literal_eval(str(z["meta"]))
 
     def group(prefix):
         out = {}
-        for k in z.files:
+        for k in z:
             if k.startswith(prefix):
                 t = torch.from_numpy(z[k])
                 out[k[len(prefix):]] = t.to(dtype) if t.is_floating_point() else t

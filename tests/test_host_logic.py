@@ -13,7 +13,7 @@ from recnet_b200 import train as T
 from recnet_b200.data import shard_range, synthetic_batch
 from recnet_b200.parallel import GradAllReducer
 from oracle import recnet_oracle as O
-from tests.golden_util import load_golden
+from tests.golden_util import golden_cases, load_golden
 
 
 def test_state_dict_matches_reference_fixture_keys_and_shapes():
@@ -38,28 +38,37 @@ def test_default_shapes_are_the_msvd_ones():
     assert sum(p.numel() for p in dec.parameters()) == 9527692              # SURVEY 8a A0
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference not mounted (GPU box)")
 def test_same_seed_same_initial_weights_as_reference():
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_decoder", "/root/reference/models/decoder.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    args = ("LSTM", 1, 64, 20, 1, 32, 16, 101, 0.5, 0.5, 0.5)
-    torch.manual_seed(3)
-    a = ref.Decoder(*args).state_dict()
-    torch.manual_seed(3)
-    b = recnet_b200.Decoder(*args).state_dict()
-    for k in a:
-        assert torch.equal(a[k], b[k]), k
+    """Every fixture's decoder weights are what the reference's own constructor drew after torch.manual_seed(seed), with fp64 as
+    the default dtype (tests/golden/make_golden.py): the same seed draws the same weights here, bit for bit."""
+    for name in golden_cases():
+        g = load_golden(name)
+        m = g["meta"]
+        saved = torch.get_default_dtype()
+        torch.set_default_dtype(torch.float64)
+        try:
+            torch.manual_seed(m["seed"])
+            b = recnet_b200.Decoder(m["dec_model"], m["dec_layers"], m["E"], m["EMB"], 1, m["H"], m["A"], m["V"], 0.5, 0.5, 0.5).state_dict()
+        finally:
+            torch.set_default_dtype(saved)
+        assert list(b) == list(g["dec"]), name
+        for k, a in g["dec"].items():
+            assert torch.equal(a, b[k]), (name, k)
 
 
 def test_config_keeps_reference_attribute_names():
-    C = recnet_b200.TrainConfig
+    # the defaults as config.py declares them: other tests reconfigure the shared TrainConfig in place
+    import importlib.util
+    from recnet_b200 import config
+    spec = importlib.util.spec_from_file_location("recnet_config_defaults", config.__file__)
+    fresh = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(fresh)
+    C = fresh.TrainConfig
     for name, val in dict(decoder_model="GRU", reconstructor_model="LSTM", caption_max_len=30, batch_size=100, embedding_size=468,
                           encoder_output_size=1536, encoder_output_len=28, decoder_hidden_size=512, decoder_attn_size=128,
                           reconstructor_hidden_size=1536, reconstructor_attn_size=128, decoder_teacher_forcing_ratio=1.0,
                           gradient_clip=50.0, decoder_learning_rate=1e-5, reconstructor_learning_rate=1e-6).items():
-        assert getattr(C, name) == val
+        assert hasattr(recnet_b200.TrainConfig, name) and getattr(C, name) == val, name
     assert C.init_word2idx == {'<PAD>': 0, '<SOS>': 1, '<EOS>': 2}
 
 
