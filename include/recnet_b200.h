@@ -40,6 +40,12 @@ typedef enum {
 typedef enum { RECNET_PREC_FP32 = 0, RECNET_PREC_BF16 = 1 } recnet_precision;
 #define RECNET_MAX_LAYERS 4
 typedef enum { RECNET_CELL_LSTM = 0, RECNET_CELL_GRU = 1 } recnet_cell;   /* models/decoder.py:32-35: anything but "LSTM" is GRU */
+/* Flag OR'd into the `cell` field of recnet_decoder_desc / recnet_local_desc (the low byte holds the recnet_cell value):
+ * the paper's softmax attention, alpha = softmax over frames (decoder) / decoder steps (local reconstructor) of the scores e,
+ * context = sum alpha * v (no 1/T).  Without it (the default) the attention is the reference's: context = mean(e * v).
+ * Any other bit above the low byte makes the call return RECNET_ERR_UNSUPPORTED. */
+#define RECNET_ATTN_SOFTMAX 0x100
+#define RECNET_CELL_MASK 0xff
 
 /* Library / device checks.  recnet_query_device fails with RECNET_ERR_UNSUPPORTED_ARCH unless the
  * device is compute capability 10.x (sm_100a cubins only; no PTX fallback, no other arch). */
@@ -84,8 +90,9 @@ int recnet_splitk_reduce(const float* partial, int splits, int64_t split_stride,
  * U-projection, which is hoisted):  e = w.tanh(Wh + Uv + b);  ctx = mean_tau(e * V)   [no softmax: SURVEY 0.1].
  *   wh_partials [n_wh][B,A] fp32 (split-K partials of h W^T, summed here); uv[b*uv_bs + tau*uv_ts + a] fp32;
  *   v[b*v_bs + tau*v_ts + d] in `precision` storage; ctx_out[b*ctx_ld + d] in `precision` storage.
- *   wh_out [B,A], e_out [B,Tn] fp32: saved for backward (nullable).  normalize=1 -> softmax over frames
- *   (paper variant, forward only).  p_drop/rng/site/drop_base: train-mode dropout on ctx (local reconstructor). */
+ *   wh_out [B,A], e_out [B,Tn] fp32: saved for backward (nullable).  normalize=1 -> the paper's attention:
+ *   alpha = softmax_tau(e), ctx = sum_tau alpha * V, and e_out holds alpha (its backward: recnet_attn_bwd_softmax).
+ *   p_drop/rng/site/drop_base: train-mode dropout on ctx (local reconstructor). */
 int recnet_attn_fwd(int precision, const float* wh_partials, int n_wh, int64_t wh_stride, const float* uv,
                     int64_t uv_bs, int64_t uv_ts, const float* attn_b, const float* attn_w, const void* v,
                     int64_t v_bs, int64_t v_ts, int B, int Tn, int A, int D, int normalize, float* wh_out,
@@ -101,6 +108,13 @@ int recnet_attn_bwd(int precision, const float* dctx_partials, int n_p, int64_t 
                     const float* attn_b, const float* attn_w, int B, int Tn, int A, int D, float* dwh_out,
                     void* dwh_op, float* duv_acc, float* dw_acc, int first, float* dctx_out, float p_drop,
                     const uint64_t* rng, uint32_t site, int64_t drop_base, void* stream);
+/* Backward of recnet_attn_fwd(normalize=1), same arguments as recnet_attn_bwd plus alpha [B,Tn] fp32 = the e_out that forward
+ * wrote: d alpha = dctx . V, d e = alpha (d alpha - sum_tau alpha d alpha), then the same score backward. */
+int recnet_attn_bwd_softmax(int precision, const float* dctx_partials, int n_p, int64_t p_stride, int64_t p_ld, const void* v,
+                            int64_t v_bs, int64_t v_ts, const float* alpha, const float* wh, const float* uv, int64_t uv_bs,
+                            int64_t uv_ts, const float* attn_b, const float* attn_w, int B, int Tn, int A, int D, float* dwh_out,
+                            void* dwh_op, float* duv_acc, float* dw_acc, int first, float* dctx_out, float p_drop,
+                            const uint64_t* rng, uint32_t site, int64_t drop_base, void* stream);
 
 /* Fused LSTM gate activation + cell update (the pointwise half of nn.LSTM, decoder.py:66; gate order i,f,g,o).
  *   pre = sum_s partials[s] + gx + b1 + b2.  gates_out [B,4H] (stash, `precision` storage), c_out/h_out fp32,
@@ -143,7 +157,7 @@ typedef struct {
   int32_t precision;                    /* recnet_precision */
   int32_t train;                        /* 1 = apply dropout (embedding, logits) */
   float embedding_scale, p_emb_drop, p_out_drop;
-  int32_t cell;                         /* recnet_cell: LSTM (i,f,g,o; state h,c) or GRU (r,z,n; state h) */
+  int32_t cell;                         /* recnet_cell: LSTM (i,f,g,o; state h,c) or GRU (r,z,n; state h); | RECNET_ATTN_SOFTMAX */
   int32_t n_layers;                     /* stacked decoder layers (decoder.py:36-40), 0/1 = one; > 1: LSTM only */
   float p_layer_drop;                   /* nn.LSTM(dropout=) between layers, train mode only */
 } recnet_decoder_desc;
@@ -209,7 +223,7 @@ typedef struct {
   int32_t B, S, R, H, A, L;             /* S = encoder_output_len steps, R = hidden (= feature dim), H = decoder hidden */
   int32_t precision, train;
   float p_drop;
-  int32_t cell;                         /* recnet_cell of the reconstructor RNN */
+  int32_t cell;                         /* recnet_cell of the reconstructor RNN; | RECNET_ATTN_SOFTMAX (one softmax over L per decoder layer) */
   int32_t dec_layers;                   /* decoder layers NLd: hiddens is (L, NLd, B, H) and every outer step runs NLd pseudo-steps */
 } recnet_local_desc;
 typedef struct {

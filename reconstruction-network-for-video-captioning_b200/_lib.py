@@ -46,6 +46,7 @@ class decoder_desc(C.Structure):
 
 
 CELL_LSTM, CELL_GRU = 0, 1
+ATTN_SOFTMAX = 0x100           # OR'd into the descriptors' `cell`: the paper's softmax attention instead of the reference's mean
 
 
 MAX_LAYERS = 4
@@ -91,6 +92,8 @@ SIGNATURES = {
     "recnet_splitk_reduce": (_i, [_p, _i, _l, _l, _p, _l, _i, _i, _i, _p]),
     "recnet_attn_fwd": (_i, [_i, _p, _i, _l, _p, _l, _l, _p, _p, _p, _l, _l, _i, _i, _i, _i, _i, _p, _p, _p, _l, _f, _p, _u, _l, _p]),
     "recnet_attn_bwd": (_i, [_i, _p, _i, _l, _l, _p, _l, _l, _p, _p, _l, _l, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p, _i, _p, _f, _p, _u, _l, _p]),
+    "recnet_attn_bwd_softmax": (_i, [_i, _p, _i, _l, _l, _p, _l, _l, _p, _p, _p, _l, _l, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p, _i, _p, _f, _p,
+                                     _u, _l, _p]),
     "recnet_lstm_cell_fwd": (_i, [_i, _p, _i, _l, _l, _p, _l, _p, _p, _p, _i, _i, _p, _p, _p, _l, _p, _l, _p, _l, _p]),
     "recnet_lstm_cell_bwd": (_i, [_i, _p, _l, _p, _p, _l, _p, _i, _l, _l, _i, _p, _i, _l, _l, _p, _i, _p, _p, _p, _i, _i, _p, _l, _p]),
     "recnet_gru_cell_fwd": (_i, [_i, _p, _i, _l, _l, _p, _i, _l, _l, _p, _l, _p, _p, _p, _l, _i, _i, _p, _p, _l, _p, _l, _p]),

@@ -3,7 +3,7 @@
 Attribute names and default values follow the reference's ``config.py`` (TrainConfig, config.py:27-93;
 EvalConfig, config.py:160-173) so that code written against ``from config import TrainConfig as C`` keeps
 working; everything that only served the reference's data loading, logging and checkpoint naming is left
-out (out of scope, SURVEY.md section 2).  Two additions: ``precision`` and ``optimizer_impl``.
+out (out of scope, SURVEY.md section 2).  Additions: ``precision``, ``optimizer_impl`` and the two ``*_attn_softmax`` switches.
 """
 
 
@@ -43,6 +43,7 @@ class TrainConfig:
     decoder_dropout = 0.5
     decoder_out_dropout = 0.5
     decoder_teacher_forcing_ratio = 1.0
+    decoder_attn_softmax = False     # B200 addition: True = the paper's softmax attention; False = the reference's mean (SURVEY.md 0.1)
 
     # --- reconstructor (config.py:74-82) ---
     use_recon = True
@@ -52,6 +53,7 @@ class TrainConfig:
     reconstructor_decoder_dropout = 0.5
     reconstructor_dropout = 0.5
     reconstructor_attn_size = 128
+    reconstructor_attn_softmax = False   # B200 addition, local reconstructor only: as decoder_attn_softmax
 
     # --- optimisation (config.py:85-94) ---
     n_iterations = 100000

@@ -4,8 +4,9 @@
 //     ctx[b,:] = (1/Tn) * sum_tau e[b,tau] * V[b,tau,:]       (mean over frames)
 // with Uv = V U^T hoisted out of the time loop and Wh = h W^T arriving as split-K partials of the
 // tensor-core GEMM.  HBM/L2-bound: V is streamed once with 16-byte coalesced loads, scores live in
-// shared memory, the weighted sum accumulates in registers.  normalize = 1 adds a warp-shuffle softmax
-// over frames (the paper's variant; not what the reference computes, never used for parity).
+// shared memory, the weighted sum accumulates in registers.  normalize = 1 turns the scores into a max-subtracted
+// softmax over frames and the mean into the weighted sum (the paper's attention, opt-in: attn_softmax); e_out then
+// holds alpha, and the backward takes it (BwdArgs::alpha) instead of recomputing the softmax.
 #pragma once
 #include "common.cuh"
 
@@ -123,15 +124,15 @@ __device__ __forceinline__ void attn_fwd_body(const FwdArgs& a, int bx, int b, f
     }
   }
   blk_sync(bar_id);
-  if (a.normalize) {   // optional softmax over frames (paper variant)
+  if (a.normalize) {   // softmax over frames (paper variant): alpha replaces e
     if (warp == 0) {
       float m = -INFINITY;
       for (int t = lane; t < a.Tn; t += 32) m = fmaxf(m, e[t]);
       m = warp_max(m);
       float z = 0.f;
-      for (int t = lane; t < a.Tn; t += 32) z += __expf(e[t] - m);
+      for (int t = lane; t < a.Tn; t += 32) z += act_exp<FAST>(e[t] - m);
       z = warp_sum(z);
-      for (int t = lane; t < a.Tn; t += 32) e[t] = __expf(e[t] - m) / z;
+      for (int t = lane; t < a.Tn; t += 32) e[t] = act_exp<FAST>(e[t] - m) / z;
     }
     blk_sync(bar_id);
   }
@@ -198,6 +199,7 @@ __global__ void __launch_bounds__(FWD_THREADS) attn_fwd_kernel(FwdArgs a) {
 // Backward.  One CTA per sample:
 //   dctx = sum of split-K partials of d[ctx;h] (first D columns)      (x dropout mask in train)
 //   de[tau] = inv_T * dctx . V[b,tau,:]
+//     softmax (alpha != null, inv_T = 1): d alpha[tau] = dctx . V[b,tau,:];  de[tau] = alpha[tau] (d alpha[tau] - sum_s alpha[s] d alpha[s])
 //   ds[tau,a] = de[tau] * w[a] * (1 - s^2),  s = tanh(Wh + Uv + b)   (recomputed, not stored)
 //   dWh[b,a] = sum_tau ds ; dUv[b,tau,a] += ds ; dw_acc[b,a] += sum_tau de[tau]*s
 struct BwdArgs {
@@ -213,6 +215,7 @@ struct BwdArgs {
   int dwh_acc;                         // dWh_out += (several attentions share one query: stacked-decoder pseudo-steps)
   float* dctx_out;                     // [B,D] fp32 (nullable): summed/masked dctx, for the deferred dV pass
   float* de_out;                       // [B,Tn] (nullable)
+  const float* alpha;                  // [B,Tn] softmax weights of the forward (nullable = the reference's mean, no softmax)
   float p_drop; const unsigned long long* rng; unsigned int site; long long drop_base;
 };
 
@@ -330,6 +333,16 @@ __device__ __forceinline__ void attn_bwd_body(const BwdArgs& a, int b, float* sm
     }
   }
   blk_sync(bar_id);
+  if (a.alpha) {       // softmax backward: de holds d alpha; de_out (if any) keeps d alpha
+    if (warp == 0) {
+      const float* al = a.alpha + (long long)b * a.Tn;
+      float s1 = 0.f;
+      for (int t = lane; t < a.Tn; t += 32) s1 += al[t] * de[t];
+      s1 = warp_sum(s1);
+      for (int t = lane; t < a.Tn; t += 32) de[t] = al[t] * (de[t] - s1);
+    }
+    blk_sync(bar_id);
+  }
   // ---- ds / dWh / dUv / dw ----
   for (int i0 = 0; i0 < a.A; i0 += per) {
     const int i = i0 + i3;
@@ -387,6 +400,7 @@ __global__ void __launch_bounds__(BWD_THREADS) attn_bwd_kernel(BwdArgs a) {
 
 // Deferred value-gradient of the local reconstructor's attention (values = decoder hiddens, which need grad):
 //   dV[l,b,:] (+)= inv_T * sum_t beta_t[b,l] * dx_t[b,:]        one pass after the time loop instead of Tsteps RMWs
+// (softmax attention: beta = alpha, inv_T = 1)
 // beta [S,B,Tn] fp32, dx [S,B,D] fp32, dV[b*dv_bs + l*dv_ts + d] fp32.
 // step_mul / step_off: stash row of outer step t is t * step_mul + step_off (pseudo-steps of a stacked decoder)
 __global__ void attn_dv_kernel(const float* __restrict__ beta, const float* __restrict__ dx, float* __restrict__ dV,
@@ -504,7 +518,7 @@ static int launch_fwd(FwdArgs a, cudaStream_t st) {
 
 template <typename TV, typename TO>
 static int launch_bwd(const BwdArgs& a, cudaStream_t st) {
-  if (lean_ok<TV>(a.Tn, a.A, a.D, a.v_bs, a.v_ts, a.uv_bs, a.uv_ts) && a.p_ld % 2 == 0 && a.p_stride % 2 == 0 && a.D <= 6144)
+  if (!a.alpha && lean_ok<TV>(a.Tn, a.A, a.D, a.v_bs, a.v_ts, a.uv_bs, a.uv_ts) && a.p_ld % 2 == 0 && a.p_stride % 2 == 0 && a.D <= 6144)
     return launch_lean_bwd<TV, TO>(a, st);
   if (a.Tn > MAX_T || a.Tn < 1) return RECNET_ERR_BAD_SHAPE;
   constexpr int VN = Vec16<TV>::N;

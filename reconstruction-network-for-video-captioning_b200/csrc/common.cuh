@@ -8,6 +8,11 @@
 
 #include "../../include/recnet_b200.h"
 
+// Descriptors as the drivers see them: the entry points split RECNET_ATTN_SOFTMAX off the public `cell` field once, so `cell` holds the
+// plain recnet_cell value and `softmax` says whether the attention is the paper's softmax (true) or the reference's mean (false).
+struct DecDesc : recnet_decoder_desc { bool softmax = false; };
+struct LocalDesc : recnet_local_desc { bool softmax = false; };
+
 typedef __nv_bfloat16 bf16;
 
 #define RN_CUDA_OK(expr)                                  \
@@ -197,8 +202,15 @@ template <bool FAST> __device__ __forceinline__ float act_sigmoid(float x) {
   if (FAST) return fmaf(0.5f, act_tanh<true>(0.5f * x), 0.5f);
   return 1.f / (1.f + expf(-x));
 }
+template <bool FAST> __device__ __forceinline__ float act_exp(float x) { return FAST ? __expf(x) : expf(x); }
 template <typename T> struct FastMath { static constexpr bool value = false; };
 template <> struct FastMath<bf16> { static constexpr bool value = true; };
+// max-subtracted softmax of a row of <= 32 scores held one per lane (valid = lane < row length; invalid lanes return 0)
+template <bool FAST> __device__ __forceinline__ float warp_softmax(float x, bool valid) {
+  const float m = warp_max(valid ? x : -INFINITY);
+  const float p = valid ? act_exp<FAST>(x - m) : 0.f;
+  return p / warp_sum(p);
+}
 
 // ---- Philox4x32-10 counter RNG (Salmon et al. 2011), used for in-kernel dropout masks --------
 struct Philox {

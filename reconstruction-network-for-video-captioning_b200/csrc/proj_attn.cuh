@@ -12,6 +12,9 @@
 //   K4  [dWh_t | dG_t] [W_a ; W_hh]     one split-K GEMM, K = A + 4H -> dh_{t-1}
 // i.e. 2 + 2 dependent kernels per step instead of 4 + 4, and the per-step weight traffic drops from 8.4 MB to 2.2 MB.
 // dW_ctx = dG^T ctx with ctx_t[b] = (1/T) sum_tau e_t[b,tau] v[b,tau] (pf_escore_kernel<.., true>, in the forward pass next to the vocabulary GEMM).
+// The paper's softmax attention (SM = true, opt-in) keeps all of this: alpha_t = softmax_tau(e_t) takes the place of e_t and the scale is
+// 1 instead of 1/T (the drivers pass inv_T = 1); the e stash holds alpha, and the backward turns d alpha into d e with
+// d e[tau] = alpha[tau] (d alpha[tau] - sum_s alpha[s] d alpha[s]) before the unchanged score backward.
 //
 // VW and the gate stash are stored "unit-interleaved": [.., H, 4] (the 4 gate columns i,f,g,o of one hidden unit
 // adjacent) so that one thread fetches its unit's 4 columns of a frame with ONE 8-byte (bf16) / 16-byte (fp32) load.
@@ -95,7 +98,7 @@ struct FwdArgs {
   const float* b_hh;                                      // [4H]
   const float* c_prev;                                    // [B, H]
   int B, Tn, A, H; float inv_T;
-  float* Wh_out; float* e_out;                            // [B, A], [B, Tn]  stash for BPTT (nullable)
+  float* Wh_out; float* e_out;                            // [B, A], [B, Tn]  stash for BPTT (nullable); e_out holds alpha when SM
   void* gates_out;                                        // [B, H, 4] TO      activated gates, unit-interleaved (nullable)
   float* c_out; float* h_out;                             // [B, H] fp32
   void* h_op;                                             // [B, H] TO: next step's GEMM operand row / vocabulary-projection row
@@ -104,7 +107,7 @@ struct FwdArgs {
 // NCH = float4 chunks of the attention axis per lane: 1 (A <= 128) or 2 (A <= 256).
 // Index math is 32-bit unsigned on purpose (r1 ncu: 42% of the first version's instructions were 64-bit address arithmetic);
 // the drivers check that every tensor has < 2^31 elements.  `Uv` already contains the attention bias (folded in at the hoist).
-template <typename TV, typename TO, int NCH, int MINB>
+template <typename TV, typename TO, int NCH, int MINB, bool SM>
 __global__ void __launch_bounds__(THREADS, MINB) pf_fwd_kernel(FwdArgs a) {
   constexpr bool FAST = FastMath<TO>::value;
   pdl_wait();
@@ -191,7 +194,7 @@ __global__ void __launch_bounds__(THREADS, MINB) pf_fwd_kernel(FwdArgs a) {
         s = warp_sum(s);
         if (lane == 0) {
           e_s[tau & 1][tau >> 1] = s;
-          if (blockIdx.x == 0 && a.e_out) a.e_out[b * Tn + tau] = s;
+          if (!SM && blockIdx.x == 0 && a.e_out) a.e_out[b * Tn + tau] = s;
         }
       }
     }
@@ -203,6 +206,19 @@ __global__ void __launch_bounds__(THREADS, MINB) pf_fwd_kernel(FwdArgs a) {
       for (unsigned i = 0; i < NCH; ++i) uv[f][i] = uvb[min(warp + (f0 + f) * NW, Tn - 1) * nchunk + min(lane + 32 * i, nchunk - 1)];
   }
   __syncthreads();
+  if constexpr (SM) {             // softmax over the (<= 64) frames: warp 0, lane owns frames lane and lane + 32
+    if (warp == 0) {
+      const unsigned t1 = lane + 32;
+      const bool ok0 = lane < Tn, ok1 = t1 < Tn;
+      const float x0 = ok0 ? e_s[lane & 1][lane >> 1] : -INFINITY, x1 = ok1 ? e_s[t1 & 1][t1 >> 1] : -INFINITY;
+      const float m = warp_max(fmaxf(x0, x1));
+      const float p0 = ok0 ? act_exp<FAST>(x0 - m) : 0.f, p1 = ok1 ? act_exp<FAST>(x1 - m) : 0.f;
+      const float z = warp_sum(p0 + p1);
+      if (ok0) { e_s[lane & 1][lane >> 1] = p0 / z; if (blockIdx.x == 0 && a.e_out) a.e_out[b * Tn + lane] = p0 / z; }
+      if (ok1) { e_s[t1 & 1][t1 >> 1] = p1 / z; if (blockIdx.x == 0 && a.e_out) a.e_out[b * Tn + t1] = p1 / z; }
+    }
+    __syncthreads();
+  }
   // (4) weighted sum over this thread's frames (weights of frames >= Tn are zero, their clamped quads are finite)
   float acc[4] = {0.f, 0.f, 0.f, 0.f};
   for (unsigned t0 = 0;;) {
@@ -257,6 +273,7 @@ struct BwdArgs {
   float* dWh_out;                                       // [B, A] fp32 (attn_b gradient)
   float* dUv_acc; int uv_first;                         // [B, Tn, A] accumulated over steps
   float* dw_acc; int dw_first;                          // [B, A]     accumulated over steps
+  const float* alpha;                                   // [B, Tn] softmax weights of the step (SM only)
 };
 
 // sum over the 32 lanes of v[k] for every k; lane l ends up with the total of v[l] (31 shuffles instead of 160)
@@ -336,7 +353,7 @@ __device__ __forceinline__ float4 cell_bwd_unit(const BwdArgs& a, const CellIn<T
 // dynamic shared memory: H float4 (gate gradients) + 2 * BNW * A floats (per-warp dWh / dw partials)
 constexpr int BTHREADS = 512;
 constexpr int BNW = BTHREADS / 32;
-template <typename TV, typename TO, int NF, int NCH>
+template <typename TV, typename TO, int NF, int NCH, bool SM>
 __global__ void __launch_bounds__(BTHREADS) pf_bwd_kernel(BwdArgs a) {
   constexpr bool FAST = FastMath<TO>::value;
   constexpr int QP = 32 / NF;                           // VW quads per lane, frame and pass (32 quads = 64 registers in flight)
@@ -368,6 +385,11 @@ __global__ void __launch_bounds__(BTHREADS) pf_bwd_kernel(BwdArgs a) {
     ww[i] = reinterpret_cast<const float4*>(a.attn_w)[cc];
 #pragma unroll
     for (unsigned f = 0; f < NF; ++f) uv[f][i] = uvb[tauc[f] * nchunk + cc];
+  }
+  float al[NF];
+  if constexpr (SM) {
+#pragma unroll
+    for (unsigned f = 0; f < NF; ++f) al[f] = warp + f * BNW < Tn ? a.alpha[b * Tn + warp + f * BNW] : 0.f;
   }
   // ---- (A) LSTM cell backward, one unit per thread and pass
   for (unsigned j0 = 0; j0 < H; j0 += BTHREADS) {
@@ -408,6 +430,19 @@ __global__ void __launch_bounds__(BTHREADS) pf_bwd_kernel(BwdArgs a) {
   }
 #pragma unroll
   for (unsigned f = 0; f < NF; ++f) de[f] = warp_sum(de[f]) * a.inv_T;
+  if constexpr (SM) {             // de = d alpha so far: d e = alpha (d alpha - sum_s alpha[s] d alpha[s]), the sum over every warp's frames
+    __shared__ float sad[BNW];
+    float s1 = 0.f;
+#pragma unroll
+    for (unsigned f = 0; f < NF; ++f) s1 = fmaf(al[f], de[f], s1);
+    if (lane == 0) sad[warp] = s1;
+    __syncthreads();
+    float tot = 0.f;
+#pragma unroll
+    for (unsigned w = 0; w < BNW; ++w) tot += sad[w];
+#pragma unroll
+    for (unsigned f = 0; f < NF; ++f) de[f] = al[f] * (de[f] - tot);
+  }
   // ---- (C) score backward of the same frames: ds = de * w * (1 - tanh^2); dWh = sum_tau ds; dUv[tau] += ds; dw += de * tanh
   float4 dwh[NCH], dww[NCH];
 #pragma unroll
@@ -556,32 +591,42 @@ static inline int check_shape(int Tn, int A, int H) {
   return 0;
 }
 
-template <typename TV, typename TO>
+// sm = softmax attention (a.inv_T must then be 1)
+template <typename TV, typename TO, bool SM = false>
 static int launch_fwd(const FwdArgs& a, cudaStream_t st) {
   RN_TRY(check_shape(a.Tn, a.A, a.H));
   ProfScope prof(KC_PF_FWD, a.B, a.Tn, a.H, st);
   static int minb = -1;
   if (minb < 0) { const char* e = getenv("RECNET_PF_MINB"); minb = e ? atoi(e) : 3; }
   const dim3 grid(rn_cdiv(a.H, UPB), a.B);
-  if (a.A <= 128 && minb == 3) RN_CUDA_OK(launch_pdl(pf_fwd_kernel<TV, TO, 1, 3>, grid, dim3(THREADS), 0, st, a));
-  else if (a.A <= 128) RN_CUDA_OK(launch_pdl(pf_fwd_kernel<TV, TO, 1, 2>, grid, dim3(THREADS), 0, st, a));
-  else RN_CUDA_OK(launch_pdl(pf_fwd_kernel<TV, TO, 2, 2>, grid, dim3(THREADS), 0, st, a));
+  if (a.A <= 128 && minb == 3) RN_CUDA_OK(launch_pdl(pf_fwd_kernel<TV, TO, 1, 3, SM>, grid, dim3(THREADS), 0, st, a));
+  else if (a.A <= 128) RN_CUDA_OK(launch_pdl(pf_fwd_kernel<TV, TO, 1, 2, SM>, grid, dim3(THREADS), 0, st, a));
+  else RN_CUDA_OK(launch_pdl(pf_fwd_kernel<TV, TO, 2, 2, SM>, grid, dim3(THREADS), 0, st, a));
   RN_LAUNCH_OK();
   return 0;
 }
-static inline size_t bwd_smem_bytes(int H, int A) { return (size_t)H * sizeof(float4) + (size_t)2 * BNW * A * sizeof(float); }
 template <typename TV, typename TO>
-static int launch_bwd(const BwdArgs& a, cudaStream_t st) {
+static int launch_fwd(const FwdArgs& a, bool softmax, cudaStream_t st) {
+  return softmax ? launch_fwd<TV, TO, true>(a, st) : launch_fwd<TV, TO, false>(a, st);
+}
+static inline size_t bwd_smem_bytes(int H, int A) { return (size_t)H * sizeof(float4) + (size_t)2 * BNW * A * sizeof(float); }
+// a.alpha != nullptr: softmax attention (a.inv_T must then be 1)
+template <typename TV, typename TO, bool SM>
+static int launch_bwd_sm(const BwdArgs& a, cudaStream_t st) {
   RN_TRY(check_shape(a.Tn, a.A, a.H));
   const size_t smem = bwd_smem_bytes(a.H, a.A);
   if (smem > 46 * 1024) return RECNET_ERR_BAD_SHAPE;
   const bool nf2 = a.Tn <= 2 * BNW, ch1 = a.A <= 128;
   ProfScope prof(KC_PF_BWD, a.B, a.Tn, a.H, st);
-  if (nf2 && ch1) RN_CUDA_OK(launch_pdl(pf_bwd_kernel<TV, TO, 2, 1>, dim3(a.B), dim3(BTHREADS), smem, st, a));
-  else if (nf2) RN_CUDA_OK(launch_pdl(pf_bwd_kernel<TV, TO, 2, 2>, dim3(a.B), dim3(BTHREADS), smem, st, a));
-  else if (ch1) RN_CUDA_OK(launch_pdl(pf_bwd_kernel<TV, TO, 4, 1>, dim3(a.B), dim3(BTHREADS), smem, st, a));
-  else RN_CUDA_OK(launch_pdl(pf_bwd_kernel<TV, TO, 4, 2>, dim3(a.B), dim3(BTHREADS), smem, st, a));
+  if (nf2 && ch1) RN_CUDA_OK(launch_pdl(pf_bwd_kernel<TV, TO, 2, 1, SM>, dim3(a.B), dim3(BTHREADS), smem, st, a));
+  else if (nf2) RN_CUDA_OK(launch_pdl(pf_bwd_kernel<TV, TO, 2, 2, SM>, dim3(a.B), dim3(BTHREADS), smem, st, a));
+  else if (ch1) RN_CUDA_OK(launch_pdl(pf_bwd_kernel<TV, TO, 4, 1, SM>, dim3(a.B), dim3(BTHREADS), smem, st, a));
+  else RN_CUDA_OK(launch_pdl(pf_bwd_kernel<TV, TO, 4, 2, SM>, dim3(a.B), dim3(BTHREADS), smem, st, a));
   RN_LAUNCH_OK();
   return 0;
+}
+template <typename TV, typename TO>
+static int launch_bwd(const BwdArgs& a, cudaStream_t st) {
+  return a.alpha ? launch_bwd_sm<TV, TO, true>(a, st) : launch_bwd_sm<TV, TO, false>(a, st);
 }
 }  // namespace pf

@@ -10,6 +10,18 @@
 
 #define ST(s) reinterpret_cast<cudaStream_t>(s)
 
+// The public descriptors carry RECNET_ATTN_SOFTMAX in their `cell` field; every entry point splits it off here, once.
+template <typename Pub, typename Int>
+static int split_desc(const Pub* d, Int* out) {
+  if (!d) return RECNET_ERR_BAD_SHAPE;
+  static_cast<Pub&>(*out) = *d;
+  const int32_t flags = d->cell & ~RECNET_CELL_MASK;
+  if (flags & ~RECNET_ATTN_SOFTMAX) return RECNET_ERR_UNSUPPORTED;
+  out->cell = d->cell & RECNET_CELL_MASK;
+  out->softmax = flags != 0;
+  return 0;
+}
+
 extern "C" {
 
 int recnet_abi_version(void) { return 1; }
@@ -101,8 +113,10 @@ int recnet_plan_persistent_loops(const recnet_local_desc* d, int32_t* out) {
   // out[6..11] backward: covered?, gate-row splits, column groups, resident k-blocks per CTA, ring stages, CTAs
   if (!d || !out) return RECNET_ERR_BAD_SHAPE;
   for (int i = 0; i < 12; ++i) out[i] = 0;
-  const rp::Shape s{d->B, d->S, d->R, d->H, d->A, d->L};
-  const bool lstm_bf16 = d->precision == RECNET_PREC_BF16 && d->cell == RECNET_CELL_LSTM && d->dec_layers <= 1;
+  LocalDesc dd;
+  RN_TRY(split_desc(d, &dd));            // both attention variants have persistent loops
+  const rp::Shape s{dd.B, dd.S, dd.R, dd.H, dd.A, dd.L};
+  const bool lstm_bf16 = dd.precision == RECNET_PREC_BF16 && dd.cell == RECNET_CELL_LSTM && dd.dec_layers <= 1;
   if (lstm_bf16 && rp::local_fwd_ok(s)) {
     const int ks = rp::pick_ks(s.R, s.H), res = rp::max_res_kb_fwd(s.R, s.H, ks);
     out[0] = 1; out[1] = ks; out[2] = s.R / rp::UNITS; out[3] = res; out[4] = rp::pick_stages_fwd(s.B, ks, res); out[5] = out[2] * ks;
@@ -149,6 +163,23 @@ int recnet_attn_bwd(int precision, const float* dctx_partials, int n_p, int64_t 
   a.Wh = wh; a.Uv = uv; a.uv_bs = uv_bs; a.uv_ts = uv_ts; a.attn_b = attn_b; a.attn_w = attn_w; a.B = B; a.Tn = Tn; a.A = A;
   a.D = D; a.inv_T = 1.f / Tn; a.dWh_out = dwh_out; a.dWh_op = dwh_op; a.dUv_acc = duv_acc; a.uv_first = first; a.dw_first = first; a.dw_acc = dw_acc;
   a.dctx_out = dctx_out; a.de_out = nullptr; a.p_drop = p_drop; a.rng = reinterpret_cast<const unsigned long long*>(rng);
+  a.site = site; a.drop_base = drop_base;
+  if (precision == RECNET_PREC_FP32) return (attn::launch_bwd<float, float>(a, ST(stream)));
+  if (precision == RECNET_PREC_BF16) return (attn::launch_bwd<bf16, bf16>(a, ST(stream)));
+  return RECNET_ERR_UNSUPPORTED;
+}
+
+int recnet_attn_bwd_softmax(int precision, const float* dctx_partials, int n_p, int64_t p_stride, int64_t p_ld, const void* v,
+                            int64_t v_bs, int64_t v_ts, const float* alpha, const float* wh, const float* uv, int64_t uv_bs,
+                            int64_t uv_ts, const float* attn_b, const float* attn_w, int B, int Tn, int A, int D, float* dwh_out,
+                            void* dwh_op, float* duv_acc, float* dw_acc, int first, float* dctx_out, float p_drop,
+                            const uint64_t* rng, uint32_t site, int64_t drop_base, void* stream) {
+  if (!alpha) return RECNET_ERR_BAD_SHAPE;
+  attn::BwdArgs a{};
+  a.dXp = dctx_partials; a.n_p = n_p; a.p_stride = p_stride; a.p_ld = p_ld; a.V = v; a.v_bs = v_bs; a.v_ts = v_ts;
+  a.Wh = wh; a.Uv = uv; a.uv_bs = uv_bs; a.uv_ts = uv_ts; a.attn_b = attn_b; a.attn_w = attn_w; a.B = B; a.Tn = Tn; a.A = A;
+  a.D = D; a.inv_T = 1.f; a.dWh_out = dwh_out; a.dWh_op = dwh_op; a.dUv_acc = duv_acc; a.uv_first = first; a.dw_first = first; a.dw_acc = dw_acc;
+  a.dctx_out = dctx_out; a.de_out = nullptr; a.alpha = alpha; a.p_drop = p_drop; a.rng = reinterpret_cast<const unsigned long long*>(rng);
   a.site = site; a.drop_base = drop_base;
   if (precision == RECNET_PREC_FP32) return (attn::launch_bwd<float, float>(a, ST(stream)));
   if (precision == RECNET_PREC_BF16) return (attn::launch_bwd<bf16, bf16>(a, ST(stream)));
@@ -209,92 +240,102 @@ int recnet_gru_cell_bwd(int precision, const float* dh_ext, int64_t dh_ld, const
 
 // ---- decoder ---------------------------------------------------------------------------------------------------
 int64_t recnet_decoder_workspace_bytes(const recnet_decoder_desc* d) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
   if (!d) return RECNET_ERR_BAD_SHAPE;
-  if (dec::pf_ok(*d)) {
-    if (d->precision == RECNET_PREC_FP32) return (int64_t)dec::plan_pf<float>(*d, nullptr).bytes;
-    if (d->precision == RECNET_PREC_BF16) return (int64_t)dec::plan_pf<bf16>(*d, nullptr).bytes;
+  if (dec::pf_ok(dd)) {
+    if (dd.precision == RECNET_PREC_FP32) return (int64_t)dec::plan_pf<float>(dd, nullptr).bytes;
+    if (dd.precision == RECNET_PREC_BF16) return (int64_t)dec::plan_pf<bf16>(dd, nullptr).bytes;
     return RECNET_ERR_UNSUPPORTED;
   }
-  if (d->precision == RECNET_PREC_FP32) return (int64_t)dec::plan<float>(*d, nullptr).bytes;
-  if (d->precision == RECNET_PREC_BF16) return (int64_t)dec::plan<bf16>(*d, nullptr).bytes;
+  if (dd.precision == RECNET_PREC_FP32) return (int64_t)dec::plan<float>(dd, nullptr).bytes;
+  if (dd.precision == RECNET_PREC_BF16) return (int64_t)dec::plan<bf16>(dd, nullptr).bytes;
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_decoder_fwd(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, const int64_t* tokens_in,
                        const int64_t* targets, const float* ce_weight, const uint64_t* rng, void* workspace,
                        int64_t workspace_bytes, float* hiddens, float* ce_out, void* stream) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
   const long long* ti = reinterpret_cast<const long long*>(tokens_in);
   const long long* tg = reinterpret_cast<const long long*>(targets);
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (d->n_layers > 1) {
-    if (d->precision == RECNET_PREC_FP32)
-      return dec::forward_ml<float>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
-    if (d->precision == RECNET_PREC_BF16)
-      return dec::forward_ml<bf16>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
+  if (dd.n_layers > 1) {
+    if (dd.precision == RECNET_PREC_FP32)
+      return dec::forward_ml<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
+    if (dd.precision == RECNET_PREC_BF16)
+      return dec::forward_ml<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
     return RECNET_ERR_UNSUPPORTED;
   }
-  if (dec::pf_ok(*d)) {
-    if (d->precision == RECNET_PREC_FP32)
-      return dec::forward_pf<float>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
-    if (d->precision == RECNET_PREC_BF16)
-      return dec::forward_pf<bf16>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
+  if (dec::pf_ok(dd)) {
+    if (dd.precision == RECNET_PREC_FP32)
+      return dec::forward_pf<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
+    if (dd.precision == RECNET_PREC_BF16)
+      return dec::forward_pf<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
     return RECNET_ERR_UNSUPPORTED;
   }
-  if (d->precision == RECNET_PREC_FP32)
-    return dec::forward<float>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
-  if (d->precision == RECNET_PREC_BF16)
-    return dec::forward<bf16>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
+  if (dd.precision == RECNET_PREC_FP32)
+    return dec::forward<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
+  if (dd.precision == RECNET_PREC_BF16)
+    return dec::forward<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_decoder_fwd_phase(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, const int64_t* tokens_in,
                              const int64_t* targets, const float* ce_weight, const uint64_t* rng, void* workspace,
                              int64_t workspace_bytes, float* hiddens, float* ce_out, int phases, void* stream) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
   if (phases < 1 || phases > 3) return RECNET_ERR_BAD_SHAPE;
-  if (d->n_layers > 1 || !dec::pf_ok(*d)) {          // not split on these paths: everything belongs to bit 0
+  if (dd.n_layers > 1 || !dec::pf_ok(dd)) {          // not split on these paths: everything belongs to bit 0
     if (!(phases & 1)) return 0;
     return recnet_decoder_fwd(d, w, feats, tokens_in, targets, ce_weight, rng, workspace, workspace_bytes, hiddens, ce_out, stream);
   }
   const long long* ti = reinterpret_cast<const long long*>(tokens_in);
   const long long* tg = reinterpret_cast<const long long*>(targets);
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (d->precision == RECNET_PREC_FP32)
-    return dec::forward_pf<float>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream), phases);
-  if (d->precision == RECNET_PREC_BF16)
-    return dec::forward_pf<bf16>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream), phases);
+  if (dd.precision == RECNET_PREC_FP32)
+    return dec::forward_pf<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream), phases);
+  if (dd.precision == RECNET_PREC_BF16)
+    return dec::forward_pf<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream), phases);
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_decoder_bwd(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, const int64_t* tokens_in,
                        const int64_t* targets, const float* ce_weight, const uint64_t* rng, void* workspace,
                        int64_t workspace_bytes, const float* g_ce, const float* g_hiddens, const float* hiddens,
                        const recnet_decoder_tensors* grads, void* stream) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
   const long long* ti = reinterpret_cast<const long long*>(tokens_in);
   const long long* tg = reinterpret_cast<const long long*>(targets);
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (d->n_layers > 1) {
-    if (d->precision == RECNET_PREC_FP32)
-      return dec::backward_ml<float>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
-    if (d->precision == RECNET_PREC_BF16)
-      return dec::backward_ml<bf16>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
+  if (dd.n_layers > 1) {
+    if (dd.precision == RECNET_PREC_FP32)
+      return dec::backward_ml<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
+    if (dd.precision == RECNET_PREC_BF16)
+      return dec::backward_ml<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
     return RECNET_ERR_UNSUPPORTED;
   }
-  if (dec::pf_ok(*d)) {
-    if (d->precision == RECNET_PREC_FP32)
-      return dec::backward_pf<float>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
-    if (d->precision == RECNET_PREC_BF16)
-      return dec::backward_pf<bf16>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
+  if (dec::pf_ok(dd)) {
+    if (dd.precision == RECNET_PREC_FP32)
+      return dec::backward_pf<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
+    if (dd.precision == RECNET_PREC_BF16)
+      return dec::backward_pf<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
     return RECNET_ERR_UNSUPPORTED;
   }
-  if (d->precision == RECNET_PREC_FP32)
-    return dec::backward<float>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, hiddens, *grads, ST(stream));
-  if (d->precision == RECNET_PREC_BF16)
-    return dec::backward<bf16>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, hiddens, *grads, ST(stream));
+  if (dd.precision == RECNET_PREC_FP32)
+    return dec::backward<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, hiddens, *grads, ST(stream));
+  if (dd.precision == RECNET_PREC_BF16)
+    return dec::backward<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, hiddens, *grads, ST(stream));
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_decoder_bwd_phase(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, const int64_t* tokens_in,
                              const int64_t* targets, const float* ce_weight, const uint64_t* rng, void* workspace,
                              int64_t workspace_bytes, const float* g_ce, const float* g_hiddens, const float* hiddens,
                              const recnet_decoder_tensors* grads, int phases, void* stream) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
   if (phases < 1 || phases > 15) return RECNET_ERR_BAD_SHAPE;
-  if (d->n_layers > 1 || !dec::pf_ok(*d)) {          // not split on these paths: everything belongs to bit 0
+  if (dd.n_layers > 1 || !dec::pf_ok(dd)) {          // not split on these paths: everything belongs to bit 0
     if (!(phases & 1)) return 0;
     return recnet_decoder_bwd(d, w, feats, tokens_in, targets, ce_weight, rng, workspace, workspace_bytes, g_ce, g_hiddens, hiddens,
                               grads, stream);
@@ -302,58 +343,72 @@ int recnet_decoder_bwd_phase(const recnet_decoder_desc* d, const recnet_decoder_
   const long long* ti = reinterpret_cast<const long long*>(tokens_in);
   const long long* tg = reinterpret_cast<const long long*>(targets);
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (d->precision == RECNET_PREC_FP32)
-    return dec::backward_pf<float>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream), phases);
-  if (d->precision == RECNET_PREC_BF16)
-    return dec::backward_pf<bf16>(*d, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream), phases);
+  if (dd.precision == RECNET_PREC_FP32)
+    return dec::backward_pf<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream), phases);
+  if (dd.precision == RECNET_PREC_BF16)
+    return dec::backward_pf<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream), phases);
   return RECNET_ERR_UNSUPPORTED;
 }
-int recnet_decoder_bwd_is_split(const recnet_decoder_desc* d) { return (d->n_layers > 1 || !dec::pf_ok(*d)) ? 0 : 1; }
+int recnet_decoder_bwd_is_split(const recnet_decoder_desc* d) {
+  DecDesc dd;
+  if (split_desc(d, &dd)) return 0;
+  return (dd.n_layers > 1 || !dec::pf_ok(dd)) ? 0 : 1;
+}
 float* recnet_decoder_logits(const recnet_decoder_desc* d, void* workspace, int64_t* ld) {
-  if (dec::pf_ok(*d)) {
-    if (d->precision == RECNET_PREC_FP32) { auto w = dec::plan_pf<float>(*d, workspace); if (ld) *ld = w.Vld; return w.logits; }
-    auto w = dec::plan_pf<bf16>(*d, workspace); if (ld) *ld = w.Vld; return w.logits;
+  DecDesc dd;
+  if (split_desc(d, &dd)) return nullptr;
+  if (dec::pf_ok(dd)) {
+    if (dd.precision == RECNET_PREC_FP32) { auto w = dec::plan_pf<float>(dd, workspace); if (ld) *ld = w.Vld; return w.logits; }
+    auto w = dec::plan_pf<bf16>(dd, workspace); if (ld) *ld = w.Vld; return w.logits;
   }
-  if (d->precision == RECNET_PREC_FP32) { auto w = dec::plan<float>(*d, workspace); if (ld) *ld = w.Vld; return w.logits; }
-  auto w = dec::plan<bf16>(*d, workspace); if (ld) *ld = w.Vld; return w.logits;
+  if (dd.precision == RECNET_PREC_FP32) { auto w = dec::plan<float>(dd, workspace); if (ld) *ld = w.Vld; return w.logits; }
+  auto w = dec::plan<bf16>(dd, workspace); if (ld) *ld = w.Vld; return w.logits;
 }
 int64_t recnet_greedy_workspace_bytes(const recnet_decoder_desc* d) {
-  if (d->precision == RECNET_PREC_FP32) return (int64_t)dec::plan_greedy<float>(*d, nullptr, 64).bytes;
-  if (d->precision == RECNET_PREC_BF16) {
-    const int64_t a = (int64_t)dec::plan_greedy<bf16>(*d, nullptr, 64).bytes;
-    const int64_t b = dec::greedy_pf_ok(*d) ? (int64_t)dec::plan_greedy_pf<bf16>(*d, nullptr, 64).bytes : 0;
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
+  if (dd.precision == RECNET_PREC_FP32) return (int64_t)dec::plan_greedy<float>(dd, nullptr, 64).bytes;
+  if (dd.precision == RECNET_PREC_BF16) {
+    const int64_t a = (int64_t)dec::plan_greedy<bf16>(dd, nullptr, 64).bytes;
+    const int64_t b = dec::greedy_pf_ok(dd) ? (int64_t)dec::plan_greedy_pf<bf16>(dd, nullptr, 64).bytes : 0;
     return a > b ? a : b;
   }
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_decoder_greedy(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, int max_steps,
                           void* workspace, int64_t workspace_bytes, int64_t* ids_out, int32_t* n_steps_out, void* stream) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
   if (max_steps < 1 || max_steps > 64) return RECNET_ERR_BAD_SHAPE;
-  if (d->precision == RECNET_PREC_FP32)
-    return dec::greedy<float>(*d, *w, feats, max_steps, workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), n_steps_out, ST(stream));
-  if (d->precision == RECNET_PREC_BF16) {
+  if (dd.precision == RECNET_PREC_FP32)
+    return dec::greedy<float>(dd, *w, feats, max_steps, workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), n_steps_out, ST(stream));
+  if (dd.precision == RECNET_PREC_BF16) {
     recnet_decoder_desc d1 = *d; d1.L = 1; d1.train = 0;
     if (dec::greedy_pf_ok(d1))      // projected-feature kernels, 4 launches per step
-      return dec::greedy_pf(*d, *w, feats, max_steps, workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), n_steps_out, ST(stream));
-    return dec::greedy<bf16>(*d, *w, feats, max_steps, workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), n_steps_out, ST(stream));
+      return dec::greedy_pf(dd, *w, feats, max_steps, workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), n_steps_out, ST(stream));
+    return dec::greedy<bf16>(dd, *w, feats, max_steps, workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), n_steps_out, ST(stream));
   }
   return RECNET_ERR_UNSUPPORTED;
 }
 
 // byte offset of the loop kernel's int32 error flag inside the workspace (0 = ok, 2 = mbarrier timeout, 3 = grid-barrier timeout)
 int64_t recnet_decoder_error_offset(const recnet_decoder_desc* d) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
   uint8_t* base = reinterpret_cast<uint8_t*>(4096);
-  if (dec::pf_ok(*d)) {
-    if (d->precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(dec::plan_pf<float>(*d, base).err) - base;
-    return reinterpret_cast<uint8_t*>(dec::plan_pf<bf16>(*d, base).err) - base;
+  if (dec::pf_ok(dd)) {
+    if (dd.precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(dec::plan_pf<float>(dd, base).err) - base;
+    return reinterpret_cast<uint8_t*>(dec::plan_pf<bf16>(dd, base).err) - base;
   }
-  if (d->precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(dec::plan<float>(*d, base).err) - base;
-  return reinterpret_cast<uint8_t*>(dec::plan<bf16>(*d, base).err) - base;
+  if (dd.precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(dec::plan<float>(dd, base).err) - base;
+  return reinterpret_cast<uint8_t*>(dec::plan<bf16>(dd, base).err) - base;
 }
 int64_t recnet_local_error_offset(const recnet_local_desc* d) {
+  LocalDesc dd;
+  RN_TRY(split_desc(d, &dd));
   uint8_t* base = reinterpret_cast<uint8_t*>(4096);
-  if (d->precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(rec::plan_local<float>(*d, base).err) - base;
-  return reinterpret_cast<uint8_t*>(rec::plan_local<bf16>(*d, base).err) - base;
+  if (dd.precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(rec::plan_local<float>(dd, base).err) - base;
+  return reinterpret_cast<uint8_t*>(rec::plan_local<bf16>(dd, base).err) - base;
 }
 int64_t recnet_global_error_offset(const recnet_global_desc* d) {
   uint8_t* base = reinterpret_cast<uint8_t*>(4096);
@@ -363,64 +418,76 @@ int64_t recnet_global_error_offset(const recnet_global_desc* d) {
 
 // ---- local reconstructor ---------------------------------------------------------------------------------------
 int64_t recnet_beam_workspace_bytes(const recnet_decoder_desc* d, int beam_width, int max_steps) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
   if (beam_width < 1 || beam_width > dec::BEAM_MAX_K || max_steps < 1 || max_steps > 64) return RECNET_ERR_BAD_SHAPE;
-  if (d->precision == RECNET_PREC_FP32) return (int64_t)dec::plan_beam<float>(*d, nullptr, beam_width, max_steps).bytes;
-  if (d->precision == RECNET_PREC_BF16) return (int64_t)dec::plan_beam<bf16>(*d, nullptr, beam_width, max_steps).bytes;
+  if (dd.precision == RECNET_PREC_FP32) return (int64_t)dec::plan_beam<float>(dd, nullptr, beam_width, max_steps).bytes;
+  if (dd.precision == RECNET_PREC_BF16) return (int64_t)dec::plan_beam<bf16>(dd, nullptr, beam_width, max_steps).bytes;
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_decoder_beam(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats_tiled, int beam_width, int max_steps,
                         int64_t eos_id, void* workspace, int64_t workspace_bytes, int64_t* seq_out, int32_t* n_steps_out, void* stream) {
-  if (d->n_layers > 1) return RECNET_ERR_UNSUPPORTED;
-  if (d->precision == RECNET_PREC_FP32)
-    return dec::beam<float>(*d, *w, feats_tiled, beam_width, max_steps, (long long)eos_id, workspace, workspace_bytes,
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
+  if (dd.n_layers > 1) return RECNET_ERR_UNSUPPORTED;
+  if (dd.precision == RECNET_PREC_FP32)
+    return dec::beam<float>(dd, *w, feats_tiled, beam_width, max_steps, (long long)eos_id, workspace, workspace_bytes,
                             reinterpret_cast<long long*>(seq_out), n_steps_out, ST(stream));
-  if (d->precision == RECNET_PREC_BF16)
-    return dec::beam<bf16>(*d, *w, feats_tiled, beam_width, max_steps, (long long)eos_id, workspace, workspace_bytes,
+  if (dd.precision == RECNET_PREC_BF16)
+    return dec::beam<bf16>(dd, *w, feats_tiled, beam_width, max_steps, (long long)eos_id, workspace, workspace_bytes,
                            reinterpret_cast<long long*>(seq_out), n_steps_out, ST(stream));
   return RECNET_ERR_UNSUPPORTED;
 }
 
 int64_t recnet_local_workspace_bytes(const recnet_local_desc* d) {
-  if (d->precision == RECNET_PREC_FP32) return (int64_t)rec::plan_local<float>(*d, nullptr).bytes;
-  if (d->precision == RECNET_PREC_BF16) return (int64_t)rec::plan_local<bf16>(*d, nullptr).bytes;
+  LocalDesc dd;
+  RN_TRY(split_desc(d, &dd));
+  if (dd.precision == RECNET_PREC_FP32) return (int64_t)rec::plan_local<float>(dd, nullptr).bytes;
+  if (dd.precision == RECNET_PREC_BF16) return (int64_t)rec::plan_local<bf16>(dd, nullptr).bytes;
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_local_fwd(const recnet_local_desc* d, const recnet_local_tensors* w, const float* hiddens, const float* feats,
                      const uint64_t* rng, void* workspace, int64_t workspace_bytes, float* mse_out, void* stream) {
+  LocalDesc dd;
+  RN_TRY(split_desc(d, &dd));
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (d->dec_layers > 1) {
-    if (d->precision == RECNET_PREC_FP32) return rec::local_forward_ml<float>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
-    if (d->precision == RECNET_PREC_BF16) return rec::local_forward_ml<bf16>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
+  if (dd.dec_layers > 1) {
+    if (dd.precision == RECNET_PREC_FP32) return rec::local_forward_ml<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
+    if (dd.precision == RECNET_PREC_BF16) return rec::local_forward_ml<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
     return RECNET_ERR_UNSUPPORTED;
   }
-  if (d->precision == RECNET_PREC_FP32) return rec::local_forward<float>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
-  if (d->precision == RECNET_PREC_BF16) return rec::local_forward<bf16>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
+  if (dd.precision == RECNET_PREC_FP32) return rec::local_forward<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
+  if (dd.precision == RECNET_PREC_BF16) return rec::local_forward<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_local_bwd(const recnet_local_desc* d, const recnet_local_tensors* w, const float* hiddens, const float* feats,
                      const uint64_t* rng, void* workspace, int64_t workspace_bytes, const float* g_mse,
                      const recnet_local_tensors* grads, float* g_hiddens, void* stream) {
+  LocalDesc dd;
+  RN_TRY(split_desc(d, &dd));
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (d->dec_layers > 1) {
-    if (d->precision == RECNET_PREC_FP32) return rec::local_backward_ml<float>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
-    if (d->precision == RECNET_PREC_BF16) return rec::local_backward_ml<bf16>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
+  if (dd.dec_layers > 1) {
+    if (dd.precision == RECNET_PREC_FP32) return rec::local_backward_ml<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
+    if (dd.precision == RECNET_PREC_BF16) return rec::local_backward_ml<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
     return RECNET_ERR_UNSUPPORTED;
   }
-  if (d->precision == RECNET_PREC_FP32) return rec::local_backward<float>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
-  if (d->precision == RECNET_PREC_BF16) return rec::local_backward<bf16>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
+  if (dd.precision == RECNET_PREC_FP32) return rec::local_backward<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
+  if (dd.precision == RECNET_PREC_BF16) return rec::local_backward<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_local_bwd_phase(const recnet_local_desc* d, const recnet_local_tensors* w, const float* hiddens, const float* feats,
                            const uint64_t* rng, void* workspace, int64_t workspace_bytes, const float* g_mse,
                            const recnet_local_tensors* grads, float* g_hiddens, int phases, void* stream) {
+  LocalDesc dd;
+  RN_TRY(split_desc(d, &dd));
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
   if (phases < 1 || phases > 3) return RECNET_ERR_BAD_SHAPE;
-  if (d->dec_layers > 1) {                 // stacked decoders: not split -- everything belongs to phase bit 0
+  if (dd.dec_layers > 1) {                 // stacked decoders: not split -- everything belongs to phase bit 0
     if (!(phases & 1)) return 0;
     return recnet_local_bwd(d, w, hiddens, feats, rng, workspace, workspace_bytes, g_mse, grads, g_hiddens, stream);
   }
-  if (d->precision == RECNET_PREC_FP32) return rec::local_backward<float>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream), phases);
-  if (d->precision == RECNET_PREC_BF16) return rec::local_backward<bf16>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream), phases);
+  if (dd.precision == RECNET_PREC_FP32) return rec::local_backward<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream), phases);
+  if (dd.precision == RECNET_PREC_BF16) return rec::local_backward<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream), phases);
   return RECNET_ERR_UNSUPPORTED;
 }
 int recnet_set_background_ctas(int n) {
@@ -429,8 +496,10 @@ int recnet_set_background_ctas(int n) {
   return 0;
 }
 float* recnet_local_outputs(const recnet_local_desc* d, void* workspace) {
-  if (d->precision == RECNET_PREC_FP32) return rec::plan_local<float>(*d, workspace).out;
-  return rec::plan_local<bf16>(*d, workspace).out;
+  LocalDesc dd;
+  if (split_desc(d, &dd)) return nullptr;
+  if (dd.precision == RECNET_PREC_FP32) return rec::plan_local<float>(dd, workspace).out;
+  return rec::plan_local<bf16>(dd, workspace).out;
 }
 
 // ---- global reconstructor --------------------------------------------------------------------------------------

@@ -147,7 +147,7 @@ static int prepare(const recnet_decoder_desc& d, const recnet_decoder_tensors& p
 // one decoder step for the sample rows [b0, b0+nb) of chain `ch`: attention -> gate GEMM -> cell.
 // Pointer arguments are the FULL-batch row-0 addresses of step t; the row offset is applied here.
 template <typename T>
-static int step(mega::Emitter<T>& em, const recnet_decoder_desc& d, const recnet_decoder_tensors& p, Ws<T>& w, int t, int ch,
+static int step(mega::Emitter<T>& em, const DecDesc& d, const recnet_decoder_tensors& p, Ws<T>& w, int t, int ch,
                 int b0, int nb, const float* gx_t, T* x_t, T* x_next, float* Wh_t, float* e_t, T* gates_t, const float* c_prev,
                 float* c_next, float* h_out) {
   const int H = d.H, E = d.E, A = d.A, Tn = d.T;
@@ -164,7 +164,7 @@ static int step(mega::Emitter<T>& em, const recnet_decoder_desc& d, const recnet
   fa.Uv = w.Uv + (size_t)b0 * Tn * A; fa.uv_bs = (long long)Tn * A; fa.uv_ts = A;
   fa.attn_b = p.attn_b; fa.attn_w = p.attn_w;
   fa.V = w.feats + (size_t)b0 * Tn * E; fa.v_bs = (long long)Tn * E; fa.v_ts = E;
-  fa.B = nb; fa.Tn = Tn; fa.A = A; fa.D = E; fa.inv_T = 1.f / Tn; fa.normalize = 0;
+  fa.B = nb; fa.Tn = Tn; fa.A = A; fa.D = E; fa.inv_T = d.softmax ? 1.f : 1.f / Tn; fa.normalize = d.softmax;
   fa.Wh_out = Wh_t ? Wh_t + (size_t)b0 * A : nullptr; fa.e_out = e_t ? e_t + (size_t)b0 * Tn : nullptr;
   fa.ctx_out = xr; fa.ctx_ld = w.KX; fa.p_drop = 0.f;
   RN_TRY(em.attn_fwd(fa));
@@ -197,7 +197,7 @@ static int step(mega::Emitter<T>& em, const recnet_decoder_desc& d, const recnet
 }
 
 template <typename T>
-static int forward(const recnet_decoder_desc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
+static int forward(const DecDesc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
                    const long long* targets, const float* ce_weight, const unsigned long long* rng, void* ws, long long ws_bytes,
                    float* hiddens, float* ce_out, cudaStream_t st) {
   RN_TRY(check(d));
@@ -255,7 +255,7 @@ static int forward(const recnet_decoder_desc& d, const recnet_decoder_tensors& p
 }
 
 template <typename T>
-static int backward(const recnet_decoder_desc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
+static int backward(const DecDesc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
                     const long long* targets, const float* ce_weight, const unsigned long long* rng, void* ws, long long ws_bytes,
                     const float* g_ce, const float* g_hiddens, const float* hiddens_fp32, const recnet_decoder_tensors& g,
                     cudaStream_t st) {
@@ -311,10 +311,10 @@ static int backward(const recnet_decoder_desc& d, const recnet_decoder_tensors& 
         ab.dXp = dXx; ab.n_p = w.pl_dxx.splits; ab.p_stride = (long long)nb * E; ab.p_ld = E;
         ab.V = w.feats + (size_t)b0 * Tn * E; ab.v_bs = (long long)Tn * E; ab.v_ts = E;
         ab.Wh = w.Wh + r * A; ab.Uv = w.Uv + (size_t)b0 * Tn * A; ab.uv_bs = (long long)Tn * A; ab.uv_ts = A;
-        ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = Tn; ab.A = A; ab.D = E; ab.inv_T = 1.f / Tn;
+        ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = Tn; ab.A = A; ab.D = E; ab.inv_T = d.softmax ? 1.f : 1.f / Tn;
         ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv + (size_t)b0 * Tn * A;
         ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc + (size_t)b0 * A;
-        ab.dctx_out = nullptr; ab.de_out = nullptr; ab.p_drop = 0.f;
+        ab.dctx_out = nullptr; ab.de_out = nullptr; ab.p_drop = 0.f; ab.alpha = d.softmax ? w.e + r * Tn : nullptr;
         RN_TRY(em.attn_bwd(ab));
         if (t > 0) RN_TRY(em.gemm_partials(w.dWh_op + r * A, A, 0, w.Wa, H, 1, dQp, nb, H, A, w.pl_dq));
         continue;
@@ -335,10 +335,10 @@ static int backward(const recnet_decoder_desc& d, const recnet_decoder_tensors& 
       ab.dXp = dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)nb * w.KX; ab.p_ld = w.KX;
       ab.V = w.feats + (size_t)b0 * Tn * E; ab.v_bs = (long long)Tn * E; ab.v_ts = E;
       ab.Wh = w.Wh + r * A; ab.Uv = w.Uv + (size_t)b0 * Tn * A; ab.uv_bs = (long long)Tn * A; ab.uv_ts = A;
-      ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = Tn; ab.A = A; ab.D = E; ab.inv_T = 1.f / Tn;
+      ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = Tn; ab.A = A; ab.D = E; ab.inv_T = d.softmax ? 1.f : 1.f / Tn;
       ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv + (size_t)b0 * Tn * A;
       ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc + (size_t)b0 * A;
-      ab.dctx_out = nullptr; ab.de_out = nullptr; ab.p_drop = 0.f;
+      ab.dctx_out = nullptr; ab.de_out = nullptr; ab.p_drop = 0.f; ab.alpha = d.softmax ? w.e + r * Tn : nullptr;
       RN_TRY(em.attn_bwd(ab));
       // attention-query path into h_{t-1}: dWh_t @ attn_W, consumed (as split-K partials) by the next cell backward
       if (t > 0) RN_TRY(em.gemm_partials(w.dWh_op + r * A, A, 0, w.Wa, H, 1, dQp, nb, H, A, w.pl_dq));
@@ -432,9 +432,9 @@ static GreedyWs<T> plan_greedy(const recnet_decoder_desc& d, void* base, int max
 }
 
 template <typename T>
-static int greedy(const recnet_decoder_desc& d0, const recnet_decoder_tensors& p, const float* feats, int max_steps, void* ws,
+static int greedy(const DecDesc& d0, const recnet_decoder_tensors& p, const float* feats, int max_steps, void* ws,
                   long long ws_bytes, long long* ids_out, int* n_steps_out, cudaStream_t st) {
-  recnet_decoder_desc d = d0; d.L = 1; d.train = 0;
+  DecDesc d = d0; d.L = 1; d.train = 0;
   RN_TRY(check(d));
   GreedyWs<T> g = plan_greedy<T>(d0, ws, max_steps);
   if ((long long)g.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
@@ -593,9 +593,9 @@ static BeamWs<T> plan_beam(const recnet_decoder_desc& d, void* base, int K, int 
 
 // d0.B = K * B0 rows; feats [K * B0, T, E] = the B0 samples tiled K times; seq_out [B0, max_steps] int64 (-1 beyond n_steps)
 template <typename T>
-static int beam(const recnet_decoder_desc& d0, const recnet_decoder_tensors& p, const float* feats, int K, int max_steps, long long eos,
+static int beam(const DecDesc& d0, const recnet_decoder_tensors& p, const float* feats, int K, int max_steps, long long eos,
                 void* ws, long long ws_bytes, long long* seq_out, int* n_steps_out, cudaStream_t st) {
-  recnet_decoder_desc d = d0; d.L = 1; d.train = 0;
+  DecDesc d = d0; d.L = 1; d.train = 0;
   RN_TRY(check(d));
   if (K < 1 || K > BEAM_MAX_K || d.B % K || max_steps < 1 || max_steps > 64 || K > d.V) return RECNET_ERR_BAD_SHAPE;
   BeamWs<T> bw = plan_beam<T>(d0, ws, K, max_steps);

@@ -16,6 +16,8 @@
 // per CTA, which a 13-sample x 136-row slice cannot fill either way round, hence the warp-level MMA here (the batched GEMMs around
 // the loop and the reconstructor loops use tcgen05).
 //
+// SM = true: the paper's softmax attention (opt-in): after barrier #2 every sample warp holds its whole score row (Tn <= 32) and turns it
+// into alpha with one warp max / sum-exp; the context sum takes alpha with scale 1 (the host passes inv_T = 1) and the e stash holds alpha.
 // Stash layout = what pf_fwd_kernel / pf_bwd_kernel leave (Hop, c, hiddens, Wh, e, gates; dGW, dWh, dUv, dw_acc), so either loop
 // implementation can run in front of / behind the other and the batched GEMMs after the loop are unchanged.
 #pragma once
@@ -99,7 +101,7 @@ struct FwdArgs {
   float* c;                       // [(L+1) B, H] fp32 cell states, row block 0 = zeros
   float* hiddens;                 // [L B, H] fp32
   bf16* Hop;                      // [(L+1) B, H] operand rows, row block 0 = zeros
-  float* Wh; float* e;            // [L B, A], [L B, Tn] stash
+  float* Wh; float* e;            // [L B, A], [L B, Tn] stash (alpha when SM)
   bf16* gates;                    // [L B, H, 4] stash
   int B, L, Tn, MS;               // MS = samples per cluster
   float inv_T;
@@ -121,7 +123,7 @@ __host__ __device__ inline SmemF smem_fwd() {
 }
 
 // NQ = frames held in registers per thread (a multiple of 4 >= Tn)
-template <int NQ>
+template <int NQ, bool SM>
 __global__ void __launch_bounds__(THREADS, 1) decoder_fwd_cluster_kernel(const FwdArgs a) {
   extern __shared__ __align__(16) unsigned char smem[];
   const SmemF S = smem_fwd();
@@ -259,12 +261,22 @@ __global__ void __launch_bounds__(THREADS, 1) decoder_fwd_cluster_kernel(const F
       const float val = f ? sc[1] : sc[0];
       if (act && tau < Tn) {
         st_c_f32(mapa(es_sa + (uint32_t)((s_w * MAXT + tau) * 4), (uint32_t)(lane >> 1)), val);
-        if (lane < 2) a.e[((size_t)t * B + b) * Tn + tau] = val;
+        if (!SM && lane < 2) a.e[((size_t)t * B + b) * Tn + tau] = val;
       }
     }
     stamp(23);
     cluster_barrier();                                          // #2 (also orders this step's og writes before the reads below)
     stamp(24);
+    if constexpr (SM) {       // this warp's row only: the next remote stores into es come after barrier #1 of the next step
+      float* er = es + s_w * MAXT;
+      const float al = warp_softmax<true>(er[lane], lane < Tn);
+      __syncwarp();
+      if (act) {
+        if (lane < Tn) er[lane] = al;
+        if (r == 0 && lane < Tn) a.e[((size_t)t * B + b) * Tn + lane] = al;
+      }
+      __syncwarp();
+    }
     // ---- P3: context sum over the frames (features from registers), gates, c_t, h_t
     {
       float acc[4] = {0.f, 0.f, 0.f, 0.f};
@@ -355,9 +367,9 @@ static int pick_ms(K kern, size_t smem, int B) {
   return ms <= MAX_MS ? ms : 0;
 }
 
-template <int NQ>
+template <int NQ, bool SM>
 static int launch_fwd_nq(FwdArgs a, cudaStream_t st) {
-  auto kern = decoder_fwd_cluster_kernel<NQ>;
+  auto kern = decoder_fwd_cluster_kernel<NQ, SM>;
   const size_t smem = smem_fwd().total;
   static bool configured = false;
   static int ms_cache_B = -1, ms_cache = 0;
@@ -380,7 +392,9 @@ static int launch_fwd_nq(FwdArgs a, cudaStream_t st) {
   RN_LAUNCH_OK();
   return 0;
 }
-static int launch_fwd(const FwdArgs& a, cudaStream_t st) {
-  return a.Tn <= 28 ? launch_fwd_nq<28>(a, st) : launch_fwd_nq<32>(a, st);
+// softmax: the paper's attention (a.inv_T must then be 1)
+static int launch_fwd(const FwdArgs& a, bool softmax, cudaStream_t st) {
+  if (softmax) return a.Tn <= 28 ? launch_fwd_nq<28, true>(a, st) : launch_fwd_nq<32, true>(a, st);
+  return a.Tn <= 28 ? launch_fwd_nq<28, false>(a, st) : launch_fwd_nq<32, false>(a, st);
 }
 }  // namespace dcl

@@ -11,7 +11,7 @@ namespace dec {
 enum : unsigned { SITE_LAYER0 = 16 };     // dropout site of the input of layer l = SITE_LAYER0 + l
 
 template <typename T>
-static int forward_ml(const recnet_decoder_desc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
+static int forward_ml(const DecDesc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
                       const long long* targets, const float* ce_weight, const unsigned long long* rng, void* ws, long long ws_bytes,
                       float* hiddens, float* ce_out, cudaStream_t st) {
   RN_TRY(check(d));
@@ -49,7 +49,8 @@ static int forward_ml(const recnet_decoder_desc& d, const recnet_decoder_tensors
     attn::FwdArgs fa{};
     fa.WhP = w.WhP; fa.n_whp = n_whp; fa.whp_stride = (long long)B * A;
     fa.Uv = w.Uv; fa.uv_bs = (long long)Tn * A; fa.uv_ts = A; fa.attn_b = p.attn_b; fa.attn_w = p.attn_w;
-    fa.V = w.feats; fa.v_bs = (long long)Tn * E; fa.v_ts = E; fa.B = B; fa.Tn = Tn; fa.A = A; fa.D = E; fa.inv_T = 1.f / Tn;
+    fa.V = w.feats; fa.v_bs = (long long)Tn * E; fa.v_ts = E; fa.B = B; fa.Tn = Tn; fa.A = A; fa.D = E;
+    fa.inv_T = d.softmax ? 1.f : 1.f / Tn; fa.normalize = d.softmax;
     fa.Wh_out = w.Wh + (size_t)t * B * A; fa.e_out = w.e + (size_t)t * B * Tn; fa.ctx_out = x0; fa.ctx_ld = w.KX;
     RN_TRY(em.attn_fwd(fa));
     for (int l = 0; l < NL; ++l) {
@@ -85,7 +86,7 @@ static int forward_ml(const recnet_decoder_desc& d, const recnet_decoder_tensors
 }
 
 template <typename T>
-static int backward_ml(const recnet_decoder_desc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
+static int backward_ml(const DecDesc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
                        const long long* targets, const float* ce_weight, const unsigned long long* rng, void* ws, long long ws_bytes,
                        const float* g_ce, const float* g_hiddens, const recnet_decoder_tensors& g, cudaStream_t st) {
   RN_TRY(check(d));
@@ -138,7 +139,8 @@ static int backward_ml(const recnet_decoder_desc& d, const recnet_decoder_tensor
     ab.dXp = w.dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)B * w.KX; ab.p_ld = w.KX;
     ab.V = w.feats; ab.v_bs = (long long)Tn * E; ab.v_ts = E;
     ab.Wh = w.Wh + (size_t)t * B * A; ab.Uv = w.Uv; ab.uv_bs = (long long)Tn * A; ab.uv_ts = A;
-    ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = B; ab.Tn = Tn; ab.A = A; ab.D = E; ab.inv_T = 1.f / Tn;
+    ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = B; ab.Tn = Tn; ab.A = A; ab.D = E;
+    ab.inv_T = d.softmax ? 1.f : 1.f / Tn; ab.alpha = d.softmax ? w.e + (size_t)t * B * Tn : nullptr;
     ab.dWh_out = w.dWh + (size_t)t * B * A; ab.dWh_op = w.dWh_op + (size_t)t * B * A; ab.dUv_acc = w.dUv;
     ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc;
     RN_TRY(em.attn_bwd(ab));

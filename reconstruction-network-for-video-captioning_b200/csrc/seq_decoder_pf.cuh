@@ -120,7 +120,7 @@ static inline int gemm_to_operand(const bf16* A, long long lda, const bf16* B, l
 }
 
 template <typename T>
-static int forward_pf(const recnet_decoder_desc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
+static int forward_pf(const DecDesc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
                       const long long* targets, const float* ce_weight, const unsigned long long* rng, void* ws, long long ws_bytes,
                       float* hiddens, float* ce_out, cudaStream_t st, int phases = 3) {
   // phases (recnet_decoder_fwd_phase): 1 = staging, hoisted projections and the time loop (-> hiddens), 2 = vocabulary projection, per-step
@@ -130,6 +130,7 @@ static int forward_pf(const recnet_decoder_desc& d, const recnet_decoder_tensors
   if ((long long)w.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
   const int B = d.B, L = d.L, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, EMB = d.EMB;
   const float p_emb = d.train ? d.p_emb_drop : 0.f, p_out = d.train ? d.p_out_drop : 0.f;
+  const float inv_T = d.softmax ? 1.f : 1.f / Tn;             // softmax: alpha weights, summed without the 1/T of the mean
   const long long ldih = EMB + E;
   if (phases & 1) {
   // operand copies of the weights / features (the optimiser changes the fp32 masters every step)
@@ -165,8 +166,8 @@ static int forward_pf(const recnet_decoder_desc& d, const recnet_decoder_tensors
       // the whole time loop as ONE kernel of independent 16-CTA clusters, [W_a ; W_hh] resident in distributed shared memory
       dcl::FwdArgs ca{};
       ca.Wcat = w.Wcat; ca.Uv = w.Uv; ca.attn_w = p.attn_w; ca.VW = w.VW; ca.Gx = w.Gx; ca.b_hh = p.b_hh; ca.c = w.c; ca.hiddens = hiddens;
-      ca.Hop = w.Hop; ca.Wh = w.Wh; ca.e = w.e; ca.gates = w.gates; ca.B = B; ca.L = L; ca.Tn = Tn; ca.inv_T = 1.f / Tn;
-      const int rc = dcl::launch_fwd(ca, st);
+      ca.Hop = w.Hop; ca.Wh = w.Wh; ca.e = w.e; ca.gates = w.gates; ca.B = B; ca.L = L; ca.Tn = Tn; ca.inv_T = inv_T;
+      const int rc = dcl::launch_fwd(ca, d.softmax, st);
       if (rc == 0) clustered = true;
       else if (rc != RECNET_ERR_UNSUPPORTED) return rc;
     }
@@ -179,10 +180,10 @@ static int forward_pf(const recnet_decoder_desc& d, const recnet_decoder_tensors
     fa.P = w.P; fa.n_p = t > 0 ? w.pl_h.splits : 0; fa.p_stride = (long long)B * w.NP; fa.NP = w.NP;
     fa.Uv = w.Uv; fa.attn_w = p.attn_w; fa.VW = w.VW;
     fa.Gx = w.Gx + r * 4 * H; fa.b_hh = p.b_hh; fa.c_prev = w.c + r * H;
-    fa.B = B; fa.Tn = Tn; fa.A = A; fa.H = H; fa.inv_T = 1.f / Tn;
+    fa.B = B; fa.Tn = Tn; fa.A = A; fa.H = H; fa.inv_T = inv_T;
     fa.Wh_out = w.Wh + r * A; fa.e_out = w.e + r * Tn; fa.gates_out = w.gates + r * 4 * H;
     fa.c_out = w.c + (r + B) * H; fa.h_out = hiddens + r * H; fa.h_op = w.Hop + (r + B) * H;
-    RN_TRY((pf::launch_fwd<T, T>(fa, st)));
+    RN_TRY((pf::launch_fwd<T, T>(fa, d.softmax, st)));
   }
   }   // phases & 1
   if (!(phases & 2)) return 0;
@@ -202,7 +203,7 @@ static int forward_pf(const recnet_decoder_desc& d, const recnet_decoder_tensors
     // measured; the two-wave grid costs the GEMM a 20 us late start at worst)
     const int spc = 1;
     pf::pf_escore_kernel<T, true><<<dim3(rn_cdiv(E, 512), rn_cdiv(B, spc)), 256, pf::escore_smem(L, Tn, true), s3>>>(w.e, w.feats, E, 0, w.ctx, L, B,
-                                                                                                               Tn, E, 1.f / Tn, spc);
+                                                                                                               Tn, E, inv_T, spc);
     RN_LAUNCH_OK();
   }
   if (targets && ce_weight && ce_out) {
@@ -218,7 +219,7 @@ static int forward_pf(const recnet_decoder_desc& d, const recnet_decoder_tensors
 }
 
 template <typename T>
-static int backward_pf(const recnet_decoder_desc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
+static int backward_pf(const DecDesc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
                        const long long* targets, const float* ce_weight, const unsigned long long* rng, void* ws, long long ws_bytes,
                        const float* g_ce, const float* g_hiddens, const recnet_decoder_tensors& g, cudaStream_t st, int phases = 15) {
   // phases (recnet_decoder_bwd_phase): 1 = CE backward + gradient wrt the states through the vocabulary projection, 2 = the BPTT loop,
@@ -251,7 +252,7 @@ static int backward_pf(const recnet_decoder_desc& d, const recnet_decoder_tensor
     ba.dc = w.dc; ba.first = last ? 1 : 0;
     ba.gates = w.gates + r * 4 * H; ba.c_prev = w.c + r * H; ba.c_new = w.c + (r + B) * H;
     ba.VW = w.VW; ba.Wh = w.Wh + r * A; ba.Uv = w.Uv; ba.attn_w = p.attn_w;
-    ba.B = B; ba.Tn = Tn; ba.A = A; ba.H = H; ba.inv_T = 1.f / Tn;
+    ba.B = B; ba.Tn = Tn; ba.A = A; ba.H = H; ba.inv_T = d.softmax ? 1.f : 1.f / Tn; ba.alpha = d.softmax ? w.e + r * Tn : nullptr;
     ba.dGW = w.dGW + r * NP; ba.dgw_ld = NP; ba.dWh_out = w.dWh + r * A;
     ba.dUv_acc = w.dUv; ba.uv_first = last ? 1 : 0; ba.dw_acc = w.dw_acc; ba.dw_first = last ? 1 : 0;
     RN_TRY((pf::launch_bwd<T, T>(ba, st)));
@@ -338,10 +339,10 @@ static inline bool greedy_pf_ok(const recnet_decoder_desc& d) {
   return on && d.precision == RECNET_PREC_BF16 && pf_ok(d) && (long long)d.V * 4 * d.H < (1ll << 31);
 }
 
-static int greedy_pf(const recnet_decoder_desc& d0, const recnet_decoder_tensors& p, const float* feats, int max_steps, void* ws,
+static int greedy_pf(const DecDesc& d0, const recnet_decoder_tensors& p, const float* feats, int max_steps, void* ws,
                      long long ws_bytes, long long* ids_out, int* n_steps_out, cudaStream_t st) {
   typedef bf16 T;
-  recnet_decoder_desc d = d0; d.L = 1; d.train = 0;
+  DecDesc d = d0; d.L = 1; d.train = 0;
   RN_TRY(check(d));
   GreedyPfWs<T> w = plan_greedy_pf<T>(d, ws, max_steps);
   if ((long long)w.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
@@ -378,10 +379,10 @@ static int greedy_pf(const recnet_decoder_desc& d0, const recnet_decoder_tensors
     fa.P = w.P; fa.n_p = t > 0 ? w.pl_h.splits : 0; fa.p_stride = (long long)B * w.NP; fa.NP = w.NP;
     fa.Uv = w.Uv; fa.attn_w = p.attn_w; fa.VW = w.VW;
     fa.Gx = w.EW; fa.gx_rows = w.tok; fa.b_hh = p.b_hh; fa.c_prev = c_p;
-    fa.B = B; fa.Tn = Tn; fa.A = A; fa.H = H; fa.inv_T = 1.f / Tn;
+    fa.B = B; fa.Tn = Tn; fa.A = A; fa.H = H; fa.inv_T = d.softmax ? 1.f : 1.f / Tn;
     fa.Wh_out = nullptr; fa.e_out = nullptr; fa.gates_out = nullptr;
     fa.c_out = c_n; fa.h_out = w.hid; fa.h_op = h_n;
-    RN_TRY((pf::launch_fwd<T, T>(fa, st)));
+    RN_TRY((pf::launch_fwd<T, T>(fa, d.softmax, st)));
     RN_TRY(gemm_full<T>(h_n, H, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
     argmax_feedback_kernel<<<B, 256, 0, st>>>(w.logits, w.Vld, V, ids_out + (size_t)t * B, w.tok, w.nonpad + t);
     RN_LAUNCH_OK();

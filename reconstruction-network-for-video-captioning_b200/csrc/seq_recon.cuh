@@ -132,7 +132,7 @@ static inline int check_local(const recnet_local_desc& d) {
 }
 
 template <typename T>
-static int local_forward(const recnet_local_desc& d, const recnet_local_tensors& p, const float* hiddens, const float* feats,
+static int local_forward(const LocalDesc& d, const recnet_local_tensors& p, const float* hiddens, const float* feats,
                          const unsigned long long* rng, void* ws, long long ws_bytes, float* mse_out, cudaStream_t st) {
   RN_TRY(check_local(d));
   LocalWs<T> w = plan_local<T>(d, ws);
@@ -160,11 +160,11 @@ static int local_forward(const recnet_local_desc& d, const recnet_local_tensors&
     if (persist) {
       // ONE cooperative launch for all S steps, [W_ih | W_hh] resident in shared memory (seq_recon_persist.cuh); same stash layout
       rp::FwdParams fp{};
-      fp.B = B; fp.S = S; fp.R = R; fp.H = H; fp.A = A; fp.L = L; fp.inv_L = 1.f / L; fp.p_drop = p_drop;
+      fp.B = B; fp.S = S; fp.R = R; fp.H = H; fp.A = A; fp.L = L; fp.inv_L = d.softmax ? 1.f : 1.f / L; fp.p_drop = p_drop;
       fp.X = w.X; fp.Hd = w.Hd; fp.Uv = w.Uv; fp.Wa = w.Wa; fp.attn_b = p.attn_b; fp.attn_w = p.attn_w; fp.b_ih = p.b_ih; fp.b_hh = p.b_hh;
       fp.Wh = w.Wh; fp.beta = w.beta; fp.gates = w.gates; fp.c = w.c; fp.XP = w.pXP; fp.WhP = w.pWhP; fp.sync = w.psync; fp.err = w.err;
       fp.rng = rng; fp.site = SITE_LOCAL_X;
-      RN_TRY(rp::launch_local_fwd(fp, w.Wrec, st));
+      RN_TRY(rp::launch_local_fwd(fp, w.Wrec, d.softmax, st));
       RN_TRY(gemm_full<T>(w.X + (size_t)B * w.KX + H, w.KX, 0, w.Wout, R, 0, w.out, R, p.out_b, S * B, R, R, 0, w.splitk, st));
       if (mse_out) {
         loss::mse_local_fwd_kernel<<<MSE_BLOCKS, 256, 0, st>>>(w.out, feats, S, B, R, w.partial);
@@ -200,7 +200,7 @@ static int local_forward(const recnet_local_desc& d, const recnet_local_tensors&
       fa.Uv = w.Uv + (size_t)b0 * A; fa.uv_bs = A; fa.uv_ts = (long long)B * A;          // Uv is [L,B,A]
       fa.attn_b = p.attn_b; fa.attn_w = p.attn_w;
       fa.V = w.Hd + (size_t)b0 * H; fa.v_bs = H; fa.v_ts = (long long)B * H;             // values = decoder states [L,B,H]
-      fa.B = nb; fa.Tn = L; fa.A = A; fa.D = H; fa.inv_T = 1.f / L; fa.normalize = 0;
+      fa.B = nb; fa.Tn = L; fa.A = A; fa.D = H; fa.inv_T = d.softmax ? 1.f : 1.f / L; fa.normalize = d.softmax;
       fa.Wh_out = w.Wh + r * A; fa.e_out = w.beta + r * L;
       fa.ctx_out = x_t; fa.ctx_ld = w.KX;
       fa.p_drop = p_drop; fa.rng = rng; fa.site = SITE_LOCAL_X; fa.drop_base = (long long)r * H;
@@ -248,7 +248,7 @@ static int local_backward_weights(const recnet_local_desc& d, const LocalWs<T>& 
 // parameter gradients over the stashed operands.  recnet_local_bwd runs both; a trainer may run bit 1 on a second stream underneath
 // the decoder's backward loop (recnet_local_bwd_phase, functional.deferred_weight_grads).
 template <typename T>
-static int local_backward(const recnet_local_desc& d, const recnet_local_tensors& p, const float* hiddens, const float* feats,
+static int local_backward(const LocalDesc& d, const recnet_local_tensors& p, const float* hiddens, const float* feats,
                           const unsigned long long* rng, void* ws, long long ws_bytes, const float* g_mse,
                           const recnet_local_tensors& g, float* g_hiddens, cudaStream_t st, int phases = 3) {
   RN_TRY(check_local(d));
@@ -271,10 +271,11 @@ static int local_backward(const recnet_local_desc& d, const recnet_local_tensors
     if (persist) {
       // ONE cooperative launch for the whole BPTT loop, [W_ih | W_hh] resident in shared memory (seq_recon_persist.cuh)
       rp::BwdParams bp{};
-      bp.B = B; bp.S = S; bp.R = R; bp.H = H; bp.A = A; bp.L = L; bp.inv_L = 1.f / L; bp.p_drop = p_drop;
+      bp.B = B; bp.S = S; bp.R = R; bp.H = H; bp.A = A; bp.L = L; bp.inv_L = d.softmax ? 1.f : 1.f / L; bp.p_drop = p_drop;
       bp.Hd = w.Hd; bp.Uv = w.Uv; bp.Wa = w.Wa; bp.attn_b = p.attn_b; bp.attn_w = p.attn_w; bp.Wh = w.Wh; bp.gates = w.gates; bp.c = w.c;
       bp.dHext = w.dHext; bp.dG = w.dG; bp.dx = w.dx; bp.dWh = w.dWh; bp.dWh_op = w.dWh_op; bp.dUv = w.dUv; bp.dw_acc = w.dw_acc;
       bp.DP = w.pXP; bp.sync = w.psync + rp::SYNC_WORDS; bp.err = w.err; bp.rng = rng; bp.site = SITE_LOCAL_X;
+      bp.alpha = d.softmax ? w.beta : nullptr;
       RN_TRY(rp::launch_local_bwd(bp, w.Wrec, st));
     }
   }
@@ -306,10 +307,10 @@ static int local_backward(const recnet_local_desc& d, const recnet_local_tensors
         ab.dXp = dXx; ab.n_p = w.pl_dxx.splits; ab.p_stride = (long long)nb * H; ab.p_ld = H;
         ab.V = w.Hd + (size_t)b0 * H; ab.v_bs = H; ab.v_ts = (long long)B * H;
         ab.Wh = w.Wh + r * A; ab.Uv = w.Uv + (size_t)b0 * A; ab.uv_bs = A; ab.uv_ts = (long long)B * A;
-        ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = 1.f / L;
+        ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = d.softmax ? 1.f : 1.f / L;
         ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv + (size_t)b0 * A;
         ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc + (size_t)b0 * A;
-        ab.dctx_out = w.dx + r * H; ab.de_out = nullptr;
+        ab.dctx_out = w.dx + r * H; ab.de_out = nullptr; ab.alpha = d.softmax ? w.beta + r * L : nullptr;
         ab.p_drop = p_drop; ab.rng = rng; ab.site = SITE_LOCAL_X; ab.drop_base = (long long)r * H;
         RN_TRY(em.attn_bwd(ab));
         if (t > 0) RN_TRY(em.gemm_partials(w.dWh_op + r * A, A, 0, w.Wa, R, 1, dQp, nb, R, A, w.pl_dq));
@@ -329,10 +330,10 @@ static int local_backward(const recnet_local_desc& d, const recnet_local_tensors
       ab.dXp = dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)nb * w.KX; ab.p_ld = w.KX;
       ab.V = w.Hd + (size_t)b0 * H; ab.v_bs = H; ab.v_ts = (long long)B * H;
       ab.Wh = w.Wh + r * A; ab.Uv = w.Uv + (size_t)b0 * A; ab.uv_bs = A; ab.uv_ts = (long long)B * A;
-      ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = 1.f / L;
+      ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = d.softmax ? 1.f : 1.f / L;
       ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv + (size_t)b0 * A;
       ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc + (size_t)b0 * A;
-      ab.dctx_out = w.dx + r * H; ab.de_out = nullptr;
+      ab.dctx_out = w.dx + r * H; ab.de_out = nullptr; ab.alpha = d.softmax ? w.beta + r * L : nullptr;
       ab.p_drop = p_drop; ab.rng = rng; ab.site = SITE_LOCAL_X; ab.drop_base = (long long)r * H;
       RN_TRY(em.attn_bwd(ab));
       if (t > 0) RN_TRY(em.gemm_partials(w.dWh_op + r * A, A, 0, w.Wa, R, 1, dQp, nb, R, A, w.pl_dq));
@@ -340,10 +341,10 @@ static int local_backward(const recnet_local_desc& d, const recnet_local_tensors
   }
   RN_TRY(em0.flush(w.table, w.table_bytes, w.bar, w.err, 4));
   if (w.nch > 1) RN_TRY(cs.join(st, w.nch));
-  // gradient wrt the decoder states: through U (keys) and through the weighted mean (values)
+  // gradient wrt the decoder states: through U (keys) and through the weighted mean / softmax-weighted sum (values)
   RN_TRY(misc::cast_pad<T>(w.dUv, A, w.dUv_op, A, (long long)L * B, A, A, st));
   RN_TRY(gemm_full<T>(w.dUv_op, A, 0, w.U, H, 1, g_hiddens, H, nullptr, L * B, H, A, 0, w.splitk2, st));
-  RN_TRY(attn::launch_dv(w.beta, w.dx, g_hiddens, H, (long long)B * H, S, B, L, H, 1.f / L, 1, 1, 0, st));
+  RN_TRY(attn::launch_dv(w.beta, w.dx, g_hiddens, H, (long long)B * H, S, B, L, H, d.softmax ? 1.f : 1.f / L, 1, 1, 0, st));
   if (phases & 2) RN_TRY(local_backward_weights<T>(d, w, g, st));
   return 0;
 }
@@ -489,7 +490,7 @@ static int global_forward(const recnet_global_desc& d, const recnet_global_tenso
       fp.B = B; fp.S = L; fp.R = R; fp.H = 0; fp.A = 0; fp.L = 1; fp.inv_L = 1.f; fp.p_drop = 0.f;
       fp.X = w.X; fp.b_ih = p.b_ih; fp.b_hh = p.b_hh; fp.gates = w.gates; fp.c = w.c; fp.XP = w.pXP; fp.sync = w.psync; fp.err = w.err;
       fp.global_mode = 1; fp.Gx = w.Gx;
-      RN_TRY(rp::launch_local_fwd(fp, w.Whh, st));
+      RN_TRY(rp::launch_local_fwd(fp, w.Whh, false, st));
     }
   }
   Chains& cs = chains();

@@ -18,7 +18,7 @@ __global__ void copy_rows_kernel(const T* __restrict__ src, long long src_row_st
 }
 
 template <typename T>
-static int local_forward_ml(const recnet_local_desc& d, const recnet_local_tensors& p, const float* hiddens, const float* feats,
+static int local_forward_ml(const LocalDesc& d, const recnet_local_tensors& p, const float* hiddens, const float* feats,
                             const unsigned long long* rng, void* ws, long long ws_bytes, float* mse_out, cudaStream_t st) {
   RN_TRY(check_local(d));
   LocalWs<T> w = plan_local<T>(d, ws);
@@ -54,7 +54,7 @@ static int local_forward_ml(const recnet_local_desc& d, const recnet_local_tenso
       fa.Uv = w.Uv + (size_t)l * B * A; fa.uv_bs = A; fa.uv_ts = (long long)NLd * B * A;          // Uv is (L, NLd, B, A)
       fa.attn_b = p.attn_b; fa.attn_w = p.attn_w;
       fa.V = w.Hd + (size_t)l * B * H; fa.v_bs = H; fa.v_ts = (long long)NLd * B * H;             // layer l of (L, NLd, B, H)
-      fa.B = B; fa.Tn = L; fa.A = A; fa.D = H; fa.inv_T = 1.f / L;
+      fa.B = B; fa.Tn = L; fa.A = A; fa.D = H; fa.inv_T = d.softmax ? 1.f : 1.f / L; fa.normalize = d.softmax;   // softmax per layer
       fa.Wh_out = w.Wh + q * B * A; fa.e_out = w.beta + q * B * L; fa.ctx_out = x_q; fa.ctx_ld = w.KX;
       fa.p_drop = p_drop; fa.rng = rng; fa.site = SITE_LOCAL_X; fa.drop_base = (long long)q * B * H;
       RN_TRY(em.attn_fwd(fa));
@@ -84,7 +84,7 @@ static int local_forward_ml(const recnet_local_desc& d, const recnet_local_tenso
 }
 
 template <typename T>
-static int local_backward_ml(const recnet_local_desc& d, const recnet_local_tensors& p, const float* hiddens, const float* feats,
+static int local_backward_ml(const LocalDesc& d, const recnet_local_tensors& p, const float* hiddens, const float* feats,
                              const unsigned long long* rng, void* ws, long long ws_bytes, const float* g_mse,
                              const recnet_local_tensors& g, float* g_hiddens, cudaStream_t st) {
   RN_TRY(check_local(d));
@@ -118,7 +118,8 @@ static int local_backward_ml(const recnet_local_desc& d, const recnet_local_tens
     ab.dXp = w.dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)B * w.KX; ab.p_ld = w.KX;
     ab.V = w.Hd + (size_t)l * B * H; ab.v_bs = H; ab.v_ts = (long long)NLd * B * H;
     ab.Wh = w.Wh + (size_t)q * B * A; ab.Uv = w.Uv + (size_t)l * B * A; ab.uv_bs = A; ab.uv_ts = (long long)NLd * B * A;
-    ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = B; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = 1.f / L;
+    ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = B; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = d.softmax ? 1.f : 1.f / L;
+    ab.alpha = d.softmax ? w.beta + (size_t)q * B * L : nullptr;
     ab.dWh_out = w.dWh + (size_t)t * B * A; ab.dWh_op = w.dWh_op + (size_t)t * B * A;          // summed over the NLd attentions of step t
     ab.dwh_acc = (l != NLd - 1) ? 1 : 0;
     ab.dUv_acc = w.dUv + (size_t)l * B * A; ab.uv_first = (t == S - 1) ? 1 : 0;
@@ -140,7 +141,7 @@ static int local_backward_ml(const recnet_local_desc& d, const recnet_local_tens
   RN_TRY(misc::colsum<float>(w.dw_acc, A, B, A, g.attn_w, 0, w.splitk, st));
   RN_TRY(gemm_full<T>(w.dUv_op, A, 0, w.U, H, 1, g_hiddens, H, nullptr, L * NLd * B, H, A, 0, w.splitk, st));
   for (int l = 0; l < NLd; ++l)
-    RN_TRY(attn::launch_dv(w.beta, w.dx, g_hiddens + (size_t)l * B * H, H, (long long)NLd * B * H, S, B, L, H, 1.f / L, 1, NLd, l, st));
+    RN_TRY(attn::launch_dv(w.beta, w.dx, g_hiddens + (size_t)l * B * H, H, (long long)NLd * B * H, S, B, L, H, d.softmax ? 1.f : 1.f / L, 1, NLd, l, st));
   return 0;
 }
 }  // namespace rec

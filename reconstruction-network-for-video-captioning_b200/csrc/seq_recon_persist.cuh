@@ -44,7 +44,7 @@ struct FwdParams {
   const bf16* Wa;                     // [A, R]
   const float *attn_b, *attn_w, *b_ih, *b_hh;
   float* Wh;                          // [S, B, A] stash (query without the bias)
-  float* beta;                        // [S, B, L] stash (scores)
+  float* beta;                        // [S, B, L] stash (scores; alpha with the softmax attention)
   bf16* gates;                        // [S*B, 4R] activated gates
   float* c;                           // [(S+1)*B, R]
   float* XP;                          // [UG][KS][B][128] K-slice partials of the pre-activations
@@ -276,7 +276,9 @@ __device__ __forceinline__ void cell_query_phase(const FwdParams& p, const CellC
       }
 }
 
-template <int KS>
+// SM = true: the paper's softmax attention (opt-in) -- alpha over the Ln <= 32 scores in every attention warp's registers, weighted sum
+// with scale 1 (the host passes inv_L = 1), alpha stashed in `beta`
+template <int KS, bool SM>
 __global__ void __launch_bounds__(THREADS, 1)
 local_fwd_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmW, const FwdParams p) {
   extern __shared__ uint8_t smem_raw[];
@@ -522,20 +524,25 @@ local_fwd_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
         if (lane < 4) {
           const float s = lane == 0 ? sc[0] : lane == 1 ? sc[1] : lane == 2 ? sc[2] : sc[3];
           const int l = aw + 8 * lane;
-          if (l < Ln) { e_s[l] = s; p.beta[((long long)t * B + b_att) * Ln + l] = s; }
+          if (l < Ln) { e_s[l] = s; if (!SM) p.beta[((long long)t * B + b_att) * Ln + l] = s; }
         }
         nbar(5, 256);
+        float al = 0.f;                                     // SM: lane l holds alpha[l]
+        if constexpr (SM) {
+          al = warp_softmax<true>(e_s[lane], lane < Ln);
+          if (aw == 0 && lane < Ln) p.beta[((long long)t * B + b_att) * Ln + lane] = al;
+        }
         float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
 #pragma unroll
         for (int l = 0; l < 32; l += 2) {
           if (l < Ln) {
             const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v[l]));
-            const float e = e_s[l];
+            const float e = SM ? __shfl_sync(0xffffffffu, al, l) : e_s[l];
             a0 = fmaf(e, f.x, a0); a1 = fmaf(e, f.y, a1);
           }
           if (l + 1 < Ln) {
             const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v[l + 1]));
-            const float e = e_s[l + 1];
+            const float e = SM ? __shfl_sync(0xffffffffu, al, l + 1) : e_s[l + 1];
             a2 = fmaf(e, f.x, a2); a3 = fmaf(e, f.y, a3);
           }
         }
@@ -612,9 +619,9 @@ static inline size_t xp_floats(const Shape& s) { const int ks = pick_ks(s.R, s.H
 static inline size_t whp_floats(const Shape& s) { return (size_t)(s.R / UNITS + 1) * s.B * s.A; }
 constexpr int SYNC_WORDS = 64 + 32 * MAX_UG;
 
-template <int KS>
+template <int KS, bool SM>
 static int launch_ks(const CUtensorMap& mx, const CUtensorMap& mw, const FwdParams& p, cudaStream_t st) {
-  auto kern = local_fwd_kernel<KS>;
+  auto kern = local_fwd_kernel<KS, SM>;
   const int smem = smem_layout(p.B, KS, p.nst, p.res_kb).total;
   static int attr_smem = 0;
   if (attr_smem < smem) {
@@ -629,7 +636,8 @@ static int launch_ks(const CUtensorMap& mx, const CUtensorMap& mw, const FwdPara
 }
 
 // X / Wrec as the kernel-per-phase path stages them; sync must be zeroed (SYNC_WORDS words) before the launch
-static int launch_local_fwd(FwdParams p, const bf16* Wrec, cudaStream_t st) {
+// softmax: the paper's attention (p.inv_L must then be 1)
+static int launch_local_fwd(FwdParams p, const bf16* Wrec, bool softmax, cudaStream_t st) {
   p.KS = pick_ks(p.R, p.H);
   p.UG = p.R / UNITS; p.NHB = p.R / BK; p.NXB = p.H / BK; p.KX = p.H + p.R;
   p.res_kb = max_res_kb_fwd(p.R, p.H, p.KS); p.nst = pick_stages_fwd(p.B, p.KS, p.res_kb);
@@ -638,10 +646,10 @@ static int launch_local_fwd(FwdParams p, const bf16* Wrec, cudaStream_t st) {
   RN_TRY(make_map(&mx, p.X, (long long)(p.S + 1) * p.B, p.KX, p.KX, BK, p.B));
   RN_TRY(make_map(&mw, Wrec, 4LL * p.R, p.KX, p.KX, BK, UNITS));
   switch (p.KS) {
-    case 1: return launch_ks<1>(mx, mw, p, st);
-    case 2: return launch_ks<2>(mx, mw, p, st);
-    case 3: return launch_ks<3>(mx, mw, p, st);
-    case 4: return launch_ks<4>(mx, mw, p, st);
+    case 1: return softmax ? launch_ks<1, true>(mx, mw, p, st) : launch_ks<1, false>(mx, mw, p, st);
+    case 2: return softmax ? launch_ks<2, true>(mx, mw, p, st) : launch_ks<2, false>(mx, mw, p, st);
+    case 3: return softmax ? launch_ks<3, true>(mx, mw, p, st) : launch_ks<3, false>(mx, mw, p, st);
+    case 4: return softmax ? launch_ks<4, true>(mx, mw, p, st) : launch_ks<4, false>(mx, mw, p, st);
   }
   return RECNET_ERR_UNSUPPORTED;
 }
@@ -677,6 +685,7 @@ struct BwdParams {
   const unsigned long long* rng;
   unsigned site;
   int global_mode;                    // GLOBAL reconstructor: no attention / query path, H = 0 (dX = dG . W_hh only)
+  const float* alpha;                 // [S, B, L] softmax weights of the forward (nullable = the reference's mean)
 };
 constexpr int MAX_NS = 12;
 
@@ -693,6 +702,8 @@ __host__ __device__ inline SmemB smem_layout_bwd(int B, int nst, int res_kb) {
   return s;
 }
 
+// SM = true: softmax attention (p.alpha, inv_L = 1): d e = alpha (d alpha - sum_l alpha[l] d alpha[l]) before the score backward
+template <bool SM>
 __global__ void __launch_bounds__(THREADS, 1)
 local_bwd_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant__ CUtensorMap tmW, const BwdParams p) {
   extern __shared__ uint8_t smem_raw[];
@@ -974,6 +985,11 @@ local_bwd_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant_
       }
       // ======================= A: attention backward of sample b_att, step t =======================
       if (do_attn) {
+        float al[4];
+        if constexpr (SM) {
+#pragma unroll
+          for (int f = 0; f < 4; ++f) al[f] = aw + 8 * f < Ln ? p.alpha[((long long)t * B + b_att) * Ln + aw + 8 * f] : 0.f;
+        }
         if (aw == 0 && lane == 0) { wait_flag(bar2, ncta * (unsigned)(S - t), p.err, abort_); if (cta == 0) stamp(12); }
         nbar(5, 256);
         const float4 wh = reinterpret_cast<const float4*>(p.Wh + ((long long)t * B + b_att) * A)[lane];
@@ -1019,6 +1035,19 @@ local_bwd_kernel(const __grid_constant__ CUtensorMap tmG, const __grid_constant_
         for (int o = 16; o > 0; o >>= 1)
 #pragma unroll
           for (int f = 0; f < 4; ++f) de[f] += __shfl_xor_sync(0xffffffffu, de[f], o);
+        if constexpr (SM) {           // de = d alpha so far; the sum over all frames meets in `red` (free here: last read before the previous barrier)
+          float s1 = 0.f;
+#pragma unroll
+          for (int f = 0; f < 4; ++f) s1 = fmaf(al[f], de[f], s1);
+          if (lane == 0) red[aw] = s1;
+          nbar(5, 256);
+          float tot = 0.f;
+#pragma unroll
+          for (int i = 0; i < 8; ++i) tot += red[i];
+          nbar(5, 256);               // every warp has read red before it is rewritten below
+#pragma unroll
+          for (int f = 0; f < 4; ++f) de[f] = al[f] * (de[f] - tot);
+        }
         // score backward of the same frames (tanh recomputed)
         float4 dwh = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
@@ -1104,7 +1133,8 @@ static inline bool local_bwd_ok(const Shape& s) {
 static inline size_t dp_floats(const Shape& s) { const int ns = pick_ns(s.R, s.H); return ns ? (size_t)((s.R + s.H) / 128) * ns * s.B * 128 : 4; }
 
 // dG / Wrec as the kernel-per-phase path lays them out; sync must be zeroed (SYNC_WORDS words) before the launch
-static int launch_local_bwd(BwdParams p, const bf16* Wrec, cudaStream_t st) {
+template <bool SM>
+static int launch_local_bwd_sm(BwdParams p, const bf16* Wrec, cudaStream_t st) {
   p.KX = p.H + p.R; p.NS = pick_ns(p.R, p.H); p.CG = p.KX / 128; p.NB4 = 4 * p.R / BK; p.UG = p.R / UNITS; p.KT = p.CG * p.NS / p.UG;
   CUtensorMap mg, mw;
   RN_TRY(make_map(&mg, p.dG, (long long)p.S * p.B, 4LL * p.R, 4LL * p.R, BK, p.B));
@@ -1114,13 +1144,17 @@ static int launch_local_bwd(BwdParams p, const bf16* Wrec, cudaStream_t st) {
   const int smem = smem_layout_bwd(p.B, p.nst, p.res_kb).total;
   static int attr_smem = 0;
   if (attr_smem < smem) {
-    RN_CUDA_OK(cudaFuncSetAttribute(local_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    RN_CUDA_OK(cudaFuncSetAttribute(local_bwd_kernel<SM>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     attr_smem = smem;
   }
   void* args[] = {(void*)&mg, (void*)&mw, (void*)&p};
   ProfScope prof(KC_LOOP, p.S, p.CG * p.NS, 1, st);
-  RN_CUDA_OK(cudaLaunchCooperativeKernel((const void*)local_bwd_kernel, dim3(p.CG * p.NS), dim3(THREADS), args, (size_t)smem, st));
+  RN_CUDA_OK(cudaLaunchCooperativeKernel((const void*)local_bwd_kernel<SM>, dim3(p.CG * p.NS), dim3(THREADS), args, (size_t)smem, st));
   RN_LAUNCH_OK();
   return 0;
+}
+// p.alpha != nullptr: softmax attention (p.inv_L must then be 1)
+static int launch_local_bwd(const BwdParams& p, const bf16* Wrec, cudaStream_t st) {
+  return p.alpha ? launch_local_bwd_sm<true>(p, Wrec, st) : launch_local_bwd_sm<false>(p, Wrec, st);
 }
 }  // namespace rp

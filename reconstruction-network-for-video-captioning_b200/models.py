@@ -7,7 +7,9 @@ reference checkpoint loads with ``load_state_dict``.  The arithmetic runs in lib
 * ``forward`` (one timestep, models/decoder.py:45) -> operator-level kernels (``ops.py``)
 * ``forward_sequence`` (whole teacher-forced loop, what train.forward_* use) -> one C call (``functional.py``)
 
-One extra constructor kwarg, ``precision`` ("bf16" | "fp32"); everything else is positional-compatible.
+Extra constructor kwargs after the reference's: ``precision`` ("bf16" | "fp32") and, on Decoder and LocalReconstructor,
+``attn_softmax`` (default False = the reference's attention: raw scores, mean over frames / steps; True = the RecNet paper's
+softmax-normalised scores and weighted sum).  ``state_dict`` keys and shapes do not depend on either.
 
 Every (cell, n_layers) combination the reference's constructors accept runs on our kernels:
 * fused sequence drivers (one C call per loop): LSTM decoder with 1-4 layers, GRU decoder with 1 layer, 1-layer LSTM
@@ -57,6 +59,18 @@ def _is_lstm(model_name: str) -> bool:
     return model_name == "LSTM"            # models/decoder.py:32-35: anything else is a GRU
 
 
+def _cell_code(model_name, attn_softmax=False) -> int:
+    """The descriptors' `cell` field: recnet_cell, | ATTN_SOFTMAX for the paper's attention."""
+    return (L.CELL_LSTM if _is_lstm(model_name) else L.CELL_GRU) | (L.ATTN_SOFTMAX if attn_softmax else 0)
+
+
+def _attention(Wh, Uv, attn_b, attn_w, V, p, softmax):
+    """ops.additive_attention; the reference's mean attention is the plain six-argument call."""
+    if softmax:
+        return ops.additive_attention(Wh, Uv, attn_b, attn_w, V, p, softmax=True)
+    return ops.additive_attention(Wh, Uv, attn_b, attn_w, V, p)
+
+
 def _zero_state(model_name, n_layers, B, size, device):
     """train.py:28-35 / 82-89 / 112-119: zero (h, c) for LSTM, zero h for GRU."""
     z = lambda: torch.zeros(n_layers, B, size, device=device)
@@ -95,7 +109,7 @@ class Decoder(nn.Module, _RngMixin):
     """models/decoder.py:6-70."""
 
     def __init__(self, model_name, n_layers, encoder_size, embedding_size, embedding_scale, hidden_size,
-                 attn_size, output_size, embedding_dropout, dropout, out_dropout, precision="bf16"):
+                 attn_size, output_size, embedding_dropout, dropout, out_dropout, precision="bf16", attn_softmax=False):
         super().__init__()
         self.model_name = model_name
         self.n_layers = n_layers
@@ -109,6 +123,7 @@ class Decoder(nn.Module, _RngMixin):
         self.dropout_p = dropout
         self.out_dropout_p = out_dropout
         self.precision = precision
+        self.attn_softmax = bool(attn_softmax)
 
         # parameter holders, created in the reference's order (decoder.py:22-42) so equal seeds give equal draws
         self.embedding = nn.Embedding(output_size, embedding_size)
@@ -133,7 +148,7 @@ class Decoder(nn.Module, _RngMixin):
         return dict(H=self.hidden_size, A=self.attn_size, EMB=self.embedding_size, V=self.output_size,
                     precision=_precision_id(self.precision), train=self.training, embedding_scale=self.embedding_scale,
                     p_emb=self.embedding_dropout_p, p_out=self.out_dropout_p, p_layer=self.dropout_p,
-                    cell=L.CELL_LSTM if self.model_name == "LSTM" else L.CELL_GRU)       # decoder.py:32-35
+                    cell=_cell_code(self.model_name, self.attn_softmax))                   # decoder.py:32-35
 
     @property
     def uses_fused_sequence(self) -> bool:
@@ -291,7 +306,7 @@ class Decoder(nn.Module, _RngMixin):
         else:
             Uv = ops.linear(encoder_outputs.reshape(B * T, E), self.attn_U.weight, None, p).view(B, T, -1)
         Wh = ops.linear(h, self.attn_W.weight, None, p)                                                   # decoder.py:51
-        ctx = ops.additive_attention(Wh, Uv, self.attn_b, self.attn_w.weight, encoder_outputs, p)          # decoder.py:55-61
+        ctx = _attention(Wh, Uv, self.attn_b, self.attn_w.weight, encoder_outputs, p, self.attn_softmax)          # decoder.py:55-61
         # layer 0 takes [emb ; ctx], layer l the (dropped-out) output of layer l-1 (nn.LSTM / nn.GRU, decoder.py:64-66)
         h_top, hidden = _rnn_stack_step(self.rnn, torch.cat((emb, ctx), dim=1), hidden, p, self.training)
         logits = ops.linear(h_top, self.out.weight, self.out.bias, p)                                     # decoder.py:68
@@ -374,7 +389,7 @@ class LocalReconstructor(_ReconstructorBase):
     """models/local_reconstructor.py:6-55."""
 
     def __init__(self, model_name, n_layers, decoder_hidden_size, hidden_size, dropout, decoder_dropout, attn_size,
-                 precision="bf16"):
+                 precision="bf16", attn_softmax=False):
         super().__init__()
         self.model_name = model_name
         self.n_layers = n_layers
@@ -384,6 +399,7 @@ class LocalReconstructor(_ReconstructorBase):
         self.decoder_dropout_p = decoder_dropout
         self.attn_size = attn_size
         self.precision = precision
+        self.attn_softmax = bool(attn_softmax)
         self.attn_W = nn.Linear(hidden_size, attn_size, bias=False)
         self.attn_U = nn.Linear(decoder_hidden_size, attn_size, bias=False)
         self.attn_b = nn.Parameter(torch.ones(attn_size), requires_grad=True)
@@ -405,7 +421,7 @@ class LocalReconstructor(_ReconstructorBase):
             return (loss if lambda_reg is None else loss + lambda_reg * reg), reg
         hid = _sequence_hiddens(decoder_hiddens)
         meta = dict(A=self.attn_size, precision=_precision_id(self.precision), train=self.training, lambda_reg=lambda_reg,
-                    p_drop=self.decoder_dropout_p, cell=L.CELL_LSTM if self.model_name == "LSTM" else L.CELL_GRU)
+                    p_drop=self.decoder_dropout_p, cell=_cell_code(self.model_name, self.attn_softmax))
         return Fn.LocalReconstructorFn.apply(meta, hid, encoder_outputs, self._next_rng(), *self._params())
 
     def _forward_sequence_stepwise(self, decoder_hiddens, encoder_outputs):
@@ -428,10 +444,11 @@ class LocalReconstructor(_ReconstructorBase):
         Lsteps, NLd, B, H = hid.shape
         Wh = ops.linear(h_prev, self.attn_W.weight, None, p)                             # local_reconstructor.py:39-42
         xs = []
-        for j in range(NLd):             # the same query attends over the L states of every decoder layer (:43-49), mean over L
+        for j in range(NLd):             # the same query attends over the L states of every decoder layer (:43-49), mean (or softmax) over L
             hj = hid[:, j]
             Uv = ops.linear(hj.reshape(Lsteps * B, H), self.attn_U.weight, None, p).view(Lsteps, B, -1).transpose(0, 1)
-            xs.append(ops.additive_attention(Wh, Uv.contiguous(), self.attn_b, self.attn_w.weight, hj.transpose(0, 1).contiguous(), p))
+            xs.append(_attention(Wh, Uv.contiguous(), self.attn_b, self.attn_w.weight, hj.transpose(0, 1).contiguous(), p,
+                                 self.attn_softmax))
         x = torch.nn.functional.dropout(torch.stack(xs), self.decoder_dropout_p, self.training)      # (NLdec,B,H)  :50
         # nn.LSTM / nn.GRU read dim 0 of its input as TIME: NLdec pseudo-steps (:52); the output of the FIRST one is projected (:54)
         first = None

@@ -82,10 +82,11 @@ def linear(x, W, bias, precision):
 
 class AdditiveAttentionFn(torch.autograd.Function):
     """ctx[b] = mean_tau( (w . tanh(Wh[b] + Uv[b,tau] + bias)) * V[b,tau] )   (models/decoder.py:55-61).
+    softmax=True: the paper's attention, ctx[b] = sum_tau alpha[b,tau] V[b,tau] with alpha = softmax_tau(e).
     Wh (B,A) f32; Uv (B,Tn,A) f32; V (B,Tn,D) f32 (cast to the operand type internally)."""
 
     @staticmethod
-    def forward(ctx, Wh, Uv, attn_b, attn_w, V, precision):
+    def forward(ctx, Wh, Uv, attn_b, attn_w, V, precision, softmax=False):
         lib = L.lib()
         B, Tn, A = Uv.shape
         D = V.shape[2]
@@ -95,10 +96,10 @@ class AdditiveAttentionFn(torch.autograd.Function):
         e = torch.empty(B, Tn, dtype=torch.float32, device=Uv.device)
         out = torch.empty(B, D, dtype=dt, device=Uv.device)
         L.check(lib.recnet_attn_fwd(precision, Wh.data_ptr(), 1, 0, Uv.data_ptr(), Tn * A, A, attn_b.data_ptr(), attn_w.data_ptr(),
-                                    Vo.data_ptr(), Tn * D, D, B, Tn, A, D, 0, None, e.data_ptr(), out.data_ptr(), D, 0.0, None, 0, 0,
+                                    Vo.data_ptr(), Tn * D, D, B, Tn, A, D, int(softmax), None, e.data_ptr(), out.data_ptr(), D, 0.0, None, 0, 0,
                                     _stream()), "recnet_attn_fwd")
-        ctx.precision = precision
-        ctx.save_for_backward(Wh, Uv, attn_b, attn_w, Vo, e)
+        ctx.precision, ctx.softmax = precision, bool(softmax)
+        ctx.save_for_backward(Wh, Uv, attn_b, attn_w, Vo, e)         # e holds alpha when softmax
         return out.float()
 
     @staticmethod
@@ -111,17 +112,26 @@ class AdditiveAttentionFn(torch.autograd.Function):
         dWh = torch.empty(B, A, dtype=torch.float32, device=g.device)
         dUv = torch.empty_like(Uv)
         dw = torch.empty(B, A, dtype=torch.float32, device=g.device)
-        L.check(lib.recnet_attn_bwd(ctx.precision, g.data_ptr(), 1, 0, D, Vo.data_ptr(), Tn * D, D, Wh.data_ptr(), Uv.data_ptr(),
-                                    Tn * A, A, attn_b.data_ptr(), attn_w.data_ptr(), B, Tn, A, D, dWh.data_ptr(), None, dUv.data_ptr(),
-                                    dw.data_ptr(), 1, None, 0.0, None, 0, 0, _stream()), "recnet_attn_bwd")
+        if ctx.softmax:
+            L.check(lib.recnet_attn_bwd_softmax(ctx.precision, g.data_ptr(), 1, 0, D, Vo.data_ptr(), Tn * D, D, e.data_ptr(), Wh.data_ptr(),
+                                                Uv.data_ptr(), Tn * A, A, attn_b.data_ptr(), attn_w.data_ptr(), B, Tn, A, D, dWh.data_ptr(),
+                                                None, dUv.data_ptr(), dw.data_ptr(), 1, None, 0.0, None, 0, 0, _stream()),
+                    "recnet_attn_bwd_softmax")
+        else:
+            L.check(lib.recnet_attn_bwd(ctx.precision, g.data_ptr(), 1, 0, D, Vo.data_ptr(), Tn * D, D, Wh.data_ptr(), Uv.data_ptr(),
+                                        Tn * A, A, attn_b.data_ptr(), attn_w.data_ptr(), B, Tn, A, D, dWh.data_ptr(), None, dUv.data_ptr(),
+                                        dw.data_ptr(), 1, None, 0.0, None, 0, 0, _stream()), "recnet_attn_bwd")
         gV = None
         if ctx.needs_input_grad[4]:
-            gV = (e.unsqueeze(2) * g.unsqueeze(1)) / Tn        # value gradient: tiny outer product, only the local reconstructor needs it
-        return dWh, dUv, dWh.sum(0), dw.sum(0).view(1, -1), gV, None
+            # value gradient: tiny outer product, only the local reconstructor needs it (alpha * g, or e * g / Tn for the mean)
+            gV = e.unsqueeze(2) * g.unsqueeze(1)
+            if not ctx.softmax:
+                gV = gV / Tn
+        return dWh, dUv, dWh.sum(0), dw.sum(0).view(1, -1), gV, None, None
 
 
-def additive_attention(Wh, Uv, attn_b, attn_w, V, precision):
-    return AdditiveAttentionFn.apply(Wh, Uv, attn_b, attn_w, V, precision)
+def additive_attention(Wh, Uv, attn_b, attn_w, V, precision, softmax=False):
+    return AdditiveAttentionFn.apply(Wh, Uv, attn_b, attn_w, V, precision, softmax)
 
 
 class LSTMCellFn(torch.autograd.Function):

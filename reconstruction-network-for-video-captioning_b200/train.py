@@ -94,7 +94,8 @@ def build_decoder(n_vocabs):
         model_name=C.decoder_model, n_layers=C.decoder_n_layers, encoder_size=C.encoder_output_size,
         embedding_size=C.embedding_size, embedding_scale=C.embedding_scale, hidden_size=C.decoder_hidden_size,
         attn_size=C.decoder_attn_size, output_size=n_vocabs, embedding_dropout=C.embedding_dropout,
-        dropout=C.decoder_dropout, out_dropout=C.decoder_out_dropout, precision=C.precision).to(C.device)
+        dropout=C.decoder_dropout, out_dropout=C.decoder_out_dropout, precision=C.precision,
+        attn_softmax=C.decoder_attn_softmax).to(C.device)
     if _optimizer_impl() == "recnet":      # clip (train.py:269-270) folded into the Adam pass
         optimizer = ClipAdam(model.parameters(), lr=C.decoder_learning_rate, weight_decay=C.decoder_weight_decay,
                              amsgrad=C.decoder_use_amsgrad, max_grad_norm=C.gradient_clip if C.use_gradient_clip else None)
@@ -111,7 +112,8 @@ def build_reconstructor():
         model = LocalReconstructor(
             model_name=C.reconstructor_model, n_layers=C.reconstructor_n_layers, decoder_hidden_size=C.decoder_hidden_size,
             hidden_size=C.reconstructor_hidden_size, dropout=C.reconstructor_dropout,
-            decoder_dropout=C.reconstructor_decoder_dropout, attn_size=C.reconstructor_attn_size, precision=C.precision)
+            decoder_dropout=C.reconstructor_decoder_dropout, attn_size=C.reconstructor_attn_size, precision=C.precision,
+            attn_softmax=C.reconstructor_attn_softmax)
     elif C.reconstructor_type == "global":
         model = GlobalReconstructor(
             model_name=C.reconstructor_model, n_layers=C.reconstructor_n_layers, decoder_hidden_size=C.decoder_hidden_size,
