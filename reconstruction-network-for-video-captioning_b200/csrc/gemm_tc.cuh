@@ -366,8 +366,8 @@ static inline int launch(const bf16* A, long long lda, int transA, const bf16* B
   if (Cf && ((reinterpret_cast<uintptr_t>(Cf) & 15) || (ldc & 3) || (split_stride & 3))) ep.vec_ok = 0;
   if (Cb && ((reinterpret_cast<uintptr_t>(Cb) & 7) || (ldcb & 3))) ep.vec_ok = 0;
   if (bias && (reinterpret_cast<uintptr_t>(bias) & 15)) ep.vec_ok = 0;
-  // short K loops (the per-step split-K GEMMs) use a shallow ring (<= 97 KB smem) so that two CTAs -- typically of
-  // two different sample chains -- share an SM; long K loops (batched GEMMs) use the deep ring.
+  // short K loops (the per-step split-K GEMMs) use a shallow ring (<= 97 KB smem) so that two CTAs share an SM; long K
+  // loops (batched GEMMs) use the deep ring.
   static int shallow_kb = -1;
   if (shallow_kb < 0) { const char* e = getenv("RECNET_GEMM_SHALLOW_KB"); shallow_kb = e ? atoi(e) : 12; }
   const bool shallow = kb_per <= shallow_kb;

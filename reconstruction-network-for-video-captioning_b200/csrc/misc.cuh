@@ -64,7 +64,7 @@ static int cast_pad(const float* src, long long ld_src, TO* dst, long long ld_ds
 // whose cost is its launch latency, not its bytes.  A Stager collects them and issues ONE kernel (table passed by value):
 //   dst[r', 0:cols] = (TO) src[r, 0:cols], dst[r', cols:cols_pad] = 0;   r' = r, or for interleave_H > 0 the unit-interleaved
 //   order  dst row 4j+g <- src row g*H+j  (W_ctx, makes the VW GEMM emit [.., H, 4]);   src == nullptr -> zero fill.
-// Items that cannot take 16-byte vectors fall back to a scalar launch of their own; RECNET_STAGE_MULTI=0 launches item by item.
+// Items that cannot take 16-byte vectors fall back to a scalar launch of their own.
 struct StageItem { const float* src; void* dst; unsigned ld_src, ld_dst, rows, cols4, cp4, interleave_H; };
 constexpr int STAGE_MAX = 12;
 struct StageTable { StageItem it[STAGE_MAX]; unsigned blk0[STAGE_MAX + 1]; int n; };
@@ -133,18 +133,9 @@ struct Stager {
   void zero(void* p, size_t bytes) { add(nullptr, 0, reinterpret_cast<TO*>(p), (long long)(bytes / sizeof(TO)), 1, 0, (int)(bytes / sizeof(TO))); }
   int launch(cudaStream_t st) {
     if (overflow) return RECNET_ERR_BAD_SHAPE;
-    static int multi = -1;
-    if (multi < 0) { const char* e = getenv("RECNET_STAGE_MULTI"); multi = e ? atoi(e) : 1; }
-    if (t.n > 0 && multi) {
+    if (t.n > 0) {
       stage_multi_kernel<TO><<<t.blk0[t.n], 256, 0, st>>>(t);
       RN_LAUNCH_OK();
-    } else {
-      for (int i = 0; i < t.n; ++i) {           // one launch per item (A/B switch)
-        StageTable one;
-        one.n = 1; one.it[0] = t.it[i]; one.blk0[0] = 0; one.blk0[1] = t.blk0[i + 1] - t.blk0[i];
-        stage_multi_kernel<TO><<<one.blk0[1], 256, 0, st>>>(one);
-        RN_LAUNCH_OK();
-      }
     }
     for (int i = 0; i < n_sc; ++i) {
       const Scalar& x = sc[i];

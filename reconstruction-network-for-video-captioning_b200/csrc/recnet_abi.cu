@@ -59,8 +59,6 @@ int recnet_profile_collect(float* out, int max_records) {
   return n;
 }
 
-// developer probe: a loop-kernel launch with n_phases empty phases (grid barrier after each if sync_after) -- measures
-// the per-phase overhead of the persistent loop kernel.  scratch: >= n_phases * 1024 + 1024 bytes of device memory.
 // developer / test probe: the inverted-dropout scales (0 or 1/(1-p)) the kernels apply to elements 0..n-1 of dropout `site`
 // for the (seed, offset) pair in rng -- the same device function the forward and backward kernels call
 __global__ void debug_dropout_mask_kernel(const unsigned long long* rng, unsigned int site, long long n, float p, float* out) {

@@ -32,44 +32,6 @@ template <typename T> struct Prec;
 template <> struct Prec<float> { static constexpr int id = RECNET_PREC_FP32; static constexpr int kpad = 4; };
 template <> struct Prec<bf16> { static constexpr int id = RECNET_PREC_BF16; static constexpr int kpad = 64; };
 
-// ---- concurrent sample chains --------------------------------------------------------------------------
-// The time loops are latency-bound: each step is a chain of ~4 small dependent kernels that cannot fill 148 SMs.
-// Samples are independent through both loops, so the batch is cut into `n` contiguous sub-batches ("chains")
-// whose loops run concurrently on forked streams (parallel branches of the captured CUDA graph) and share the
-// batched GEMMs before and after the loop.  MEASURED (profiles/r1_b_chains.md): on B200 the graph is bound by
-// per-node launch/dependency overhead, so more chains = more nodes = SLOWER (1: 4.47 ms, 2: 5.11, 4: 5.95, 8: 8.55
-// per step).  Default is therefore 1; RECNET_CHAINS=n keeps the experiment reproducible.
-struct Chains {
-  static constexpr int MAX = 8;
-  cudaStream_t s[MAX];
-  cudaEvent_t fork_ev, join_ev[MAX];
-  bool ready = false;
-  int init() {
-    if (ready) return 0;
-    for (int i = 0; i < MAX; ++i) {
-      RN_CUDA_OK(cudaStreamCreateWithFlags(&s[i], cudaStreamNonBlocking));
-      RN_CUDA_OK(cudaEventCreateWithFlags(&join_ev[i], cudaEventDisableTiming));
-    }
-    RN_CUDA_OK(cudaEventCreateWithFlags(&fork_ev, cudaEventDisableTiming));
-    ready = true;
-    return 0;
-  }
-  int fork(cudaStream_t main, int n) {
-    RN_TRY(init());
-    RN_CUDA_OK(cudaEventRecord(fork_ev, main));
-    for (int i = 0; i < n; ++i) RN_CUDA_OK(cudaStreamWaitEvent(s[i], fork_ev, 0));
-    return 0;
-  }
-  int join(cudaStream_t main, int n) {
-    for (int i = 0; i < n; ++i) {
-      RN_CUDA_OK(cudaEventRecord(join_ev[i], s[i]));
-      RN_CUDA_OK(cudaStreamWaitEvent(main, join_ev[i], 0));
-    }
-    return 0;
-  }
-};
-inline Chains& chains() { static Chains c; return c; }
-
 // ---- side stream for the batched work around the time loops (default on; RECNET_SIDE=0 puts everything on `main`) -------------
 // Before and after each time loop a driver issues a dozen mutually independent batched kernels (weight-gradient GEMMs, column
 // sums, operand staging); several of them are small grids (the 128-row attention weight gradients run on 32-64 CTAs) or end in
@@ -113,34 +75,14 @@ struct Side {
 };
 inline Side& side() { static Side x; return x; }
 
-static inline int num_chains(int B) {
-  static int env = -1;
-  if (env < 0) { const char* e = getenv("RECNET_CHAINS"); env = e ? atoi(e) : 0; }
-  int n = env > 0 ? env : 1;
-  if (n > Chains::MAX) n = Chains::MAX;
-  if (n > B) n = B;
-  return n < 1 ? 1 : n;
-}
-// rows [lo, lo+cnt) of chain c out of n
-static inline void chain_rows(int B, int n, int c, int* lo, int* cnt) {
-  const int base = B / n, rem = B % n;
-  *lo = c * base + (c < rem ? c : rem);
-  *cnt = base + (c < rem ? 1 : 0);
-}
-static inline int chain_rows_max(int B, int n) { return (B + n - 1) / n; }
-
 // ---- split-K / tile policy ---------------------------------------------------------------------------
 struct GemmPlan { int bn; int splits; };
-// target = CTAs one GEMM should spread over: the whole GPU for a single chain, half of it when several chains
-// keep the machine busy (fewer split-K partials for the consumer kernels to sum).
-template <typename T> static inline GemmPlan plan_gemm(int M, int N, int K, int target = NUM_SMS);
-template <> inline GemmPlan plan_gemm<bf16>(int M, int N, int K, int target) {
+template <typename T> static inline GemmPlan plan_gemm(int M, int N, int K);
+template <> inline GemmPlan plan_gemm<bf16>(int M, int N, int K) {
   GemmPlan p;
   p.bn = (N >= 1024) ? 128 : 64;
   const int nkb0 = rn_cdiv(K, tc::BK);
-  static int big_bn = -1;
-  if (big_bn < 0) { const char* e = getenv("RECNET_GEMM_COSTMODEL"); big_bn = e ? atoi(e) : 1; }
-  if (big_bn && nkb0 >= 16 && rn_cdiv(M, tc::BM) * rn_cdiv(N, 64) >= 2 * target) {
+  if (nkb0 >= 16 && rn_cdiv(M, tc::BM) * rn_cdiv(N, 64) >= 2 * NUM_SMS) {
     // Batched GEMMs (weight gradients, hoisted projections).  r1 ncu: the main loop is bound by what one SM can pull from L2
     // (~50 B/clk), not by the tensor pipe, so wider N tiles (fewer A re-reads per MMA) win unless they cost a whole extra wave.
     // cost per k-block ~ max(MMA cycles = 2 bn, (A 12.8 KB + B 128 bn bytes) / 50 B/clk); total ~ waves * cost.
@@ -148,7 +90,7 @@ template <> inline GemmPlan plan_gemm<bf16>(int M, int N, int K, int target) {
     for (int bn = 64; bn <= 256; bn *= 2) {
       const int tiles = rn_cdiv(M, tc::BM) * rn_cdiv(N, bn);
       const float per = fmaxf(2.f * bn, (12800.f + 128.f * bn) / 50.f);
-      const float cost = (float)rn_cdiv(tiles, target) * per;
+      const float cost = (float)rn_cdiv(tiles, NUM_SMS) * per;
       if (cost < best * 0.97f) { best = cost; p.bn = bn; }
     }
     p.splits = 1;
@@ -156,18 +98,18 @@ template <> inline GemmPlan plan_gemm<bf16>(int M, int N, int K, int target) {
   }
   const int tiles = rn_cdiv(M, tc::BM) * rn_cdiv(N, p.bn);
   const int nkb = rn_cdiv(K, tc::BK);
-  int s = target / tiles;
+  int s = NUM_SMS / tiles;
   if (s < 1) s = 1;
   if (s > nkb) s = nkb;
   const int kb_per = rn_cdiv(nkb, s);
   p.splits = rn_cdiv(nkb, kb_per);
   return p;
 }
-template <> inline GemmPlan plan_gemm<float>(int M, int N, int K, int target) {
+template <> inline GemmPlan plan_gemm<float>(int M, int N, int K) {
   GemmPlan p;
   p.bn = 0;
   const int tiles = rn_cdiv(M, sg::BM) * rn_cdiv(N, sg::BN);
-  int s = (2 * target) / tiles;
+  int s = (2 * NUM_SMS) / tiles;
   const int maxs = K / 64 > 0 ? K / 64 : 1;
   if (s < 1) s = 1;
   if (s > maxs) s = maxs;
@@ -216,6 +158,7 @@ static inline int splitk_reduce(const float* P, int splits, long long split_stri
 constexpr size_t SPLITK_SCRATCH_FLOATS = (size_t)NUM_SMS * 2 * 128 * 128;   // enough for any plan with splits > 1
 
 // ---- tile / split-K plan of the BATCHED GEMMs (gemm_full: weight gradients, hoisted projections, vocabulary projection) ----------
+template <typename T> static inline GemmPlan plan_gemm_full(int M, int N, int K) { return plan_gemm<T>(M, N, K); }
 // Cost model fitted to a sweep of every batched GEMM of the MSVD train step over (N-tile width, split count) on the B200
 // (tools/gemm_sweep.py, profiles/r1_g_gemm_sweep.md).  What the sweep showed: the main loop is bound by L2 -> SM delivery, not by
 // the tensor pipe.  With all 148 SMs pulling, one k-block (64 deep) costs ~857 / 1030 / 1240 cycles for 64 / 128 / 256-wide tiles
@@ -223,7 +166,7 @@ constexpr size_t SPLITK_SCRATCH_FLOATS = (size_t)NUM_SMS * 2 * 128 * 128;   // e
 // cycles); every wave pays prologue + epilogue (~2000 + 16 bn cycles); a split-K plan adds the reduce pass (~5 us + bytes at
 // 3.5 TB/s).  Wider tiles win whenever they do not cost an extra wave; split-K only pays for GEMMs with a handful of tiles.
 // Candidates are visited from the simplest plan up and must beat the incumbent by 5 % (the fit is good to about +-4 us).
-static inline GemmPlan plan_gemm_full_bf16(int M, int N, int K) {
+template <> inline GemmPlan plan_gemm_full<bf16>(int M, int N, int K) {
   static const float CF[3] = {857.f, 1030.f, 1240.f}, FL[3] = {745.f, 857.f, 944.f};
   static const int SPL[6] = {1, 2, 3, 4, 6, 8};
   const int mt = rn_cdiv(M, tc::BM), nkb = rn_cdiv(K, tc::BK);
@@ -269,12 +212,6 @@ static inline GemmPlan plan_gemm_full_bf16(int M, int N, int K) {
     else best.bn = (nkb >= 16 && 2 * pairs >= 3 * (NUM_SMS / 2)) ? 2256 : 1256;
   }
   return best;
-}
-template <typename T> static inline GemmPlan plan_gemm_full(int M, int N, int K) { return plan_gemm<T>(M, N, K); }
-template <> inline GemmPlan plan_gemm_full<bf16>(int M, int N, int K) {
-  static int mode = -1;                                    // RECNET_GEMM_COSTMODEL: 2 (default) this model, 1 the r1_f model, 0 fixed tiles
-  if (mode < 0) { const char* e = getenv("RECNET_GEMM_COSTMODEL"); mode = e ? atoi(e) : 2; }
-  return mode >= 2 ? plan_gemm_full_bf16(M, N, K) : plan_gemm<bf16>(M, N, K);
 }
 
 // Full GEMM into a dense destination: splits the K loop when the tile grid alone cannot fill the GPU,

@@ -8,7 +8,6 @@
 //   * BPTT mirrors it; all weight gradients are batched GEMMs over the stashed operands after the loop.
 #pragma once
 #include "gru_cell.cuh"
-#include "mega.cuh"
 #include "runtime.cuh"
 
 namespace dec {
@@ -20,7 +19,6 @@ template <typename T>
 struct Ws {
   // geometry
   int EMBp, KX, Vp, Vld;
-  int nch, Bc;                       // concurrent sample chains, max rows per chain
   int G;                             // gates per unit: 4 (LSTM) or 3 (GRU)
   GemmPlan pl_wh, pl_gate, pl_dx, pl_dq;
   GemmPlan pl_gx, pl_gh, pl_dxx, pl_dxh;   // GRU: x-part / h-part kept separate (n gate)
@@ -32,7 +30,7 @@ struct Ws {
   // backward scratch
   T* dlogits; float* dHext; T* dG; T* dG2; float* dXp; float* dXp2; float* dQp; float* dWh; T* dWh_op; float* dUv; T* dUv_op; float* dw_acc;
   float* dc; float* dXe; float* splitk;
-  uint8_t* table; size_t table_bytes; unsigned* bar; int* err;     // loop-kernel phase table, grid-barrier counter, error flag
+  int* err;                          // error flag (recnet_decoder_error_offset)
   // layers 1 .. NL-1 of a stacked decoder (index l-1): operand rows X_l[t] = [h^{l-1}_t ; h^l_{t-1}], K = 2H
   int NL;
   GemmPlan pl_gate_x, pl_dx_x;
@@ -49,18 +47,15 @@ static Ws<T> plan(const recnet_decoder_desc& d, void* base) {
   w.KX = E + H;
   w.Vp = round_up(V, 8);
   w.Vld = round_up(V, 4);
-  w.nch = num_chains(B);
-  w.Bc = chain_rows_max(B, w.nch);
-  const int tgt = w.nch > 1 ? NUM_SMS / 2 : NUM_SMS;
-  w.pl_wh = plan_gemm<T>(w.Bc, A, H, tgt);
-  w.pl_gate = plan_gemm<T>(w.Bc, 4 * H, w.KX, tgt);
-  w.pl_dx = plan_gemm<T>(w.Bc, w.KX, 4 * H, tgt);
-  w.pl_dq = plan_gemm<T>(w.Bc, H, A, tgt);
+  w.pl_wh = plan_gemm<T>(B, A, H);
+  w.pl_gate = plan_gemm<T>(B, 4 * H, w.KX);
+  w.pl_dx = plan_gemm<T>(B, w.KX, 4 * H);
+  w.pl_dq = plan_gemm<T>(B, H, A);
   w.G = d.cell == RECNET_CELL_GRU ? 3 : 4;
-  w.pl_gx = plan_gemm<T>(w.Bc, 3 * H, E, tgt);
-  w.pl_gh = plan_gemm<T>(w.Bc, 3 * H, H, tgt);
-  w.pl_dxx = plan_gemm<T>(w.Bc, E, 3 * H, tgt);
-  w.pl_dxh = plan_gemm<T>(w.Bc, H, 3 * H, tgt);
+  w.pl_gx = plan_gemm<T>(B, 3 * H, E);
+  w.pl_gh = plan_gemm<T>(B, 3 * H, H);
+  w.pl_dxx = plan_gemm<T>(B, E, 3 * H);
+  w.pl_dxh = plan_gemm<T>(B, H, 3 * H);
   const bool gru_ = d.cell == RECNET_CELL_GRU;
   Bump m(base);
   w.Wemb = m.take<T>((size_t)4 * H * w.EMBp);
@@ -73,11 +68,11 @@ static Ws<T> plan(const recnet_decoder_desc& d, void* base) {
   w.Xe = m.take<T>((size_t)L * B * w.EMBp);
   w.Gx = m.take<float>((size_t)L * B * 4 * H);
   w.X = m.take<T>((size_t)(L + 1) * B * w.KX);
-  w.WhP = m.take<float>((size_t)w.nch * w.pl_wh.splits * w.Bc * A);
+  w.WhP = m.take<float>((size_t)w.pl_wh.splits * B * A);
   w.Wh = m.take<float>((size_t)L * B * A);
   w.e = m.take<float>((size_t)L * B * Tn);
-  w.P = m.take<float>((size_t)w.nch * (gru_ ? w.pl_gx.splits : w.pl_gate.splits) * w.Bc * 4 * H + (size_t)16 * B * 4 * H);
-  w.P2 = m.take<float>(gru_ ? (size_t)w.nch * w.pl_gh.splits * w.Bc * 3 * H : 1);
+  w.P = m.take<float>((size_t)(gru_ ? w.pl_gx.splits : w.pl_gate.splits) * B * 4 * H + (size_t)16 * B * 4 * H);
+  w.P2 = m.take<float>(gru_ ? (size_t)w.pl_gh.splits * B * 3 * H : 1);
   w.gates = m.take<T>((size_t)L * B * 4 * H);
   w.c = m.take<float>((size_t)(L + 1) * B * H);
   w.logits = m.take<float>((size_t)L * B * w.Vld);
@@ -86,10 +81,10 @@ static Ws<T> plan(const recnet_decoder_desc& d, void* base) {
   w.dlogits = m.take<T>((size_t)L * B * w.Vp);
   w.dHext = m.take<float>((size_t)L * B * H);
   w.dG = m.take<T>((size_t)L * B * 4 * H);
-  w.dXp = m.take<float>((size_t)w.nch * (gru_ ? w.pl_dxx.splits : w.pl_dx.splits) * w.Bc * w.KX);
-  w.dXp2 = m.take<float>(gru_ ? (size_t)w.nch * w.pl_dxh.splits * w.Bc * H : 1);
+  w.dXp = m.take<float>((size_t)(gru_ ? w.pl_dxx.splits : w.pl_dx.splits) * B * w.KX);
+  w.dXp2 = m.take<float>(gru_ ? (size_t)w.pl_dxh.splits * B * H : 1);
   w.dG2 = m.take<T>(gru_ ? (size_t)L * B * 3 * H : 1);
-  w.dQp = m.take<float>((size_t)w.nch * w.pl_dq.splits * w.Bc * H);
+  w.dQp = m.take<float>((size_t)w.pl_dq.splits * B * H);
   w.dWh = m.take<float>((size_t)L * B * A);
   w.dWh_op = m.take<T>((size_t)L * B * A);
   w.dUv = m.take<float>((size_t)B * Tn * A);
@@ -98,13 +93,10 @@ static Ws<T> plan(const recnet_decoder_desc& d, void* base) {
   w.dc = m.take<float>((size_t)B * H);
   w.dXe = m.take<float>((size_t)L * B * w.EMBp);
   w.splitk = m.take<float>(SPLITK_SCRATCH_FLOATS);
-  w.table_bytes = mega::table_bytes(L);
-  w.table = m.take<uint8_t>(w.table_bytes);
-  w.bar = m.take<unsigned>(64);
   w.err = m.take<int>(64);
   w.NL = d.n_layers < 1 ? 1 : d.n_layers;
-  w.pl_gate_x = plan_gemm<T>(w.Bc, 4 * H, 2 * H, tgt);
-  w.pl_dx_x = plan_gemm<T>(w.Bc, 2 * H, 4 * H, tgt);
+  w.pl_gate_x = plan_gemm<T>(B, 4 * H, 2 * H);
+  w.pl_dx_x = plan_gemm<T>(B, 2 * H, 4 * H);
   for (int l = 1; l < w.NL && l < RECNET_MAX_LAYERS; ++l) {
     w.Wrec_x[l - 1] = m.take<T>((size_t)4 * H * 2 * H);
     w.X_x[l - 1] = m.take<T>((size_t)(L + 1) * B * 2 * H);
@@ -144,56 +136,48 @@ static int prepare(const recnet_decoder_desc& d, const recnet_decoder_tensors& p
   return 0;
 }
 
-// one decoder step for the sample rows [b0, b0+nb) of chain `ch`: attention -> gate GEMM -> cell.
-// Pointer arguments are the FULL-batch row-0 addresses of step t; the row offset is applied here.
+// one decoder step: attention -> gate GEMM -> cell.  Pointer arguments are the row-0 addresses of step t.
 template <typename T>
-static int step(mega::Emitter<T>& em, const DecDesc& d, const recnet_decoder_tensors& p, Ws<T>& w, int t, int ch,
-                int b0, int nb, const float* gx_t, T* x_t, T* x_next, float* Wh_t, float* e_t, T* gates_t, const float* c_prev,
-                float* c_next, float* h_out) {
-  const int H = d.H, E = d.E, A = d.A, Tn = d.T;
-  float* WhP = w.WhP + (size_t)ch * w.pl_wh.splits * w.Bc * A;
-  float* P = w.P + (size_t)ch * w.pl_gate.splits * w.Bc * 4 * H;
-  T* xr = x_t + (size_t)b0 * w.KX;
+static int step(const DecDesc& d, const recnet_decoder_tensors& p, Ws<T>& w, int t, const float* gx_t, T* x_t, T* x_next, float* Wh_t,
+                float* e_t, T* gates_t, const float* c_prev, float* c_next, float* h_out, cudaStream_t st) {
+  const int B = d.B, H = d.H, E = d.E, A = d.A, Tn = d.T;
   int n_whp = 0;
   if (t > 0) {   // h_{-1} = 0 -> W h = 0, skip the GEMM
-    RN_TRY(em.gemm_partials(xr + E, w.KX, 0, w.Wa, H, 0, WhP, nb, A, H, w.pl_wh));
+    RN_TRY(gemm_partials<T>(x_t + E, w.KX, 0, w.Wa, H, 0, w.WhP, B, A, H, w.pl_wh, st));
     n_whp = w.pl_wh.splits;
   }
   attn::FwdArgs fa{};
-  fa.WhP = WhP; fa.n_whp = n_whp; fa.whp_stride = (long long)nb * A;
-  fa.Uv = w.Uv + (size_t)b0 * Tn * A; fa.uv_bs = (long long)Tn * A; fa.uv_ts = A;
+  fa.WhP = w.WhP; fa.n_whp = n_whp; fa.whp_stride = (long long)B * A;
+  fa.Uv = w.Uv; fa.uv_bs = (long long)Tn * A; fa.uv_ts = A;
   fa.attn_b = p.attn_b; fa.attn_w = p.attn_w;
-  fa.V = w.feats + (size_t)b0 * Tn * E; fa.v_bs = (long long)Tn * E; fa.v_ts = E;
-  fa.B = nb; fa.Tn = Tn; fa.A = A; fa.D = E; fa.inv_T = d.softmax ? 1.f : 1.f / Tn; fa.normalize = d.softmax;
-  fa.Wh_out = Wh_t ? Wh_t + (size_t)b0 * A : nullptr; fa.e_out = e_t ? e_t + (size_t)b0 * Tn : nullptr;
-  fa.ctx_out = xr; fa.ctx_ld = w.KX; fa.p_drop = 0.f;
-  RN_TRY(em.attn_fwd(fa));
+  fa.V = w.feats; fa.v_bs = (long long)Tn * E; fa.v_ts = E;
+  fa.B = B; fa.Tn = Tn; fa.A = A; fa.D = E; fa.inv_T = d.softmax ? 1.f : 1.f / Tn; fa.normalize = d.softmax;
+  fa.Wh_out = Wh_t; fa.e_out = e_t;
+  fa.ctx_out = x_t; fa.ctx_ld = w.KX; fa.p_drop = 0.f;
+  RN_TRY((attn::launch_fwd<T, T>(fa, st)));
   if (d.cell == RECNET_CELL_GRU) {
     // x-part: ctx_t @ W_ctx^T (K = E) ; h-part: h_{t-1} @ W_hh^T (K = H): same operand rows, same weight copy, two column ranges
-    float* Px = w.P + (size_t)ch * w.pl_gx.splits * w.Bc * 3 * H;
-    float* Ph = w.P2 + (size_t)ch * w.pl_gh.splits * w.Bc * 3 * H;
-    RN_TRY(em.gemm_partials(xr, w.KX, 0, w.Wrec, w.KX, 0, Px, nb, 3 * H, E, w.pl_gx));
-    if (t > 0) RN_TRY(em.gemm_partials(xr + E, w.KX, 0, w.Wrec + E, w.KX, 0, Ph, nb, 3 * H, H, w.pl_gh));
+    RN_TRY(gemm_partials<T>(x_t, w.KX, 0, w.Wrec, w.KX, 0, w.P, B, 3 * H, E, w.pl_gx, st));
+    if (t > 0) RN_TRY(gemm_partials<T>(x_t + E, w.KX, 0, w.Wrec + E, w.KX, 0, w.P2, B, 3 * H, H, w.pl_gh, st));
     gru::FwdArgs ga{};
-    ga.Px = Px; ga.n_px = w.pl_gx.splits; ga.px_stride = (long long)nb * 3 * H; ga.px_ld = 3 * H;
-    ga.Ph = t > 0 ? Ph : nullptr; ga.n_ph = t > 0 ? w.pl_gh.splits : 0; ga.ph_stride = (long long)nb * 3 * H; ga.ph_ld = 3 * H;
-    ga.Gx = gx_t + (size_t)b0 * 3 * H; ga.gx_ld = 3 * H; ga.b_ih = nullptr; ga.b_hh = p.b_hh;
-    ga.h_prev = c_prev + (size_t)b0 * H; ga.hp_ld = H; ga.B = nb; ga.H = H;
-    ga.stash = gates_t ? gates_t + (size_t)b0 * 4 * H : nullptr;
-    ga.h_out = h_out + (size_t)b0 * H; ga.h_ld = H;
-    ga.h_op = x_next + (size_t)b0 * w.KX + E; ga.hop_ld = w.KX;
-    return gru::launch_fwd<T, T>(ga, em.st);
+    ga.Px = w.P; ga.n_px = w.pl_gx.splits; ga.px_stride = (long long)B * 3 * H; ga.px_ld = 3 * H;
+    ga.Ph = t > 0 ? w.P2 : nullptr; ga.n_ph = t > 0 ? w.pl_gh.splits : 0; ga.ph_stride = (long long)B * 3 * H; ga.ph_ld = 3 * H;
+    ga.Gx = gx_t; ga.gx_ld = 3 * H; ga.b_ih = nullptr; ga.b_hh = p.b_hh;
+    ga.h_prev = c_prev; ga.hp_ld = H; ga.B = B; ga.H = H;
+    ga.stash = gates_t;
+    ga.h_out = h_out; ga.h_ld = H;
+    ga.h_op = x_next + E; ga.hop_ld = w.KX;
+    return gru::launch_fwd<T, T>(ga, st);
   }
-  RN_TRY(em.gemm_partials(xr, w.KX, 0, w.Wrec, w.KX, 0, P, nb, 4 * H, w.KX, w.pl_gate));
+  RN_TRY(gemm_partials<T>(x_t, w.KX, 0, w.Wrec, w.KX, 0, w.P, B, 4 * H, w.KX, w.pl_gate, st));
   cell::FwdArgs ca{};
-  ca.P = P; ca.n_p = w.pl_gate.splits; ca.p_stride = (long long)nb * 4 * H; ca.p_ld = 4 * H;
-  ca.Gx = gx_t + (size_t)b0 * 4 * H; ca.gx_ld = 4 * H; ca.b1 = nullptr; ca.b2 = p.b_hh;
-  ca.c_prev = c_prev + (size_t)b0 * H; ca.B = nb; ca.H = H;
-  ca.gates_out = gates_t ? gates_t + (size_t)b0 * 4 * H : nullptr; ca.c_out = c_next + (size_t)b0 * H;
-  ca.h_out = h_out + (size_t)b0 * H; ca.h_ld = H;
-  ca.h_op = x_next + (size_t)b0 * w.KX + E; ca.hop_ld = w.KX; ca.h_op2 = nullptr;
-  RN_TRY(em.cell_fwd(ca));
-  return 0;
+  ca.P = w.P; ca.n_p = w.pl_gate.splits; ca.p_stride = (long long)B * 4 * H; ca.p_ld = 4 * H;
+  ca.Gx = gx_t; ca.gx_ld = 4 * H; ca.b1 = nullptr; ca.b2 = p.b_hh;
+  ca.c_prev = c_prev; ca.B = B; ca.H = H;
+  ca.gates_out = gates_t; ca.c_out = c_next;
+  ca.h_out = h_out; ca.h_ld = H;
+  ca.h_op = x_next + E; ca.hop_ld = w.KX; ca.h_op2 = nullptr;
+  return cell::launch_fwd<T, T>(ca, st);
 }
 
 template <typename T>
@@ -217,29 +201,16 @@ static int forward(const DecDesc& d, const recnet_decoder_tensors& p, const floa
   // initial state: h_{-1} = 0 (operand slot of X[0]), c_{-1} = 0
   RN_CUDA_OK(cudaMemsetAsync(w.X, 0, (size_t)B * w.KX * sizeof(T), st));
   RN_CUDA_OK(cudaMemsetAsync(w.c, 0, (size_t)B * H * sizeof(float), st));
-  // time loop.  One chain (default): the whole loop is ONE persistent loop-kernel launch (bf16 build) or one kernel
-  // per phase (fp32 build / RECNET_MEGA=0).  Several chains (RECNET_CHAINS, experimental): forked streams, eager.
+  // time loop: one kernel per phase
   RN_CUDA_OK(cudaMemsetAsync(w.err, 0, sizeof(int), st));
-  Chains& cs = chains();
-  if (w.nch > 1) RN_TRY(cs.fork(st, w.nch));
-  {
-    mega::Emitter<T> em0(w.nch == 1 && !is_gru, st, (size_t)E + Tn + 8 * attn::BWD_THREADS + 2 * A);
-    for (int t = 0; t < L; ++t) {
-      T* x_t = w.X + (size_t)t * B * w.KX;
-      for (int ch = 0; ch < w.nch; ++ch) {
-        int b0, nb;
-        chain_rows(B, w.nch, ch, &b0, &nb);
-        mega::Emitter<T> emc(false, w.nch > 1 ? cs.s[ch] : st);
-        // LSTM: c_{t-1} -> c_t live in w.c; GRU: the fp32 state is h itself (previous row of `hiddens`, zeros = w.c at t = 0)
-        const float* s_prev = is_gru ? (t == 0 ? w.c : hiddens + (size_t)(t - 1) * B * H) : w.c + (size_t)t * B * H;
-        RN_TRY(step<T>(w.nch == 1 ? em0 : emc, d, p, w, t, ch, b0, nb, w.Gx + (size_t)t * B * GH, x_t, x_t + (size_t)B * w.KX,
-                       w.Wh + (size_t)t * B * A, w.e + (size_t)t * B * Tn, w.gates + (size_t)t * B * 4 * H,
-                       s_prev, w.c + (size_t)(t + 1) * B * H, hiddens + (size_t)t * B * H));
-      }
-    }
-    RN_TRY(em0.flush(w.table, w.table_bytes, w.bar, w.err, 1));
+  for (int t = 0; t < L; ++t) {
+    T* x_t = w.X + (size_t)t * B * w.KX;
+    // LSTM: c_{t-1} -> c_t live in w.c; GRU: the fp32 state is h itself (previous row of `hiddens`, zeros = w.c at t = 0)
+    const float* s_prev = is_gru ? (t == 0 ? w.c : hiddens + (size_t)(t - 1) * B * H) : w.c + (size_t)t * B * H;
+    RN_TRY(step<T>(d, p, w, t, w.Gx + (size_t)t * B * GH, x_t, x_t + (size_t)B * w.KX, w.Wh + (size_t)t * B * A,
+                   w.e + (size_t)t * B * Tn, w.gates + (size_t)t * B * 4 * H, s_prev, w.c + (size_t)(t + 1) * B * H,
+                   hiddens + (size_t)t * B * H, st));
   }
-  if (w.nch > 1) RN_TRY(cs.join(st, w.nch));
   // vocabulary projection over all steps, then the masked CE (train.py:54-60,68)
   RN_TRY(gemm_full<T>(w.X + (size_t)B * w.KX + E, w.KX, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, L * B, V, H, 0,
                       w.splitk, st));
@@ -276,76 +247,63 @@ static int backward(const DecDesc& d, const recnet_decoder_tensors& p, const flo
   RN_TRY(gemm_full<T>(w.dlogits, w.Vp, 0, w.Wout, H, 1, w.dHext, H, nullptr, LB, H, V, 0, w.splitk, st));
   RN_TRY(gemm_full<T>(w.dlogits, w.Vp, 1, Hall, w.KX, 1, g.out_w, H, nullptr, V, H, LB, 0, w.splitk, st));
   RN_TRY(misc::colsum<T>(w.dlogits, w.Vp, LB, V, g.out_b, 0, w.splitk, st));
-  // ---- BPTT: the same sample chains, each with private split-K scratch ------------------------------------------
-  Chains& cs = chains();
-  if (w.nch > 1) RN_TRY(cs.fork(st, w.nch));
+  // ---- BPTT: one kernel per phase -------------------------------------------------------------------------
   const bool is_gru = d.cell == RECNET_CELL_GRU;
   const int GH = w.G * H;
-  mega::Emitter<T> em0(w.nch == 1 && !is_gru, st, (size_t)E + Tn + 8 * attn::BWD_THREADS + 2 * A);
   for (int t = L - 1; t >= 0; --t) {
     const bool last = (t == L - 1);
-    for (int ch = 0; ch < w.nch; ++ch) {
-      int b0, nb;
-      chain_rows(B, w.nch, ch, &b0, &nb);
-      mega::Emitter<T> emc(false, w.nch > 1 ? cs.s[ch] : st);
-      mega::Emitter<T>& em = w.nch == 1 ? em0 : emc;
-      float* dXp = w.dXp + (size_t)ch * w.pl_dx.splits * w.Bc * w.KX;
-      float* dQp = w.dQp + (size_t)ch * w.pl_dq.splits * w.Bc * H;
-      const size_t r = (size_t)t * B + b0;           // first (t, b) row of this chain
-      if (is_gru) {
-        float* dXx = w.dXp + (size_t)ch * w.pl_dxx.splits * w.Bc * w.KX;      // x-part dgrad partials [splits][nb, E]
-        float* dXh = w.dXp2 + (size_t)ch * w.pl_dxh.splits * w.Bc * H;         // h-part dgrad partials [splits][nb, H]
-        gru::BwdArgs gb{};
-        gb.dh_ext = w.dHext + r * H; gb.dh_ld = H;
-        gb.dh_ext2 = g_hiddens ? g_hiddens + r * H : nullptr; gb.dh2_ld = H;
-        gb.dHp = last ? nullptr : dXh; gb.n_p = w.pl_dxh.splits; gb.p_stride = (long long)nb * H; gb.p_ld = H;
-        gb.dQp = last ? nullptr : dQp; gb.n_q = w.pl_dq.splits; gb.q_stride = (long long)nb * H; gb.q_ld = H;
-        gb.carry = w.dc + (size_t)b0 * H; gb.first = last ? 1 : 0;
-        gb.stash = w.gates + r * 4 * H;
-        gb.h_prev = t == 0 ? w.c + (size_t)b0 * H : hiddens_fp32 + ((size_t)(t - 1) * B + b0) * H; gb.hp_ld = H;
-        gb.B = nb; gb.H = H; gb.dGi = w.dG + r * 3 * H; gb.dGh = w.dG2 + r * 3 * H; gb.dg_ld = 3 * H;
-        RN_TRY((gru::launch_bwd<T, T>(gb, em.st)));
-        RN_TRY(em.gemm_partials(w.dG + r * 3 * H, 3 * H, 0, w.Wrec, w.KX, 1, dXx, nb, E, 3 * H, w.pl_dxx));           // dctx = dGi @ W_ctx
-        if (t > 0) RN_TRY(em.gemm_partials(w.dG2 + r * 3 * H, 3 * H, 0, w.Wrec + E, w.KX, 1, dXh, nb, H, 3 * H, w.pl_dxh));  // dh += dGh @ W_hh
-        attn::BwdArgs ab{};
-        ab.dXp = dXx; ab.n_p = w.pl_dxx.splits; ab.p_stride = (long long)nb * E; ab.p_ld = E;
-        ab.V = w.feats + (size_t)b0 * Tn * E; ab.v_bs = (long long)Tn * E; ab.v_ts = E;
-        ab.Wh = w.Wh + r * A; ab.Uv = w.Uv + (size_t)b0 * Tn * A; ab.uv_bs = (long long)Tn * A; ab.uv_ts = A;
-        ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = Tn; ab.A = A; ab.D = E; ab.inv_T = d.softmax ? 1.f : 1.f / Tn;
-        ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv + (size_t)b0 * Tn * A;
-        ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc + (size_t)b0 * A;
-        ab.dctx_out = nullptr; ab.de_out = nullptr; ab.p_drop = 0.f; ab.alpha = d.softmax ? w.e + r * Tn : nullptr;
-        RN_TRY(em.attn_bwd(ab));
-        if (t > 0) RN_TRY(em.gemm_partials(w.dWh_op + r * A, A, 0, w.Wa, H, 1, dQp, nb, H, A, w.pl_dq));
-        continue;
-      }
-      cell::BwdArgs cb{};
-      cb.dh_ext = w.dHext + r * H; cb.dh_ld = H; cb.dh_scale = nullptr;
-      cb.dh_ext2 = g_hiddens ? g_hiddens + r * H : nullptr; cb.dh2_ld = H;
-      cb.dXp = last ? nullptr : dXp; cb.n_p = w.pl_dx.splits; cb.p_stride = (long long)nb * w.KX; cb.p_ld = w.KX; cb.col0 = E;
-      cb.dQp = last ? nullptr : dQp; cb.n_q = w.pl_dq.splits; cb.q_stride = (long long)nb * H; cb.q_ld = H;
-      cb.dc = w.dc + (size_t)b0 * H; cb.first = last ? 1 : 0;
-      cb.gates = w.gates + r * 4 * H;
-      cb.c_prev = w.c + r * H; cb.c_new = w.c + ((size_t)(t + 1) * B + b0) * H;
-      cb.B = nb; cb.H = H; cb.dG = w.dG + r * 4 * H; cb.dg_ld = 4 * H;
-      RN_TRY(em.cell_bwd(cb));
-      // d[ctx ; h_{t-1}] = dG_t @ [W_ctx | W_hh]
-      RN_TRY(em.gemm_partials(w.dG + r * 4 * H, 4 * H, 0, w.Wrec, w.KX, 1, dXp, nb, w.KX, 4 * H, w.pl_dx));
+    const size_t r = (size_t)t * B;                // first (t, b) row of step t
+    if (is_gru) {
+      float* dXx = w.dXp;                          // x-part dgrad partials [splits][B, E]
+      float* dXh = w.dXp2;                         // h-part dgrad partials [splits][B, H]
+      gru::BwdArgs gb{};
+      gb.dh_ext = w.dHext + r * H; gb.dh_ld = H;
+      gb.dh_ext2 = g_hiddens ? g_hiddens + r * H : nullptr; gb.dh2_ld = H;
+      gb.dHp = last ? nullptr : dXh; gb.n_p = w.pl_dxh.splits; gb.p_stride = (long long)B * H; gb.p_ld = H;
+      gb.dQp = last ? nullptr : w.dQp; gb.n_q = w.pl_dq.splits; gb.q_stride = (long long)B * H; gb.q_ld = H;
+      gb.carry = w.dc; gb.first = last ? 1 : 0;
+      gb.stash = w.gates + r * 4 * H;
+      gb.h_prev = t == 0 ? w.c : hiddens_fp32 + (size_t)(t - 1) * B * H; gb.hp_ld = H;
+      gb.B = B; gb.H = H; gb.dGi = w.dG + r * 3 * H; gb.dGh = w.dG2 + r * 3 * H; gb.dg_ld = 3 * H;
+      RN_TRY((gru::launch_bwd<T, T>(gb, st)));
+      RN_TRY(gemm_partials<T>(w.dG + r * 3 * H, 3 * H, 0, w.Wrec, w.KX, 1, dXx, B, E, 3 * H, w.pl_dxx, st));           // dctx = dGi @ W_ctx
+      if (t > 0) RN_TRY(gemm_partials<T>(w.dG2 + r * 3 * H, 3 * H, 0, w.Wrec + E, w.KX, 1, dXh, B, H, 3 * H, w.pl_dxh, st));  // dh += dGh @ W_hh
       attn::BwdArgs ab{};
-      ab.dXp = dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)nb * w.KX; ab.p_ld = w.KX;
-      ab.V = w.feats + (size_t)b0 * Tn * E; ab.v_bs = (long long)Tn * E; ab.v_ts = E;
-      ab.Wh = w.Wh + r * A; ab.Uv = w.Uv + (size_t)b0 * Tn * A; ab.uv_bs = (long long)Tn * A; ab.uv_ts = A;
-      ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = Tn; ab.A = A; ab.D = E; ab.inv_T = d.softmax ? 1.f : 1.f / Tn;
-      ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv + (size_t)b0 * Tn * A;
-      ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc + (size_t)b0 * A;
+      ab.dXp = dXx; ab.n_p = w.pl_dxx.splits; ab.p_stride = (long long)B * E; ab.p_ld = E;
+      ab.V = w.feats; ab.v_bs = (long long)Tn * E; ab.v_ts = E;
+      ab.Wh = w.Wh + r * A; ab.Uv = w.Uv; ab.uv_bs = (long long)Tn * A; ab.uv_ts = A;
+      ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = B; ab.Tn = Tn; ab.A = A; ab.D = E; ab.inv_T = d.softmax ? 1.f : 1.f / Tn;
+      ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv;
+      ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc;
       ab.dctx_out = nullptr; ab.de_out = nullptr; ab.p_drop = 0.f; ab.alpha = d.softmax ? w.e + r * Tn : nullptr;
-      RN_TRY(em.attn_bwd(ab));
-      // attention-query path into h_{t-1}: dWh_t @ attn_W, consumed (as split-K partials) by the next cell backward
-      if (t > 0) RN_TRY(em.gemm_partials(w.dWh_op + r * A, A, 0, w.Wa, H, 1, dQp, nb, H, A, w.pl_dq));
+      RN_TRY((attn::launch_bwd<T, T>(ab, st)));
+      if (t > 0) RN_TRY(gemm_partials<T>(w.dWh_op + r * A, A, 0, w.Wa, H, 1, w.dQp, B, H, A, w.pl_dq, st));
+      continue;
     }
+    cell::BwdArgs cb{};
+    cb.dh_ext = w.dHext + r * H; cb.dh_ld = H; cb.dh_scale = nullptr;
+    cb.dh_ext2 = g_hiddens ? g_hiddens + r * H : nullptr; cb.dh2_ld = H;
+    cb.dXp = last ? nullptr : w.dXp; cb.n_p = w.pl_dx.splits; cb.p_stride = (long long)B * w.KX; cb.p_ld = w.KX; cb.col0 = E;
+    cb.dQp = last ? nullptr : w.dQp; cb.n_q = w.pl_dq.splits; cb.q_stride = (long long)B * H; cb.q_ld = H;
+    cb.dc = w.dc; cb.first = last ? 1 : 0;
+    cb.gates = w.gates + r * 4 * H;
+    cb.c_prev = w.c + r * H; cb.c_new = w.c + (size_t)(t + 1) * B * H;
+    cb.B = B; cb.H = H; cb.dG = w.dG + r * 4 * H; cb.dg_ld = 4 * H;
+    RN_TRY((cell::launch_bwd<T, T>(cb, st)));
+    // d[ctx ; h_{t-1}] = dG_t @ [W_ctx | W_hh]
+    RN_TRY(gemm_partials<T>(w.dG + r * 4 * H, 4 * H, 0, w.Wrec, w.KX, 1, w.dXp, B, w.KX, 4 * H, w.pl_dx, st));
+    attn::BwdArgs ab{};
+    ab.dXp = w.dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)B * w.KX; ab.p_ld = w.KX;
+    ab.V = w.feats; ab.v_bs = (long long)Tn * E; ab.v_ts = E;
+    ab.Wh = w.Wh + r * A; ab.Uv = w.Uv; ab.uv_bs = (long long)Tn * A; ab.uv_ts = A;
+    ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = B; ab.Tn = Tn; ab.A = A; ab.D = E; ab.inv_T = d.softmax ? 1.f : 1.f / Tn;
+    ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv;
+    ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc;
+    ab.dctx_out = nullptr; ab.de_out = nullptr; ab.p_drop = 0.f; ab.alpha = d.softmax ? w.e + r * Tn : nullptr;
+    RN_TRY((attn::launch_bwd<T, T>(ab, st)));
+    // attention-query path into h_{t-1}: dWh_t @ attn_W, consumed (as split-K partials) by the next cell backward
+    if (t > 0) RN_TRY(gemm_partials<T>(w.dWh_op + r * A, A, 0, w.Wa, H, 1, w.dQp, B, H, A, w.pl_dq, st));
   }
-  RN_TRY(em0.flush(w.table, w.table_bytes, w.bar, w.err, 2));
-  if (w.nch > 1) RN_TRY(cs.join(st, w.nch));
   // ---- batched weight gradients over the stashed operands ----------------------------------------------------
   const long long ldih = EMB + E;
   // LSTM: one gate-gradient matrix dG [LB,4H]; GRU: dGi (input side) in w.dG and dGh (hidden side, n column scaled by r) in w.dG2
@@ -457,10 +415,8 @@ static int greedy(const DecDesc& d0, const recnet_decoder_tensors& p, const floa
                                                     nullptr, SITE_EMB);
     RN_LAUNCH_OK();
     RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
-    mega::Emitter<T> em(false, st);
     // GRU keeps its fp32 state h in the c ping-pong rows (h_prev = c_p, h' -> c_n)
-    RN_TRY(step<T>(em, d, p, w, t, 0, 0, B, w.Gx, x_t, x_n, nullptr, nullptr, nullptr, c_p, c_n,
-                   d.cell == RECNET_CELL_GRU ? c_n : g.h_scratch));
+    RN_TRY(step<T>(d, p, w, t, w.Gx, x_t, x_n, nullptr, nullptr, nullptr, c_p, c_n, d.cell == RECNET_CELL_GRU ? c_n : g.h_scratch, st));
     RN_TRY(gemm_full<T>(x_n + E, w.KX, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
     argmax_feedback_kernel<<<B, 256, 0, st>>>(w.logits, w.Vld, V, ids_out + (size_t)t * B, g.tok, g.nonpad + t);
     RN_LAUNCH_OK();
@@ -620,8 +576,7 @@ static int beam(const DecDesc& d0, const recnet_decoder_tensors& p, const float*
                                                     nullptr, SITE_EMB);
     RN_LAUNCH_OK();
     RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
-    mega::Emitter<T> em(false, st);
-    RN_TRY(step<T>(em, d, p, w, t, 0, 0, B, w.Gx, x0, x1, nullptr, nullptr, nullptr, c0, c1, d.cell == RECNET_CELL_GRU ? c1 : g.h_scratch));
+    RN_TRY(step<T>(d, p, w, t, w.Gx, x0, x1, nullptr, nullptr, nullptr, c0, c1, d.cell == RECNET_CELL_GRU ? c1 : g.h_scratch, st));
     RN_TRY(gemm_full<T>(x1 + E, w.KX, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
     const int in = t & 1, out = (t + 1) & 1;
     beam_select_kernel<<<B0, BEAM_THREADS, 0, st>>>(w.logits, w.Vld, V, B0, K, t, max_steps, eos, bw.cum[in], bw.cum[out], bw.eos[in], bw.eos[out],

@@ -36,14 +36,13 @@ static int forward_ml(const DecDesc& d, const recnet_decoder_tensors& p, const f
     RN_CUDA_OK(cudaMemsetAsync(w.X_x[l - 1], 0, (size_t)B * 2 * H * sizeof(T), st));
     RN_CUDA_OK(cudaMemsetAsync(w.c_x[l - 1], 0, (size_t)B * H * sizeof(float), st));
   }
-  mega::Emitter<T> em(false, st);
   T* Xtop = w.X_x[top - 1];
   for (int t = 0; t < L; ++t) {
     T* x0 = w.X + (size_t)t * B * w.KX;
     // attention with the top layer's previous state as query
     int n_whp = 0;
     if (t > 0) {
-      RN_TRY(em.gemm_partials(Xtop + (size_t)t * B * 2 * H + H, 2 * H, 0, w.Wa, H, 0, w.WhP, B, A, H, w.pl_wh));
+      RN_TRY(gemm_partials<T>(Xtop + (size_t)t * B * 2 * H + H, 2 * H, 0, w.Wa, H, 0, w.WhP, B, A, H, w.pl_wh, st));
       n_whp = w.pl_wh.splits;
     }
     attn::FwdArgs fa{};
@@ -52,13 +51,13 @@ static int forward_ml(const DecDesc& d, const recnet_decoder_tensors& p, const f
     fa.V = w.feats; fa.v_bs = (long long)Tn * E; fa.v_ts = E; fa.B = B; fa.Tn = Tn; fa.A = A; fa.D = E;
     fa.inv_T = d.softmax ? 1.f : 1.f / Tn; fa.normalize = d.softmax;
     fa.Wh_out = w.Wh + (size_t)t * B * A; fa.e_out = w.e + (size_t)t * B * Tn; fa.ctx_out = x0; fa.ctx_ld = w.KX;
-    RN_TRY(em.attn_fwd(fa));
+    RN_TRY((attn::launch_fwd<T, T>(fa, st)));
     for (int l = 0; l < NL; ++l) {
       const int K = l == 0 ? w.KX : 2 * H;
       T* xl = l == 0 ? x0 : w.X_x[l - 1] + (size_t)t * B * 2 * H;
       const T* Wl = l == 0 ? w.Wrec : w.Wrec_x[l - 1];
       const GemmPlan pl = l == 0 ? w.pl_gate : w.pl_gate_x;
-      RN_TRY(em.gemm_partials(xl, K, 0, Wl, K, 0, w.P, B, 4 * H, K, pl));
+      RN_TRY(gemm_partials<T>(xl, K, 0, Wl, K, 0, w.P, B, 4 * H, K, pl, st));
       float* cl = l == 0 ? w.c : w.c_x[l - 1];
       cell::FwdArgs ca{};
       ca.P = w.P; ca.n_p = pl.splits; ca.p_stride = (long long)B * 4 * H; ca.p_ld = 4 * H;
@@ -72,7 +71,7 @@ static int forward_ml(const DecDesc& d, const recnet_decoder_tensors& p, const f
         ca.h_op2 = w.X_x[l] + (size_t)t * B * 2 * H; ca.hop2_ld = 2 * H;
         ca.op2_drop = p_lay; ca.rng = rng; ca.site = SITE_LAYER0 + l + 1; ca.drop_base = (long long)t * B * H;
       }
-      RN_TRY(em.cell_fwd(ca));
+      RN_TRY((cell::launch_fwd<T, T>(ca, st)));
     }
   }
   RN_TRY(gemm_full<T>(Xtop + (size_t)B * 2 * H + H, 2 * H, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, L * B, V, H, 0, w.splitk, st));
@@ -106,7 +105,6 @@ static int backward_ml(const DecDesc& d, const recnet_decoder_tensors& p, const 
   RN_TRY(gemm_full<T>(w.dlogits, w.Vp, 0, w.Wout, H, 1, w.dHext, H, nullptr, LB, H, V, 0, w.splitk, st));
   RN_TRY(gemm_full<T>(w.dlogits, w.Vp, 1, Htop, 2 * H, 1, g.out_w, H, nullptr, V, H, LB, 0, w.splitk, st));
   RN_TRY(misc::colsum<T>(w.dlogits, w.Vp, LB, V, g.out_b, 0, w.splitk, st));
-  mega::Emitter<T> em(false, st);
   for (int t = L - 1; t >= 0; --t) {
     const bool last = (t == L - 1);
     for (int l = top; l >= 0; --l) {
@@ -131,9 +129,9 @@ static int backward_ml(const DecDesc& d, const recnet_decoder_tensors& p, const 
       cb.B = B; cb.H = H;
       T* dGl = (l == 0 ? w.dG : w.dG_x[l - 1]) + (size_t)t * B * 4 * H;
       cb.dG = dGl; cb.dg_ld = 4 * H;
-      RN_TRY(em.cell_bwd(cb));
+      RN_TRY((cell::launch_bwd<T, T>(cb, st)));
       const T* Wl = l == 0 ? w.Wrec : w.Wrec_x[l - 1];
-      RN_TRY(em.gemm_partials(dGl, 4 * H, 0, Wl, K, 1, dXl, B, K, 4 * H, pl));
+      RN_TRY(gemm_partials<T>(dGl, 4 * H, 0, Wl, K, 1, dXl, B, K, 4 * H, pl, st));
     }
     attn::BwdArgs ab{};
     ab.dXp = w.dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)B * w.KX; ab.p_ld = w.KX;
@@ -143,8 +141,8 @@ static int backward_ml(const DecDesc& d, const recnet_decoder_tensors& p, const 
     ab.inv_T = d.softmax ? 1.f : 1.f / Tn; ab.alpha = d.softmax ? w.e + (size_t)t * B * Tn : nullptr;
     ab.dWh_out = w.dWh + (size_t)t * B * A; ab.dWh_op = w.dWh_op + (size_t)t * B * A; ab.dUv_acc = w.dUv;
     ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc;
-    RN_TRY(em.attn_bwd(ab));
-    if (t > 0) RN_TRY(em.gemm_partials(w.dWh_op + (size_t)t * B * A, A, 0, w.Wa, H, 1, w.dQp, B, H, A, w.pl_dq));
+    RN_TRY((attn::launch_bwd<T, T>(ab, st)));
+    if (t > 0) RN_TRY(gemm_partials<T>(w.dWh_op + (size_t)t * B * A, A, 0, w.Wa, H, 1, w.dQp, B, H, A, w.pl_dq, st));
   }
   // ---- weight gradients ----
   const long long ldih = EMB + E;

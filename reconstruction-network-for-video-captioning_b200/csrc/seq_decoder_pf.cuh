@@ -31,7 +31,6 @@ static inline bool pf_enabled() {
 }
 static inline bool pf_ok(const recnet_decoder_desc& d) {
   if (!pf_enabled() || d.cell != RECNET_CELL_LSTM || d.n_layers > 1) return false;
-  if (num_chains(d.B) != 1) return false;
   const int al = d.precision == RECNET_PREC_BF16 ? 8 : 4;
   if ((long long)d.B * d.T * 4 * d.H >= (1ll << 31) || (long long)d.L * d.B * (d.A + 4 * d.H) >= (1ll << 31)) return false;   // 32-bit index math
   if ((d.E & 1) || pf::escore_smem(d.L, d.T, true) > 46 * 1024) return false;          // pf_escore_kernel: column pairs, e[L x T] in shared memory
@@ -47,8 +46,8 @@ static PfWs<T> plan_pf(const recnet_decoder_desc& d, void* base) {
   w.Vp = round_up(V, 8);
   w.Vld = round_up(V, 4);
   w.NP = A + 4 * H;
-  w.pl_h = plan_gemm<T>(B, w.NP, H, NUM_SMS);
-  w.pl_dh = plan_gemm<T>(B, H, w.NP, NUM_SMS);
+  w.pl_h = plan_gemm<T>(B, w.NP, H);
+  w.pl_dh = plan_gemm<T>(B, H, w.NP);
   if (Prec<T>::id == RECNET_PREC_BF16) {
     // K = H is only 8 k-blocks: 64-wide N tiles x few splits (34 x 4 CTAs at H = 512) instead of 128-wide x 8 -- half the
     // partial traffic for the fused kernel to sum
@@ -310,7 +309,7 @@ static GreedyPfWs<T> plan_greedy_pf(const recnet_decoder_desc& d, void* base, in
   w.EMBp = round_up(d.EMB, Prec<T>::kpad);
   w.Vld = round_up(V, 4);
   w.NP = A + 4 * H;
-  w.pl_h = plan_gemm<T>(B, w.NP, H, NUM_SMS);
+  w.pl_h = plan_gemm<T>(B, w.NP, H);
   Bump m(base);
   w.Wemb = m.take<T>((size_t)4 * H * w.EMBp);
   w.WctxI = m.take<T>((size_t)4 * H * E);

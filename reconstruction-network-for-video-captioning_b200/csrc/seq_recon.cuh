@@ -7,7 +7,6 @@
 // projection and all weight gradients batched over time.  One decoder layer (the reference default).
 #pragma once
 #include "gru_cell.cuh"
-#include "mega.cuh"
 #include "runtime.cuh"
 #include "seq_recon_persist.cuh"
 
@@ -19,14 +18,14 @@ enum : unsigned { SITE_LOCAL_X = 3, SITE_GLOBAL_MP = 4 };
 // ================================================ local =========================================================
 template <typename T>
 struct LocalWs {
-  int KX, nch, Bc, G;
+  int KX, G;
   GemmPlan pl_wh, pl_gate, pl_dx, pl_dq;
   GemmPlan pl_gx, pl_gh, pl_dxx, pl_dxh;      // GRU: input / hidden sides kept separate
   T *Wrec, *U, *Wa, *Wout, *Hd;
   float* Uv; T* X; float* WhP; float* Wh; float* beta; float* P; float* P2; T* gates; float* c; float* out; float* partial;
   T* dOut; float* dHext; T* dG; T* dG2; float* dXp; float* dXp2; float* dQp; float* dWh; T* dWh_op; float* dUv; T* dUv_op; float* dw_acc; float* dc;
   float* dx; float* splitk; float* splitk2;        // splitk2: scratch of the side stream (runtime.cuh:Side)
-  uint8_t* table; size_t table_bytes; unsigned* bar; int* err;
+  int* err;
   T* Hout; T* Hq;                 // stacked decoder only: compact rows of h after pseudo-step (t,0) / at the start of outer step t
   float* pXP; float* pWhP; unsigned* psync;      // weight-resident persistent loop (seq_recon_persist.cuh): partial exchange + flags
   size_t bytes;
@@ -36,12 +35,12 @@ constexpr int MSE_BLOCKS = 592;
 // the weight-resident persistent forward loop covers: bf16, LSTM over a 1-layer decoder, shapes whose [W_ih | W_hh] fits the SMs' shared memory
 template <typename T>
 static inline bool persist_fwd_ok(const recnet_local_desc& d) {
-  if (!std::is_same<T, bf16>::value || d.cell != RECNET_CELL_LSTM || d.dec_layers > 1 || num_chains(d.B) != 1) return false;
+  if (!std::is_same<T, bf16>::value || d.cell != RECNET_CELL_LSTM || d.dec_layers > 1) return false;
   return rp::local_fwd_ok(rp::Shape{d.B, d.S, d.R, d.H, d.A, d.L});
 }
 template <typename T>
 static inline bool persist_bwd_ok(const recnet_local_desc& d) {
-  if (!std::is_same<T, bf16>::value || d.cell != RECNET_CELL_LSTM || d.dec_layers > 1 || num_chains(d.B) != 1) return false;
+  if (!std::is_same<T, bf16>::value || d.cell != RECNET_CELL_LSTM || d.dec_layers > 1) return false;
   static int on = -1;
   if (on < 0) { const char* e = getenv("RECNET_PERSIST_BWD"); on = e ? atoi(e) : 1; }
   return on && rp::local_bwd_ok(rp::Shape{d.B, d.S, d.R, d.H, d.A, d.L});
@@ -54,23 +53,20 @@ static LocalWs<T> plan_local(const recnet_local_desc& d, void* base) {
   // with a stacked decoder every outer step runs NLd pseudo-steps and the hiddens carry a layer axis: size by S*NLd / L*NLd
   const int B = d.B, S = d.S * NLd, R = d.R, H = d.H, A = d.A, L = d.L * NLd;
   w.KX = H + R;
-  w.nch = num_chains(B);
-  w.Bc = chain_rows_max(B, w.nch);
-  const int tgt = w.nch > 1 ? NUM_SMS / 2 : NUM_SMS;
-  w.pl_wh = plan_gemm<T>(w.Bc, A, R, tgt);
+  w.pl_wh = plan_gemm<T>(B, A, R);
   if (w.pl_wh.splits > 8) {      // the attention kernel sums these partials with one batch of 8 loads per lane
     const int nkb = rn_cdiv(R, 64);
     w.pl_wh.splits = rn_cdiv(nkb, rn_cdiv(nkb, 8));
   }
-  w.pl_gate = plan_gemm<T>(w.Bc, 4 * R, w.KX, tgt);
-  w.pl_dx = plan_gemm<T>(w.Bc, w.KX, 4 * R, tgt);
-  w.pl_dq = plan_gemm<T>(w.Bc, R, A, tgt);
+  w.pl_gate = plan_gemm<T>(B, 4 * R, w.KX);
+  w.pl_dx = plan_gemm<T>(B, w.KX, 4 * R);
+  w.pl_dq = plan_gemm<T>(B, R, A);
   const bool gru_ = d.cell == RECNET_CELL_GRU;
   w.G = gru_ ? 3 : 4;
-  w.pl_gx = plan_gemm<T>(w.Bc, 3 * R, H, tgt);
-  w.pl_gh = plan_gemm<T>(w.Bc, 3 * R, R, tgt);
-  w.pl_dxx = plan_gemm<T>(w.Bc, H, 3 * R, tgt);
-  w.pl_dxh = plan_gemm<T>(w.Bc, R, 3 * R, tgt);
+  w.pl_gx = plan_gemm<T>(B, 3 * R, H);
+  w.pl_gh = plan_gemm<T>(B, 3 * R, R);
+  w.pl_dxx = plan_gemm<T>(B, H, 3 * R);
+  w.pl_dxh = plan_gemm<T>(B, R, 3 * R);
   Bump m(base);
   w.Wrec = m.take<T>((size_t)4 * R * w.KX);
   w.U = m.take<T>((size_t)A * H);
@@ -79,11 +75,11 @@ static LocalWs<T> plan_local(const recnet_local_desc& d, void* base) {
   w.Hd = m.take<T>((size_t)L * B * H);
   w.Uv = m.take<float>((size_t)L * B * A);
   w.X = m.take<T>((size_t)(S + 1) * B * w.KX);
-  w.WhP = m.take<float>((size_t)w.nch * (w.pl_wh.splits > rn_cdiv(R, cell::THREADS) ? w.pl_wh.splits : rn_cdiv(R, cell::THREADS)) * w.Bc * A);
+  w.WhP = m.take<float>((size_t)(w.pl_wh.splits > rn_cdiv(R, cell::THREADS) ? w.pl_wh.splits : rn_cdiv(R, cell::THREADS)) * B * A);
   w.Wh = m.take<float>((size_t)S * B * A);
   w.beta = m.take<float>((size_t)S * B * L);
-  w.P = m.take<float>((size_t)w.nch * (gru_ ? w.pl_gx.splits : w.pl_gate.splits) * w.Bc * 4 * R);
-  w.P2 = m.take<float>(gru_ ? (size_t)w.nch * w.pl_gh.splits * w.Bc * 3 * R : 1);
+  w.P = m.take<float>((size_t)(gru_ ? w.pl_gx.splits : w.pl_gate.splits) * B * 4 * R);
+  w.P2 = m.take<float>(gru_ ? (size_t)w.pl_gh.splits * B * 3 * R : 1);
   w.gates = m.take<T>((size_t)S * B * 4 * R);
   w.c = m.take<float>((size_t)(S + 1) * B * R);
   w.out = m.take<float>((size_t)S * B * R);
@@ -91,10 +87,10 @@ static LocalWs<T> plan_local(const recnet_local_desc& d, void* base) {
   w.dOut = m.take<T>((size_t)S * B * R);
   w.dHext = m.take<float>((size_t)S * B * R);
   w.dG = m.take<T>((size_t)S * B * 4 * R);
-  w.dXp = m.take<float>((size_t)w.nch * (gru_ ? w.pl_dxx.splits : w.pl_dx.splits) * w.Bc * w.KX);
-  w.dXp2 = m.take<float>(gru_ ? (size_t)w.nch * w.pl_dxh.splits * w.Bc * R : 1);
+  w.dXp = m.take<float>((size_t)(gru_ ? w.pl_dxx.splits : w.pl_dx.splits) * B * w.KX);
+  w.dXp2 = m.take<float>(gru_ ? (size_t)w.pl_dxh.splits * B * R : 1);
   w.dG2 = m.take<T>(gru_ ? (size_t)S * B * 3 * R : 1);
-  w.dQp = m.take<float>((size_t)w.nch * w.pl_dq.splits * w.Bc * R);
+  w.dQp = m.take<float>((size_t)w.pl_dq.splits * B * R);
   w.dWh = m.take<float>((size_t)S * B * A);
   w.dWh_op = m.take<T>((size_t)S * B * A);
   w.dUv = m.take<float>((size_t)L * B * A);
@@ -104,9 +100,6 @@ static LocalWs<T> plan_local(const recnet_local_desc& d, void* base) {
   w.dx = m.take<float>((size_t)S * B * H);
   w.splitk = m.take<float>(SPLITK_SCRATCH_FLOATS);
   w.splitk2 = m.take<float>(SPLITK_SCRATCH_FLOATS);
-  w.table_bytes = mega::table_bytes(S);
-  w.table = m.take<uint8_t>(w.table_bytes);
-  w.bar = m.take<unsigned>(64);
   w.err = m.take<int>(64);
   w.Hout = m.take<T>(NLd > 1 ? (size_t)d.S * B * R : 1);
   w.Hq = m.take<T>(NLd > 1 ? (size_t)d.S * B * R : 1);
@@ -175,62 +168,47 @@ static int local_forward(const LocalDesc& d, const recnet_local_tensors& p, cons
       return 0;
     }
   }
-  Chains& cs = chains();
-  if (w.nch > 1) RN_TRY(cs.fork(st, w.nch));
-  mega::Emitter<T> em0(w.nch == 1 && !is_gru, st, (size_t)H + L + 8 * attn::BWD_THREADS + 2 * A);
   for (int t = 0; t < S; ++t) {
-    for (int ch = 0; ch < w.nch; ++ch) {
-      int b0, nb;
-      chain_rows(B, w.nch, ch, &b0, &nb);
-      mega::Emitter<T> emc(false, w.nch > 1 ? cs.s[ch] : st);
-      mega::Emitter<T>& em = w.nch == 1 ? em0 : emc;
-      float* WhP = w.WhP + (size_t)ch * w.pl_wh.splits * w.Bc * A;
-      float* P = w.P + (size_t)ch * w.pl_gate.splits * w.Bc * 4 * R;
-      const size_t r = (size_t)t * B + b0;
-      T* x_t = w.X + r * w.KX;
-      T* x_n = x_t + (size_t)B * w.KX;
-      // attention query W.h_{t-1}: its own small GEMM, partials summed by the attention kernel
-      int n_whp = 0;
-      if (t > 0) {
-        RN_TRY(em.gemm_partials(x_t + H, w.KX, 0, w.Wa, R, 0, WhP, nb, A, R, w.pl_wh));
-        n_whp = w.pl_wh.splits;
-      }
-      attn::FwdArgs fa{};
-      fa.WhP = WhP; fa.n_whp = n_whp; fa.whp_stride = (long long)nb * A;
-      fa.Uv = w.Uv + (size_t)b0 * A; fa.uv_bs = A; fa.uv_ts = (long long)B * A;          // Uv is [L,B,A]
-      fa.attn_b = p.attn_b; fa.attn_w = p.attn_w;
-      fa.V = w.Hd + (size_t)b0 * H; fa.v_bs = H; fa.v_ts = (long long)B * H;             // values = decoder states [L,B,H]
-      fa.B = nb; fa.Tn = L; fa.A = A; fa.D = H; fa.inv_T = d.softmax ? 1.f : 1.f / L; fa.normalize = d.softmax;
-      fa.Wh_out = w.Wh + r * A; fa.e_out = w.beta + r * L;
-      fa.ctx_out = x_t; fa.ctx_ld = w.KX;
-      fa.p_drop = p_drop; fa.rng = rng; fa.site = SITE_LOCAL_X; fa.drop_base = (long long)r * H;
-      RN_TRY(em.attn_fwd(fa));
-      if (is_gru) {
-        float* Px = w.P + (size_t)ch * w.pl_gx.splits * w.Bc * 3 * R;
-        float* Ph = w.P2 + (size_t)ch * w.pl_gh.splits * w.Bc * 3 * R;
-        RN_TRY(em.gemm_partials(x_t, w.KX, 0, w.Wrec, w.KX, 0, Px, nb, 3 * R, H, w.pl_gx));
-        if (t > 0) RN_TRY(em.gemm_partials(x_t + H, w.KX, 0, w.Wrec + H, w.KX, 0, Ph, nb, 3 * R, R, w.pl_gh));
-        gru::FwdArgs ga{};
-        ga.Px = Px; ga.n_px = w.pl_gx.splits; ga.px_stride = (long long)nb * 3 * R; ga.px_ld = 3 * R;
-        ga.Ph = t > 0 ? Ph : nullptr; ga.n_ph = t > 0 ? w.pl_gh.splits : 0; ga.ph_stride = (long long)nb * 3 * R; ga.ph_ld = 3 * R;
-        ga.Gx = nullptr; ga.b_ih = p.b_ih; ga.b_hh = p.b_hh;
-        ga.h_prev = w.c + r * R; ga.hp_ld = R; ga.B = nb; ga.H = R;            // fp32 state h lives in the c rows
-        ga.stash = w.gates + r * 4 * R; ga.h_out = w.c + ((size_t)(t + 1) * B + b0) * R; ga.h_ld = R;
-        ga.h_op = x_n + H; ga.hop_ld = w.KX;
-        RN_TRY((gru::launch_fwd<T, T>(ga, em.st)));
-        continue;
-      }
-      RN_TRY(em.gemm_partials(x_t, w.KX, 0, w.Wrec, w.KX, 0, P, nb, 4 * R, w.KX, w.pl_gate));
-      cell::FwdArgs ca{};
-      ca.P = P; ca.n_p = w.pl_gate.splits; ca.p_stride = (long long)nb * 4 * R; ca.p_ld = 4 * R;
-      ca.Gx = nullptr; ca.b1 = p.b_ih; ca.b2 = p.b_hh; ca.c_prev = w.c + r * R; ca.B = nb; ca.H = R;
-      ca.gates_out = w.gates + r * 4 * R; ca.c_out = w.c + ((size_t)(t + 1) * B + b0) * R; ca.h_out = nullptr;
-      ca.h_op = x_n + H; ca.hop_ld = w.KX; ca.h_op2 = nullptr;
-      RN_TRY(em.cell_fwd(ca));
+    const size_t r = (size_t)t * B;
+    T* x_t = w.X + r * w.KX;
+    T* x_n = x_t + (size_t)B * w.KX;
+    // attention query W.h_{t-1}: its own small GEMM, partials summed by the attention kernel
+    int n_whp = 0;
+    if (t > 0) {
+      RN_TRY(gemm_partials<T>(x_t + H, w.KX, 0, w.Wa, R, 0, w.WhP, B, A, R, w.pl_wh, st));
+      n_whp = w.pl_wh.splits;
     }
+    attn::FwdArgs fa{};
+    fa.WhP = w.WhP; fa.n_whp = n_whp; fa.whp_stride = (long long)B * A;
+    fa.Uv = w.Uv; fa.uv_bs = A; fa.uv_ts = (long long)B * A;          // Uv is [L,B,A]
+    fa.attn_b = p.attn_b; fa.attn_w = p.attn_w;
+    fa.V = w.Hd; fa.v_bs = H; fa.v_ts = (long long)B * H;             // values = decoder states [L,B,H]
+    fa.B = B; fa.Tn = L; fa.A = A; fa.D = H; fa.inv_T = d.softmax ? 1.f : 1.f / L; fa.normalize = d.softmax;
+    fa.Wh_out = w.Wh + r * A; fa.e_out = w.beta + r * L;
+    fa.ctx_out = x_t; fa.ctx_ld = w.KX;
+    fa.p_drop = p_drop; fa.rng = rng; fa.site = SITE_LOCAL_X; fa.drop_base = (long long)r * H;
+    RN_TRY((attn::launch_fwd<T, T>(fa, st)));
+    if (is_gru) {
+      RN_TRY(gemm_partials<T>(x_t, w.KX, 0, w.Wrec, w.KX, 0, w.P, B, 3 * R, H, w.pl_gx, st));
+      if (t > 0) RN_TRY(gemm_partials<T>(x_t + H, w.KX, 0, w.Wrec + H, w.KX, 0, w.P2, B, 3 * R, R, w.pl_gh, st));
+      gru::FwdArgs ga{};
+      ga.Px = w.P; ga.n_px = w.pl_gx.splits; ga.px_stride = (long long)B * 3 * R; ga.px_ld = 3 * R;
+      ga.Ph = t > 0 ? w.P2 : nullptr; ga.n_ph = t > 0 ? w.pl_gh.splits : 0; ga.ph_stride = (long long)B * 3 * R; ga.ph_ld = 3 * R;
+      ga.Gx = nullptr; ga.b_ih = p.b_ih; ga.b_hh = p.b_hh;
+      ga.h_prev = w.c + r * R; ga.hp_ld = R; ga.B = B; ga.H = R;            // fp32 state h lives in the c rows
+      ga.stash = w.gates + r * 4 * R; ga.h_out = w.c + (size_t)(t + 1) * B * R; ga.h_ld = R;
+      ga.h_op = x_n + H; ga.hop_ld = w.KX;
+      RN_TRY((gru::launch_fwd<T, T>(ga, st)));
+      continue;
+    }
+    RN_TRY(gemm_partials<T>(x_t, w.KX, 0, w.Wrec, w.KX, 0, w.P, B, 4 * R, w.KX, w.pl_gate, st));
+    cell::FwdArgs ca{};
+    ca.P = w.P; ca.n_p = w.pl_gate.splits; ca.p_stride = (long long)B * 4 * R; ca.p_ld = 4 * R;
+    ca.Gx = nullptr; ca.b1 = p.b_ih; ca.b2 = p.b_hh; ca.c_prev = w.c + r * R; ca.B = B; ca.H = R;
+    ca.gates_out = w.gates + r * 4 * R; ca.c_out = w.c + (size_t)(t + 1) * B * R; ca.h_out = nullptr;
+    ca.h_op = x_n + H; ca.hop_ld = w.KX; ca.h_op2 = nullptr;
+    RN_TRY((cell::launch_fwd<T, T>(ca, st)));
   }
-  RN_TRY(em0.flush(w.table, w.table_bytes, w.bar, w.err, 3));
-  if (w.nch > 1) RN_TRY(cs.join(st, w.nch));
   RN_TRY(gemm_full<T>(w.X + (size_t)B * w.KX + H, w.KX, 0, w.Wout, R, 0, w.out, R, p.out_b, S * B, R, R, 0, w.splitk, st));
   if (mse_out) {
     loss::mse_local_fwd_kernel<<<MSE_BLOCKS, 256, 0, st>>>(w.out, feats, S, B, R, w.partial);
@@ -261,8 +239,6 @@ static int local_backward(const LocalDesc& d, const recnet_local_tensors& p, con
   loss::mse_local_bwd_kernel<T><<<MSE_BLOCKS, 256, 0, st>>>(w.out, feats, S, B, R, g_mse, 2.f / ((float)S * B * R), w.dOut);
   RN_LAUNCH_OK();
   RN_TRY(gemm_full<T>(w.dOut, R, 0, w.Wout, R, 1, w.dHext, R, nullptr, SB, R, R, 0, w.splitk, st));
-  Chains& cs = chains();
-  if (w.nch > 1) RN_TRY(cs.fork(st, w.nch));
   const bool is_gru = d.cell == RECNET_CELL_GRU;
   const int GR = w.G * R;
   bool persist = false;
@@ -279,68 +255,57 @@ static int local_backward(const LocalDesc& d, const recnet_local_tensors& p, con
       RN_TRY(rp::launch_local_bwd(bp, w.Wrec, st));
     }
   }
-  mega::Emitter<T> em0(w.nch == 1 && !is_gru, st, (size_t)H + L + 8 * attn::BWD_THREADS + 2 * A);
   for (int t = S - 1; t >= 0 && !persist; --t) {
     const bool last = (t == S - 1);
-    for (int ch = 0; ch < w.nch; ++ch) {
-      int b0, nb;
-      chain_rows(B, w.nch, ch, &b0, &nb);
-      mega::Emitter<T> emc(false, w.nch > 1 ? cs.s[ch] : st);
-      mega::Emitter<T>& em = w.nch == 1 ? em0 : emc;
-      float* dXp = w.dXp + (size_t)ch * w.pl_dx.splits * w.Bc * w.KX;
-      float* dQp = w.dQp + (size_t)ch * w.pl_dq.splits * w.Bc * R;
-      const size_t r = (size_t)t * B + b0;
-      if (is_gru) {
-        float* dXx = w.dXp + (size_t)ch * w.pl_dxx.splits * w.Bc * w.KX;
-        float* dXh = w.dXp2 + (size_t)ch * w.pl_dxh.splits * w.Bc * R;
-        gru::BwdArgs gb{};
-        gb.dh_ext = w.dHext + r * R; gb.dh_ld = R;
-        gb.dHp = last ? nullptr : dXh; gb.n_p = w.pl_dxh.splits; gb.p_stride = (long long)nb * R; gb.p_ld = R;
-        gb.dQp = last ? nullptr : dQp; gb.n_q = w.pl_dq.splits; gb.q_stride = (long long)nb * R; gb.q_ld = R;
-        gb.carry = w.dc + (size_t)b0 * R; gb.first = last ? 1 : 0;
-        gb.stash = w.gates + r * 4 * R; gb.h_prev = w.c + r * R; gb.hp_ld = R;
-        gb.B = nb; gb.H = R; gb.dGi = w.dG + r * 3 * R; gb.dGh = w.dG2 + r * 3 * R; gb.dg_ld = 3 * R;
-        RN_TRY((gru::launch_bwd<T, T>(gb, em.st)));
-        RN_TRY(em.gemm_partials(w.dG + r * 3 * R, 3 * R, 0, w.Wrec, w.KX, 1, dXx, nb, H, 3 * R, w.pl_dxx));
-        if (t > 0) RN_TRY(em.gemm_partials(w.dG2 + r * 3 * R, 3 * R, 0, w.Wrec + H, w.KX, 1, dXh, nb, R, 3 * R, w.pl_dxh));
-        attn::BwdArgs ab{};
-        ab.dXp = dXx; ab.n_p = w.pl_dxx.splits; ab.p_stride = (long long)nb * H; ab.p_ld = H;
-        ab.V = w.Hd + (size_t)b0 * H; ab.v_bs = H; ab.v_ts = (long long)B * H;
-        ab.Wh = w.Wh + r * A; ab.Uv = w.Uv + (size_t)b0 * A; ab.uv_bs = A; ab.uv_ts = (long long)B * A;
-        ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = d.softmax ? 1.f : 1.f / L;
-        ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv + (size_t)b0 * A;
-        ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc + (size_t)b0 * A;
-        ab.dctx_out = w.dx + r * H; ab.de_out = nullptr; ab.alpha = d.softmax ? w.beta + r * L : nullptr;
-        ab.p_drop = p_drop; ab.rng = rng; ab.site = SITE_LOCAL_X; ab.drop_base = (long long)r * H;
-        RN_TRY(em.attn_bwd(ab));
-        if (t > 0) RN_TRY(em.gemm_partials(w.dWh_op + r * A, A, 0, w.Wa, R, 1, dQp, nb, R, A, w.pl_dq));
-        continue;
-      }
-      cell::BwdArgs cb{};
-      cb.dh_ext = w.dHext + r * R; cb.dh_ld = R;
-      cb.dXp = last ? nullptr : dXp; cb.n_p = w.pl_dx.splits; cb.p_stride = (long long)nb * w.KX; cb.p_ld = w.KX; cb.col0 = H;
-      cb.dQp = last ? nullptr : dQp; cb.n_q = w.pl_dq.splits; cb.q_stride = (long long)nb * R; cb.q_ld = R;
-      cb.dc = w.dc + (size_t)b0 * R; cb.first = last ? 1 : 0;
-      cb.gates = w.gates + r * 4 * R;
-      cb.c_prev = w.c + r * R; cb.c_new = w.c + ((size_t)(t + 1) * B + b0) * R;
-      cb.B = nb; cb.H = R; cb.dG = w.dG + r * 4 * R; cb.dg_ld = 4 * R;
-      RN_TRY(em.cell_bwd(cb));
-      RN_TRY(em.gemm_partials(w.dG + r * 4 * R, 4 * R, 0, w.Wrec, w.KX, 1, dXp, nb, w.KX, 4 * R, w.pl_dx));
+    const size_t r = (size_t)t * B;
+    if (is_gru) {
+      float* dXx = w.dXp;
+      float* dXh = w.dXp2;
+      gru::BwdArgs gb{};
+      gb.dh_ext = w.dHext + r * R; gb.dh_ld = R;
+      gb.dHp = last ? nullptr : dXh; gb.n_p = w.pl_dxh.splits; gb.p_stride = (long long)B * R; gb.p_ld = R;
+      gb.dQp = last ? nullptr : w.dQp; gb.n_q = w.pl_dq.splits; gb.q_stride = (long long)B * R; gb.q_ld = R;
+      gb.carry = w.dc; gb.first = last ? 1 : 0;
+      gb.stash = w.gates + r * 4 * R; gb.h_prev = w.c + r * R; gb.hp_ld = R;
+      gb.B = B; gb.H = R; gb.dGi = w.dG + r * 3 * R; gb.dGh = w.dG2 + r * 3 * R; gb.dg_ld = 3 * R;
+      RN_TRY((gru::launch_bwd<T, T>(gb, st)));
+      RN_TRY(gemm_partials<T>(w.dG + r * 3 * R, 3 * R, 0, w.Wrec, w.KX, 1, dXx, B, H, 3 * R, w.pl_dxx, st));
+      if (t > 0) RN_TRY(gemm_partials<T>(w.dG2 + r * 3 * R, 3 * R, 0, w.Wrec + H, w.KX, 1, dXh, B, R, 3 * R, w.pl_dxh, st));
       attn::BwdArgs ab{};
-      ab.dXp = dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)nb * w.KX; ab.p_ld = w.KX;
-      ab.V = w.Hd + (size_t)b0 * H; ab.v_bs = H; ab.v_ts = (long long)B * H;
-      ab.Wh = w.Wh + r * A; ab.Uv = w.Uv + (size_t)b0 * A; ab.uv_bs = A; ab.uv_ts = (long long)B * A;
-      ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = nb; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = d.softmax ? 1.f : 1.f / L;
-      ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv + (size_t)b0 * A;
-      ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc + (size_t)b0 * A;
+      ab.dXp = dXx; ab.n_p = w.pl_dxx.splits; ab.p_stride = (long long)B * H; ab.p_ld = H;
+      ab.V = w.Hd; ab.v_bs = H; ab.v_ts = (long long)B * H;
+      ab.Wh = w.Wh + r * A; ab.Uv = w.Uv; ab.uv_bs = A; ab.uv_ts = (long long)B * A;
+      ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = B; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = d.softmax ? 1.f : 1.f / L;
+      ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv;
+      ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc;
       ab.dctx_out = w.dx + r * H; ab.de_out = nullptr; ab.alpha = d.softmax ? w.beta + r * L : nullptr;
       ab.p_drop = p_drop; ab.rng = rng; ab.site = SITE_LOCAL_X; ab.drop_base = (long long)r * H;
-      RN_TRY(em.attn_bwd(ab));
-      if (t > 0) RN_TRY(em.gemm_partials(w.dWh_op + r * A, A, 0, w.Wa, R, 1, dQp, nb, R, A, w.pl_dq));
+      RN_TRY((attn::launch_bwd<T, T>(ab, st)));
+      if (t > 0) RN_TRY(gemm_partials<T>(w.dWh_op + r * A, A, 0, w.Wa, R, 1, w.dQp, B, R, A, w.pl_dq, st));
+      continue;
     }
+    cell::BwdArgs cb{};
+    cb.dh_ext = w.dHext + r * R; cb.dh_ld = R;
+    cb.dXp = last ? nullptr : w.dXp; cb.n_p = w.pl_dx.splits; cb.p_stride = (long long)B * w.KX; cb.p_ld = w.KX; cb.col0 = H;
+    cb.dQp = last ? nullptr : w.dQp; cb.n_q = w.pl_dq.splits; cb.q_stride = (long long)B * R; cb.q_ld = R;
+    cb.dc = w.dc; cb.first = last ? 1 : 0;
+    cb.gates = w.gates + r * 4 * R;
+    cb.c_prev = w.c + r * R; cb.c_new = w.c + (size_t)(t + 1) * B * R;
+    cb.B = B; cb.H = R; cb.dG = w.dG + r * 4 * R; cb.dg_ld = 4 * R;
+    RN_TRY((cell::launch_bwd<T, T>(cb, st)));
+    RN_TRY(gemm_partials<T>(w.dG + r * 4 * R, 4 * R, 0, w.Wrec, w.KX, 1, w.dXp, B, w.KX, 4 * R, w.pl_dx, st));
+    attn::BwdArgs ab{};
+    ab.dXp = w.dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)B * w.KX; ab.p_ld = w.KX;
+    ab.V = w.Hd; ab.v_bs = H; ab.v_ts = (long long)B * H;
+    ab.Wh = w.Wh + r * A; ab.Uv = w.Uv; ab.uv_bs = A; ab.uv_ts = (long long)B * A;
+    ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = B; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = d.softmax ? 1.f : 1.f / L;
+    ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv;
+    ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc;
+    ab.dctx_out = w.dx + r * H; ab.de_out = nullptr; ab.alpha = d.softmax ? w.beta + r * L : nullptr;
+    ab.p_drop = p_drop; ab.rng = rng; ab.site = SITE_LOCAL_X; ab.drop_base = (long long)r * H;
+    RN_TRY((attn::launch_bwd<T, T>(ab, st)));
+    if (t > 0) RN_TRY(gemm_partials<T>(w.dWh_op + r * A, A, 0, w.Wa, R, 1, w.dQp, B, R, A, w.pl_dq, st));
   }
-  RN_TRY(em0.flush(w.table, w.table_bytes, w.bar, w.err, 4));
-  if (w.nch > 1) RN_TRY(cs.join(st, w.nch));
   // gradient wrt the decoder states: through U (keys) and through the weighted mean / softmax-weighted sum (values)
   RN_TRY(misc::cast_pad<T>(w.dUv, A, w.dUv_op, A, (long long)L * B, A, A, st));
   RN_TRY(gemm_full<T>(w.dUv_op, A, 0, w.U, H, 1, g_hiddens, H, nullptr, L * B, H, A, 0, w.splitk2, st));
@@ -381,11 +346,11 @@ static int local_backward_weights(const recnet_local_desc& d, const LocalWs<T>& 
 // ================================================ global ========================================================
 template <typename T>
 struct GlobalWs {
-  int nch, Bc, G;
+  int G;
   GemmPlan pl_gate, pl_dx;
   T *Wih, *Whh, *Wout; float* mp; T* Xg; float* Gx; T* X; float* P; T* gates; float* c; float* out; float* diff; float* partial;
   T* dOut; float* dHext; T* dG; T* dG2; float* dXp; float* dc; float* dXg; float* dmp; float* splitk;
-  uint8_t* table; size_t table_bytes; unsigned* bar; int* err;
+  int* err;
   float* pXP; unsigned* psync;                    // weight-resident persistent loops (seq_recon_persist.cuh)
   size_t bytes;
 };
@@ -393,7 +358,7 @@ constexpr int GMSE_THREADS = 256;
 
 template <typename T>
 static inline bool persist_global_ok(const recnet_global_desc& d, bool bwd) {
-  if (!std::is_same<T, bf16>::value || d.cell != RECNET_CELL_LSTM || num_chains(d.B) != 1) return false;
+  if (!std::is_same<T, bf16>::value || d.cell != RECNET_CELL_LSTM) return false;
   static int on = -1;
   if (on < 0) { const char* e = getenv("RECNET_PERSIST_GLOBAL"); on = e ? atoi(e) : 1; }
   if (!on) return false;
@@ -404,13 +369,10 @@ template <typename T>
 static GlobalWs<T> plan_global(const recnet_global_desc& d, void* base) {
   GlobalWs<T> w;
   const int B = d.B, L = d.L, R = d.R, H = d.H;
-  w.nch = num_chains(B);
-  w.Bc = chain_rows_max(B, w.nch);
-  const int tgt = w.nch > 1 ? NUM_SMS / 2 : NUM_SMS;
   const bool gru_ = d.cell == RECNET_CELL_GRU;
   w.G = gru_ ? 3 : 4;
-  w.pl_gate = plan_gemm<T>(w.Bc, w.G * R, R, tgt);
-  w.pl_dx = plan_gemm<T>(w.Bc, R, w.G * R, tgt);
+  w.pl_gate = plan_gemm<T>(B, w.G * R, R);
+  w.pl_dx = plan_gemm<T>(B, R, w.G * R);
   Bump m(base);
   w.Wih = m.take<T>((size_t)4 * R * 2 * H);
   w.Whh = m.take<T>((size_t)4 * R * R);
@@ -419,7 +381,7 @@ static GlobalWs<T> plan_global(const recnet_global_desc& d, void* base) {
   w.Xg = m.take<T>((size_t)L * B * 2 * H);
   w.Gx = m.take<float>((size_t)L * B * 4 * R);
   w.X = m.take<T>((size_t)(L + 1) * B * R);
-  w.P = m.take<float>((size_t)w.nch * w.pl_gate.splits * w.Bc * 4 * R);
+  w.P = m.take<float>((size_t)w.pl_gate.splits * B * 4 * R);
   w.gates = m.take<T>((size_t)L * B * 4 * R);
   w.c = m.take<float>((size_t)(L + 1) * B * R);
   w.out = m.take<float>((size_t)L * B * R);
@@ -428,15 +390,12 @@ static GlobalWs<T> plan_global(const recnet_global_desc& d, void* base) {
   w.dOut = m.take<T>((size_t)L * B * R);
   w.dHext = m.take<float>((size_t)L * B * R);
   w.dG = m.take<T>((size_t)L * B * 4 * R);
-  w.dXp = m.take<float>((size_t)w.nch * w.pl_dx.splits * w.Bc * R);
+  w.dXp = m.take<float>((size_t)w.pl_dx.splits * B * R);
   w.dc = m.take<float>((size_t)B * R);
   w.dG2 = m.take<T>(gru_ ? (size_t)L * B * 3 * R : 1);
   w.dXg = m.take<float>((size_t)L * B * 2 * H);
   w.dmp = m.take<float>((size_t)B * H);
   w.splitk = m.take<float>(SPLITK_SCRATCH_FLOATS);
-  w.table_bytes = mega::table_bytes(L);
-  w.table = m.take<uint8_t>(w.table_bytes);
-  w.bar = m.take<unsigned>(64);
   w.err = m.take<int>(64);
   {
     size_t n = 4;
@@ -493,45 +452,33 @@ static int global_forward(const recnet_global_desc& d, const recnet_global_tenso
       RN_TRY(rp::launch_local_fwd(fp, w.Whh, false, st));
     }
   }
-  Chains& cs = chains();
-  if (w.nch > 1) RN_TRY(cs.fork(st, w.nch));
-  mega::Emitter<T> em0(w.nch == 1 && !is_gru, st);
   for (int t = 0; t < L && !persist; ++t) {
-    for (int ch = 0; ch < w.nch; ++ch) {
-      int b0, nb;
-      chain_rows(B, w.nch, ch, &b0, &nb);
-      mega::Emitter<T> emc(false, w.nch > 1 ? cs.s[ch] : st);
-      mega::Emitter<T>& em = w.nch == 1 ? em0 : emc;
-      float* P = w.P + (size_t)ch * w.pl_gate.splits * w.Bc * 4 * R;
-      const size_t r = (size_t)t * B + b0;
-      T* x_t = w.X + r * R;
-      int n_p = 0;
-      if (t > 0) {
-        RN_TRY(em.gemm_partials(x_t, R, 0, w.Whh, R, 0, P, nb, GR, R, w.pl_gate));
-        n_p = w.pl_gate.splits;
-      }
-      if (is_gru) {
-        gru::FwdArgs ga{};
-        ga.Px = nullptr; ga.n_px = 0;
-        ga.Ph = n_p ? P : nullptr; ga.n_ph = n_p; ga.ph_stride = (long long)nb * 3 * R; ga.ph_ld = 3 * R;
-        ga.Gx = w.Gx + r * 3 * R; ga.gx_ld = 3 * R; ga.b_ih = nullptr; ga.b_hh = p.b_hh;
-        ga.h_prev = w.c + r * R; ga.hp_ld = R; ga.B = nb; ga.H = R;
-        ga.stash = w.gates + r * 4 * R; ga.h_out = w.c + ((size_t)(t + 1) * B + b0) * R; ga.h_ld = R;
-        ga.h_op = x_t + (size_t)B * R; ga.hop_ld = R;
-        RN_TRY((gru::launch_fwd<T, T>(ga, em.st)));
-        continue;
-      }
-      cell::FwdArgs ca{};
-      ca.P = P; ca.n_p = n_p; ca.p_stride = (long long)nb * 4 * R; ca.p_ld = 4 * R;
-      ca.Gx = w.Gx + r * 4 * R; ca.gx_ld = 4 * R; ca.b1 = nullptr; ca.b2 = p.b_hh;
-      ca.c_prev = w.c + r * R; ca.B = nb; ca.H = R;
-      ca.gates_out = w.gates + r * 4 * R; ca.c_out = w.c + ((size_t)(t + 1) * B + b0) * R; ca.h_out = nullptr;
-      ca.h_op = x_t + (size_t)B * R; ca.hop_ld = R; ca.h_op2 = nullptr;
-      RN_TRY(em.cell_fwd(ca));
+    const size_t r = (size_t)t * B;
+    T* x_t = w.X + r * R;
+    int n_p = 0;
+    if (t > 0) {
+      RN_TRY(gemm_partials<T>(x_t, R, 0, w.Whh, R, 0, w.P, B, GR, R, w.pl_gate, st));
+      n_p = w.pl_gate.splits;
     }
+    if (is_gru) {
+      gru::FwdArgs ga{};
+      ga.Px = nullptr; ga.n_px = 0;
+      ga.Ph = n_p ? w.P : nullptr; ga.n_ph = n_p; ga.ph_stride = (long long)B * 3 * R; ga.ph_ld = 3 * R;
+      ga.Gx = w.Gx + r * 3 * R; ga.gx_ld = 3 * R; ga.b_ih = nullptr; ga.b_hh = p.b_hh;
+      ga.h_prev = w.c + r * R; ga.hp_ld = R; ga.B = B; ga.H = R;
+      ga.stash = w.gates + r * 4 * R; ga.h_out = w.c + (size_t)(t + 1) * B * R; ga.h_ld = R;
+      ga.h_op = x_t + (size_t)B * R; ga.hop_ld = R;
+      RN_TRY((gru::launch_fwd<T, T>(ga, st)));
+      continue;
+    }
+    cell::FwdArgs ca{};
+    ca.P = w.P; ca.n_p = n_p; ca.p_stride = (long long)B * 4 * R; ca.p_ld = 4 * R;
+    ca.Gx = w.Gx + r * 4 * R; ca.gx_ld = 4 * R; ca.b1 = nullptr; ca.b2 = p.b_hh;
+    ca.c_prev = w.c + r * R; ca.B = B; ca.H = R;
+    ca.gates_out = w.gates + r * 4 * R; ca.c_out = w.c + (size_t)(t + 1) * B * R; ca.h_out = nullptr;
+    ca.h_op = x_t + (size_t)B * R; ca.hop_ld = R; ca.h_op2 = nullptr;
+    RN_TRY((cell::launch_fwd<T, T>(ca, st)));
   }
-  RN_TRY(em0.flush(w.table, w.table_bytes, w.bar, w.err, 5));
-  if (w.nch > 1) RN_TRY(cs.join(st, w.nch));
   RN_TRY(gemm_full<T>(w.X + (size_t)B * R, R, 0, w.Wout, R, 0, w.out, R, p.out_b, L * B, R, R, 0, w.splitk, st));
   if (loss_out) {
     const int nb = rn_cdiv((long long)B * R, GMSE_THREADS);
@@ -559,8 +506,6 @@ static int global_backward(const recnet_global_desc& d, const recnet_global_tens
   RN_TRY(gemm_full<T>(w.dOut, R, 0, w.Wout, R, 1, w.dHext, R, nullptr, LB, R, R, 0, w.splitk, st));
   RN_TRY(gemm_full<T>(w.dOut, R, 1, w.X + (size_t)B * R, R, 1, g.out_w, R, nullptr, R, R, LB, 0, w.splitk, st));
   RN_TRY(misc::colsum<T>(w.dOut, R, LB, R, g.out_b, 0, w.splitk, st));
-  Chains& cs = chains();
-  if (w.nch > 1) RN_TRY(cs.fork(st, w.nch));
   const bool is_gru = d.cell == RECNET_CELL_GRU;
   const int GR = w.G * R;
   bool persist = false;
@@ -574,40 +519,30 @@ static int global_backward(const recnet_global_desc& d, const recnet_global_tens
       RN_TRY(rp::launch_local_bwd(bp, w.Whh, st));
     }
   }
-  mega::Emitter<T> em0(w.nch == 1 && !is_gru, st);
   for (int t = L - 1; t >= 0 && !persist; --t) {
     const bool last = (t == L - 1);
-    for (int ch = 0; ch < w.nch; ++ch) {
-      int b0, nb;
-      chain_rows(B, w.nch, ch, &b0, &nb);
-      mega::Emitter<T> emc(false, w.nch > 1 ? cs.s[ch] : st);
-      mega::Emitter<T>& em = w.nch == 1 ? em0 : emc;
-      float* dXp = w.dXp + (size_t)ch * w.pl_dx.splits * w.Bc * R;
-      const size_t r = (size_t)t * B + b0;
-      if (is_gru) {
-        gru::BwdArgs gb{};
-        gb.dh_ext = w.dHext + r * R; gb.dh_ld = R;
-        gb.dHp = last ? nullptr : dXp; gb.n_p = w.pl_dx.splits; gb.p_stride = (long long)nb * R; gb.p_ld = R;
-        gb.dQp = nullptr; gb.carry = w.dc + (size_t)b0 * R; gb.first = last ? 1 : 0;
-        gb.stash = w.gates + r * 4 * R; gb.h_prev = w.c + r * R; gb.hp_ld = R;
-        gb.B = nb; gb.H = R; gb.dGi = w.dG + r * 3 * R; gb.dGh = w.dG2 + r * 3 * R; gb.dg_ld = 3 * R;
-        RN_TRY((gru::launch_bwd<T, T>(gb, em.st)));
-        if (t > 0) RN_TRY(em.gemm_partials(w.dG2 + r * 3 * R, 3 * R, 0, w.Whh, R, 1, dXp, nb, R, 3 * R, w.pl_dx));
-        continue;
-      }
-      cell::BwdArgs cb{};
-      cb.dh_ext = w.dHext + r * R; cb.dh_ld = R;
-      cb.dXp = last ? nullptr : dXp; cb.n_p = w.pl_dx.splits; cb.p_stride = (long long)nb * R; cb.p_ld = R; cb.col0 = 0;
-      cb.dQp = nullptr; cb.dc = w.dc + (size_t)b0 * R; cb.first = last ? 1 : 0;
-      cb.gates = w.gates + r * 4 * R;
-      cb.c_prev = w.c + r * R; cb.c_new = w.c + ((size_t)(t + 1) * B + b0) * R;
-      cb.B = nb; cb.H = R; cb.dG = w.dG + r * 4 * R; cb.dg_ld = 4 * R;
-      RN_TRY(em.cell_bwd(cb));
-      if (t > 0) RN_TRY(em.gemm_partials(w.dG + r * 4 * R, 4 * R, 0, w.Whh, R, 1, dXp, nb, R, 4 * R, w.pl_dx));
+    const size_t r = (size_t)t * B;
+    if (is_gru) {
+      gru::BwdArgs gb{};
+      gb.dh_ext = w.dHext + r * R; gb.dh_ld = R;
+      gb.dHp = last ? nullptr : w.dXp; gb.n_p = w.pl_dx.splits; gb.p_stride = (long long)B * R; gb.p_ld = R;
+      gb.dQp = nullptr; gb.carry = w.dc; gb.first = last ? 1 : 0;
+      gb.stash = w.gates + r * 4 * R; gb.h_prev = w.c + r * R; gb.hp_ld = R;
+      gb.B = B; gb.H = R; gb.dGi = w.dG + r * 3 * R; gb.dGh = w.dG2 + r * 3 * R; gb.dg_ld = 3 * R;
+      RN_TRY((gru::launch_bwd<T, T>(gb, st)));
+      if (t > 0) RN_TRY(gemm_partials<T>(w.dG2 + r * 3 * R, 3 * R, 0, w.Whh, R, 1, w.dXp, B, R, 3 * R, w.pl_dx, st));
+      continue;
     }
+    cell::BwdArgs cb{};
+    cb.dh_ext = w.dHext + r * R; cb.dh_ld = R;
+    cb.dXp = last ? nullptr : w.dXp; cb.n_p = w.pl_dx.splits; cb.p_stride = (long long)B * R; cb.p_ld = R; cb.col0 = 0;
+    cb.dQp = nullptr; cb.dc = w.dc; cb.first = last ? 1 : 0;
+    cb.gates = w.gates + r * 4 * R;
+    cb.c_prev = w.c + r * R; cb.c_new = w.c + (size_t)(t + 1) * B * R;
+    cb.B = B; cb.H = R; cb.dG = w.dG + r * 4 * R; cb.dg_ld = 4 * R;
+    RN_TRY((cell::launch_bwd<T, T>(cb, st)));
+    if (t > 0) RN_TRY(gemm_partials<T>(w.dG + r * 4 * R, 4 * R, 0, w.Whh, R, 1, w.dXp, B, R, 4 * R, w.pl_dx, st));
   }
-  RN_TRY(em0.flush(w.table, w.table_bytes, w.bar, w.err, 6));
-  if (w.nch > 1) RN_TRY(cs.join(st, w.nch));
   const T* dGh = is_gru ? w.dG2 : w.dG;
   RN_TRY(misc::colsum<T>(w.dG, GR, LB, GR, g.b_ih, 0, w.splitk, st));
   if (is_gru) { RN_TRY(misc::colsum<T>(dGh, GR, LB, GR, g.b_hh, 0, w.splitk, st)); }

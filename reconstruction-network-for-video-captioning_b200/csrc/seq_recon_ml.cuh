@@ -35,7 +35,6 @@ static int local_forward_ml(const LocalDesc& d, const recnet_local_tensors& p, c
   RN_CUDA_OK(cudaMemsetAsync(w.X, 0, (size_t)B * w.KX * sizeof(T), st));
   RN_CUDA_OK(cudaMemsetAsync(w.c, 0, (size_t)B * R * sizeof(float), st));
   RN_CUDA_OK(cudaMemsetAsync(w.err, 0, sizeof(int), st));
-  mega::Emitter<T> em(false, st);
   int n_whp = 0;
   for (int t = 0; t < S; ++t) {
     for (int l = 0; l < NLd; ++l) {
@@ -45,7 +44,7 @@ static int local_forward_ml(const LocalDesc& d, const recnet_local_tensors& p, c
       if (l == 0) {
         n_whp = 0;
         if (t > 0) {      // ONE query per outer step: the state before the pseudo-steps
-          RN_TRY(em.gemm_partials(x_q + H, w.KX, 0, w.Wa, R, 0, w.WhP, B, A, R, w.pl_wh));
+          RN_TRY(gemm_partials<T>(x_q + H, w.KX, 0, w.Wa, R, 0, w.WhP, B, A, R, w.pl_wh, st));
           n_whp = w.pl_wh.splits;
         }
       }
@@ -57,15 +56,15 @@ static int local_forward_ml(const LocalDesc& d, const recnet_local_tensors& p, c
       fa.B = B; fa.Tn = L; fa.A = A; fa.D = H; fa.inv_T = d.softmax ? 1.f : 1.f / L; fa.normalize = d.softmax;   // softmax per layer
       fa.Wh_out = w.Wh + q * B * A; fa.e_out = w.beta + q * B * L; fa.ctx_out = x_q; fa.ctx_ld = w.KX;
       fa.p_drop = p_drop; fa.rng = rng; fa.site = SITE_LOCAL_X; fa.drop_base = (long long)q * B * H;
-      RN_TRY(em.attn_fwd(fa));
-      RN_TRY(em.gemm_partials(x_q, w.KX, 0, w.Wrec, w.KX, 0, w.P, B, 4 * R, w.KX, w.pl_gate));
+      RN_TRY((attn::launch_fwd<T, T>(fa, st)));
+      RN_TRY(gemm_partials<T>(x_q, w.KX, 0, w.Wrec, w.KX, 0, w.P, B, 4 * R, w.KX, w.pl_gate, st));
       cell::FwdArgs ca{};
       ca.P = w.P; ca.n_p = w.pl_gate.splits; ca.p_stride = (long long)B * 4 * R; ca.p_ld = 4 * R;
       ca.b1 = p.b_ih; ca.b2 = p.b_hh; ca.c_prev = w.c + q * B * R; ca.B = B; ca.H = R;
       ca.gates_out = w.gates + q * B * 4 * R; ca.c_out = w.c + (q + 1) * B * R;
       ca.h_op = x_n + H; ca.hop_ld = w.KX;
       if (l == 0) { ca.h_op2 = w.Hout + (size_t)t * B * R; ca.hop2_ld = R; }                       // `output[0]`
-      RN_TRY(em.cell_fwd(ca));
+      RN_TRY((cell::launch_fwd<T, T>(ca, st)));
     }
   }
   // query-state rows (state at the start of every outer step) for the attn_W gradient
@@ -98,7 +97,6 @@ static int local_backward_ml(const LocalDesc& d, const recnet_local_tensors& p, 
   RN_TRY(gemm_full<T>(w.dOut, R, 0, w.Wout, R, 1, w.dHext, R, nullptr, SB, R, R, 0, w.splitk, st));
   RN_TRY(gemm_full<T>(w.dOut, R, 1, w.Hout, R, 1, g.out_w, R, nullptr, R, R, SB, 0, w.splitk, st));
   RN_TRY(misc::colsum<T>(w.dOut, R, SB, R, g.out_b, 0, w.splitk, st));
-  mega::Emitter<T> em(false, st);
   for (int q = Sp - 1; q >= 0; --q) {
     const int t = q / NLd, l = q % NLd;
     const bool last = (q == Sp - 1);
@@ -112,8 +110,8 @@ static int local_backward_ml(const LocalDesc& d, const recnet_local_tensors& p, 
     cb.gates = w.gates + (size_t)q * B * 4 * R;
     cb.c_prev = w.c + (size_t)q * B * R; cb.c_new = w.c + (size_t)(q + 1) * B * R;
     cb.B = B; cb.H = R; cb.dG = w.dG + (size_t)q * B * 4 * R; cb.dg_ld = 4 * R;
-    RN_TRY(em.cell_bwd(cb));
-    RN_TRY(em.gemm_partials(w.dG + (size_t)q * B * 4 * R, 4 * R, 0, w.Wrec, w.KX, 1, w.dXp, B, w.KX, 4 * R, w.pl_dx));
+    RN_TRY((cell::launch_bwd<T, T>(cb, st)));
+    RN_TRY(gemm_partials<T>(w.dG + (size_t)q * B * 4 * R, 4 * R, 0, w.Wrec, w.KX, 1, w.dXp, B, w.KX, 4 * R, w.pl_dx, st));
     attn::BwdArgs ab{};
     ab.dXp = w.dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)B * w.KX; ab.p_ld = w.KX;
     ab.V = w.Hd + (size_t)l * B * H; ab.v_bs = H; ab.v_ts = (long long)NLd * B * H;
@@ -126,8 +124,8 @@ static int local_backward_ml(const LocalDesc& d, const recnet_local_tensors& p, 
     ab.dw_acc = w.dw_acc; ab.dw_first = last ? 1 : 0;
     ab.dctx_out = w.dx + (size_t)q * B * H;
     ab.p_drop = p_drop; ab.rng = rng; ab.site = SITE_LOCAL_X; ab.drop_base = (long long)q * B * H;
-    RN_TRY(em.attn_bwd(ab));
-    if (l == 0 && t > 0) RN_TRY(em.gemm_partials(w.dWh_op + (size_t)t * B * A, A, 0, w.Wa, R, 1, w.dQp, B, R, A, w.pl_dq));
+    RN_TRY((attn::launch_bwd<T, T>(ab, st)));
+    if (l == 0 && t > 0) RN_TRY(gemm_partials<T>(w.dWh_op + (size_t)t * B * A, A, 0, w.Wa, R, 1, w.dQp, B, R, A, w.pl_dq, st));
   }
   const int SpB = Sp * B;
   RN_TRY(misc::colsum<T>(w.dG, 4 * R, SpB, 4 * R, g.b_ih, 0, w.splitk, st));

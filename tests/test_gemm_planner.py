@@ -1,4 +1,4 @@
-"""The tile / split-K plan of the batched GEMMs (csrc/runtime.cuh:plan_gemm_full_bf16) is host code: pin its decisions for the shapes of the
+"""The tile / split-K plan of the batched GEMMs (csrc/runtime.cuh:plan_gemm_full<bf16>) is host code: pin its decisions for the shapes of the
 MSVD train step to what the sweeps on the B200 found best (profiles/r2_h_gemm_sweep.md, r1_g_gemm_sweep.md).  No GPU needed."""
 import ctypes as C
 
