@@ -31,8 +31,7 @@ __device__ __forceinline__ float4 sum_partials4(const float* __restrict__ q, int
 }
 
 static inline bool lean_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("RECNET_LEAN_ATTN"); v = e ? atoi(e) : 1; }
+  static const int v = rn_env_int("RECNET_LEAN_ATTN", 1);
   return v != 0;
 }
 

@@ -65,6 +65,13 @@ struct ProfScope {
 
 static inline int rn_cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 
+// The RECNET_* environment switches (INTEGRATION.md) are read through this: the integer value of `name`, or `dflt` when it is unset.
+// The call sites keep the value in a function-local `static const`, so each switch is read once per process.
+inline int rn_env_int(const char* name, int dflt) {
+  const char* e = getenv(name);
+  return e ? atoi(e) : dflt;
+}
+
 // ---- type conversion -------------------------------------------------------------------------
 // Upper bound on the CTAs of ONE launch of the batched kernels (0 = none): set by a trainer around work it runs on a second stream UNDERNEATH a
 // latency-bound foreground kernel sequence (recnet_set_background_ctas; functional.py "background lane").  Persistent GEMMs, split-K plans and the
@@ -160,8 +167,7 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 __device__ __forceinline__ void pdl_launch_next() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 inline bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("RECNET_PDL"); v = e ? atoi(e) : 0; }   // measured: 4.53 ms/step with PDL vs 4.14 without -> opt-in
+  static const int v = rn_env_int("RECNET_PDL", 0);   // measured: 4.53 ms/step with PDL vs 4.14 without -> opt-in
   return v != 0;
 }
 // launch with the programmatic-stream-serialization attribute (falls back to a plain launch when RECNET_PDL=0)

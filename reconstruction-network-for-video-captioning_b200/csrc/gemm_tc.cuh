@@ -368,8 +368,7 @@ static inline int launch(const bf16* A, long long lda, int transA, const bf16* B
   if (bias && (reinterpret_cast<uintptr_t>(bias) & 15)) ep.vec_ok = 0;
   // short K loops (the per-step split-K GEMMs) use a shallow ring (<= 97 KB smem) so that two CTAs share an SM; long K
   // loops (batched GEMMs) use the deep ring.
-  static int shallow_kb = -1;
-  if (shallow_kb < 0) { const char* e = getenv("RECNET_GEMM_SHALLOW_KB"); shallow_kb = e ? atoi(e) : 12; }
+  static const int shallow_kb = rn_env_int("RECNET_GEMM_SHALLOW_KB", 12);
   const bool shallow = kb_per <= shallow_kb;
   if (BN == 64) return shallow ? launch_bn<64, 4>(transA, transB, ma, mb, ep, M, N, K, splits, kb_per, st)
                                : launch_bn<64, 8>(transA, transB, ma, mb, ep, M, N, K, splits, kb_per, st);

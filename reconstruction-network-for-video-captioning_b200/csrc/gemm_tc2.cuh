@@ -314,8 +314,6 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
 }
 
 // ---- host side -----------------------------------------------------------------------------------
-inline int& background_ctas() { return rn_background_ctas(); }       // common.cuh
-
 // output tensor [rows, cols] row-major (ld elements): fp32 boxes of 32 x 32, bf16 boxes of 32 rows x 64 columns -- 128-byte rows
 static inline int make_out_map(CUtensorMap* map, const void* ptr, long long rows, long long cols, long long ld, bool is_bf16) {
   tc::EncodeTiledFn enc = tc::get_encode_fn();
@@ -352,7 +350,7 @@ static int launch_cfg(const CUtensorMap& ma, const CUtensorMap& mb, const CUtens
   }
   const int tiles_m = rn_cdiv(M, BM * CTAS), tiles_n = rn_cdiv(N, BN);
   int units = min(tiles_m * tiles_n, TC2_SMS / CTAS);
-  if (background_ctas() > 0) units = min(units, max(1, background_ctas() / CTAS));
+  if (rn_background_ctas() > 0) units = min(units, max(1, rn_background_ctas() / CTAS));
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(units * CTAS);
   cfg.blockDim = dim3(THREADS);

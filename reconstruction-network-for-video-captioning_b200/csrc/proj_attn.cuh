@@ -596,8 +596,7 @@ template <typename TV, typename TO, bool SM = false>
 static int launch_fwd(const FwdArgs& a, cudaStream_t st) {
   RN_TRY(check_shape(a.Tn, a.A, a.H));
   ProfScope prof(KC_PF_FWD, a.B, a.Tn, a.H, st);
-  static int minb = -1;
-  if (minb < 0) { const char* e = getenv("RECNET_PF_MINB"); minb = e ? atoi(e) : 3; }
+  static const int minb = rn_env_int("RECNET_PF_MINB", 3);
   const dim3 grid(rn_cdiv(a.H, UPB), a.B);
   if (a.A <= 128 && minb == 3) RN_CUDA_OK(launch_pdl(pf_fwd_kernel<TV, TO, 1, 3, SM>, grid, dim3(THREADS), 0, st, a));
   else if (a.A <= 128) RN_CUDA_OK(launch_pdl(pf_fwd_kernel<TV, TO, 1, 2, SM>, grid, dim3(THREADS), 0, st, a));

@@ -10,16 +10,43 @@
 
 #define ST(s) reinterpret_cast<cudaStream_t>(s)
 
-// The public descriptors carry RECNET_ATTN_SOFTMAX in their `cell` field; every entry point splits it off here, once.
+// f(float{}) or f(bf16{}) by precision -- the generic lambda takes `using T = decltype(t)` -- and `bad` for any other precision.
+template <typename R, typename F>
+static R by_prec(int precision, R bad, F&& f) {
+  if (precision == RECNET_PREC_FP32) return f(float{});
+  if (precision == RECNET_PREC_BF16) return f(bf16{});
+  return bad;
+}
+
+// Every entry point that takes a descriptor checks it here: a null descriptor is RECNET_ERR_BAD_SHAPE, an unknown precision
+// RECNET_ERR_UNSUPPORTED (the pointer accessors return nullptr for both).
+template <typename Pub>
+static int check_desc(const Pub* d) {
+  if (!d) return RECNET_ERR_BAD_SHAPE;
+  return by_prec<int>(d->precision, RECNET_ERR_UNSUPPORTED, [](auto) { return 0; });
+}
+// The decoder and local descriptors also carry RECNET_ATTN_SOFTMAX in their `cell` field; it is split off here, once.
 template <typename Pub, typename Int>
 static int split_desc(const Pub* d, Int* out) {
-  if (!d) return RECNET_ERR_BAD_SHAPE;
+  RN_TRY(check_desc(d));
   static_cast<Pub&>(*out) = *d;
   const int32_t flags = d->cell & ~RECNET_CELL_MASK;
   if (flags & ~RECNET_ATTN_SOFTMAX) return RECNET_ERR_UNSUPPORTED;
   out->cell = d->cell & RECNET_CELL_MASK;
   out->softmax = flags != 0;
   return 0;
+}
+
+// The workspace layout of the decoder's training drivers: the projected-feature plan, or the general plan (which the stacked driver shares).
+struct DecLayout { int64_t bytes; float* logits; int64_t ld; int* err; };
+template <typename T>
+static DecLayout dec_layout(const DecDesc& dd, void* base) {
+  if (dec::dec_path(dd) == dec::DecPath::PF) {
+    const auto w = dec::plan_pf<T>(dd, base);
+    return {(int64_t)w.bytes, w.logits, w.Vld, w.err};
+  }
+  const auto w = dec::plan<T>(dd, base);
+  return {(int64_t)w.bytes, w.logits, w.Vld, w.err};
 }
 
 extern "C" {
@@ -94,16 +121,18 @@ int recnet_query_device(int device, int* sm_count, int* cc_major, int* cc_minor)
 int recnet_gemm(int precision, const void* A, int64_t lda, int transA, const void* B, int64_t ldb, int transB, float* C,
                 int64_t ldc, void* c_op, int64_t ldc_op, const float* bias, int M, int N, int K, int splits,
                 int64_t split_stride, int accumulate, int bn_hint, void* stream) {
-  if (precision == RECNET_PREC_FP32) {
-    if (c_op) return RECNET_ERR_UNSUPPORTED;
-    return sg::launch(reinterpret_cast<const float*>(A), lda, transA, reinterpret_cast<const float*>(B), ldb, transB, C, ldc,
-                      bias, M, N, K, splits, split_stride, accumulate, ST(stream));
-  }
-  if (precision == RECNET_PREC_BF16)
-    return tc::launch(reinterpret_cast<const bf16*>(A), lda, transA, reinterpret_cast<const bf16*>(B), ldb, transB, C, ldc,
-                      reinterpret_cast<bf16*>(c_op), ldc_op, bias, M, N, K, splits, split_stride, accumulate, bn_hint,
-                      ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(precision, RECNET_ERR_UNSUPPORTED, [&](auto t) -> int {
+    using T = decltype(t);
+    if constexpr (std::is_same<T, float>::value) {
+      if (c_op) return RECNET_ERR_UNSUPPORTED;
+      return sg::launch(reinterpret_cast<const float*>(A), lda, transA, reinterpret_cast<const float*>(B), ldb, transB, C, ldc,
+                        bias, M, N, K, splits, split_stride, accumulate, ST(stream));
+    } else {
+      return tc::launch(reinterpret_cast<const bf16*>(A), lda, transA, reinterpret_cast<const bf16*>(B), ldb, transB, C, ldc,
+                        reinterpret_cast<bf16*>(c_op), ldc_op, bias, M, N, K, splits, split_stride, accumulate, bn_hint,
+                        ST(stream));
+    }
+  });
 }
 
 int recnet_plan_persistent_loops(const recnet_local_desc* d, int32_t* out) {
@@ -113,13 +142,13 @@ int recnet_plan_persistent_loops(const recnet_local_desc* d, int32_t* out) {
   for (int i = 0; i < 12; ++i) out[i] = 0;
   LocalDesc dd;
   RN_TRY(split_desc(d, &dd));            // both attention variants have persistent loops
+  if (dd.precision != RECNET_PREC_BF16) return 0;
   const rp::Shape s{dd.B, dd.S, dd.R, dd.H, dd.A, dd.L};
-  const bool lstm_bf16 = dd.precision == RECNET_PREC_BF16 && dd.cell == RECNET_CELL_LSTM && dd.dec_layers <= 1;
-  if (lstm_bf16 && rp::local_fwd_ok(s)) {
+  if (rec::persist_fwd_ok<bf16>(dd)) {
     const int ks = rp::pick_ks(s.R, s.H), res = rp::max_res_kb_fwd(s.R, s.H, ks);
     out[0] = 1; out[1] = ks; out[2] = s.R / rp::UNITS; out[3] = res; out[4] = rp::pick_stages_fwd(s.B, ks, res); out[5] = out[2] * ks;
   }
-  if (lstm_bf16 && rp::local_bwd_ok(s)) {
+  if (rec::persist_bwd_ok<bf16>(dd)) {
     const int ns = rp::pick_ns(s.R, s.H), res = (4 * s.R / rp::BK + ns - 1) / ns;
     out[6] = 1; out[7] = ns; out[8] = (s.R + s.H) / 128; out[9] = res; out[10] = rp::pick_stages_bwd(s.B, res); out[11] = out[8] * ns;
   }
@@ -146,25 +175,30 @@ int recnet_attn_fwd(int precision, const float* wh_partials, int n_wh, int64_t w
   a.attn_b = attn_b; a.attn_w = attn_w; a.V = v; a.v_bs = v_bs; a.v_ts = v_ts; a.B = B; a.Tn = Tn; a.A = A; a.D = D;
   a.inv_T = 1.f / Tn; a.normalize = normalize; a.Wh_out = wh_out; a.e_out = e_out; a.ctx_out = ctx_out; a.ctx_ld = ctx_ld;
   a.p_drop = p_drop; a.rng = reinterpret_cast<const unsigned long long*>(rng); a.site = site; a.drop_base = drop_base;
-  if (precision == RECNET_PREC_FP32) return attn::launch_fwd<float, float>(a, ST(stream));
-  if (precision == RECNET_PREC_BF16) return attn::launch_fwd<bf16, bf16>(a, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(precision, RECNET_ERR_UNSUPPORTED, [&](auto t) { using T = decltype(t); return attn::launch_fwd<T, T>(a, ST(stream)); });
 }
 
+// the backward of both attention variants: the reference's mean (alpha = nullptr, context scaled by 1/Tn) and the softmax (alpha, scale 1)
+static int attn_bwd(int precision, const float* dctx_partials, int n_p, int64_t p_stride, int64_t p_ld, const void* v, int64_t v_bs,
+                    int64_t v_ts, const float* alpha, float inv_T, const float* wh, const float* uv, int64_t uv_bs, int64_t uv_ts,
+                    const float* attn_b, const float* attn_w, int B, int Tn, int A, int D, float* dwh_out, void* dwh_op, float* duv_acc,
+                    float* dw_acc, int first, float* dctx_out, float p_drop, const uint64_t* rng, uint32_t site, int64_t drop_base,
+                    void* stream) {
+  attn::BwdArgs a{};
+  a.dXp = dctx_partials; a.n_p = n_p; a.p_stride = p_stride; a.p_ld = p_ld; a.V = v; a.v_bs = v_bs; a.v_ts = v_ts;
+  a.Wh = wh; a.Uv = uv; a.uv_bs = uv_bs; a.uv_ts = uv_ts; a.attn_b = attn_b; a.attn_w = attn_w; a.B = B; a.Tn = Tn; a.A = A;
+  a.D = D; a.inv_T = inv_T; a.dWh_out = dwh_out; a.dWh_op = dwh_op; a.dUv_acc = duv_acc; a.uv_first = first; a.dw_first = first; a.dw_acc = dw_acc;
+  a.dctx_out = dctx_out; a.de_out = nullptr; a.alpha = alpha; a.p_drop = p_drop; a.rng = reinterpret_cast<const unsigned long long*>(rng);
+  a.site = site; a.drop_base = drop_base;
+  return by_prec<int>(precision, RECNET_ERR_UNSUPPORTED, [&](auto t) { using T = decltype(t); return attn::launch_bwd<T, T>(a, ST(stream)); });
+}
 int recnet_attn_bwd(int precision, const float* dctx_partials, int n_p, int64_t p_stride, int64_t p_ld, const void* v,
                     int64_t v_bs, int64_t v_ts, const float* wh, const float* uv, int64_t uv_bs, int64_t uv_ts,
                     const float* attn_b, const float* attn_w, int B, int Tn, int A, int D, float* dwh_out, void* dwh_op,
                     float* duv_acc, float* dw_acc, int first, float* dctx_out, float p_drop, const uint64_t* rng,
                     uint32_t site, int64_t drop_base, void* stream) {
-  attn::BwdArgs a{};
-  a.dXp = dctx_partials; a.n_p = n_p; a.p_stride = p_stride; a.p_ld = p_ld; a.V = v; a.v_bs = v_bs; a.v_ts = v_ts;
-  a.Wh = wh; a.Uv = uv; a.uv_bs = uv_bs; a.uv_ts = uv_ts; a.attn_b = attn_b; a.attn_w = attn_w; a.B = B; a.Tn = Tn; a.A = A;
-  a.D = D; a.inv_T = 1.f / Tn; a.dWh_out = dwh_out; a.dWh_op = dwh_op; a.dUv_acc = duv_acc; a.uv_first = first; a.dw_first = first; a.dw_acc = dw_acc;
-  a.dctx_out = dctx_out; a.de_out = nullptr; a.p_drop = p_drop; a.rng = reinterpret_cast<const unsigned long long*>(rng);
-  a.site = site; a.drop_base = drop_base;
-  if (precision == RECNET_PREC_FP32) return (attn::launch_bwd<float, float>(a, ST(stream)));
-  if (precision == RECNET_PREC_BF16) return (attn::launch_bwd<bf16, bf16>(a, ST(stream)));
-  return RECNET_ERR_UNSUPPORTED;
+  return attn_bwd(precision, dctx_partials, n_p, p_stride, p_ld, v, v_bs, v_ts, nullptr, 1.f / Tn, wh, uv, uv_bs, uv_ts, attn_b, attn_w,
+                  B, Tn, A, D, dwh_out, dwh_op, duv_acc, dw_acc, first, dctx_out, p_drop, rng, site, drop_base, stream);
 }
 
 int recnet_attn_bwd_softmax(int precision, const float* dctx_partials, int n_p, int64_t p_stride, int64_t p_ld, const void* v,
@@ -173,15 +207,8 @@ int recnet_attn_bwd_softmax(int precision, const float* dctx_partials, int n_p, 
                             void* dwh_op, float* duv_acc, float* dw_acc, int first, float* dctx_out, float p_drop,
                             const uint64_t* rng, uint32_t site, int64_t drop_base, void* stream) {
   if (!alpha) return RECNET_ERR_BAD_SHAPE;
-  attn::BwdArgs a{};
-  a.dXp = dctx_partials; a.n_p = n_p; a.p_stride = p_stride; a.p_ld = p_ld; a.V = v; a.v_bs = v_bs; a.v_ts = v_ts;
-  a.Wh = wh; a.Uv = uv; a.uv_bs = uv_bs; a.uv_ts = uv_ts; a.attn_b = attn_b; a.attn_w = attn_w; a.B = B; a.Tn = Tn; a.A = A;
-  a.D = D; a.inv_T = 1.f; a.dWh_out = dwh_out; a.dWh_op = dwh_op; a.dUv_acc = duv_acc; a.uv_first = first; a.dw_first = first; a.dw_acc = dw_acc;
-  a.dctx_out = dctx_out; a.de_out = nullptr; a.alpha = alpha; a.p_drop = p_drop; a.rng = reinterpret_cast<const unsigned long long*>(rng);
-  a.site = site; a.drop_base = drop_base;
-  if (precision == RECNET_PREC_FP32) return (attn::launch_bwd<float, float>(a, ST(stream)));
-  if (precision == RECNET_PREC_BF16) return (attn::launch_bwd<bf16, bf16>(a, ST(stream)));
-  return RECNET_ERR_UNSUPPORTED;
+  return attn_bwd(precision, dctx_partials, n_p, p_stride, p_ld, v, v_bs, v_ts, alpha, 1.f, wh, uv, uv_bs, uv_ts, attn_b, attn_w,
+                  B, Tn, A, D, dwh_out, dwh_op, duv_acc, dw_acc, first, dctx_out, p_drop, rng, site, drop_base, stream);
 }
 
 int recnet_lstm_cell_fwd(int precision, const float* partials, int n_p, int64_t p_stride, int64_t p_ld, const float* gx,
@@ -192,9 +219,7 @@ int recnet_lstm_cell_fwd(int precision, const float* partials, int n_p, int64_t 
   a.P = partials; a.n_p = n_p; a.p_stride = p_stride; a.p_ld = p_ld; a.Gx = gx; a.gx_ld = gx_ld; a.b1 = b1; a.b2 = b2;
   a.c_prev = c_prev; a.B = B; a.H = H; a.gates_out = gates_out; a.c_out = c_out; a.h_out = h_out; a.h_ld = h_ld;
   a.h_op = h_op; a.hop_ld = hop_ld; a.h_op2 = h_op2; a.hop2_ld = hop2_ld;
-  if (precision == RECNET_PREC_FP32) return cell::launch_fwd<float, float>(a, ST(stream));
-  if (precision == RECNET_PREC_BF16) return cell::launch_fwd<bf16, bf16>(a, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(precision, RECNET_ERR_UNSUPPORTED, [&](auto t) { using T = decltype(t); return cell::launch_fwd<T, T>(a, ST(stream)); });
 }
 
 int recnet_lstm_cell_bwd(int precision, const float* dh_ext, int64_t dh_ld, const float* dh_scale, const float* dh_ext2,
@@ -205,9 +230,7 @@ int recnet_lstm_cell_bwd(int precision, const float* dh_ext, int64_t dh_ld, cons
   a.dh_ext = dh_ext; a.dh_ld = dh_ld; a.dh_scale = dh_scale; a.dh_ext2 = dh_ext2; a.dh2_ld = dh2_ld; a.dXp = dxp; a.n_p = n_p;
   a.p_stride = p_stride; a.p_ld = p_ld; a.col0 = col0; a.dQp = dqp; a.n_q = n_q; a.q_stride = q_stride; a.q_ld = q_ld; a.dc = dc; a.first = first; a.gates = gates;
   a.c_prev = c_prev; a.c_new = c_new; a.B = B; a.H = H; a.dG = dg_out; a.dg_ld = dg_ld;
-  if (precision == RECNET_PREC_FP32) return cell::launch_bwd<float, float>(a, ST(stream));
-  if (precision == RECNET_PREC_BF16) return cell::launch_bwd<bf16, bf16>(a, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(precision, RECNET_ERR_UNSUPPORTED, [&](auto t) { using T = decltype(t); return cell::launch_bwd<T, T>(a, ST(stream)); });
 }
 
 int recnet_gru_cell_fwd(int precision, const float* px, int n_px, int64_t px_stride, int64_t px_ld, const float* ph, int n_ph,
@@ -218,9 +241,7 @@ int recnet_gru_cell_fwd(int precision, const float* px, int n_px, int64_t px_str
   a.Px = px; a.n_px = n_px; a.px_stride = px_stride; a.px_ld = px_ld; a.Ph = ph; a.n_ph = n_ph; a.ph_stride = ph_stride; a.ph_ld = ph_ld;
   a.Gx = gx; a.gx_ld = gx_ld; a.b_ih = b_ih; a.b_hh = b_hh; a.h_prev = h_prev; a.hp_ld = hp_ld; a.B = B; a.H = H; a.stash = stash;
   a.h_out = h_out; a.h_ld = h_ld; a.h_op = h_op; a.hop_ld = hop_ld;
-  if (precision == RECNET_PREC_FP32) return gru::launch_fwd<float, float>(a, ST(stream));
-  if (precision == RECNET_PREC_BF16) return gru::launch_fwd<bf16, bf16>(a, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(precision, RECNET_ERR_UNSUPPORTED, [&](auto t) { using T = decltype(t); return gru::launch_fwd<T, T>(a, ST(stream)); });
 }
 
 int recnet_gru_cell_bwd(int precision, const float* dh_ext, int64_t dh_ld, const float* dh_ext2, int64_t dh2_ld, const float* dhp,
@@ -231,52 +252,19 @@ int recnet_gru_cell_bwd(int precision, const float* dh_ext, int64_t dh_ld, const
   a.dh_ext = dh_ext; a.dh_ld = dh_ld; a.dh_ext2 = dh_ext2; a.dh2_ld = dh2_ld; a.dHp = dhp; a.n_p = n_p; a.p_stride = p_stride; a.p_ld = p_ld;
   a.dQp = dqp; a.n_q = n_q; a.q_stride = q_stride; a.q_ld = q_ld; a.carry = carry; a.first = first; a.stash = stash; a.h_prev = h_prev;
   a.hp_ld = hp_ld; a.B = B; a.H = H; a.dGi = dgi; a.dGh = dgh; a.dg_ld = dg_ld;
-  if (precision == RECNET_PREC_FP32) return gru::launch_bwd<float, float>(a, ST(stream));
-  if (precision == RECNET_PREC_BF16) return gru::launch_bwd<bf16, bf16>(a, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(precision, RECNET_ERR_UNSUPPORTED, [&](auto t) { using T = decltype(t); return gru::launch_bwd<T, T>(a, ST(stream)); });
 }
 
 // ---- decoder ---------------------------------------------------------------------------------------------------
 int64_t recnet_decoder_workspace_bytes(const recnet_decoder_desc* d) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
-  if (!d) return RECNET_ERR_BAD_SHAPE;
-  if (dec::pf_ok(dd)) {
-    if (dd.precision == RECNET_PREC_FP32) return (int64_t)dec::plan_pf<float>(dd, nullptr).bytes;
-    if (dd.precision == RECNET_PREC_BF16) return (int64_t)dec::plan_pf<bf16>(dd, nullptr).bytes;
-    return RECNET_ERR_UNSUPPORTED;
-  }
-  if (dd.precision == RECNET_PREC_FP32) return (int64_t)dec::plan<float>(dd, nullptr).bytes;
-  if (dd.precision == RECNET_PREC_BF16) return (int64_t)dec::plan<bf16>(dd, nullptr).bytes;
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) { return dec_layout<decltype(t)>(dd, nullptr).bytes; });
 }
 int recnet_decoder_fwd(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, const int64_t* tokens_in,
                        const int64_t* targets, const float* ce_weight, const uint64_t* rng, void* workspace,
                        int64_t workspace_bytes, float* hiddens, float* ce_out, void* stream) {
-  DecDesc dd;
-  RN_TRY(split_desc(d, &dd));
-  const long long* ti = reinterpret_cast<const long long*>(tokens_in);
-  const long long* tg = reinterpret_cast<const long long*>(targets);
-  const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (dd.n_layers > 1) {
-    if (dd.precision == RECNET_PREC_FP32)
-      return dec::forward_ml<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
-    if (dd.precision == RECNET_PREC_BF16)
-      return dec::forward_ml<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
-    return RECNET_ERR_UNSUPPORTED;
-  }
-  if (dec::pf_ok(dd)) {
-    if (dd.precision == RECNET_PREC_FP32)
-      return dec::forward_pf<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
-    if (dd.precision == RECNET_PREC_BF16)
-      return dec::forward_pf<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
-    return RECNET_ERR_UNSUPPORTED;
-  }
-  if (dd.precision == RECNET_PREC_FP32)
-    return dec::forward<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
-  if (dd.precision == RECNET_PREC_BF16)
-    return dec::forward<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return recnet_decoder_fwd_phase(d, w, feats, tokens_in, targets, ce_weight, rng, workspace, workspace_bytes, hiddens, ce_out, 3, stream);
 }
 int recnet_decoder_fwd_phase(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, const int64_t* tokens_in,
                              const int64_t* targets, const float* ce_weight, const uint64_t* rng, void* workspace,
@@ -284,47 +272,29 @@ int recnet_decoder_fwd_phase(const recnet_decoder_desc* d, const recnet_decoder_
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
   if (phases < 1 || phases > 3) return RECNET_ERR_BAD_SHAPE;
-  if (dd.n_layers > 1 || !dec::pf_ok(dd)) {          // not split on these paths: everything belongs to bit 0
-    if (!(phases & 1)) return 0;
-    return recnet_decoder_fwd(d, w, feats, tokens_in, targets, ce_weight, rng, workspace, workspace_bytes, hiddens, ce_out, stream);
-  }
+  const dec::DecPath path = dec::dec_path(dd);
+  if (path != dec::DecPath::PF && !(phases & 1)) return 0;          // not split on these paths: everything belongs to bit 0
   const long long* ti = reinterpret_cast<const long long*>(tokens_in);
   const long long* tg = reinterpret_cast<const long long*>(targets);
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (dd.precision == RECNET_PREC_FP32)
-    return dec::forward_pf<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream), phases);
-  if (dd.precision == RECNET_PREC_BF16)
-    return dec::forward_pf<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream), phases);
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    using T = decltype(t);
+    switch (path) {
+      case dec::DecPath::ML:
+        return dec::forward_ml<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
+      case dec::DecPath::PF:
+        return dec::forward_pf<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream), phases);
+      default:
+        return dec::forward<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
+    }
+  });
 }
 int recnet_decoder_bwd(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, const int64_t* tokens_in,
                        const int64_t* targets, const float* ce_weight, const uint64_t* rng, void* workspace,
                        int64_t workspace_bytes, const float* g_ce, const float* g_hiddens, const float* hiddens,
                        const recnet_decoder_tensors* grads, void* stream) {
-  DecDesc dd;
-  RN_TRY(split_desc(d, &dd));
-  const long long* ti = reinterpret_cast<const long long*>(tokens_in);
-  const long long* tg = reinterpret_cast<const long long*>(targets);
-  const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (dd.n_layers > 1) {
-    if (dd.precision == RECNET_PREC_FP32)
-      return dec::backward_ml<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
-    if (dd.precision == RECNET_PREC_BF16)
-      return dec::backward_ml<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
-    return RECNET_ERR_UNSUPPORTED;
-  }
-  if (dec::pf_ok(dd)) {
-    if (dd.precision == RECNET_PREC_FP32)
-      return dec::backward_pf<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
-    if (dd.precision == RECNET_PREC_BF16)
-      return dec::backward_pf<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
-    return RECNET_ERR_UNSUPPORTED;
-  }
-  if (dd.precision == RECNET_PREC_FP32)
-    return dec::backward<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, hiddens, *grads, ST(stream));
-  if (dd.precision == RECNET_PREC_BF16)
-    return dec::backward<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, hiddens, *grads, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return recnet_decoder_bwd_phase(d, w, feats, tokens_in, targets, ce_weight, rng, workspace, workspace_bytes, g_ce, g_hiddens, hiddens,
+                                  grads, 15, stream);
 }
 int recnet_decoder_bwd_phase(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, const int64_t* tokens_in,
                              const int64_t* targets, const float* ce_weight, const uint64_t* rng, void* workspace,
@@ -333,60 +303,68 @@ int recnet_decoder_bwd_phase(const recnet_decoder_desc* d, const recnet_decoder_
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
   if (phases < 1 || phases > 15) return RECNET_ERR_BAD_SHAPE;
-  if (dd.n_layers > 1 || !dec::pf_ok(dd)) {          // not split on these paths: everything belongs to bit 0
-    if (!(phases & 1)) return 0;
-    return recnet_decoder_bwd(d, w, feats, tokens_in, targets, ce_weight, rng, workspace, workspace_bytes, g_ce, g_hiddens, hiddens,
-                              grads, stream);
-  }
+  const dec::DecPath path = dec::dec_path(dd);
+  if (path != dec::DecPath::PF && !(phases & 1)) return 0;          // not split on these paths: everything belongs to bit 0
   const long long* ti = reinterpret_cast<const long long*>(tokens_in);
   const long long* tg = reinterpret_cast<const long long*>(targets);
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (dd.precision == RECNET_PREC_FP32)
-    return dec::backward_pf<float>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream), phases);
-  if (dd.precision == RECNET_PREC_BF16)
-    return dec::backward_pf<bf16>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream), phases);
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    using T = decltype(t);
+    switch (path) {
+      case dec::DecPath::ML:
+        return dec::backward_ml<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
+      case dec::DecPath::PF:
+        return dec::backward_pf<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream),
+                                   phases);
+      default:
+        return dec::backward<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, hiddens, *grads,
+                                ST(stream));
+    }
+  });
 }
 int recnet_decoder_bwd_is_split(const recnet_decoder_desc* d) {
   DecDesc dd;
   if (split_desc(d, &dd)) return 0;
-  return (dd.n_layers > 1 || !dec::pf_ok(dd)) ? 0 : 1;
+  return dec::dec_path(dd) == dec::DecPath::PF ? 1 : 0;
 }
 float* recnet_decoder_logits(const recnet_decoder_desc* d, void* workspace, int64_t* ld) {
   DecDesc dd;
   if (split_desc(d, &dd)) return nullptr;
-  if (dec::pf_ok(dd)) {
-    if (dd.precision == RECNET_PREC_FP32) { auto w = dec::plan_pf<float>(dd, workspace); if (ld) *ld = w.Vld; return w.logits; }
-    auto w = dec::plan_pf<bf16>(dd, workspace); if (ld) *ld = w.Vld; return w.logits;
-  }
-  if (dd.precision == RECNET_PREC_FP32) { auto w = dec::plan<float>(dd, workspace); if (ld) *ld = w.Vld; return w.logits; }
-  auto w = dec::plan<bf16>(dd, workspace); if (ld) *ld = w.Vld; return w.logits;
+  return by_prec<float*>(dd.precision, nullptr, [&](auto t) {
+    const DecLayout w = dec_layout<decltype(t)>(dd, workspace);
+    if (ld) *ld = w.ld;
+    return w.logits;
+  });
 }
 int64_t recnet_greedy_workspace_bytes(const recnet_decoder_desc* d) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
-  if (dd.precision == RECNET_PREC_FP32) return (int64_t)dec::plan_greedy<float>(dd, nullptr, 64).bytes;
-  if (dd.precision == RECNET_PREC_BF16) {
-    const int64_t a = (int64_t)dec::plan_greedy<bf16>(dd, nullptr, 64).bytes;
-    const int64_t b = dec::greedy_pf_ok(dd) ? (int64_t)dec::plan_greedy_pf<bf16>(dd, nullptr, 64).bytes : 0;
-    return a > b ? a : b;
-  }
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    using T = decltype(t);
+    const int64_t a = (int64_t)dec::plan_greedy<T>(dd, nullptr, 64).bytes;
+    if constexpr (std::is_same<T, bf16>::value) {      // room for either bf16 driver: recnet_decoder_greedy picks one per call
+      const int64_t b = dec::greedy_pf_ok(dd) ? (int64_t)dec::plan_greedy_pf<bf16>(dd, nullptr, 64).bytes : 0;
+      return a > b ? a : b;
+    }
+    return a;
+  });
 }
 int recnet_decoder_greedy(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, int max_steps,
                           void* workspace, int64_t workspace_bytes, int64_t* ids_out, int32_t* n_steps_out, void* stream) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
   if (max_steps < 1 || max_steps > 64) return RECNET_ERR_BAD_SHAPE;
-  if (dd.precision == RECNET_PREC_FP32)
-    return dec::greedy<float>(dd, *w, feats, max_steps, workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), n_steps_out, ST(stream));
-  if (dd.precision == RECNET_PREC_BF16) {
-    recnet_decoder_desc d1 = *d; d1.L = 1; d1.train = 0;
-    if (dec::greedy_pf_ok(d1))      // projected-feature kernels, 4 launches per step
-      return dec::greedy_pf(dd, *w, feats, max_steps, workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), n_steps_out, ST(stream));
-    return dec::greedy<bf16>(dd, *w, feats, max_steps, workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), n_steps_out, ST(stream));
-  }
-  return RECNET_ERR_UNSUPPORTED;
+  long long* ids = reinterpret_cast<long long*>(ids_out);
+  return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    using T = decltype(t);
+    if constexpr (std::is_same<T, bf16>::value) {
+      DecDesc d1 = dd; d1.L = 1; d1.train = 0;
+      // softmax decoders keep dec::greedy: moving them onto greedy_pf changes their launches and needs its own measurement
+      if (dec::greedy_pf_ok(d1) && !dd.softmax)      // projected-feature kernels, 4 launches per step
+        return dec::greedy_pf(dd, *w, feats, max_steps, workspace, workspace_bytes, ids, n_steps_out, ST(stream));
+    }
+    return dec::greedy<T>(dd, *w, feats, max_steps, workspace, workspace_bytes, ids, n_steps_out, ST(stream));
+  });
 }
 
 // byte offset of the loop kernel's int32 error flag inside the workspace (0 = ok, 2 = mbarrier timeout, 3 = grid-barrier timeout)
@@ -394,136 +372,116 @@ int64_t recnet_decoder_error_offset(const recnet_decoder_desc* d) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
   uint8_t* base = reinterpret_cast<uint8_t*>(4096);
-  if (dec::pf_ok(dd)) {
-    if (dd.precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(dec::plan_pf<float>(dd, base).err) - base;
-    return reinterpret_cast<uint8_t*>(dec::plan_pf<bf16>(dd, base).err) - base;
-  }
-  if (dd.precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(dec::plan<float>(dd, base).err) - base;
-  return reinterpret_cast<uint8_t*>(dec::plan<bf16>(dd, base).err) - base;
+  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED,
+                          [&](auto t) { return reinterpret_cast<uint8_t*>(dec_layout<decltype(t)>(dd, base).err) - base; });
 }
 int64_t recnet_local_error_offset(const recnet_local_desc* d) {
   LocalDesc dd;
   RN_TRY(split_desc(d, &dd));
   uint8_t* base = reinterpret_cast<uint8_t*>(4096);
-  if (dd.precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(rec::plan_local<float>(dd, base).err) - base;
-  return reinterpret_cast<uint8_t*>(rec::plan_local<bf16>(dd, base).err) - base;
+  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED,
+                          [&](auto t) { return reinterpret_cast<uint8_t*>(rec::plan_local<decltype(t)>(dd, base).err) - base; });
 }
 int64_t recnet_global_error_offset(const recnet_global_desc* d) {
+  RN_TRY(check_desc(d));
   uint8_t* base = reinterpret_cast<uint8_t*>(4096);
-  if (d->precision == RECNET_PREC_FP32) return reinterpret_cast<uint8_t*>(rec::plan_global<float>(*d, base).err) - base;
-  return reinterpret_cast<uint8_t*>(rec::plan_global<bf16>(*d, base).err) - base;
+  return by_prec<int64_t>(d->precision, RECNET_ERR_UNSUPPORTED,
+                          [&](auto t) { return reinterpret_cast<uint8_t*>(rec::plan_global<decltype(t)>(*d, base).err) - base; });
 }
 
-// ---- local reconstructor ---------------------------------------------------------------------------------------
 int64_t recnet_beam_workspace_bytes(const recnet_decoder_desc* d, int beam_width, int max_steps) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
   if (beam_width < 1 || beam_width > dec::BEAM_MAX_K || max_steps < 1 || max_steps > 64) return RECNET_ERR_BAD_SHAPE;
-  if (dd.precision == RECNET_PREC_FP32) return (int64_t)dec::plan_beam<float>(dd, nullptr, beam_width, max_steps).bytes;
-  if (dd.precision == RECNET_PREC_BF16) return (int64_t)dec::plan_beam<bf16>(dd, nullptr, beam_width, max_steps).bytes;
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED,
+                          [&](auto t) { return (int64_t)dec::plan_beam<decltype(t)>(dd, nullptr, beam_width, max_steps).bytes; });
 }
 int recnet_decoder_beam(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats_tiled, int beam_width, int max_steps,
                         int64_t eos_id, void* workspace, int64_t workspace_bytes, int64_t* seq_out, int32_t* n_steps_out, void* stream) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
   if (dd.n_layers > 1) return RECNET_ERR_UNSUPPORTED;
-  if (dd.precision == RECNET_PREC_FP32)
-    return dec::beam<float>(dd, *w, feats_tiled, beam_width, max_steps, (long long)eos_id, workspace, workspace_bytes,
-                            reinterpret_cast<long long*>(seq_out), n_steps_out, ST(stream));
-  if (dd.precision == RECNET_PREC_BF16)
-    return dec::beam<bf16>(dd, *w, feats_tiled, beam_width, max_steps, (long long)eos_id, workspace, workspace_bytes,
-                           reinterpret_cast<long long*>(seq_out), n_steps_out, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    return dec::beam<decltype(t)>(dd, *w, feats_tiled, beam_width, max_steps, (long long)eos_id, workspace, workspace_bytes,
+                                  reinterpret_cast<long long*>(seq_out), n_steps_out, ST(stream));
+  });
 }
 
+// ---- local reconstructor ---------------------------------------------------------------------------------------
 int64_t recnet_local_workspace_bytes(const recnet_local_desc* d) {
   LocalDesc dd;
   RN_TRY(split_desc(d, &dd));
-  if (dd.precision == RECNET_PREC_FP32) return (int64_t)rec::plan_local<float>(dd, nullptr).bytes;
-  if (dd.precision == RECNET_PREC_BF16) return (int64_t)rec::plan_local<bf16>(dd, nullptr).bytes;
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED,
+                          [&](auto t) { return (int64_t)rec::plan_local<decltype(t)>(dd, nullptr).bytes; });
 }
 int recnet_local_fwd(const recnet_local_desc* d, const recnet_local_tensors* w, const float* hiddens, const float* feats,
                      const uint64_t* rng, void* workspace, int64_t workspace_bytes, float* mse_out, void* stream) {
   LocalDesc dd;
   RN_TRY(split_desc(d, &dd));
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (dd.dec_layers > 1) {
-    if (dd.precision == RECNET_PREC_FP32) return rec::local_forward_ml<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
-    if (dd.precision == RECNET_PREC_BF16) return rec::local_forward_ml<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
-    return RECNET_ERR_UNSUPPORTED;
-  }
-  if (dd.precision == RECNET_PREC_FP32) return rec::local_forward<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
-  if (dd.precision == RECNET_PREC_BF16) return rec::local_forward<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    using T = decltype(t);
+    if (dd.dec_layers > 1) return rec::local_forward_ml<T>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
+    return rec::local_forward<T>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
+  });
 }
 int recnet_local_bwd(const recnet_local_desc* d, const recnet_local_tensors* w, const float* hiddens, const float* feats,
                      const uint64_t* rng, void* workspace, int64_t workspace_bytes, const float* g_mse,
                      const recnet_local_tensors* grads, float* g_hiddens, void* stream) {
-  LocalDesc dd;
-  RN_TRY(split_desc(d, &dd));
-  const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (dd.dec_layers > 1) {
-    if (dd.precision == RECNET_PREC_FP32) return rec::local_backward_ml<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
-    if (dd.precision == RECNET_PREC_BF16) return rec::local_backward_ml<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
-    return RECNET_ERR_UNSUPPORTED;
-  }
-  if (dd.precision == RECNET_PREC_FP32) return rec::local_backward<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
-  if (dd.precision == RECNET_PREC_BF16) return rec::local_backward<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return recnet_local_bwd_phase(d, w, hiddens, feats, rng, workspace, workspace_bytes, g_mse, grads, g_hiddens, 3, stream);
 }
 int recnet_local_bwd_phase(const recnet_local_desc* d, const recnet_local_tensors* w, const float* hiddens, const float* feats,
                            const uint64_t* rng, void* workspace, int64_t workspace_bytes, const float* g_mse,
                            const recnet_local_tensors* grads, float* g_hiddens, int phases, void* stream) {
   LocalDesc dd;
   RN_TRY(split_desc(d, &dd));
-  const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
   if (phases < 1 || phases > 3) return RECNET_ERR_BAD_SHAPE;
-  if (dd.dec_layers > 1) {                 // stacked decoders: not split -- everything belongs to phase bit 0
-    if (!(phases & 1)) return 0;
-    return recnet_local_bwd(d, w, hiddens, feats, rng, workspace, workspace_bytes, g_mse, grads, g_hiddens, stream);
-  }
-  if (dd.precision == RECNET_PREC_FP32) return rec::local_backward<float>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream), phases);
-  if (dd.precision == RECNET_PREC_BF16) return rec::local_backward<bf16>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream), phases);
-  return RECNET_ERR_UNSUPPORTED;
+  if (dd.dec_layers > 1 && !(phases & 1)) return 0;     // stacked decoders: not split -- everything belongs to phase bit 0
+  const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
+  return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    using T = decltype(t);
+    if (dd.dec_layers > 1)
+      return rec::local_backward_ml<T>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
+    return rec::local_backward<T>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream), phases);
+  });
 }
 int recnet_set_background_ctas(int n) {
   if (n < 0 || n > 4096) return RECNET_ERR_BAD_SHAPE;
-  tc2::background_ctas() = n;
+  rn_background_ctas() = n;
   return 0;
 }
 float* recnet_local_outputs(const recnet_local_desc* d, void* workspace) {
   LocalDesc dd;
   if (split_desc(d, &dd)) return nullptr;
-  if (dd.precision == RECNET_PREC_FP32) return rec::plan_local<float>(dd, workspace).out;
-  return rec::plan_local<bf16>(dd, workspace).out;
+  return by_prec<float*>(dd.precision, nullptr, [&](auto t) { return rec::plan_local<decltype(t)>(dd, workspace).out; });
 }
 
 // ---- global reconstructor --------------------------------------------------------------------------------------
 int64_t recnet_global_workspace_bytes(const recnet_global_desc* d) {
-  if (d->precision == RECNET_PREC_FP32) return (int64_t)rec::plan_global<float>(*d, nullptr).bytes;
-  if (d->precision == RECNET_PREC_BF16) return (int64_t)rec::plan_global<bf16>(*d, nullptr).bytes;
-  return RECNET_ERR_UNSUPPORTED;
+  RN_TRY(check_desc(d));
+  return by_prec<int64_t>(d->precision, RECNET_ERR_UNSUPPORTED,
+                          [&](auto t) { return (int64_t)rec::plan_global<decltype(t)>(*d, nullptr).bytes; });
 }
 int recnet_global_fwd(const recnet_global_desc* d, const recnet_global_tensors* w, const float* hiddens, const float* feats,
                       const uint64_t* rng, void* workspace, int64_t workspace_bytes, float* loss_out, void* stream) {
+  RN_TRY(check_desc(d));
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (d->precision == RECNET_PREC_FP32) return rec::global_forward<float>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, loss_out, ST(stream));
-  if (d->precision == RECNET_PREC_BF16) return rec::global_forward<bf16>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, loss_out, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(d->precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    return rec::global_forward<decltype(t)>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, loss_out, ST(stream));
+  });
 }
 int recnet_global_bwd(const recnet_global_desc* d, const recnet_global_tensors* w, const float* hiddens, const float* feats,
                       const uint64_t* rng, void* workspace, int64_t workspace_bytes, const float* g_loss,
                       const recnet_global_tensors* grads, float* g_hiddens, void* stream) {
+  RN_TRY(check_desc(d));
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
-  if (d->precision == RECNET_PREC_FP32) return rec::global_backward<float>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, g_loss, *grads, g_hiddens, ST(stream));
-  if (d->precision == RECNET_PREC_BF16) return rec::global_backward<bf16>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, g_loss, *grads, g_hiddens, ST(stream));
-  return RECNET_ERR_UNSUPPORTED;
+  return by_prec<int>(d->precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    return rec::global_backward<decltype(t)>(*d, *w, hiddens, feats, r, workspace, workspace_bytes, g_loss, *grads, g_hiddens, ST(stream));
+  });
 }
 float* recnet_global_outputs(const recnet_global_desc* d, void* workspace) {
-  if (d->precision == RECNET_PREC_FP32) return rec::plan_global<float>(*d, workspace).out;
-  return rec::plan_global<bf16>(*d, workspace).out;
+  if (check_desc(d)) return nullptr;
+  return by_prec<float*>(d->precision, nullptr, [&](auto t) { return rec::plan_global<decltype(t)>(*d, workspace).out; });
 }
 
 // ---- regulariser -----------------------------------------------------------------------------------------------

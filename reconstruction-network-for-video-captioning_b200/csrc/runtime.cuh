@@ -46,8 +46,7 @@ struct Side {
   cudaEvent_t fork_ev = nullptr, join_ev = nullptr;
   int dev = -1;
   static bool enabled() {
-    static int on = -1;
-    if (on < 0) { const char* e = getenv("RECNET_SIDE"); on = e ? atoi(e) : 1; }
+    static const int on = rn_env_int("RECNET_SIDE", 1);
     return on != 0;
   }
   int fork(cudaStream_t main, cudaStream_t* out) {
@@ -202,8 +201,7 @@ template <> inline GemmPlan plan_gemm_full<bf16>(int M, int N, int K) {
   // skinny -- sweep in profiles/r2_h_gemm_sweep.md: it wins or ties on every batched GEMM with M, N >= 256; the four 128-row
   // attention weight gradients and the 128-column key projections stay on the split-K / 64-wide plans above.  256-wide tiles once
   // they fill 2/3 of the SMs; CTA pairs (half the B traffic per SM) only for long K loops with at least 1.5 rounds of pair tiles.
-  static int persist = -1;
-  if (persist < 0) { const char* e = getenv("RECNET_GEMM_PERSIST"); persist = e ? atoi(e) : 1; }
+  static const int persist = rn_env_int("RECNET_GEMM_PERSIST", 1);
   if (persist && M >= 256 && N >= 256) {
     const int t256 = mt * rn_cdiv(N, 256);
     const int pairs = rn_cdiv(M, 256) * rn_cdiv(N, 256);

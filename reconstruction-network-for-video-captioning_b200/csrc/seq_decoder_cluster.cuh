@@ -327,8 +327,7 @@ __global__ void __launch_bounds__(THREADS, 1) decoder_fwd_cluster_kernel(const F
 }
 
 static inline bool cluster_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("RECNET_DEC_CLUSTER"); v = e ? atoi(e) : 1; }
+  static const int v = rn_env_int("RECNET_DEC_CLUSTER", 1);
   return v != 0;
 }
 // shapes the cluster kernels are written for (MSVD decoder); everything else runs the kernel-per-phase loop
@@ -360,8 +359,8 @@ static int pick_ms(K kern, size_t smem, int B) {
   cfg.attrs = at; cfg.numAttrs = 1;
   int n = 0;
   if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess) { cudaGetLastError(); return 0; }
-  if (const char* e = getenv("RECNET_DEC_CLUSTERS")) n = atoi(e);          // developer override
-  if (getenv("RECNET_DEBUG_CLUSTERS")) fprintf(stderr, "[recnet] decoder cluster kernel: max active %d-CTA clusters = %d\n", CS, n);
+  n = rn_env_int("RECNET_DEC_CLUSTERS", n);          // developer override
+  if (rn_env_int("RECNET_DEBUG_CLUSTERS", 0)) fprintf(stderr, "[recnet] decoder cluster kernel: max active %d-CTA clusters = %d\n", CS, n);
   if (n < 1) return 0;
   const int ms = (B + n - 1) / n;
   return ms <= MAX_MS ? ms : 0;

@@ -25,8 +25,7 @@ struct PfWs {
 
 // eligibility of the projected-feature path; everything else runs the general drivers (seq_decoder.cuh / seq_decoder_ml.cuh)
 static inline bool pf_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("RECNET_PF"); v = e ? atoi(e) : 1; }
+  static const int v = rn_env_int("RECNET_PF", 1);
   return v != 0;
 }
 static inline bool pf_ok(const recnet_decoder_desc& d) {
@@ -36,6 +35,12 @@ static inline bool pf_ok(const recnet_decoder_desc& d) {
   if ((d.E & 1) || pf::escore_smem(d.L, d.T, true) > 46 * 1024) return false;          // pf_escore_kernel: column pairs, e[L x T] in shared memory
   return d.T >= 1 && d.T <= pf::MAX_T && d.A >= 4 && d.A <= pf::MAX_A && d.A % al == 0 && d.H % al == 0 &&
          pf::bwd_smem_bytes(d.H, d.A) <= 46 * 1024;
+}
+// the training driver a descriptor runs: stacked layers (seq_decoder_ml.cuh), projected-feature (here) or general (seq_decoder.cuh)
+enum class DecPath { ML, PF, GENERAL };
+static inline DecPath dec_path(const recnet_decoder_desc& d) {
+  if (d.n_layers > 1) return DecPath::ML;
+  return pf_ok(d) ? DecPath::PF : DecPath::GENERAL;
 }
 
 template <typename T>
@@ -59,10 +64,9 @@ static PfWs<T> plan_pf(const recnet_decoder_desc& d, void* base) {
     const int nkb2 = rn_cdiv(w.NP, tc::BK);
     if (w.pl_dh.splits > pf::MAXS) w.pl_dh.splits = rn_cdiv(nkb2, rn_cdiv(nkb2, pf::MAXS));
     // tuning overrides (tools/ sweeps): RECNET_PF_SPLITS_H / RECNET_PF_SPLITS_DH / RECNET_PF_BN_H
-    static int eh = -1, edh = -1, ebn = -1;
-    if (eh < 0) { const char* e = getenv("RECNET_PF_SPLITS_H"); eh = e ? atoi(e) : 0; }
-    if (edh < 0) { const char* e = getenv("RECNET_PF_SPLITS_DH"); edh = e ? atoi(e) : 0; }
-    if (ebn < 0) { const char* e = getenv("RECNET_PF_BN_H"); ebn = e ? atoi(e) : 0; }
+    static const int eh = rn_env_int("RECNET_PF_SPLITS_H", 0);
+    static const int edh = rn_env_int("RECNET_PF_SPLITS_DH", 0);
+    static const int ebn = rn_env_int("RECNET_PF_BN_H", 0);
     if (ebn == 64 || ebn == 128) w.pl_h.bn = ebn;
     if (eh > 0) w.pl_h.splits = rn_cdiv(nkb, rn_cdiv(nkb, eh > nkb ? nkb : eh));
     if (edh > 0) w.pl_dh.splits = rn_cdiv(nkb2, rn_cdiv(nkb2, edh > nkb2 ? nkb2 : edh));
@@ -333,8 +337,7 @@ static GreedyPfWs<T> plan_greedy_pf(const recnet_decoder_desc& d, void* base, in
   return w;
 }
 static inline bool greedy_pf_ok(const recnet_decoder_desc& d) {
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("RECNET_GREEDY_PF"); on = e ? atoi(e) : 1; }
+  static const int on = rn_env_int("RECNET_GREEDY_PF", 1);
   return on && d.precision == RECNET_PREC_BF16 && pf_ok(d) && (long long)d.V * 4 * d.H < (1ll << 31);
 }
 

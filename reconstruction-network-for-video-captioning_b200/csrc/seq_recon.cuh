@@ -41,8 +41,7 @@ static inline bool persist_fwd_ok(const recnet_local_desc& d) {
 template <typename T>
 static inline bool persist_bwd_ok(const recnet_local_desc& d) {
   if (!std::is_same<T, bf16>::value || d.cell != RECNET_CELL_LSTM || d.dec_layers > 1) return false;
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("RECNET_PERSIST_BWD"); on = e ? atoi(e) : 1; }
+  static const int on = rn_env_int("RECNET_PERSIST_BWD", 1);
   return on && rp::local_bwd_ok(rp::Shape{d.B, d.S, d.R, d.H, d.A, d.L});
 }
 
@@ -327,7 +326,7 @@ static int local_backward_weights(const recnet_local_desc& d, const LocalWs<T>& 
   // Column sums first: on a trainer's background lane they stay within the lane's CTA budget (misc.cuh) and the first ~60 us still run next
   // to the decoder's CE backward rather than its loop.
   cudaStream_t s2 = st;
-  const bool lane = tc2::background_ctas() > 0;   // on the lane: one capped GEMM at a time (the foreground loop's 512-thread, 128-register
+  const bool lane = rn_background_ctas() > 0;   // on the lane: one capped GEMM at a time (the foreground loop's 512-thread, 128-register
   if (!lane) RN_TRY(side().fork(st, &s2));        // CTAs need SMs that are completely empty)
   RN_TRY(misc::colsum<T>(w.dG, GR, SB, GR, g.b_ih, 0, w.splitk, st, is_gru ? nullptr : g.b_hh));     // LSTM: b_hh gets the same gradient
   if (is_gru) RN_TRY(misc::colsum<T>(dGh, GR, SB, GR, g.b_hh, 0, w.splitk, st));
@@ -359,8 +358,7 @@ constexpr int GMSE_THREADS = 256;
 template <typename T>
 static inline bool persist_global_ok(const recnet_global_desc& d, bool bwd) {
   if (!std::is_same<T, bf16>::value || d.cell != RECNET_CELL_LSTM) return false;
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("RECNET_PERSIST_GLOBAL"); on = e ? atoi(e) : 1; }
+  static const int on = rn_env_int("RECNET_PERSIST_GLOBAL", 1);
   if (!on) return false;
   return bwd ? rp::global_bwd_ok(d.B, d.L, d.R) : rp::global_fwd_ok(d.B, d.L, d.R);
 }

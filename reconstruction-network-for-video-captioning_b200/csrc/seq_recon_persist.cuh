@@ -564,8 +564,7 @@ local_fwd_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
 
 // ---- host side ---------------------------------------------------------------------------------------------------
 static inline bool persist_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("RECNET_PERSIST"); v = e ? atoi(e) : 1; }
+  static const int v = rn_env_int("RECNET_PERSIST", 1);
   return v != 0;
 }
 static inline int sm_count() {
