@@ -1,10 +1,8 @@
 // extern "C" entry points of librecnet_b200.so (declared in include/recnet_b200.h).
 #include "runtime.cuh"
 #include "seq_decoder.cuh"
-#include "seq_decoder_ml.cuh"
 #include "seq_decoder_pf.cuh"
 #include "seq_recon.cuh"
-#include "seq_recon_ml.cuh"
 #include "optim.cuh"
 #include "allreduce.cuh"
 
@@ -37,7 +35,7 @@ static int split_desc(const Pub* d, Int* out) {
   return 0;
 }
 
-// The workspace layout of the decoder's training drivers: the projected-feature plan, or the general plan (which the stacked driver shares).
+// The workspace layout of the decoder's training drivers: the projected-feature plan, or the general plan (single-layer and stacked).
 struct DecLayout { int64_t bytes; float* logits; int64_t ld; int* err; };
 template <typename T>
 static DecLayout dec_layout(const DecDesc& dd, void* base) {
@@ -280,8 +278,6 @@ int recnet_decoder_fwd_phase(const recnet_decoder_desc* d, const recnet_decoder_
   return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
     using T = decltype(t);
     switch (path) {
-      case dec::DecPath::ML:
-        return dec::forward_ml<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream));
       case dec::DecPath::PF:
         return dec::forward_pf<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, hiddens, ce_out, ST(stream), phases);
       default:
@@ -311,8 +307,6 @@ int recnet_decoder_bwd_phase(const recnet_decoder_desc* d, const recnet_decoder_
   return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
     using T = decltype(t);
     switch (path) {
-      case dec::DecPath::ML:
-        return dec::backward_ml<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream));
       case dec::DecPath::PF:
         return dec::backward_pf<T>(dd, *w, feats, ti, tg, ce_weight, r, workspace, workspace_bytes, g_ce, g_hiddens, *grads, ST(stream),
                                    phases);
@@ -421,7 +415,6 @@ int recnet_local_fwd(const recnet_local_desc* d, const recnet_local_tensors* w, 
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
   return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
     using T = decltype(t);
-    if (dd.dec_layers > 1) return rec::local_forward_ml<T>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
     return rec::local_forward<T>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, mse_out, ST(stream));
   });
 }
@@ -436,12 +429,13 @@ int recnet_local_bwd_phase(const recnet_local_desc* d, const recnet_local_tensor
   LocalDesc dd;
   RN_TRY(split_desc(d, &dd));
   if (phases < 1 || phases > 3) return RECNET_ERR_BAD_SHAPE;
-  if (dd.dec_layers > 1 && !(phases & 1)) return 0;     // stacked decoders: not split -- everything belongs to phase bit 0
+  if (dd.dec_layers > 1) {                              // stacked decoders: not split -- everything belongs to phase bit 0
+    if (!(phases & 1)) return 0;
+    phases = 3;
+  }
   const unsigned long long* r = reinterpret_cast<const unsigned long long*>(rng);
   return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
     using T = decltype(t);
-    if (dd.dec_layers > 1)
-      return rec::local_backward_ml<T>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream));
     return rec::local_backward<T>(dd, *w, hiddens, feats, r, workspace, workspace_bytes, g_mse, *grads, g_hiddens, ST(stream), phases);
   });
 }

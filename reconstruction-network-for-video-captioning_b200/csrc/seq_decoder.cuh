@@ -6,6 +6,10 @@
 //     decoder.py:64), split-K partials summed inside the fused cell kernel
 //   * vocabulary projection batched over all steps (M = L*B), fused CE forward/backward over stacked logits
 //   * BPTT mirrors it; all weight gradients are batched GEMMs over the stashed operands after the loop.
+// Stacked (n_layers = NL > 1, LSTM only): models/decoder.py:36-40,66 with num_layers = NL.  Layer 0 is the step above (input
+// [emb ; ctx]); layer l >= 1 consumes h^{l-1}_t (inter-layer dropout in train mode) and its own h^l_{t-1} as ONE K-concatenated GEMM
+// over operand rows X_l[t] = [h^{l-1}_t ; h^l_{t-1}].  The attention query and the vocabulary projection use the TOP layer
+// (decoder.py:51,68); `hiddens` returns every layer, (L, NL, B, H) (train.py:61-64).
 #pragma once
 #include "gru_cell.cuh"
 #include "runtime.cuh"
@@ -13,7 +17,7 @@
 namespace dec {
 using namespace rt;
 
-enum : unsigned { SITE_EMB = 1, SITE_LOGITS = 2 };
+enum : unsigned { SITE_EMB = 1, SITE_LOGITS = 2, SITE_LAYER0 = 16 };   // dropout site of the input of layer l = SITE_LAYER0 + l
 
 template <typename T>
 struct Ws {
@@ -136,14 +140,25 @@ static int prepare(const recnet_decoder_desc& d, const recnet_decoder_tensors& p
   return 0;
 }
 
-// one decoder step: attention -> gate GEMM -> cell.  Pointer arguments are the row-0 addresses of step t.
+// Where the top layer's h rows live: block t (B rows of ld *ld) holds h^top_{t-1}, block 0 the zero initial state.  The attention
+// query, the vocabulary GEMMs and the attn_W gradient read from here.
 template <typename T>
-static int step(const DecDesc& d, const recnet_decoder_tensors& p, Ws<T>& w, int t, const float* gx_t, T* x_t, T* x_next, float* Wh_t,
-                float* e_t, T* gates_t, const float* c_prev, float* c_next, float* h_out, cudaStream_t st) {
+static const T* top_h(const recnet_decoder_desc& d, const Ws<T>& w, long long* ld) {
+  if (w.NL == 1) { *ld = w.KX; return w.X + d.E; }
+  *ld = 2 * d.H;
+  return w.X_x[w.NL - 2] + d.H;
+}
+
+// one decoder step: attention -> gate GEMM -> layer-0 cell.  Pointer arguments are the row-0 addresses of step t; q_t (ld q_ld) holds
+// the attention query h^top_{t-1}.  In a stack, up_t is layer 1's input slot X_1[t], written through the inter-layer dropout.
+template <typename T>
+static int step(const DecDesc& d, const recnet_decoder_tensors& p, Ws<T>& w, int t, const T* q_t, long long q_ld, const float* gx_t,
+                T* x_t, T* x_next, float* Wh_t, float* e_t, T* gates_t, const float* c_prev, float* c_next, float* h_out, cudaStream_t st,
+                T* up_t = nullptr, const unsigned long long* rng = nullptr) {
   const int B = d.B, H = d.H, E = d.E, A = d.A, Tn = d.T;
   int n_whp = 0;
   if (t > 0) {   // h_{-1} = 0 -> W h = 0, skip the GEMM
-    RN_TRY(gemm_partials<T>(x_t + E, w.KX, 0, w.Wa, H, 0, w.WhP, B, A, H, w.pl_wh, st));
+    RN_TRY(gemm_partials<T>(q_t, q_ld, 0, w.Wa, H, 0, w.WhP, B, A, H, w.pl_wh, st));
     n_whp = w.pl_wh.splits;
   }
   attn::FwdArgs fa{};
@@ -177,6 +192,10 @@ static int step(const DecDesc& d, const recnet_decoder_tensors& p, Ws<T>& w, int
   ca.gates_out = gates_t; ca.c_out = c_next;
   ca.h_out = h_out; ca.h_ld = H;
   ca.h_op = x_next + E; ca.hop_ld = w.KX; ca.h_op2 = nullptr;
+  if (up_t) {
+    ca.h_op2 = up_t; ca.hop2_ld = 2 * H;
+    ca.op2_drop = d.train ? d.p_layer_drop : 0.f; ca.rng = rng; ca.site = SITE_LAYER0 + 1; ca.drop_base = (long long)t * B * H;
+  }
   return cell::launch_fwd<T, T>(ca, st);
 }
 
@@ -187,9 +206,15 @@ static int forward(const DecDesc& d, const recnet_decoder_tensors& p, const floa
   RN_TRY(check(d));
   Ws<T> w = plan<T>(d, ws);
   if ((long long)w.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
-  const int B = d.B, L = d.L, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T;
-  const float p_emb = d.train ? d.p_emb_drop : 0.f, p_out = d.train ? d.p_out_drop : 0.f;
+  const int B = d.B, L = d.L, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, NL = w.NL;
+  const float p_emb = d.train ? d.p_emb_drop : 0.f, p_out = d.train ? d.p_out_drop : 0.f, p_lay = d.train ? d.p_layer_drop : 0.f;
   RN_TRY(prepare<T>(d, p, feats, w, st));
+  for (int l = 1; l < NL; ++l) {
+    RN_TRY(misc::cast_pad<T>(p.w_ih_x[l - 1], H, w.Wrec_x[l - 1], 2 * H, 4 * H, H, H, st));
+    RN_TRY(misc::cast_pad<T>(p.w_hh_x[l - 1], H, w.Wrec_x[l - 1] + H, 2 * H, 4 * H, H, H, st));
+  }
+  long long ldq;
+  const T* Htop = top_h(d, w, &ldq);
   // hoisted projections
   RN_TRY(gemm_full<T>(w.feats, E, 0, w.U, E, 0, w.Uv, A, nullptr, B * Tn, A, E, 0, w.splitk, st));
   misc::embed_gather_kernel<T><<<L * B, 128, 0, st>>>(p.embedding, tokens_in, w.Xe, w.EMBp, L * B, d.EMB, w.EMBp, V,
@@ -203,17 +228,37 @@ static int forward(const DecDesc& d, const recnet_decoder_tensors& p, const floa
   RN_CUDA_OK(cudaMemsetAsync(w.c, 0, (size_t)B * H * sizeof(float), st));
   // time loop: one kernel per phase
   RN_CUDA_OK(cudaMemsetAsync(w.err, 0, sizeof(int), st));
+  for (int l = 1; l < NL; ++l) {
+    RN_CUDA_OK(cudaMemsetAsync(w.X_x[l - 1], 0, (size_t)B * 2 * H * sizeof(T), st));
+    RN_CUDA_OK(cudaMemsetAsync(w.c_x[l - 1], 0, (size_t)B * H * sizeof(float), st));
+  }
   for (int t = 0; t < L; ++t) {
     T* x_t = w.X + (size_t)t * B * w.KX;
     // LSTM: c_{t-1} -> c_t live in w.c; GRU: the fp32 state is h itself (previous row of `hiddens`, zeros = w.c at t = 0)
     const float* s_prev = is_gru ? (t == 0 ? w.c : hiddens + (size_t)(t - 1) * B * H) : w.c + (size_t)t * B * H;
-    RN_TRY(step<T>(d, p, w, t, w.Gx + (size_t)t * B * GH, x_t, x_t + (size_t)B * w.KX, w.Wh + (size_t)t * B * A,
-                   w.e + (size_t)t * B * Tn, w.gates + (size_t)t * B * 4 * H, s_prev, w.c + (size_t)(t + 1) * B * H,
-                   hiddens + (size_t)t * B * H, st));
+    RN_TRY(step<T>(d, p, w, t, Htop + (size_t)t * B * ldq, ldq, w.Gx + (size_t)t * B * GH, x_t, x_t + (size_t)B * w.KX,
+                   w.Wh + (size_t)t * B * A, w.e + (size_t)t * B * Tn, w.gates + (size_t)t * B * 4 * H, s_prev,
+                   w.c + (size_t)(t + 1) * B * H, hiddens + (size_t)t * NL * B * H, st,
+                   NL > 1 ? w.X_x[0] + (size_t)t * B * 2 * H : nullptr, rng));
+    for (int l = 1; l < NL; ++l) {
+      T* xl = w.X_x[l - 1] + (size_t)t * B * 2 * H;
+      RN_TRY(gemm_partials<T>(xl, 2 * H, 0, w.Wrec_x[l - 1], 2 * H, 0, w.P, B, 4 * H, 2 * H, w.pl_gate_x, st));
+      cell::FwdArgs ca{};
+      ca.P = w.P; ca.n_p = w.pl_gate_x.splits; ca.p_stride = (long long)B * 4 * H; ca.p_ld = 4 * H;
+      ca.b1 = p.b_ih_x[l - 1]; ca.b2 = p.b_hh_x[l - 1];
+      ca.c_prev = w.c_x[l - 1] + (size_t)t * B * H; ca.c_out = w.c_x[l - 1] + (size_t)(t + 1) * B * H; ca.B = B; ca.H = H;
+      ca.gates_out = w.gates_x[l - 1] + (size_t)t * B * 4 * H;
+      ca.h_out = hiddens + ((size_t)t * NL + l) * B * H; ca.h_ld = H;
+      ca.h_op = xl + (size_t)B * 2 * H + H; ca.hop_ld = 2 * H;                            // own recurrent slot of step t+1
+      if (l + 1 < NL) {                                                                     // input slot of the layer above, same t
+        ca.h_op2 = w.X_x[l] + (size_t)t * B * 2 * H; ca.hop2_ld = 2 * H;
+        ca.op2_drop = p_lay; ca.rng = rng; ca.site = SITE_LAYER0 + l + 1; ca.drop_base = (long long)t * B * H;
+      }
+      RN_TRY((cell::launch_fwd<T, T>(ca, st)));
+    }
   }
   // vocabulary projection over all steps, then the masked CE (train.py:54-60,68)
-  RN_TRY(gemm_full<T>(w.X + (size_t)B * w.KX + E, w.KX, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, L * B, V, H, 0,
-                      w.splitk, st));
+  RN_TRY(gemm_full<T>(Htop + (size_t)B * ldq, ldq, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, L * B, V, H, 0, w.splitk, st));
   if (targets && ce_weight && ce_out) {
     ProfScope prof(KC_CE, L * B, V, 0, st);
     loss::ce_fwd_kernel<<<L * B, loss::CE_THREADS, 0, st>>>(w.logits, w.Vld, targets, ce_weight, V, p_out, rng, SITE_LOGITS,
@@ -233,10 +278,11 @@ static int backward(const DecDesc& d, const recnet_decoder_tensors& p, const flo
   RN_TRY(check(d));
   Ws<T> w = plan<T>(d, ws);
   if ((long long)w.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
-  const int B = d.B, L = d.L, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, EMB = d.EMB;
-  const float p_emb = d.train ? d.p_emb_drop : 0.f, p_out = d.train ? d.p_out_drop : 0.f;
+  const int B = d.B, L = d.L, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, EMB = d.EMB, NL = w.NL, top = NL - 1;
+  const float p_emb = d.train ? d.p_emb_drop : 0.f, p_out = d.train ? d.p_out_drop : 0.f, p_lay = d.train ? d.p_layer_drop : 0.f;
   const int LB = L * B;
-  const T* Hall = w.X + (size_t)B * w.KX + E;     // h_t rows, ld = KX
+  long long ldq;
+  const T* Htop = top_h(d, w, &ldq);
   // ---- CE backward and the vocabulary projection --------------------------------------------------------
   {
     ProfScope prof(KC_CE, LB, V, 1, st);
@@ -245,7 +291,7 @@ static int backward(const DecDesc& d, const recnet_decoder_tensors& p, const flo
   }
   RN_LAUNCH_OK();
   RN_TRY(gemm_full<T>(w.dlogits, w.Vp, 0, w.Wout, H, 1, w.dHext, H, nullptr, LB, H, V, 0, w.splitk, st));
-  RN_TRY(gemm_full<T>(w.dlogits, w.Vp, 1, Hall, w.KX, 1, g.out_w, H, nullptr, V, H, LB, 0, w.splitk, st));
+  RN_TRY(gemm_full<T>(w.dlogits, w.Vp, 1, Htop + (size_t)B * ldq, ldq, 1, g.out_w, H, nullptr, V, H, LB, 0, w.splitk, st));
   RN_TRY(misc::colsum<T>(w.dlogits, w.Vp, LB, V, g.out_b, 0, w.splitk, st));
   // ---- BPTT: one kernel per phase -------------------------------------------------------------------------
   const bool is_gru = d.cell == RECNET_CELL_GRU;
@@ -280,18 +326,31 @@ static int backward(const DecDesc& d, const recnet_decoder_tensors& p, const flo
       if (t > 0) RN_TRY(gemm_partials<T>(w.dWh_op + r * A, A, 0, w.Wa, H, 1, w.dQp, B, H, A, w.pl_dq, st));
       continue;
     }
-    cell::BwdArgs cb{};
-    cb.dh_ext = w.dHext + r * H; cb.dh_ld = H; cb.dh_scale = nullptr;
-    cb.dh_ext2 = g_hiddens ? g_hiddens + r * H : nullptr; cb.dh2_ld = H;
-    cb.dXp = last ? nullptr : w.dXp; cb.n_p = w.pl_dx.splits; cb.p_stride = (long long)B * w.KX; cb.p_ld = w.KX; cb.col0 = E;
-    cb.dQp = last ? nullptr : w.dQp; cb.n_q = w.pl_dq.splits; cb.q_stride = (long long)B * H; cb.q_ld = H;
-    cb.dc = w.dc; cb.first = last ? 1 : 0;
-    cb.gates = w.gates + r * 4 * H;
-    cb.c_prev = w.c + r * H; cb.c_new = w.c + (size_t)(t + 1) * B * H;
-    cb.B = B; cb.H = H; cb.dG = w.dG + r * 4 * H; cb.dg_ld = 4 * H;
-    RN_TRY((cell::launch_bwd<T, T>(cb, st)));
-    // d[ctx ; h_{t-1}] = dG_t @ [W_ctx | W_hh]
-    RN_TRY(gemm_partials<T>(w.dG + r * 4 * H, 4 * H, 0, w.Wrec, w.KX, 1, w.dXp, B, w.KX, 4 * H, w.pl_dx, st));
+    for (int l = top; l >= 0; --l) {     // operand rows: [ctx ; h_{t-1}] for layer 0, [h^{l-1}_t ; h^l_{t-1}] above
+      const int K = l == 0 ? w.KX : 2 * H;
+      const GemmPlan pl = l == 0 ? w.pl_dx : w.pl_dx_x;
+      float* dXl = l == 0 ? w.dXp : w.dXp_x[l - 1];
+      T* dGl = (l == 0 ? w.dG : w.dG_x[l - 1]) + r * 4 * H;
+      const float* cl = l == 0 ? w.c : w.c_x[l - 1];
+      cell::BwdArgs cb{};
+      if (l == top) { cb.dh_ext = w.dHext + r * H; cb.dh_ld = H; }
+      cb.dh_ext2 = g_hiddens ? g_hiddens + ((size_t)t * NL + l) * B * H : nullptr; cb.dh2_ld = H;
+      // own recurrent path: h-part of this layer's dgrad at step t+1
+      cb.dXp = last ? nullptr : dXl; cb.n_p = pl.splits; cb.p_stride = (long long)B * K; cb.p_ld = K; cb.col0 = l == 0 ? E : H;
+      if (l == top) {          // attention query of step t+1
+        cb.dQp = last ? nullptr : w.dQp; cb.n_q = w.pl_dq.splits; cb.q_stride = (long long)B * H; cb.q_ld = H;
+      } else {                 // input of the layer above at the SAME step (x-part of its dgrad), through the inter-layer dropout
+        cb.dQp = w.dXp_x[l]; cb.n_q = w.pl_dx_x.splits; cb.q_stride = (long long)B * 2 * H; cb.q_ld = 2 * H;
+        cb.q_drop = p_lay; cb.rng = rng; cb.q_site = SITE_LAYER0 + l + 1; cb.q_base = (long long)t * B * H;
+      }
+      cb.dc = l == 0 ? w.dc : w.dc_x[l - 1]; cb.first = last ? 1 : 0;
+      cb.gates = (l == 0 ? w.gates : w.gates_x[l - 1]) + r * 4 * H;
+      cb.c_prev = cl + r * H; cb.c_new = cl + (size_t)(t + 1) * B * H;
+      cb.B = B; cb.H = H; cb.dG = dGl; cb.dg_ld = 4 * H;
+      RN_TRY((cell::launch_bwd<T, T>(cb, st)));
+      // d[x ; h_{t-1}] = dG_t @ W_rec of layer l ([W_ctx | W_hh] for layer 0)
+      RN_TRY(gemm_partials<T>(dGl, 4 * H, 0, l == 0 ? w.Wrec : w.Wrec_x[l - 1], K, 1, dXl, B, K, 4 * H, pl, st));
+    }
     attn::BwdArgs ab{};
     ab.dXp = w.dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)B * w.KX; ab.p_ld = w.KX;
     ab.V = w.feats; ab.v_bs = (long long)Tn * E; ab.v_ts = E;
@@ -319,8 +378,16 @@ static int backward(const DecDesc& d, const recnet_decoder_tensors& p, const flo
   misc::embed_scatter_kernel<<<LB, 128, 0, st>>>(g.embedding, tokens_in, w.dXe, w.EMBp, LB, EMB, V, d.embedding_scale, p_emb, rng,
                                                  SITE_EMB);
   RN_LAUNCH_OK();
+  for (int l = 1; l < NL; ++l) {
+    const T* dGl = w.dG_x[l - 1];
+    const T* Xl = w.X_x[l - 1];
+    RN_TRY(misc::colsum<T>(dGl, 4 * H, LB, 4 * H, g.b_ih_x[l - 1], 0, w.splitk, st));
+    RN_CUDA_OK(cudaMemcpyAsync(g.b_hh_x[l - 1], g.b_ih_x[l - 1], (size_t)4 * H * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    RN_TRY(gemm_full<T>(dGl, 4 * H, 1, Xl, 2 * H, 1, g.w_ih_x[l - 1], H, nullptr, 4 * H, H, LB, 0, w.splitk, st));
+    RN_TRY(gemm_full<T>(dGl, 4 * H, 1, Xl + H, 2 * H, 1, g.w_hh_x[l - 1], H, nullptr, 4 * H, H, LB, 0, w.splitk, st));
+  }
   // attention parameters
-  RN_TRY(gemm_full<T>(w.dWh_op, A, 1, w.X + E, w.KX, 1, g.attn_W, H, nullptr, A, H, LB, 0, w.splitk, st));              // dW_a = dWh^T h_{t-1}
+  RN_TRY(gemm_full<T>(w.dWh_op, A, 1, Htop, ldq, 1, g.attn_W, H, nullptr, A, H, LB, 0, w.splitk, st));                 // dW_a = dWh^T h^top_{t-1}
   RN_TRY(misc::cast_pad<T>(w.dUv, A, w.dUv_op, A, (long long)B * Tn, A, A, st));
   RN_TRY(gemm_full<T>(w.dUv_op, A, 1, w.feats, E, 1, g.attn_U, E, nullptr, A, E, B * Tn, 0, w.splitk, st));             // dU = dUv^T v
   RN_TRY(misc::colsum<float>(w.dWh, A, LB, A, g.attn_b, 0, w.splitk, st));
@@ -416,7 +483,8 @@ static int greedy(const DecDesc& d0, const recnet_decoder_tensors& p, const floa
     RN_LAUNCH_OK();
     RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
     // GRU keeps its fp32 state h in the c ping-pong rows (h_prev = c_p, h' -> c_n)
-    RN_TRY(step<T>(d, p, w, t, w.Gx, x_t, x_n, nullptr, nullptr, nullptr, c_p, c_n, d.cell == RECNET_CELL_GRU ? c_n : g.h_scratch, st));
+    RN_TRY(step<T>(d, p, w, t, x_t + E, w.KX, w.Gx, x_t, x_n, nullptr, nullptr, nullptr, c_p, c_n,
+                   d.cell == RECNET_CELL_GRU ? c_n : g.h_scratch, st));
     RN_TRY(gemm_full<T>(x_n + E, w.KX, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
     argmax_feedback_kernel<<<B, 256, 0, st>>>(w.logits, w.Vld, V, ids_out + (size_t)t * B, g.tok, g.nonpad + t);
     RN_LAUNCH_OK();
@@ -576,7 +644,8 @@ static int beam(const DecDesc& d0, const recnet_decoder_tensors& p, const float*
                                                     nullptr, SITE_EMB);
     RN_LAUNCH_OK();
     RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
-    RN_TRY(step<T>(d, p, w, t, w.Gx, x0, x1, nullptr, nullptr, nullptr, c0, c1, d.cell == RECNET_CELL_GRU ? c1 : g.h_scratch, st));
+    RN_TRY(step<T>(d, p, w, t, x0 + E, w.KX, w.Gx, x0, x1, nullptr, nullptr, nullptr, c0, c1, d.cell == RECNET_CELL_GRU ? c1 : g.h_scratch,
+                   st));
     RN_TRY(gemm_full<T>(x1 + E, w.KX, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
     const int in = t & 1, out = (t + 1) & 1;
     beam_select_kernel<<<B0, BEAM_THREADS, 0, st>>>(w.logits, w.Vld, V, B0, K, t, max_steps, eos, bw.cum[in], bw.cum[out], bw.eos[in], bw.eos[out],

@@ -23,7 +23,7 @@ struct PfWs {
   size_t bytes;
 };
 
-// eligibility of the projected-feature path; everything else runs the general drivers (seq_decoder.cuh / seq_decoder_ml.cuh)
+// eligibility of the projected-feature path; everything else runs the general drivers (seq_decoder.cuh)
 static inline bool pf_enabled() {
   static const int v = rn_env_int("RECNET_PF", 1);
   return v != 0;
@@ -36,10 +36,9 @@ static inline bool pf_ok(const recnet_decoder_desc& d) {
   return d.T >= 1 && d.T <= pf::MAX_T && d.A >= 4 && d.A <= pf::MAX_A && d.A % al == 0 && d.H % al == 0 &&
          pf::bwd_smem_bytes(d.H, d.A) <= 46 * 1024;
 }
-// the training driver a descriptor runs: stacked layers (seq_decoder_ml.cuh), projected-feature (here) or general (seq_decoder.cuh)
-enum class DecPath { ML, PF, GENERAL };
+// the training driver a descriptor runs: projected-feature (here) or general (seq_decoder.cuh, single-layer and stacked)
+enum class DecPath { PF, GENERAL };
 static inline DecPath dec_path(const recnet_decoder_desc& d) {
-  if (d.n_layers > 1) return DecPath::ML;
   return pf_ok(d) ? DecPath::PF : DecPath::GENERAL;
 }
 

@@ -4,7 +4,12 @@
 //  global : train.forward_global_reconstructor (train.py:78-105) over GlobalReconstructor.forward
 //           (models/global_reconstructor.py:30-46): [h_t ; mean-pool] -> LSTM(R) -> Linear(R,R), MSE of means / L.
 // Same restructuring as the decoder: U.hiddens hoisted, [x ; h] K-concatenated gate GEMM per step, output
-// projection and all weight gradients batched over time.  One decoder layer (the reference default).
+// projection and all weight gradients batched over time.
+// Local over a STACKED decoder (hiddens (L, NLd, B, H), NLd > 1, LSTM cells only) -- the reference's quirk A7
+// (models/local_reconstructor.py:44-54): the attended input keeps the decoder-layer axis, (NLd, B, H), and nn.LSTM
+// treats that axis as TIME, so every outer step t runs NLd pseudo-steps (attention over layer l's states -> LSTM step),
+// all NLd attentions sharing ONE query (the state at the start of the outer step); the output projection reads the
+// state after pseudo-step 0 (`output[0]`).
 #pragma once
 #include "gru_cell.cuh"
 #include "runtime.cuh"
@@ -114,6 +119,25 @@ static LocalWs<T> plan_local(const recnet_local_desc& d, void* base) {
   return w;
 }
 
+// Rows of h that the output projection reads and rows of the attention query, S*B each with ld `ld`: the h slots of X over a
+// one-layer decoder; over a stacked one the compact copies Hout (`output[0]`) and Hq (state at the start of every outer step).
+template <typename T>
+struct HRows { const T* out; const T* query; long long ld; };
+template <typename T>
+static HRows<T> h_rows(const recnet_local_desc& d, const LocalWs<T>& w) {
+  if (d.dec_layers > 1) return {w.Hout, w.Hq, d.R};
+  return {w.X + (size_t)d.B * w.KX + d.H, w.X + d.H, w.KX};
+}
+
+template <typename T>
+__global__ void copy_rows_kernel(const T* __restrict__ src, long long src_row_stride, T* __restrict__ dst, long long n_rows, int cols) {
+  const long long total = n_rows * cols;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long r = i / cols; const int c = (int)(i % cols);
+    dst[i] = src[r * src_row_stride + c];
+  }
+}
+
 static inline int check_local(const recnet_local_desc& d) {
   if (d.B < 1 || d.S < 1 || d.L < 1 || d.L > attn::MAX_T) return RECNET_ERR_BAD_SHAPE;
   if (d.cell != RECNET_CELL_LSTM && d.cell != RECNET_CELL_GRU) return RECNET_ERR_UNSUPPORTED;
@@ -129,7 +153,7 @@ static int local_forward(const LocalDesc& d, const recnet_local_tensors& p, cons
   RN_TRY(check_local(d));
   LocalWs<T> w = plan_local<T>(d, ws);
   if ((long long)w.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
-  const int B = d.B, S = d.S, R = d.R, H = d.H, A = d.A, L = d.L;
+  const int B = d.B, S = d.S, R = d.R, H = d.H, A = d.A, L = d.L, NLd = d.dec_layers < 1 ? 1 : d.dec_layers;
   const float p_drop = d.train ? d.p_drop : 0.f;
   const bool is_gru = d.cell == RECNET_CELL_GRU;
   const int GR = w.G * R;
@@ -140,14 +164,14 @@ static int local_forward(const LocalDesc& d, const recnet_local_tensors& p, cons
   sg.add(p.attn_U, H, w.U, H, A, H, H);
   sg.add(p.attn_W, R, w.Wa, R, A, R, R);
   sg.add(p.out_w, R, w.Wout, R, R, R, R);
-  sg.add(hiddens, H, w.Hd, H, (long long)L * B, H, H);
+  sg.add(hiddens, H, w.Hd, H, (long long)L * NLd * B, H, H);
   sg.zero(w.X, (size_t)B * w.KX * sizeof(T));
   sg.zero(w.c, (size_t)B * R * sizeof(float));
   sg.zero(w.err, 64 * sizeof(int));
   const bool persist = persist_fwd_ok<T>(d);
   if (persist || persist_bwd_ok<T>(d)) sg.zero(w.psync, 2 * rp::SYNC_WORDS * sizeof(unsigned));
   RN_TRY(sg.launch(st));
-  RN_TRY(gemm_full<T>(w.Hd, H, 0, w.U, H, 0, w.Uv, A, nullptr, L * B, A, H, 0, w.splitk, st));     // U.hiddens, once
+  RN_TRY(gemm_full<T>(w.Hd, H, 0, w.U, H, 0, w.Uv, A, nullptr, L * NLd * B, A, H, 0, w.splitk, st));     // U.hiddens, once
   if constexpr (std::is_same<T, bf16>::value) {
     if (persist) {
       // ONE cooperative launch for all S steps, [W_ih | W_hh] resident in shared memory (seq_recon_persist.cuh); same stash layout
@@ -167,21 +191,25 @@ static int local_forward(const LocalDesc& d, const recnet_local_tensors& p, cons
       return 0;
     }
   }
-  for (int t = 0; t < S; ++t) {
-    const size_t r = (size_t)t * B;
+  int n_whp = 0;
+  for (int q = 0; q < S * NLd; ++q) {      // pseudo-step q = (outer step t, decoder layer l)
+    const int t = q / NLd, l = q - t * NLd;
+    const size_t r = (size_t)q * B;
     T* x_t = w.X + r * w.KX;
     T* x_n = x_t + (size_t)B * w.KX;
-    // attention query W.h_{t-1}: its own small GEMM, partials summed by the attention kernel
-    int n_whp = 0;
-    if (t > 0) {
-      RN_TRY(gemm_partials<T>(x_t + H, w.KX, 0, w.Wa, R, 0, w.WhP, B, A, R, w.pl_wh, st));
-      n_whp = w.pl_wh.splits;
+    // attention query W.h_{t-1}: its own small GEMM, partials summed by the attention kernel; ONE per outer step
+    if (l == 0) {
+      n_whp = 0;
+      if (t > 0) {
+        RN_TRY(gemm_partials<T>(x_t + H, w.KX, 0, w.Wa, R, 0, w.WhP, B, A, R, w.pl_wh, st));
+        n_whp = w.pl_wh.splits;
+      }
     }
     attn::FwdArgs fa{};
     fa.WhP = w.WhP; fa.n_whp = n_whp; fa.whp_stride = (long long)B * A;
-    fa.Uv = w.Uv; fa.uv_bs = A; fa.uv_ts = (long long)B * A;          // Uv is [L,B,A]
+    fa.Uv = w.Uv + (size_t)l * B * A; fa.uv_bs = A; fa.uv_ts = (long long)NLd * B * A;          // Uv is [L,NLd,B,A]
     fa.attn_b = p.attn_b; fa.attn_w = p.attn_w;
-    fa.V = w.Hd; fa.v_bs = H; fa.v_ts = (long long)B * H;             // values = decoder states [L,B,H]
+    fa.V = w.Hd + (size_t)l * B * H; fa.v_bs = H; fa.v_ts = (long long)NLd * B * H;             // values = layer l of [L,NLd,B,H]
     fa.B = B; fa.Tn = L; fa.A = A; fa.D = H; fa.inv_T = d.softmax ? 1.f : 1.f / L; fa.normalize = d.softmax;
     fa.Wh_out = w.Wh + r * A; fa.e_out = w.beta + r * L;
     fa.ctx_out = x_t; fa.ctx_ld = w.KX;
@@ -189,13 +217,13 @@ static int local_forward(const LocalDesc& d, const recnet_local_tensors& p, cons
     RN_TRY((attn::launch_fwd<T, T>(fa, st)));
     if (is_gru) {
       RN_TRY(gemm_partials<T>(x_t, w.KX, 0, w.Wrec, w.KX, 0, w.P, B, 3 * R, H, w.pl_gx, st));
-      if (t > 0) RN_TRY(gemm_partials<T>(x_t + H, w.KX, 0, w.Wrec + H, w.KX, 0, w.P2, B, 3 * R, R, w.pl_gh, st));
+      if (q > 0) RN_TRY(gemm_partials<T>(x_t + H, w.KX, 0, w.Wrec + H, w.KX, 0, w.P2, B, 3 * R, R, w.pl_gh, st));
       gru::FwdArgs ga{};
       ga.Px = w.P; ga.n_px = w.pl_gx.splits; ga.px_stride = (long long)B * 3 * R; ga.px_ld = 3 * R;
-      ga.Ph = t > 0 ? w.P2 : nullptr; ga.n_ph = t > 0 ? w.pl_gh.splits : 0; ga.ph_stride = (long long)B * 3 * R; ga.ph_ld = 3 * R;
+      ga.Ph = q > 0 ? w.P2 : nullptr; ga.n_ph = q > 0 ? w.pl_gh.splits : 0; ga.ph_stride = (long long)B * 3 * R; ga.ph_ld = 3 * R;
       ga.Gx = nullptr; ga.b_ih = p.b_ih; ga.b_hh = p.b_hh;
       ga.h_prev = w.c + r * R; ga.hp_ld = R; ga.B = B; ga.H = R;            // fp32 state h lives in the c rows
-      ga.stash = w.gates + r * 4 * R; ga.h_out = w.c + (size_t)(t + 1) * B * R; ga.h_ld = R;
+      ga.stash = w.gates + r * 4 * R; ga.h_out = w.c + (size_t)(q + 1) * B * R; ga.h_ld = R;
       ga.h_op = x_n + H; ga.hop_ld = w.KX;
       RN_TRY((gru::launch_fwd<T, T>(ga, st)));
       continue;
@@ -204,11 +232,18 @@ static int local_forward(const LocalDesc& d, const recnet_local_tensors& p, cons
     cell::FwdArgs ca{};
     ca.P = w.P; ca.n_p = w.pl_gate.splits; ca.p_stride = (long long)B * 4 * R; ca.p_ld = 4 * R;
     ca.Gx = nullptr; ca.b1 = p.b_ih; ca.b2 = p.b_hh; ca.c_prev = w.c + r * R; ca.B = B; ca.H = R;
-    ca.gates_out = w.gates + r * 4 * R; ca.c_out = w.c + (size_t)(t + 1) * B * R; ca.h_out = nullptr;
+    ca.gates_out = w.gates + r * 4 * R; ca.c_out = w.c + (size_t)(q + 1) * B * R; ca.h_out = nullptr;
     ca.h_op = x_n + H; ca.hop_ld = w.KX; ca.h_op2 = nullptr;
+    if (NLd > 1 && l == 0) { ca.h_op2 = w.Hout + (size_t)t * B * R; ca.hop2_ld = R; }        // `output[0]`
     RN_TRY((cell::launch_fwd<T, T>(ca, st)));
   }
-  RN_TRY(gemm_full<T>(w.X + (size_t)B * w.KX + H, w.KX, 0, w.Wout, R, 0, w.out, R, p.out_b, S * B, R, R, 0, w.splitk, st));
+  // stacked: query-state rows (state at the start of every outer step) for the attn_W gradient
+  for (int t = 0; t < S && NLd > 1; ++t) {
+    copy_rows_kernel<T><<<rn_cdiv((long long)B * R, 256), 256, 0, st>>>(w.X + (size_t)t * NLd * B * w.KX + H, w.KX, w.Hq + (size_t)t * B * R, B, R);
+    RN_LAUNCH_OK();
+  }
+  const HRows<T> hr = h_rows(d, w);
+  RN_TRY(gemm_full<T>(hr.out, hr.ld, 0, w.Wout, R, 0, w.out, R, p.out_b, S * B, R, R, 0, w.splitk, st));
   if (mse_out) {
     loss::mse_local_fwd_kernel<<<MSE_BLOCKS, 256, 0, st>>>(w.out, feats, S, B, R, w.partial);
     RN_LAUNCH_OK();
@@ -232,7 +267,7 @@ static int local_backward(const LocalDesc& d, const recnet_local_tensors& p, con
   LocalWs<T> w = plan_local<T>(d, ws);
   if ((long long)w.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
   if (!(phases & 1)) return (phases & 2) ? local_backward_weights<T>(d, w, g, st) : 0;
-  const int B = d.B, S = d.S, R = d.R, H = d.H, A = d.A, L = d.L;
+  const int B = d.B, S = d.S, R = d.R, H = d.H, A = d.A, L = d.L, NLd = d.dec_layers < 1 ? 1 : d.dec_layers;
   const float p_drop = d.train ? d.p_drop : 0.f;
   const int SB = S * B;
   loss::mse_local_bwd_kernel<T><<<MSE_BLOCKS, 256, 0, st>>>(w.out, feats, S, B, R, g_mse, 2.f / ((float)S * B * R), w.dOut);
@@ -254,9 +289,10 @@ static int local_backward(const LocalDesc& d, const recnet_local_tensors& p, con
       RN_TRY(rp::launch_local_bwd(bp, w.Wrec, st));
     }
   }
-  for (int t = S - 1; t >= 0 && !persist; --t) {
-    const bool last = (t == S - 1);
-    const size_t r = (size_t)t * B;
+  for (int q = S * NLd - 1; q >= 0 && !persist; --q) {      // pseudo-step q = (outer step t, decoder layer l)
+    const int t = q / NLd, l = q - t * NLd;
+    const bool last = (q == S * NLd - 1);
+    const size_t r = (size_t)q * B;
     if (is_gru) {
       float* dXx = w.dXp;
       float* dXh = w.dXp2;
@@ -284,31 +320,37 @@ static int local_backward(const LocalDesc& d, const recnet_local_tensors& p, con
       continue;
     }
     cell::BwdArgs cb{};
-    cb.dh_ext = w.dHext + r * R; cb.dh_ld = R;
+    if (l == 0) { cb.dh_ext = w.dHext + (size_t)t * B * R; cb.dh_ld = R; }                       // out-proj reads pseudo-step (t,0)
     cb.dXp = last ? nullptr : w.dXp; cb.n_p = w.pl_dx.splits; cb.p_stride = (long long)B * w.KX; cb.p_ld = w.KX; cb.col0 = H;
-    cb.dQp = last ? nullptr : w.dQp; cb.n_q = w.pl_dq.splits; cb.q_stride = (long long)B * R; cb.q_ld = R;
+    if (l == NLd - 1) {                                                                          // query of outer step t+1
+      cb.dQp = last ? nullptr : w.dQp; cb.n_q = w.pl_dq.splits; cb.q_stride = (long long)B * R; cb.q_ld = R;
+    }
     cb.dc = w.dc; cb.first = last ? 1 : 0;
     cb.gates = w.gates + r * 4 * R;
-    cb.c_prev = w.c + r * R; cb.c_new = w.c + (size_t)(t + 1) * B * R;
+    cb.c_prev = w.c + r * R; cb.c_new = w.c + (size_t)(q + 1) * B * R;
     cb.B = B; cb.H = R; cb.dG = w.dG + r * 4 * R; cb.dg_ld = 4 * R;
     RN_TRY((cell::launch_bwd<T, T>(cb, st)));
     RN_TRY(gemm_partials<T>(w.dG + r * 4 * R, 4 * R, 0, w.Wrec, w.KX, 1, w.dXp, B, w.KX, 4 * R, w.pl_dx, st));
     attn::BwdArgs ab{};
     ab.dXp = w.dXp; ab.n_p = w.pl_dx.splits; ab.p_stride = (long long)B * w.KX; ab.p_ld = w.KX;
-    ab.V = w.Hd; ab.v_bs = H; ab.v_ts = (long long)B * H;
-    ab.Wh = w.Wh + r * A; ab.Uv = w.Uv; ab.uv_bs = A; ab.uv_ts = (long long)B * A;
+    ab.V = w.Hd + (size_t)l * B * H; ab.v_bs = H; ab.v_ts = (long long)NLd * B * H;
+    ab.Wh = w.Wh + r * A; ab.Uv = w.Uv + (size_t)l * B * A; ab.uv_bs = A; ab.uv_ts = (long long)NLd * B * A;
     ab.attn_b = p.attn_b; ab.attn_w = p.attn_w; ab.B = B; ab.Tn = L; ab.A = A; ab.D = H; ab.inv_T = d.softmax ? 1.f : 1.f / L;
-    ab.dWh_out = w.dWh + r * A; ab.dWh_op = w.dWh_op + r * A; ab.dUv_acc = w.dUv;
-    ab.uv_first = last ? 1 : 0; ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc;
+    ab.dWh_out = w.dWh + (size_t)t * B * A; ab.dWh_op = w.dWh_op + (size_t)t * B * A;          // summed over the NLd attentions of step t
+    ab.dwh_acc = (l != NLd - 1) ? 1 : 0;
+    ab.dUv_acc = w.dUv + (size_t)l * B * A; ab.uv_first = (t == S - 1) ? 1 : 0;
+    ab.dw_first = last ? 1 : 0; ab.dw_acc = w.dw_acc;
     ab.dctx_out = w.dx + r * H; ab.de_out = nullptr; ab.alpha = d.softmax ? w.beta + r * L : nullptr;
     ab.p_drop = p_drop; ab.rng = rng; ab.site = SITE_LOCAL_X; ab.drop_base = (long long)r * H;
     RN_TRY((attn::launch_bwd<T, T>(ab, st)));
-    if (t > 0) RN_TRY(gemm_partials<T>(w.dWh_op + r * A, A, 0, w.Wa, R, 1, w.dQp, B, R, A, w.pl_dq, st));
+    if (l == 0 && t > 0) RN_TRY(gemm_partials<T>(w.dWh_op + (size_t)t * B * A, A, 0, w.Wa, R, 1, w.dQp, B, R, A, w.pl_dq, st));
   }
-  // gradient wrt the decoder states: through U (keys) and through the weighted mean / softmax-weighted sum (values)
-  RN_TRY(misc::cast_pad<T>(w.dUv, A, w.dUv_op, A, (long long)L * B, A, A, st));
-  RN_TRY(gemm_full<T>(w.dUv_op, A, 0, w.U, H, 1, g_hiddens, H, nullptr, L * B, H, A, 0, w.splitk2, st));
-  RN_TRY(attn::launch_dv(w.beta, w.dx, g_hiddens, H, (long long)B * H, S, B, L, H, d.softmax ? 1.f : 1.f / L, 1, 1, 0, st));
+  // gradient wrt the decoder states: through U (keys) and through the weighted mean / softmax-weighted sum (values), layer by layer
+  RN_TRY(misc::cast_pad<T>(w.dUv, A, w.dUv_op, A, (long long)L * NLd * B, A, A, st));
+  RN_TRY(gemm_full<T>(w.dUv_op, A, 0, w.U, H, 1, g_hiddens, H, nullptr, L * NLd * B, H, A, 0, w.splitk2, st));
+  for (int l = 0; l < NLd; ++l)
+    RN_TRY(attn::launch_dv(w.beta, w.dx, g_hiddens + (size_t)l * B * H, H, (long long)NLd * B * H, S, B, L, H, d.softmax ? 1.f : 1.f / L,
+                           1, NLd, l, st));
   if (phases & 2) RN_TRY(local_backward_weights<T>(d, w, g, st));
   return 0;
 }
@@ -317,27 +359,27 @@ static int local_backward(const LocalDesc& d, const recnet_local_tensors& p, con
 // gradients on `st`; the output projection and the 128-row attention gradients on the side stream
 template <typename T>
 static int local_backward_weights(const recnet_local_desc& d, const LocalWs<T>& w, const recnet_local_tensors& g, cudaStream_t st) {
-  const int B = d.B, S = d.S, R = d.R, H = d.H, A = d.A, L = d.L;
-  const int SB = S * B;
+  const int B = d.B, S = d.S, R = d.R, H = d.H, A = d.A, L = d.L, NLd = d.dec_layers < 1 ? 1 : d.dec_layers;
+  const int SB = S * B, SpB = S * NLd * B;          // outer steps / pseudo-steps (with a stacked decoder: NLd per outer step)
   const bool is_gru = d.cell == RECNET_CELL_GRU;
   const int GR = w.G * R;
-  const T* Hr = w.X + (size_t)B * w.KX + H;       // h_t rows, ld = KX
+  const HRows<T> hr = h_rows(d, w);
   const T* dGh = is_gru ? w.dG2 : w.dG;
   // Column sums first: on a trainer's background lane they stay within the lane's CTA budget (misc.cuh) and the first ~60 us still run next
   // to the decoder's CE backward rather than its loop.
   cudaStream_t s2 = st;
   const bool lane = rn_background_ctas() > 0;   // on the lane: one capped GEMM at a time (the foreground loop's 512-thread, 128-register
   if (!lane) RN_TRY(side().fork(st, &s2));        // CTAs need SMs that are completely empty)
-  RN_TRY(misc::colsum<T>(w.dG, GR, SB, GR, g.b_ih, 0, w.splitk, st, is_gru ? nullptr : g.b_hh));     // LSTM: b_hh gets the same gradient
-  if (is_gru) RN_TRY(misc::colsum<T>(dGh, GR, SB, GR, g.b_hh, 0, w.splitk, st));
+  RN_TRY(misc::colsum<T>(w.dG, GR, SpB, GR, g.b_ih, 0, w.splitk, st, is_gru ? nullptr : g.b_hh));    // LSTM: b_hh gets the same gradient
+  if (is_gru) RN_TRY(misc::colsum<T>(dGh, GR, SpB, GR, g.b_hh, 0, w.splitk, st));
   RN_TRY(misc::colsum<T>(w.dOut, R, SB, R, g.out_b, 0, w.splitk2, s2));
   RN_TRY(misc::colsum<float>(w.dWh, A, SB, A, g.attn_b, 0, w.splitk2, s2));
   RN_TRY(misc::colsum<float>(w.dw_acc, A, B, A, g.attn_w, 0, w.splitk2, s2));
-  RN_TRY(gemm_full<T>(w.dOut, R, 1, Hr, w.KX, 1, g.out_w, R, nullptr, R, R, SB, 0, w.splitk2, s2));
-  RN_TRY(gemm_full<T>(w.dWh_op, A, 1, w.X + H, w.KX, 1, g.attn_W, R, nullptr, A, R, SB, 0, w.splitk2, s2));
-  RN_TRY(gemm_full<T>(w.dUv_op, A, 1, w.Hd, H, 1, g.attn_U, H, nullptr, A, H, L * B, 0, w.splitk2, s2));
-  RN_TRY(gemm_full<T>(w.dG, GR, 1, w.X, w.KX, 1, g.w_ih, H, nullptr, GR, H, SB, 0, w.splitk, st));
-  RN_TRY(gemm_full<T>(dGh, GR, 1, w.X + H, w.KX, 1, g.w_hh, R, nullptr, GR, R, SB, 0, w.splitk, st));
+  RN_TRY(gemm_full<T>(w.dOut, R, 1, hr.out, hr.ld, 1, g.out_w, R, nullptr, R, R, SB, 0, w.splitk2, s2));
+  RN_TRY(gemm_full<T>(w.dWh_op, A, 1, hr.query, hr.ld, 1, g.attn_W, R, nullptr, A, R, SB, 0, w.splitk2, s2));
+  RN_TRY(gemm_full<T>(w.dUv_op, A, 1, w.Hd, H, 1, g.attn_U, H, nullptr, A, H, L * NLd * B, 0, w.splitk2, s2));
+  RN_TRY(gemm_full<T>(w.dG, GR, 1, w.X, w.KX, 1, g.w_ih, H, nullptr, GR, H, SpB, 0, w.splitk, st));
+  RN_TRY(gemm_full<T>(dGh, GR, 1, w.X + H, w.KX, 1, g.w_hh, R, nullptr, GR, R, SpB, 0, w.splitk, st));
   if (!lane) RN_TRY(side().join(st, s2));
   return 0;
 }

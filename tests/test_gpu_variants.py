@@ -69,7 +69,7 @@ def test_stacked_decoder_greedy_and_step_logits_fp32(name):
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])
 def test_config5_msrvtt_two_layer_decoder_local_reconstructor_against_oracle(precision):
     """BASELINE config 5 shape family: 40 frames x (1536 + 2048)-d features, 2-layer LSTM decoder, local reconstructor with
-    R = 3584 -- the fused stacked-decoder drivers (seq_decoder_ml / seq_recon_ml) at the stress widths and the FULL caption length
+    R = 3584 -- the fused drivers over a stacked decoder (seq_decoder.cuh / seq_recon.cuh) at the stress widths and the FULL caption length
     (31 decoded steps, 40 reconstructor steps); only the batch is reduced so that the CPU oracle finishes in seconds."""
     from oracle import recnet_oracle as O
     m = dict(B=8, T=40, E=3584, H=512, A=128, EMB=468, V=600, cap_len=30, dec_layers=2, rec_layers=1, dec_model="LSTM", rec_model="LSTM")
