@@ -8,12 +8,18 @@ models/global_reconstructor.py:38).  (seed, offset) is the module's ``_rng`` buf
 Sites and element order (must match the kernels):
   1 SITE_EMB      : [L, B, EMB]   embedding * scale, then dropout            (misc.cuh:embed_gather_kernel)
   2 SITE_LOGITS   : [L, B, V]     logits dropped BEFORE the cross entropy    (losses.cuh:ce_fwd_kernel)
-  3 SITE_LOCAL_X  : [S, B, H]     attended decoder state of the local reconstructor (attention_lean.cuh / seq_recon_persist.cuh)
+  3 SITE_LOCAL_X  : [S, B, H]     attended decoder state of the local reconstructor (attention_lean.cuh / seq_recon_persist.cuh);
+                    over a stacked decoder [S, NLd, B, H]: outer step t, decoder layer l is pseudo-step q = t*NLd + l
+                    (seq_recon.cuh:local_forward, drop_base = q*B*H)
   4 SITE_GLOBAL_MP: [L, B, H]     mean-pooled decoder state of the global reconstructor, a fresh mask every step (misc.cuh:global_x_kernel)
+ 17..19           : [L, B, H]     inter-layer dropout of a stacked LSTM decoder (nn.LSTM(dropout=p)): the input of layer l
+                    (1 <= l <= NL-1) uses site SITE_LAYER0 + l; it multiplies only the copy of h^{l-1}_t fed to layer l
+                    (seq_decoder.cuh: lstm_cell.cuh h_op2 in the forward, q_drop in the backward)
 """
 import numpy as np
 
 SITE_EMB, SITE_LOGITS, SITE_LOCAL_X, SITE_GLOBAL_MP = 1, 2, 3, 4
+SITE_LAYER0 = 16                     # + l: input of decoder layer l >= 1
 M32 = np.uint64(0xFFFFFFFF)
 
 

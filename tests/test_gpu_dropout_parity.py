@@ -21,14 +21,17 @@ from recnet_b200 import train as T
 from recnet_b200.optim import ClipAdam
 from oracle import recnet_oracle as O
 from tests.golden_util import load_golden, load_golden_beam, load_golden_train, philox_scales
-from tests.philox_ref import SITE_EMB, SITE_GLOBAL_MP, SITE_LOCAL_X, SITE_LOGITS, dropout_scales
+from tests.philox_ref import SITE_EMB, SITE_GLOBAL_MP, SITE_LAYER0, SITE_LOCAL_X, SITE_LOGITS, dropout_scales
 from tests.test_gpu_parity import FULL, TOL, _Vocab, _full_inputs, build, dev, rel
 
 pytestmark = pytest.mark.gpu
 
 
+# inter-layer dropout of a stacked decoder (sites 17..19): the (L, B, H) of the benchmarked 2-layer step and of the 3- and 4-layer
+# cases of test_gpu_stacked.py
 @pytest.mark.parametrize("site,n,p", [(SITE_EMB, 31 * 100 * 468, 0.5), (SITE_LOGITS, 7 * 4188 + 3, 0.5), (SITE_LOCAL_X, 28 * 100 * 512, 0.5),
-                                      (SITE_GLOBAL_MP, 12345, 0.3)])
+                                      (SITE_GLOBAL_MP, 12345, 0.3), (SITE_LAYER0 + 1, 31 * 100 * 512, 0.5),
+                                      (SITE_LAYER0 + 2, 13 * 13 * 256 + 1, 0.5), (SITE_LAYER0 + 3, 13 * 13 * 256, 0.3)])
 def test_device_dropout_masks_equal_the_numpy_philox_restatement(site, n, p):
     seed, offset = 0xDEC0 + site, 3
     rng = torch.tensor([seed, offset], dtype=torch.int64, device=dev())
