@@ -203,7 +203,9 @@ int recnet_decoder_bwd_is_split(const recnet_decoder_desc* d);
 float* recnet_decoder_logits(const recnet_decoder_desc* d, void* workspace, int64_t* ld);
 
 /* Greedy decoding (eval.greedy_search, eval.py:19-33): argmax feedback on device, zero host syncs.
- * ids_out [max_steps,B] int64; n_steps_out[1] int32 (device) = steps until every fed-back token is <PAD>. */
+ * ids_out [max_steps,B] int64; n_steps_out[1] int32 (device) = steps until every fed-back token is <PAD>.  The loop runs all max_steps
+ * steps (rows after n_steps_out[0] continue the argmax feedback).  LSTM decoders with 1-4 layers, single-layer GRU; a stacked GRU or
+ * n_layers > RECNET_MAX_LAYERS is RECNET_ERR_UNSUPPORTED. */
 int64_t recnet_greedy_workspace_bytes(const recnet_decoder_desc* d);
 int recnet_decoder_greedy(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats,
                           int max_steps, void* workspace, int64_t workspace_bytes, int64_t* ids_out,
@@ -213,7 +215,7 @@ int recnet_decoder_greedy(const recnet_decoder_desc* d, const recnet_decoder_ten
  * beam k of sample b; feats_tiled [beam_width * B0, T, E] = the B0 samples repeated beam_width times.  Scores log(sigmoid(logit)),
  * running score divided by len^0.7 at every step (len = position of the last <EOS> + 1, else t + 1), top-k over beams x vocabulary, stop
  * when every fed-back token is <PAD> -- the reference's rules.  seq_out [B0, max_steps] int64 = the top-1 sequence of every sample
- * (-1 beyond n_steps_out[0]); beam_width <= 8; single-layer decoders (LSTM or GRU). */
+ * (-1 beyond n_steps_out[0]); beam_width <= 8; LSTM decoders with 1-4 layers, single-layer GRU (others: RECNET_ERR_UNSUPPORTED). */
 int64_t recnet_beam_workspace_bytes(const recnet_decoder_desc* d, int beam_width, int max_steps);
 int recnet_decoder_beam(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats_tiled, int beam_width, int max_steps,
                         int64_t eos_id, void* workspace, int64_t workspace_bytes, int64_t* seq_out, int32_t* n_steps_out, void* stream);

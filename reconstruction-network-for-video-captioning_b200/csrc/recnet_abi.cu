@@ -394,7 +394,6 @@ int recnet_decoder_beam(const recnet_decoder_desc* d, const recnet_decoder_tenso
                         int64_t eos_id, void* workspace, int64_t workspace_bytes, int64_t* seq_out, int32_t* n_steps_out, void* stream) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
-  if (dd.n_layers > 1) return RECNET_ERR_UNSUPPORTED;
   return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
     return dec::beam<decltype(t)>(dd, *w, feats_tiled, beam_width, max_steps, (long long)eos_id, workspace, workspace_bytes,
                                   reinterpret_cast<long long*>(seq_out), n_steps_out, ST(stream));

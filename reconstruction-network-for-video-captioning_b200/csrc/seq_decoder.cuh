@@ -137,6 +137,10 @@ static int prepare(const recnet_decoder_desc& d, const recnet_decoder_tensors& p
   RN_TRY(misc::cast_pad<T>(p.attn_W, H, w.Wa, H, A, H, H, st));
   RN_TRY(misc::cast_pad<T>(p.out_w, H, w.Wout, H, V, H, H, st));
   if (feats) RN_TRY(misc::cast_pad<T>(feats, E, w.feats, E, (long long)d.B * d.T, E, E, st));
+  for (int l = 1; l < w.NL; ++l) {    // stacked layers: [W_ih | W_hh] of layer l side by side, K = 2H
+    RN_TRY(misc::cast_pad<T>(p.w_ih_x[l - 1], H, w.Wrec_x[l - 1], 2 * H, 4 * H, H, H, st));
+    RN_TRY(misc::cast_pad<T>(p.w_hh_x[l - 1], H, w.Wrec_x[l - 1] + H, 2 * H, 4 * H, H, H, st));
+  }
   return 0;
 }
 
@@ -199,6 +203,34 @@ static int step(const DecDesc& d, const recnet_decoder_tensors& p, Ws<T>& w, int
   return cell::launch_fwd<T, T>(ca, st);
 }
 
+// layers 1 .. NL-1 of one stacked step (LSTM): per layer, the K-concatenated gate GEMM over its operand rows [h^{l-1}_t ; h^l_{t-1}]
+// (block rd of X_x[l-1]) and the cell, which reads c^l_{t-1} from block rd of c_x[l-1] and writes c^l_t and h^l_t into block wr (h into
+// the own recurrent slot, second half) and h^l_t into the input slot of the layer above (block rd of X_x[l], through the inter-layer
+// dropout).  The sequence forward passes rd = t, wr = t + 1 and h_t = the (NL, B, H) rows of step t in `hiddens`, which also turns on
+// the gate stash for BPTT; the decode loops ping-pong two blocks and pass h_t = nullptr (neither is kept).
+template <typename T>
+static int upper_layers(const DecDesc& d, const recnet_decoder_tensors& p, Ws<T>& w, int t, int rd, int wr, float* h_t, float p_lay,
+                        const unsigned long long* rng, cudaStream_t st) {
+  const int B = d.B, H = d.H, NL = w.NL;
+  for (int l = 1; l < NL; ++l) {
+    T* xl = w.X_x[l - 1] + (size_t)rd * B * 2 * H;
+    RN_TRY(gemm_partials<T>(xl, 2 * H, 0, w.Wrec_x[l - 1], 2 * H, 0, w.P, B, 4 * H, 2 * H, w.pl_gate_x, st));
+    cell::FwdArgs ca{};
+    ca.P = w.P; ca.n_p = w.pl_gate_x.splits; ca.p_stride = (long long)B * 4 * H; ca.p_ld = 4 * H;
+    ca.b1 = p.b_ih_x[l - 1]; ca.b2 = p.b_hh_x[l - 1];
+    ca.c_prev = w.c_x[l - 1] + (size_t)rd * B * H; ca.c_out = w.c_x[l - 1] + (size_t)wr * B * H; ca.B = B; ca.H = H;
+    ca.gates_out = h_t ? w.gates_x[l - 1] + (size_t)rd * B * 4 * H : nullptr;
+    ca.h_out = h_t ? h_t + (size_t)l * B * H : nullptr; ca.h_ld = H;
+    ca.h_op = w.X_x[l - 1] + (size_t)wr * B * 2 * H + H; ca.hop_ld = 2 * H;          // own recurrent slot of the next step
+    if (l + 1 < NL) {                                                                   // input slot of the layer above, same t
+      ca.h_op2 = w.X_x[l] + (size_t)rd * B * 2 * H; ca.hop2_ld = 2 * H;
+      ca.op2_drop = p_lay; ca.rng = rng; ca.site = SITE_LAYER0 + l + 1; ca.drop_base = (long long)t * B * H;
+    }
+    RN_TRY((cell::launch_fwd<T, T>(ca, st)));
+  }
+  return 0;
+}
+
 template <typename T>
 static int forward(const DecDesc& d, const recnet_decoder_tensors& p, const float* feats, const long long* tokens_in,
                    const long long* targets, const float* ce_weight, const unsigned long long* rng, void* ws, long long ws_bytes,
@@ -209,10 +241,6 @@ static int forward(const DecDesc& d, const recnet_decoder_tensors& p, const floa
   const int B = d.B, L = d.L, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, NL = w.NL;
   const float p_emb = d.train ? d.p_emb_drop : 0.f, p_out = d.train ? d.p_out_drop : 0.f, p_lay = d.train ? d.p_layer_drop : 0.f;
   RN_TRY(prepare<T>(d, p, feats, w, st));
-  for (int l = 1; l < NL; ++l) {
-    RN_TRY(misc::cast_pad<T>(p.w_ih_x[l - 1], H, w.Wrec_x[l - 1], 2 * H, 4 * H, H, H, st));
-    RN_TRY(misc::cast_pad<T>(p.w_hh_x[l - 1], H, w.Wrec_x[l - 1] + H, 2 * H, 4 * H, H, H, st));
-  }
   long long ldq;
   const T* Htop = top_h(d, w, &ldq);
   // hoisted projections
@@ -240,22 +268,7 @@ static int forward(const DecDesc& d, const recnet_decoder_tensors& p, const floa
                    w.Wh + (size_t)t * B * A, w.e + (size_t)t * B * Tn, w.gates + (size_t)t * B * 4 * H, s_prev,
                    w.c + (size_t)(t + 1) * B * H, hiddens + (size_t)t * NL * B * H, st,
                    NL > 1 ? w.X_x[0] + (size_t)t * B * 2 * H : nullptr, rng));
-    for (int l = 1; l < NL; ++l) {
-      T* xl = w.X_x[l - 1] + (size_t)t * B * 2 * H;
-      RN_TRY(gemm_partials<T>(xl, 2 * H, 0, w.Wrec_x[l - 1], 2 * H, 0, w.P, B, 4 * H, 2 * H, w.pl_gate_x, st));
-      cell::FwdArgs ca{};
-      ca.P = w.P; ca.n_p = w.pl_gate_x.splits; ca.p_stride = (long long)B * 4 * H; ca.p_ld = 4 * H;
-      ca.b1 = p.b_ih_x[l - 1]; ca.b2 = p.b_hh_x[l - 1];
-      ca.c_prev = w.c_x[l - 1] + (size_t)t * B * H; ca.c_out = w.c_x[l - 1] + (size_t)(t + 1) * B * H; ca.B = B; ca.H = H;
-      ca.gates_out = w.gates_x[l - 1] + (size_t)t * B * 4 * H;
-      ca.h_out = hiddens + ((size_t)t * NL + l) * B * H; ca.h_ld = H;
-      ca.h_op = xl + (size_t)B * 2 * H + H; ca.hop_ld = 2 * H;                            // own recurrent slot of step t+1
-      if (l + 1 < NL) {                                                                     // input slot of the layer above, same t
-        ca.h_op2 = w.X_x[l] + (size_t)t * B * 2 * H; ca.hop2_ld = 2 * H;
-        ca.op2_drop = p_lay; ca.rng = rng; ca.site = SITE_LAYER0 + l + 1; ca.drop_base = (long long)t * B * H;
-      }
-      RN_TRY((cell::launch_fwd<T, T>(ca, st)));
-    }
+    RN_TRY(upper_layers<T>(d, p, w, t, t, t + 1, hiddens + (size_t)t * NL * B * H, p_lay, rng, st));
   }
   // vocabulary projection over all steps, then the masked CE (train.py:54-60,68)
   RN_TRY(gemm_full<T>(Htop + (size_t)B * ldq, ldq, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, L * B, V, H, 0, w.splitk, st));
@@ -456,6 +469,19 @@ static GreedyWs<T> plan_greedy(const recnet_decoder_desc& d, void* base, int max
   return g;
 }
 
+// zero initial state of the decode loops: both blocks of X and c, and of every X_x / c_x in a stack
+template <typename T>
+static int zero_decode_state(const DecDesc& d, Ws<T>& w, cudaStream_t st) {
+  const int B = d.B, H = d.H;
+  RN_CUDA_OK(cudaMemsetAsync(w.X, 0, (size_t)2 * B * w.KX * sizeof(T), st));
+  RN_CUDA_OK(cudaMemsetAsync(w.c, 0, (size_t)2 * B * H * sizeof(float), st));
+  for (int l = 1; l < w.NL; ++l) {
+    RN_CUDA_OK(cudaMemsetAsync(w.X_x[l - 1], 0, (size_t)2 * B * 2 * H * sizeof(T), st));
+    RN_CUDA_OK(cudaMemsetAsync(w.c_x[l - 1], 0, (size_t)2 * B * H * sizeof(float), st));
+  }
+  return 0;
+}
+
 template <typename T>
 static int greedy(const DecDesc& d0, const recnet_decoder_tensors& p, const float* feats, int max_steps, void* ws,
                   long long ws_bytes, long long* ids_out, int* n_steps_out, cudaStream_t st) {
@@ -464,28 +490,32 @@ static int greedy(const DecDesc& d0, const recnet_decoder_tensors& p, const floa
   GreedyWs<T> g = plan_greedy<T>(d0, ws, max_steps);
   if ((long long)g.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
   Ws<T>& w = g.w;
-  const int B = d.B, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T;
+  const int B = d.B, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, NL = w.NL;
   RN_TRY(prepare<T>(d, p, feats, w, st));
   RN_TRY(gemm_full<T>(w.feats, E, 0, w.U, E, 0, w.Uv, A, nullptr, B * Tn, A, E, 0, w.splitk, st));
-  RN_CUDA_OK(cudaMemsetAsync(w.X, 0, (size_t)2 * B * w.KX * sizeof(T), st));
-  RN_CUDA_OK(cudaMemsetAsync(w.c, 0, (size_t)2 * B * H * sizeof(float), st));
+  RN_TRY(zero_decode_state<T>(d, w, st));
   RN_CUDA_OK(cudaMemsetAsync(g.nonpad, 0, (size_t)max_steps * sizeof(int), st));
   fill_tokens_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(g.tok, B, 1 /* <SOS> */);
   RN_LAUNCH_OK();
-  // ping-pong the two X rows / c rows of the L=1 plan
+  // ping-pong the two blocks of every X / c buffer of the L=1 plan: step t reads block t & 1 and writes block (t + 1) & 1.  The top
+  // layer's h (attention query, vocabulary projection) sits at the same place in either block (top_h).
+  long long ldq;
+  const T* Htop = top_h(d, w, &ldq);
   for (int t = 0; t < max_steps; ++t) {
-    T* x_t = w.X + (size_t)(t & 1) * B * w.KX;
-    T* x_n = w.X + (size_t)((t + 1) & 1) * B * w.KX;
-    float* c_p = w.c + (size_t)(t & 1) * B * H;
-    float* c_n = w.c + (size_t)((t + 1) & 1) * B * H;
+    const int rd = t & 1, wr = (t + 1) & 1;
+    T* x_t = w.X + (size_t)rd * B * w.KX;
+    T* x_n = w.X + (size_t)wr * B * w.KX;
+    float* c_p = w.c + (size_t)rd * B * H;
+    float* c_n = w.c + (size_t)wr * B * H;
     misc::embed_gather_kernel<T><<<B, 128, 0, st>>>(p.embedding, g.tok, w.Xe, w.EMBp, B, d.EMB, w.EMBp, V, d.embedding_scale, 0.f,
                                                     nullptr, SITE_EMB);
     RN_LAUNCH_OK();
     RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
     // GRU keeps its fp32 state h in the c ping-pong rows (h_prev = c_p, h' -> c_n)
-    RN_TRY(step<T>(d, p, w, t, x_t + E, w.KX, w.Gx, x_t, x_n, nullptr, nullptr, nullptr, c_p, c_n,
-                   d.cell == RECNET_CELL_GRU ? c_n : g.h_scratch, st));
-    RN_TRY(gemm_full<T>(x_n + E, w.KX, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
+    RN_TRY(step<T>(d, p, w, t, Htop + (size_t)rd * B * ldq, ldq, w.Gx, x_t, x_n, nullptr, nullptr, nullptr, c_p, c_n,
+                   d.cell == RECNET_CELL_GRU ? c_n : g.h_scratch, st, NL > 1 ? w.X_x[0] + (size_t)rd * B * 2 * H : nullptr));
+    RN_TRY(upper_layers<T>(d, p, w, t, rd, wr, nullptr, 0.f, nullptr, st));
+    RN_TRY(gemm_full<T>(Htop + (size_t)wr * B * ldq, ldq, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
     argmax_feedback_kernel<<<B, 256, 0, st>>>(w.logits, w.Vld, V, ids_out + (size_t)t * B, g.tok, g.nonpad + t);
     RN_LAUNCH_OK();
   }
@@ -580,6 +610,29 @@ __global__ void beam_gather_kernel(const T* __restrict__ h_src, T* __restrict__ 
     c_dst[(long long)row * H + j] = c_src[(long long)srow * H + j];
   }
 }
+// the same for every layer of a stack in one launch: layer 0's h rows (ld KX) and c, layer l's h (second half of the X_x[l-1] rows,
+// ld 2H) and c_x[l-1].  The input-slot halves need no gather: every step rewrites them before it reads them.
+template <typename T>
+struct BeamStateRows {
+  const T* h_src[RECNET_MAX_LAYERS]; T* h_dst[RECNET_MAX_LAYERS]; long long ld[RECNET_MAX_LAYERS];
+  const float* c_src[RECNET_MAX_LAYERS]; float* c_dst[RECNET_MAX_LAYERS];
+  int n;
+};
+template <typename T>
+__global__ void beam_gather_layers_kernel(BeamStateRows<T> s, int H, int B0, int K, const int* __restrict__ src,
+                                          const int* __restrict__ nonpad, int t) {
+  if (t > 0 && nonpad[t - 1] == 0) return;                  // frozen (see beam_select_kernel)
+  const int row = blockIdx.x, k = row / B0, b = row - k * B0;
+  const int srow = src[b * K + k] * B0 + b;
+#pragma unroll
+  for (int l = 0; l < RECNET_MAX_LAYERS; ++l) {
+    if (l >= s.n) break;
+    for (int j = threadIdx.x; j < H; j += blockDim.x) {
+      s.h_dst[l][(long long)row * s.ld[l] + j] = s.h_src[l][(long long)srow * s.ld[l] + j];
+      s.c_dst[l][(long long)row * H + j] = s.c_src[l][(long long)srow * H + j];
+    }
+  }
+}
 __global__ void beam_finalize_kernel(const int* __restrict__ nonpad, int max_steps, int B0, int K, const int* __restrict__ seq0,
                                      const int* __restrict__ seq1, long long* __restrict__ out, int* __restrict__ n_steps) {
   int n = max_steps;
@@ -626,32 +679,47 @@ static int beam(const DecDesc& d0, const recnet_decoder_tensors& p, const float*
   if ((long long)bw.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
   GreedyWs<T>& g = bw.g;
   Ws<T>& w = g.w;
-  const int B = d.B, B0 = B / K, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T;
+  const int B = d.B, B0 = B / K, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, NL = w.NL;
   RN_TRY(prepare<T>(d, p, feats, w, st));
   RN_TRY(gemm_full<T>(w.feats, E, 0, w.U, E, 0, w.Uv, A, nullptr, B * Tn, A, E, 0, w.splitk, st));
-  RN_CUDA_OK(cudaMemsetAsync(w.X, 0, (size_t)2 * B * w.KX * sizeof(T), st));
-  RN_CUDA_OK(cudaMemsetAsync(w.c, 0, (size_t)2 * B * H * sizeof(float), st));
+  RN_TRY(zero_decode_state<T>(d, w, st));
   RN_CUDA_OK(cudaMemsetAsync(g.nonpad, 0, (size_t)max_steps * sizeof(int), st));
   fill_tokens_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(g.tok, B, 1 /* <SOS> */);
   RN_LAUNCH_OK();
   beam_init_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(bw.cum[0], bw.eos[0], B);
   RN_LAUNCH_OK();
-  // state buffers: step reads (x0, c0) and writes (x1, c1); the gather moves the selected beams' state back into (x0, c0)
+  // state buffers: step reads block 0 of every X / c buffer (x0, c0, ...) and writes block 1 (x1, c1, ...); the gather moves the
+  // selected beams' state back into block 0
   T* x0 = w.X; T* x1 = w.X + (size_t)B * w.KX;
   float* c0 = w.c; float* c1 = w.c + (size_t)B * H;
+  long long ldq;
+  const T* Htop = top_h(d, w, &ldq);
+  BeamStateRows<T> rows{};                 // a stack's gather: h (own recurrent slot) and c of every layer
+  rows.n = NL;
+  for (int l = 0; l < NL; ++l) {
+    T* h = l == 0 ? w.X + E : w.X_x[l - 1] + H;
+    float* c = l == 0 ? w.c : w.c_x[l - 1];
+    rows.ld[l] = l == 0 ? w.KX : 2 * H;
+    rows.h_dst[l] = h; rows.h_src[l] = h + (size_t)B * rows.ld[l];
+    rows.c_dst[l] = c; rows.c_src[l] = c + (size_t)B * H;
+  }
   for (int t = 0; t < max_steps; ++t) {
     misc::embed_gather_kernel<T><<<B, 128, 0, st>>>(p.embedding, g.tok, w.Xe, w.EMBp, B, d.EMB, w.EMBp, V, d.embedding_scale, 0.f,
                                                     nullptr, SITE_EMB);
     RN_LAUNCH_OK();
     RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
-    RN_TRY(step<T>(d, p, w, t, x0 + E, w.KX, w.Gx, x0, x1, nullptr, nullptr, nullptr, c0, c1, d.cell == RECNET_CELL_GRU ? c1 : g.h_scratch,
-                   st));
-    RN_TRY(gemm_full<T>(x1 + E, w.KX, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
+    RN_TRY(step<T>(d, p, w, t, Htop, ldq, w.Gx, x0, x1, nullptr, nullptr, nullptr, c0, c1, d.cell == RECNET_CELL_GRU ? c1 : g.h_scratch,
+                   st, NL > 1 ? w.X_x[0] : nullptr));
+    RN_TRY(upper_layers<T>(d, p, w, t, 0, 1, nullptr, 0.f, nullptr, st));
+    RN_TRY(gemm_full<T>(Htop + (size_t)B * ldq, ldq, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
     const int in = t & 1, out = (t + 1) & 1;
     beam_select_kernel<<<B0, BEAM_THREADS, 0, st>>>(w.logits, w.Vld, V, B0, K, t, max_steps, eos, bw.cum[in], bw.cum[out], bw.eos[in], bw.eos[out],
                                                     bw.seq[in], bw.seq[out], g.tok, bw.src, g.nonpad);
     RN_LAUNCH_OK();
-    beam_gather_kernel<T><<<B, 128, 0, st>>>(x1 + E, x0 + E, w.KX, c1, c0, H, B0, K, bw.src, g.nonpad, t);
+    if (NL == 1)
+      beam_gather_kernel<T><<<B, 128, 0, st>>>(x1 + E, x0 + E, w.KX, c1, c0, H, B0, K, bw.src, g.nonpad, t);
+    else
+      beam_gather_layers_kernel<T><<<B, 128, 0, st>>>(rows, H, B0, K, bw.src, g.nonpad, t);
     RN_LAUNCH_OK();
   }
   beam_finalize_kernel<<<1, 256, 0, st>>>(g.nonpad, max_steps, B0, K, bw.seq[0], bw.seq[1], seq_out, n_steps_out);

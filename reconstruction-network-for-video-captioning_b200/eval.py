@@ -48,11 +48,12 @@ def beam_search(config, beam_width, vocab, decoder, input, hidden, encoder_outpu
 
 
 def _device_beam_applies(decoder, beam_width, input, hidden, vocab) -> bool:
-    """recnet_decoder_beam covers what eval.evaluate passes (eval.py:130-140): single-layer decoder, <SOS> start, zero state, <= 8 beams."""
+    """recnet_decoder_beam covers what eval.evaluate passes (eval.py:130-140): a decoder with a fused driver (LSTM with 1-4 layers,
+    single-layer GRU), <SOS> start, zero state, <= 8 beams."""
     import os
     if os.environ.get("RECNET_BEAM_DEVICE", "1") != "1" or not hasattr(decoder, "beam"):
         return False
-    if getattr(decoder, "n_layers", 1) != 1 or not getattr(decoder, "uses_fused_sequence", False) or not 1 <= beam_width <= 8:
+    if not getattr(decoder, "uses_fused_sequence", False) or not 1 <= beam_width <= 8:
         return False
     if not input.is_cuda or vocab.word2idx.get('<PAD>', 0) != 0:
         return False

@@ -14,10 +14,12 @@ softmax-normalised scores and weighted sum).  ``state_dict`` keys and shapes do 
 Every (cell, n_layers) combination the reference's constructors accept runs on our kernels:
 * fused sequence drivers (one C call per loop): LSTM decoder with 1-4 layers, GRU decoder with 1 layer, 1-layer LSTM
   reconstructors over any such decoder, 1-layer GRU reconstructors over a 1-layer decoder -- the configurations the
-  reference's config.py / published runs use, and everything bench.py measures;
+  reference's config.py / published runs use, and everything bench.py measures.  The same decoders also decode in one C
+  call each (``greedy``, ``beam``);
 * every other variant (stacked GRU decoder, GRU reconstructor over a stacked decoder, multi-layer reconstructors, > 4
   decoder layers) runs ``forward_sequence`` as a Python loop over the per-step ``forward`` -- the same operator-level
-  CUDA kernels (ops.py), autograd glue in between.  Slower, never silent: ``uses_fused_sequence`` says which one runs.
+  CUDA kernels (ops.py), autograd glue in between; such decoders also decode step by step.  Slower, never silent:
+  ``uses_fused_sequence`` says which one runs.
 """
 from __future__ import annotations
 
@@ -220,35 +222,18 @@ class Decoder(nn.Module, _RngMixin):
 
     @torch.no_grad()
     def greedy(self, encoder_outputs, max_steps):
-        """eval.greedy_search (eval.py:19-33) on device: returns (ids (n,B) int64 on device, n)."""
+        """eval.greedy_search (eval.py:19-33) on device: returns (ids (max_steps,B) int64 on device, n).  One C call for the decoders
+        with a fused driver (LSTM with 1-4 layers, single-layer GRU); the others step through ``forward``."""
         import ctypes as C
-        if self.n_layers > 1 or not self.uses_fused_sequence:
-            # stacked decoders: step by step through Decoder.forward (our kernels), arg-max feedback on device
-            B = encoder_outputs.shape[0]
-            dev = encoder_outputs.device
-            hid = _zero_state(self.model_name, self.n_layers, B, self.hidden_size, dev)
-            tok = torch.ones(1, B, dtype=torch.long, device=dev)
-            was_training = self.training
-            self.eval()
-            ids = torch.zeros(max_steps, B, dtype=torch.long, device=dev)
-            n = max_steps
-            with self.cached_uv(encoder_outputs):
-                for t in range(max_steps):
-                    logits, hid = self.forward(tok, hid, encoder_outputs)
-                    tok = logits.argmax(dim=1).view(1, -1)
-                    ids[t] = tok[0]
-                    if bool((tok == 0).all()):
-                        n = t + 1
-                        break
-            self.train(was_training)
-            return ids, torch.tensor([n], dtype=torch.int32, device=dev)
+        if not self.uses_fused_sequence:
+            return self._greedy_stepwise(encoder_outputs, max_steps)
         lib = L.lib()
         feats = Fn._f32c(encoder_outputs, "encoder_outputs")
         B, T, E = feats.shape
         meta = self._meta()
         d = L.decoder_desc(B=B, T=T, E=E, H=meta["H"], A=meta["A"], EMB=meta["EMB"], V=meta["V"], L=1,
                            precision=meta["precision"], train=0, embedding_scale=float(meta["embedding_scale"]),
-                           p_emb_drop=0.0, p_out_drop=0.0, cell=meta["cell"])
+                           p_emb_drop=0.0, p_out_drop=0.0, cell=meta["cell"], n_layers=self.n_layers)
         nbytes = lib.recnet_greedy_workspace_bytes(C.byref(d))
         ws = torch.empty(nbytes, dtype=torch.uint8, device=feats.device)
         ids = torch.empty(max_steps, B, dtype=torch.int64, device=feats.device)
@@ -258,6 +243,29 @@ class Decoder(nn.Module, _RngMixin):
         L.check(lib.recnet_decoder_greedy(C.byref(d), C.byref(w), feats.data_ptr(), max_steps, ws.data_ptr(), nbytes,
                                           ids.data_ptr(), n.data_ptr(), Fn._stream()), "recnet_decoder_greedy")
         return ids, n
+
+    @torch.no_grad()
+    def _greedy_stepwise(self, encoder_outputs, max_steps):
+        """``greedy`` step by step through Decoder.forward (our kernels), arg-max feedback on device, one host read per step; stops
+        after the first all-<PAD> step and leaves the remaining rows 0."""
+        B = encoder_outputs.shape[0]
+        dev = encoder_outputs.device
+        hid = _zero_state(self.model_name, self.n_layers, B, self.hidden_size, dev)
+        tok = torch.ones(1, B, dtype=torch.long, device=dev)
+        was_training = self.training
+        self.eval()
+        ids = torch.zeros(max_steps, B, dtype=torch.long, device=dev)
+        n = max_steps
+        with self.cached_uv(encoder_outputs):
+            for t in range(max_steps):
+                logits, hid = self.forward(tok, hid, encoder_outputs)
+                tok = logits.argmax(dim=1).view(1, -1)
+                ids[t] = tok[0]
+                if bool((tok == 0).all()):
+                    n = t + 1
+                    break
+        self.train(was_training)
+        return ids, torch.tensor([n], dtype=torch.int32, device=dev)
 
     @torch.no_grad()
     def beam(self, encoder_outputs, beam_width, max_steps, eos_id=2):
@@ -272,7 +280,7 @@ class Decoder(nn.Module, _RngMixin):
         meta = self._meta()
         d = L.decoder_desc(B=B0 * K, T=T, E=E, H=meta["H"], A=meta["A"], EMB=meta["EMB"], V=meta["V"], L=1,
                            precision=meta["precision"], train=0, embedding_scale=float(meta["embedding_scale"]),
-                           p_emb_drop=0.0, p_out_drop=0.0, cell=meta["cell"])
+                           p_emb_drop=0.0, p_out_drop=0.0, cell=meta["cell"], n_layers=self.n_layers)
         nbytes = lib.recnet_beam_workspace_bytes(C.byref(d), K, max_steps)
         if nbytes < 0:
             L.check(int(nbytes), "recnet_beam_workspace_bytes")

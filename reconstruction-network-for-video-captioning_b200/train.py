@@ -59,8 +59,10 @@ def forward_decoder(decoder, encoder_outputs, targets, target_masks, teacher_for
             # KNOWN DIFFERENCE in train mode with teacher_forcing_ratio < 1 (the reference's default is 1.0, config.py:71): the
             # reference feeds back the argmax of the SAME pass's dropout-perturbed logits; here the tokens come from a dropout-free
             # greedy pass, so the fed-back tokens follow the eval-mode distribution.  Losses / gradients for a GIVEN token sequence
-            # are identical.  (The step-wise greedy of stacked decoders also stops once every token is <PAD> and leaves the
-            # remaining rows 0 = <PAD>, which is what the reference would decode from an all-<PAD> row only by accident.)
+            # are identical.  The device greedy keeps feeding the argmax back after an all-<PAD> step, as the reference does.
+            # (The step-wise greedy of the decoders without a fused driver -- stacked GRU, > 4 layers -- stops once every token is
+            # <PAD> and leaves the remaining rows 0 = <PAD>, which is what the reference would decode from an all-<PAD> row only by
+            # accident.)
             ids, _ = model.greedy(encoder_outputs, L)
             tokens_in = torch.cat((sos, ids[: L - 1]), dim=0)
             output_indices = ids[:L].cpu()
