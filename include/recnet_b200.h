@@ -220,6 +220,21 @@ int64_t recnet_beam_workspace_bytes(const recnet_decoder_desc* d, int beam_width
 int recnet_decoder_beam(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats_tiled, int beam_width, int max_steps,
                         int64_t eos_id, void* workspace, int64_t workspace_bytes, int64_t* seq_out, int32_t* n_steps_out, void* stream);
 
+/* Sampling (Gumbel-max) as a device loop with zero host syncs: every row draws its token of step t from softmax(z'/temperature), z' =
+ * the logits after their dropout (site 2) when d->train is set, with Gumbel noise from Philox site 5 of the `noise` (seed, offset) pair
+ * at element (t*B + row)*V + v.  In train mode every dropout mask is drawn from `rng` (the module's pair, device memory) at the element
+ * the sequence forward uses for row t*B + row, so recnet_decoder_fwd over tokens_in = [<SOS>; ids[:-1]], targets = ids with the same
+ * pair computes the logits the sampler drew from.  A row finishes once it emits eos_id or <PAD>, then emits <PAD> with log-prob 0.
+ * Outputs (device): ids_out [max_steps,B] int64, logp_out [max_steps,B] = log softmax(z'/temperature)[id], lengths_out [B] = tokens up
+ * to and including the finishing one (max_steps if none), n_steps_out[1] = the step at which the last row finished + 1.  rng and noise are
+ * device pointers.  Coverage of recnet_decoder_greedy (others: RECNET_ERR_UNSUPPORTED); temperature <= 0 or max_steps outside 1..64:
+ * RECNET_ERR_BAD_SHAPE. */
+int64_t recnet_sample_workspace_bytes(const recnet_decoder_desc* d, int max_steps);
+int recnet_decoder_sample(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, int max_steps,
+                          float temperature, int64_t eos_id, const unsigned long long* rng, const unsigned long long* noise,
+                          void* workspace, int64_t workspace_bytes, int64_t* ids_out, float* logp_out, int32_t* lengths_out,
+                          int32_t* n_steps_out, void* stream);
+
 /* Local reconstructor (models/local_reconstructor.py:37-55 + train.forward_local_reconstructor, train.py:108-131). */
 typedef struct {
   int32_t B, S, R, H, A, L;             /* S = encoder_output_len steps, R = hidden (= feature dim), H = decoder hidden */

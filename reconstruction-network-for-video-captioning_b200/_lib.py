@@ -111,6 +111,9 @@ SIGNATURES = {
     "recnet_decoder_greedy": (_i, [C.POINTER(decoder_desc), C.POINTER(decoder_tensors), _p, _i, _p, _l, _p, _p, _p]),
     "recnet_beam_workspace_bytes": (_l, [C.POINTER(decoder_desc), _i, _i]),
     "recnet_decoder_beam": (_i, [C.POINTER(decoder_desc), C.POINTER(decoder_tensors), _p, _i, _i, _l, _p, _l, _p, _p, _p]),
+    "recnet_sample_workspace_bytes": (_l, [C.POINTER(decoder_desc), _i]),
+    "recnet_decoder_sample": (_i, [C.POINTER(decoder_desc), C.POINTER(decoder_tensors), _p, _i, _f, _l, _p, _p, _p, _l, _p, _p, _p, _p,
+                                   _p]),
     "recnet_local_workspace_bytes": (_l, [C.POINTER(local_desc)]),
     "recnet_local_fwd": (_i, [C.POINTER(local_desc), C.POINTER(local_tensors), _p, _p, _p, _p, _l, _p, _p]),
     "recnet_local_bwd": (_i, [C.POINTER(local_desc), C.POINTER(local_tensors), _p, _p, _p, _p, _l, _p,

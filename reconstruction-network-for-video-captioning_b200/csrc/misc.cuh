@@ -148,11 +148,12 @@ struct Stager {
   }
 };
 
-// Xe[r, c] = emb[tok[r], c] * scale * dropmask   (c < EMB), 0 for the K padding
+// Xe[r, c] = emb[tok[r], c] * scale * dropmask   (c < EMB), 0 for the K padding.  The mask of row r is that of row row0 + r of the
+// site's tensor: a decode loop gathers one step of B rows at a time, row0 = t * B.
 template <typename TO>
 __global__ void embed_gather_kernel(const float* __restrict__ emb, const long long* __restrict__ tok, TO* __restrict__ out,
                                     long long ld_out, int rows, int EMB, int EMBp, int V, float scale, float p_drop,
-                                    const unsigned long long* rng, unsigned int site) {
+                                    const unsigned long long* rng, unsigned int site, long long row0 = 0) {
   const int r = blockIdx.x;
   long long t = tok[r];
   if (t < 0 || t >= V) t = 0;
@@ -160,7 +161,7 @@ __global__ void embed_gather_kernel(const float* __restrict__ emb, const long lo
     float v = 0.f;
     if (c < EMB) {
       v = emb[t * EMB + c] * scale;
-      if (p_drop > 0.f) v *= dropout_scale(rng, site, (uint64_t)r * EMB + c, p_drop);
+      if (p_drop > 0.f) v *= dropout_scale(rng, site, (uint64_t)(row0 + r) * EMB + c, p_drop);
     }
     out[(long long)r * ld_out + c] = from_f32<TO>(v);
   }

@@ -400,6 +400,27 @@ int recnet_decoder_beam(const recnet_decoder_desc* d, const recnet_decoder_tenso
   });
 }
 
+int64_t recnet_sample_workspace_bytes(const recnet_decoder_desc* d, int max_steps) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
+  DecDesc d1 = dd; d1.L = 1;
+  RN_TRY(dec::check(d1));
+  if (max_steps < 1 || max_steps > 64) return RECNET_ERR_BAD_SHAPE;
+  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED,
+                          [&](auto t) { return (int64_t)dec::plan_sample<decltype(t)>(dd, nullptr, max_steps).bytes; });
+}
+int recnet_decoder_sample(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, int max_steps,
+                          float temperature, int64_t eos_id, const unsigned long long* rng, const unsigned long long* noise,
+                          void* workspace, int64_t workspace_bytes, int64_t* ids_out, float* logp_out, int32_t* lengths_out,
+                          int32_t* n_steps_out, void* stream) {
+  DecDesc dd;
+  RN_TRY(split_desc(d, &dd));
+  return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    return dec::sample<decltype(t)>(dd, *w, feats, max_steps, temperature, (long long)eos_id, rng, noise, workspace, workspace_bytes,
+                                    reinterpret_cast<long long*>(ids_out), logp_out, lengths_out, n_steps_out, ST(stream));
+  });
+}
+
 // ---- local reconstructor ---------------------------------------------------------------------------------------
 int64_t recnet_local_workspace_bytes(const recnet_local_desc* d) {
   LocalDesc dd;

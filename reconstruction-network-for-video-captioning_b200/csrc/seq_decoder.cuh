@@ -18,6 +18,7 @@ namespace dec {
 using namespace rt;
 
 enum : unsigned { SITE_EMB = 1, SITE_LOGITS = 2, SITE_LAYER0 = 16 };   // dropout site of the input of layer l = SITE_LAYER0 + l
+enum : unsigned { SITE_SAMPLE = 5 };                                     // Gumbel noise of the sampler (its own (seed, offset) pair)
 
 template <typename T>
 struct Ws {
@@ -723,6 +724,161 @@ static int beam(const DecDesc& d0, const recnet_decoder_tensors& p, const float*
     RN_LAUNCH_OK();
   }
   beam_finalize_kernel<<<1, 256, 0, st>>>(g.nonpad, max_steps, B0, K, bw.seq[0], bw.seq[1], seq_out, n_steps_out);
+  RN_LAUNCH_OK();
+  return 0;
+}
+
+// ---- sampling (Gumbel-max) as a device loop: stochastic decoding and the sampling half of self-critical training ----------------
+// Per step: the decoder step on all rows (the kernels of greedy, plus the training-mode dropout masks when desc.train is set), then
+// ONE selection kernel that draws a token per row from softmax(z' / tau) by Gumbel-max, z' = the logits after their dropout.  Every
+// dropout mask is drawn at the element index the sequence forward (dec::forward) uses for row t * B + row, so a teacher-forced pass
+// over the sampled tokens with the same dropout pair differentiates the logits the sampler drew from.  A row finishes once it emits
+// <EOS> or <PAD>; after that it emits and feeds back <PAD> with log-prob 0, so a row of samples has the shape of a `targets` column.
+constexpr int SAMPLE_THREADS = 256;
+
+// -log(u) for u = ((w >> 8) + 0.5) 2^-24 in (0, 1), without rounding u itself: for u >= 1/2, 1 - u is exact in fp32 but u is not
+// (u = 1 - 2^-25 would round to 1 and make the Gumbel noise -log(-log u) infinite).
+__device__ __forceinline__ float neg_log_uniform(uint32_t w) {
+  const uint32_t k = w >> 8;
+  if (k < (1u << 23)) return -logf(((float)k + 0.5f) * (1.0f / 16777216.0f));
+  return -log1pf(-((float)((1u << 24) - 1u - k) + 0.5f) * (1.0f / 16777216.0f));
+}
+// (max, sum exp(x - max)) of a union of two parts
+__device__ __forceinline__ void lse_merge(float& m, float& s, float om, float os) {
+  const float M = fmaxf(m, om);
+  if (M == -INFINITY) return;
+  s = s * expf(m - M) + os * expf(om - M);
+  m = M;
+}
+__device__ __forceinline__ void sample_reduce_step(float& best, int& bi, float& bx, float& m, float& s, int o) {
+  const float ob = __shfl_xor_sync(0xffffffffu, best, o), ox = __shfl_xor_sync(0xffffffffu, bx, o);
+  const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+  if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; bx = ox; }
+  const float om = __shfl_xor_sync(0xffffffffu, m, o), os = __shfl_xor_sync(0xffffffffu, s, o);
+  lse_merge(m, s, om, os);
+}
+
+// One CTA per row, one pass over its V logits: training-mode dropout (site SITE_LOGITS), / tau, + Gumbel noise (site SITE_SAMPLE of the
+// `noise` pair), both at element (t * B + row) * V + v with one Philox call per 4 elements; arg-max of the noisy value (lowest index
+// wins ties) and, in the same pass, the running max / sum-exp of z' / tau for log softmax(z' / tau)[chosen].  live[t] counts the rows
+// still unfinished after step t; once it is 0 the remaining steps change nothing.
+__global__ void __launch_bounds__(SAMPLE_THREADS) sample_select_kernel(
+    const float* __restrict__ logits, long long ld, int V, int B, int t, float tau, long long eos, float p_drop,
+    const unsigned long long* __restrict__ rng, const unsigned long long* __restrict__ noise, long long* __restrict__ ids_t,
+    float* __restrict__ logp_t, long long* __restrict__ tok, int* __restrict__ finished, int* __restrict__ lengths,
+    int* __restrict__ live) {
+  if (t > 0 && live[t - 1] == 0) return;                     // frozen: every row has finished
+  const int row = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (finished[row]) {                                       // ids / logp of this step stay 0 (cleared by the driver)
+    if (tid == 0) tok[row] = 0;
+    return;
+  }
+  __shared__ float sb[SAMPLE_THREADS / 32], sx[SAMPLE_THREADS / 32], sm[SAMPLE_THREADS / 32], ss[SAMPLE_THREADS / 32];
+  __shared__ int si[SAMPLE_THREADS / 32];
+  const float* z = logits + (long long)row * ld;
+  const long long base = ((long long)t * B + row) * V;
+  const long long q0 = base >> 2, nq = ((base + V - 1) >> 2) - q0 + 1;
+  const bool drop = p_drop > 0.f;
+  const Philox dph(drop ? rng[0] : 0ull), nph(noise[0]);
+  const unsigned long long dstream = drop ? (rng[1] << 8) | SITE_LOGITS : 0ull, nstream = (noise[1] << 8) | SITE_SAMPLE;
+  const float keep = 1.f / (1.f - p_drop);
+  float best = -INFINITY, bx = 0.f, m = -INFINITY, s = 0.f;
+  int bi = 0x7fffffff;
+  for (long long q = tid; q < nq; q += SAMPLE_THREADS) {
+    const unsigned long long ctr = (unsigned long long)(q0 + q);
+    const uint4 n4 = nph(ctr, nstream);
+    const uint4 d4 = drop ? dph(ctr, dstream) : make_uint4(0u, 0u, 0u, 0u);
+    const uint32_t nw[4] = {n4.x, n4.y, n4.z, n4.w}, dw[4] = {d4.x, d4.y, d4.z, d4.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const long long v = 4 * (q0 + q) + j - base;
+      if (v < 0 || v >= V) continue;
+      float x = z[v];
+      if (drop) x *= ((float)(dw[j] >> 8) * (1.0f / 16777216.0f) >= p_drop) ? keep : 0.f;
+      x = x / tau;
+      const float y = x - logf(neg_log_uniform(nw[j]));
+      if (y > best) { best = y; bi = (int)v; bx = x; }      // v grows within a thread: strict > keeps the lowest index
+      if (x > m) { s = s * expf(m - x) + 1.f; m = x; } else { s += expf(x - m); }
+    }
+  }
+  for (int o = 16; o > 0; o >>= 1) sample_reduce_step(best, bi, bx, m, s, o);
+  if (lane == 0) { sb[warp] = best; si[warp] = bi; sx[warp] = bx; sm[warp] = m; ss[warp] = s; }
+  __syncthreads();
+  if (warp) return;
+  const bool ok = lane < SAMPLE_THREADS / 32;
+  best = ok ? sb[lane] : -INFINITY; bi = ok ? si[lane] : 0x7fffffff; bx = ok ? sx[lane] : 0.f;
+  m = ok ? sm[lane] : -INFINITY; s = ok ? ss[lane] : 0.f;
+  for (int o = 16; o > 0; o >>= 1) sample_reduce_step(best, bi, bx, m, s, o);
+  if (lane == 0) {
+    ids_t[row] = bi;
+    logp_t[row] = bx - (m + logf(s));
+    tok[row] = bi;
+    if (bi == eos || bi == 0) { finished[row] = 1; lengths[row] = t + 1; }
+    else atomicAdd(live + t, 1);
+  }
+}
+__global__ void sample_init_kernel(long long* tok, int* finished, int* lengths, int n, int max_steps) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) { tok[i] = 1; finished[i] = 0; lengths[i] = max_steps; }    // <SOS>; a row that never finishes has max_steps tokens
+}
+
+template <typename T>
+struct SampleWs { GreedyWs<T> g; int* finished; size_t bytes; };
+template <typename T>
+static SampleWs<T> plan_sample(const recnet_decoder_desc& d, void* base, int max_steps) {
+  SampleWs<T> s;
+  s.g = plan_greedy<T>(d, base, max_steps);
+  Bump m(base); m.off = s.g.bytes;
+  s.finished = m.take<int>((size_t)d.B);
+  s.bytes = m.off + 256;
+  return s;
+}
+
+// ids_out / logp_out [max_steps, B], lengths_out [B] = sampled tokens of the row, the finishing one included; n_steps_out = the step at
+// which the last row finished + 1 (max_steps if a row never finishes).  rng = the dropout pair (read when d0.train is set),
+// noise = the Gumbel pair.  Always the general step path: greedy_pf hoists the embedding projection and could not drop the embedding.
+template <typename T>
+static int sample(const DecDesc& d0, const recnet_decoder_tensors& p, const float* feats, int max_steps, float tau, long long eos,
+                  const unsigned long long* rng, const unsigned long long* noise, void* ws, long long ws_bytes, long long* ids_out,
+                  float* logp_out, int* lengths_out, int* n_steps_out, cudaStream_t st) {
+  DecDesc d = d0; d.L = 1;
+  RN_TRY(check(d));
+  if (max_steps < 1 || max_steps > 64 || !(tau > 0.f) || !noise || (d.train && !rng)) return RECNET_ERR_BAD_SHAPE;
+  SampleWs<T> sw = plan_sample<T>(d0, ws, max_steps);
+  if ((long long)sw.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
+  GreedyWs<T>& g = sw.g;
+  Ws<T>& w = g.w;
+  const int B = d.B, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, NL = w.NL;
+  const float p_emb = d.train ? d.p_emb_drop : 0.f, p_out = d.train ? d.p_out_drop : 0.f, p_lay = d.train ? d.p_layer_drop : 0.f;
+  RN_TRY(prepare<T>(d, p, feats, w, st));
+  RN_TRY(gemm_full<T>(w.feats, E, 0, w.U, E, 0, w.Uv, A, nullptr, B * Tn, A, E, 0, w.splitk, st));
+  RN_TRY(zero_decode_state<T>(d, w, st));
+  RN_CUDA_OK(cudaMemsetAsync(g.nonpad, 0, (size_t)max_steps * sizeof(int), st));        // live rows per step
+  RN_CUDA_OK(cudaMemsetAsync(ids_out, 0, (size_t)max_steps * B * sizeof(long long), st));
+  RN_CUDA_OK(cudaMemsetAsync(logp_out, 0, (size_t)max_steps * B * sizeof(float), st));
+  sample_init_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(g.tok, sw.finished, lengths_out, B, max_steps);
+  RN_LAUNCH_OK();
+  long long ldq;
+  const T* Htop = top_h(d, w, &ldq);
+  for (int t = 0; t < max_steps; ++t) {                      // the ping-pong of greedy
+    const int rd = t & 1, wr = (t + 1) & 1;
+    T* x_t = w.X + (size_t)rd * B * w.KX;
+    T* x_n = w.X + (size_t)wr * B * w.KX;
+    float* c_p = w.c + (size_t)rd * B * H;
+    float* c_n = w.c + (size_t)wr * B * H;
+    misc::embed_gather_kernel<T><<<B, 128, 0, st>>>(p.embedding, g.tok, w.Xe, w.EMBp, B, d.EMB, w.EMBp, V, d.embedding_scale, p_emb,
+                                                    rng, SITE_EMB, (long long)t * B);
+    RN_LAUNCH_OK();
+    RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
+    RN_TRY(step<T>(d, p, w, t, Htop + (size_t)rd * B * ldq, ldq, w.Gx, x_t, x_n, nullptr, nullptr, nullptr, c_p, c_n,
+                   d.cell == RECNET_CELL_GRU ? c_n : g.h_scratch, st, NL > 1 ? w.X_x[0] + (size_t)rd * B * 2 * H : nullptr, rng));
+    RN_TRY(upper_layers<T>(d, p, w, t, rd, wr, nullptr, p_lay, rng, st));
+    RN_TRY(gemm_full<T>(Htop + (size_t)wr * B * ldq, ldq, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
+    sample_select_kernel<<<B, SAMPLE_THREADS, 0, st>>>(w.logits, w.Vld, V, B, t, tau, eos, p_out, rng, noise, ids_out + (size_t)t * B,
+                                                       logp_out + (size_t)t * B, g.tok, sw.finished, lengths_out, g.nonpad);
+    RN_LAUNCH_OK();
+  }
+  greedy_finalize_kernel<<<1, 1, 0, st>>>(g.nonpad, max_steps, n_steps_out);   // first step with no live row, + 1
   RN_LAUNCH_OK();
   return 0;
 }

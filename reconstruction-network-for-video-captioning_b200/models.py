@@ -293,6 +293,54 @@ class Decoder(nn.Module, _RngMixin):
                                         seqs.data_ptr(), n.data_ptr(), Fn._stream()), "recnet_decoder_beam")
         return seqs, n
 
+    @torch.no_grad()
+    def sample(self, encoder_outputs, n_samples=1, *, max_steps, temperature=1.0, eos_id=2, seed=None):
+        """Stochastic decoding on the device, ONE C call (recnet_decoder_sample): each row draws its tokens from
+        softmax(logits / temperature) by Gumbel-max until it emits <EOS> (or <PAD>), then emits <PAD>.  In train mode the logits are
+        those of the module's training forward, dropout included (one ``_next_rng()`` per call), so ``forward_sequence`` over
+        ``[<SOS>; ids[:-1]]`` with that dropout pair differentiates exactly the distribution the tokens were drawn from.
+        Rows are tiled like ``beam``: row k * B0 + b is sample k of video b.  The Gumbel noise pair is (seed, 0), or drawn from torch's
+        default generator when ``seed`` is None (reproducible under ``torch.manual_seed``, different on every call).
+        Returns (ids (max_steps, K*B0) int64, logp (max_steps, K*B0) f32 = log-prob of each id (0 after the row finished),
+        lengths (K*B0,) int32 = tokens up to and including the finishing one, n device int32 = steps until every row finished)."""
+        if not self.uses_fused_sequence:
+            raise NotImplementedError(f"Decoder.sample: no device sampler for a {self.n_layers}-layer {self.model_name} decoder "
+                                      f"(LSTM with 1-{L.MAX_LAYERS} layers and single-layer GRU have one)")
+        if seed is None:
+            noise = torch.randint(0, 2 ** 62, (2,), dtype=torch.int64)
+        else:
+            noise = torch.tensor([int(seed), 0], dtype=torch.int64)
+        feats = Fn._f32c(encoder_outputs, "encoder_outputs")
+        tiled = feats.repeat(int(n_samples), 1, 1).contiguous()
+        return self._sample(tiled, max_steps, temperature, eos_id, noise.to(feats.device))
+
+    def _sample(self, feats, max_steps, temperature, eos_id, noise):
+        """``sample`` on rows that are already tiled, with the Gumbel (seed, offset) pair `noise` given as a device int64 (2,) tensor."""
+        import ctypes as C
+        lib = L.lib()
+        N, T, E = feats.shape
+        meta = self._meta()
+        d = L.decoder_desc(B=N, T=T, E=E, H=meta["H"], A=meta["A"], EMB=meta["EMB"], V=meta["V"], L=1,
+                           precision=meta["precision"], train=int(self.training), embedding_scale=float(meta["embedding_scale"]),
+                           p_emb_drop=float(meta["p_emb"]), p_out_drop=float(meta["p_out"]), cell=meta["cell"], n_layers=self.n_layers,
+                           p_layer_drop=float(meta["p_layer"]))
+        nbytes = lib.recnet_sample_workspace_bytes(C.byref(d), int(max_steps))
+        if nbytes < 0:
+            L.check(int(nbytes), "recnet_sample_workspace_bytes")
+        dev = feats.device
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        ids = torch.empty(max_steps, N, dtype=torch.int64, device=dev)
+        logp = torch.empty(max_steps, N, dtype=torch.float32, device=dev)
+        lengths = torch.empty(N, dtype=torch.int32, device=dev)
+        n = torch.zeros(1, dtype=torch.int32, device=dev)
+        rng = self._next_rng() if self.training else None
+        params = tuple(Fn._f32c(p, "param") for p in self._params())
+        w = Fn._pack(L.decoder_tensors, params)
+        L.check(lib.recnet_decoder_sample(C.byref(d), C.byref(w), feats.data_ptr(), int(max_steps), float(temperature), int(eos_id),
+                                          Fn._ptr(rng), noise.data_ptr(), ws.data_ptr(), nbytes, ids.data_ptr(), logp.data_ptr(),
+                                          lengths.data_ptr(), n.data_ptr(), Fn._stream()), "recnet_decoder_sample")
+        return ids, logp, lengths, n
+
     # ---- single timestep (reference API) ----
     def forward(self, input, hidden, encoder_outputs):
         """input (1,B) int64; hidden ((NL,B,H),(NL,B,H)) [LSTM] or (NL,B,H) [GRU]; encoder_outputs (B,T,E) -> (logits (B,V), hidden)."""

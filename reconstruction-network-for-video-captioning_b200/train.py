@@ -76,6 +76,48 @@ def forward_decoder(decoder, encoder_outputs, targets, target_masks, teacher_for
     return loss, hiddens, output_indices                                                                    # (L,NL,B,H), train.py:73-75
 
 
+def self_critical_weights(rewards, baseline, lengths, n_steps):
+    """ce_weight (n_steps, K*B0) of self-critical training: (rewards[row] - baseline[row % B0]) * [t < lengths[row]] / (K*B0).
+    With it the cross entropy of forward_sequence is -sum_row advantage_row / N * sum_t log p(ids[t, row]), the policy-gradient loss."""
+    N = rewards.shape[0]
+    B0 = baseline.shape[0]
+    adv = rewards.float() - baseline.float().repeat(N // B0)                      # row k * B0 + b is sample k of video b
+    steps = torch.arange(n_steps, device=lengths.device).unsqueeze(1)
+    mask = (steps < lengths.long().unsqueeze(0)).float()
+    return mask * (adv / N).unsqueeze(0), adv
+
+
+def forward_decoder_self_critical(decoder, encoder_outputs, reward_fn, n_samples=1, temperature=1.0, max_steps=None):
+    """Self-critical sequence training (Rennie et al., 2017), one forward: sample ``n_samples`` captions per video on the device in the
+    module's current mode (``Decoder.sample``), decode the greedy baseline (``Decoder.greedy``), score both with
+    ``reward_fn(sample_ids (n, K*B0), greedy_ids (max_steps, B0)) -> (rewards (K*B0,), baseline (B0,))``, then replay the samples
+    through the fused sequence kernels with ce_weight = advantage * step mask / (K*B0) (``self_critical_weights``), the dropout pair
+    the sampler read and ``+ lambda_reg * reg`` as in ``forward_decoder``.  Returns (loss, hiddens (n, NL, K*B0, H), info) with info =
+    {rewards, baseline, advantage, ids, lengths, logp}; the caller runs backward and the optimiser step (or adds a reconstructor loss on
+    ``hiddens`` over the features tiled K times) as in ``train_step``.
+    The replay computes the sampler's logits again with other kernels: in fp32 they agree to fp32 rounding; in bf16 the replay runs
+    the training kernels (the cluster / projected-feature loop and the batched vocabulary GEMM) rather than the sampler's per-step
+    kernels, so they agree to bf16 rounding only."""
+    sos_id, eos_id = C.init_word2idx['<SOS>'], C.init_word2idx['<EOS>']
+    model = decoder['model']
+    L = max_steps if max_steps is not None else C.caption_max_len + 1
+    K = int(n_samples)
+    ids, logp, lengths, n = model.sample(encoder_outputs, K, max_steps=L, temperature=temperature, eos_id=eos_id)
+    rng = model._rng.clone()               # the pair the sampler read; the buffer itself moves on with the next training forward
+    greedy_ids, _ = model.greedy(encoder_outputs, L)
+    n = int(n)
+    ids, logp = ids[:n], logp[:n]
+    rewards, baseline = reward_fn(ids, greedy_ids)
+    ce_weight, adv = self_critical_weights(rewards, baseline, lengths, n)
+    N = ids.shape[1]
+    tokens_in = torch.cat((torch.full((1, N), sos_id, dtype=torch.long, device=ids.device), ids[:-1]), dim=0)
+    meta = model._meta()
+    meta["lambda_reg"] = decoder['lambda_reg']
+    feats = encoder_outputs.repeat(K, 1, 1).contiguous()
+    loss, hiddens, _ = Fn.DecoderSequenceFn.apply(meta, feats, tokens_in, ids, ce_weight.contiguous(), rng, *model._params())
+    return loss, hiddens, {"rewards": rewards, "baseline": baseline, "advantage": adv, "ids": ids, "lengths": lengths, "logp": logp}
+
+
 def forward_global_reconstructor(decoder_hiddens, encoder_outputs, reconstructor):
     """train.py:78-105."""
     model = reconstructor['model']
