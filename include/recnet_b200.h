@@ -327,6 +327,33 @@ int recnet_param_norms_bwd(const int64_t* ptrs, const int64_t* grad_ptrs, const 
 
 /* Teacher-forcing inputs of train.forward_decoder in one launch (train.py:25,44-45,54-60,68): targets (>= L rows of B int64,
  * row-major) -> tokens_in [L,B] = (<SOS> row, targets[0..L-2]) and ce_weight [L,B] = [target > pad] / (max(n_t,1) * sum_t n_t). */
+/* CIDEr-D (coco-caption's CiderD: n = 1..4, sigma = 6, document frequencies from the reference corpus) of id captions against a
+ * reference corpus, on the device.  The corpus is a host struct of device arrays, built once on the host (recnet_b200.cider.CiderCorpus):
+ * an n-gram of ids a_1..a_n (each in 1..65535) is the key sum_j a_j << (64 - 16 j), so the order n is implied by the zero padding. */
+typedef struct {
+  int32_t n_videos;               /* >= 1 */
+  int32_t n_df;                   /* distinct n-grams over all references */
+  int32_t vocab;                  /* ids of the corpus are below this; > 65536 is RECNET_ERR_UNSUPPORTED */
+  float ref_len;                  /* log(n_videos) */
+  const uint64_t* df_keys;        /* [n_df] ascending */
+  const float* df_log;            /* [n_df] log(max(1, number of videos whose references contain the n-gram)) */
+  const int32_t* video_refs;      /* [n_videos + 1] reference range of each video (CSR) */
+  const int32_t* ref_entries;     /* [n_refs + 1] entry range of each reference (CSR) */
+  const uint64_t* entry_keys;     /* [n_entries] the reference's n-grams, ascending within each reference */
+  const float* entry_w;           /* [n_entries] count * (ref_len - df_log) */
+  const float* ref_norm;          /* [n_refs, 4] L2 norm of each order's weights */
+  const int32_t* ref_length;      /* [n_refs] bigram count (coco-caption's CiderScorer.counts2vec length) */
+} recnet_cider_corpus;
+
+/* scores_out[r] = CIDEr-D of candidate row r against the references of video video_of_row[r], r < n_rows.  Token t of row r is
+ * ids[t * ld_step + r * ld_row] (strides in elements: a time-major (steps, N) tensor and a batch-major (N, steps) one both read in
+ * place); the caption is the ids before the first eos_id, <PAD> (0) or negative id, at most `steps`.  A row whose caption holds an id
+ * above 65535, or whose video is outside 0..n_videos-1, scores NaN.  One warp per row, fixed reduction order: no atomics, so the
+ * scores are the same bit for bit from run to run.  All pointers but `c` are device pointers.  steps outside 1..64 or n_rows <= 0:
+ * RECNET_ERR_BAD_SHAPE; c->vocab > 65536: RECNET_ERR_UNSUPPORTED (both before any launch). */
+int recnet_cider_d(const recnet_cider_corpus* c, const int64_t* ids, int64_t ld_step, int64_t ld_row, int steps, int n_rows,
+                   const int32_t* video_of_row, int64_t eos_id, float* scores_out, void* stream);
+
 int recnet_teacher_forcing_prep(const int64_t* targets, int L, int B, int64_t pad, int64_t sos, int64_t* tokens_in,
                                 float* ce_weight, void* stream);
 

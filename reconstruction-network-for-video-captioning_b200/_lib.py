@@ -77,6 +77,12 @@ class global_tensors(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in FIELDS]
 
 
+class cider_corpus(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("n_videos", "n_df", "vocab")] + [("ref_len", C.c_float)] + \
+               [(n, C.c_void_p) for n in ("df_keys", "df_log", "video_refs", "ref_entries", "entry_keys", "entry_w", "ref_norm",
+                                          "ref_length")]
+
+
 _p, _i, _l, _f, _u, _d = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_uint32, C.c_double
 
 # name -> (restype, argtypes); mirrors include/recnet_b200.h one to one
@@ -136,6 +142,7 @@ SIGNATURES = {
     "recnet_param_norms_partial": (_i, [_p, _p, _p, _p, _i, _p, _p]),
     "recnet_param_norms_finalize": (_i, [_p, _p, _i, _i, _p, _p, _p, _p, _p, _p]),
     "recnet_param_norms_bwd": (_i, [_p, _p, _p, _i, _p, _p, _i, _p, _p, _f, _p, _i, _p]),
+    "recnet_cider_d": (_i, [C.POINTER(cider_corpus), _p, _l, _l, _i, _i, _p, _l, _p, _p]),
     "recnet_teacher_forcing_prep": (_i, [_p, _i, _i, _l, _l, _p, _p, _p]),
     "recnet_allreduce_avg": (_i, [_p, _p, _p, _p, _p, _p, _p, _l, _l, _i, _i, _i, _p]),
     "recnet_adam_step": (_i, [_p, _p, _p, _p, _p, _p, _i, _p, _p, _i, _d, _d, _d, _d, _d, _d, _p, _p, _i, _p]),

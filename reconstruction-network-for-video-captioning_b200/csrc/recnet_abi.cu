@@ -5,6 +5,7 @@
 #include "seq_recon.cuh"
 #include "optim.cuh"
 #include "allreduce.cuh"
+#include "cider.cuh"
 
 #define ST(s) reinterpret_cast<cudaStream_t>(s)
 
@@ -538,6 +539,14 @@ int recnet_param_norms_bwd(const int64_t* ptrs, const int64_t* grad_ptrs, const 
 }
 
 // ---- teacher-forcing inputs (train.py:25,44-45,54-60,68) ----------------------------------------------------------
+int recnet_cider_d(const recnet_cider_corpus* c, const int64_t* ids, int64_t ld_step, int64_t ld_row, int steps, int n_rows,
+                   const int32_t* video_of_row, int64_t eos_id, float* scores_out, void* stream) {
+  if (!c || c->n_videos < 1 || steps < 1 || steps > cider::kMaxSteps || n_rows <= 0) return RECNET_ERR_BAD_SHAPE;
+  if (c->vocab > 65536) return RECNET_ERR_UNSUPPORTED;
+  return cider::launch(*c, reinterpret_cast<const long long*>(ids), (long long)ld_step, (long long)ld_row, steps, n_rows, video_of_row,
+                       (long long)eos_id, scores_out, ST(stream));
+}
+
 int recnet_teacher_forcing_prep(const int64_t* targets, int L, int B, int64_t pad, int64_t sos, int64_t* tokens_in, float* ce_weight,
                                 void* stream) {
   if (L < 1 || B < 1 || !targets || !tokens_in || !ce_weight) return RECNET_ERR_BAD_SHAPE;

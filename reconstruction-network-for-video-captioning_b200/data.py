@@ -32,6 +32,25 @@ def synthetic_batch(B, T, E, V, caption_max_len=30, seed=1234, full_length_first
     return feats, targets, targets > PAD
 
 
+def synthetic_captions(n_videos, n_refs, V, seed, min_len=3, max_len=30, zipf=1.0):
+    """Seeded MSVD-shaped reference captions for CIDEr-D: ``n_refs`` per video, lengths uniform in [min_len, max_len], word ids 3..V-1
+    drawn with Zipf weights 1 / rank^zipf (frequent words recur across videos, as in real captions), each ended by <EOS>.
+    Returns refs[video][ref] = int64 numpy array."""
+    rng = np.random.default_rng(seed)
+    p = 1.0 / np.arange(1, V - 2, dtype=np.float64) ** zipf
+    p /= p.sum()
+    lens = rng.integers(min_len, max_len + 1, size=(n_videos, n_refs))
+    words = rng.choice(np.arange(3, V, dtype=np.int64), size=int(lens.sum()), p=p)
+    refs, k = [], 0
+    for v in range(n_videos):
+        rs = []
+        for n in lens[v]:
+            rs.append(np.append(words[k:k + n], EOS))
+            k += n
+        refs.append(rs)
+    return refs
+
+
 def shard_range(n_items: int, rank: int, world: int):
     """Contiguous shard [lo, hi) of n_items for `rank` of `world` (remainder spread over the first ranks)."""
     base, rem = divmod(n_items, world)
