@@ -287,6 +287,9 @@ int recnet_global_bwd(const recnet_global_desc* d, const recnet_global_tensors* 
                       const uint64_t* rng, void* workspace, int64_t workspace_bytes, const float* g_loss,
                       const recnet_global_tensors* grads, float* g_hiddens, void* stream);
 float* recnet_global_outputs(const recnet_global_desc* d, void* workspace);  /* [L,B,R] fp32 */
+/* Host-only: the same 12 ints as recnet_plan_persistent_loops for a global-reconstructor call, whose loops run the local kernels in
+ * global mode (no attention, operand rows hold h only): column groups are R / 128. */
+int recnet_plan_global_loops(const recnet_global_desc* d, int32_t* out);
 
 /* The weight-resident time loops of the bf16 build (local reconstructor, LSTM, MSVD-class shapes) run as ONE persistent
  * cooperative kernel per loop (csrc/seq_recon_persist.cuh): [W_ih | W_hh] stays in the shared memory of 144 CTAs for all steps

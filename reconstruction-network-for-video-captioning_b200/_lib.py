@@ -133,6 +133,7 @@ SIGNATURES = {
     "recnet_global_bwd": (_i, [C.POINTER(global_desc), C.POINTER(global_tensors), _p, _p, _p, _p, _l, _p,
                                C.POINTER(global_tensors), _p, _p]),
     "recnet_global_outputs": (_p, [C.POINTER(global_desc), _p]),
+    "recnet_plan_global_loops": (_i, [C.POINTER(global_desc), _p]),
     "recnet_decoder_error_offset": (_l, [C.POINTER(decoder_desc)]),
     "recnet_local_error_offset": (_l, [C.POINTER(local_desc)]),
     "recnet_global_error_offset": (_l, [C.POINTER(global_desc)]),

@@ -498,6 +498,22 @@ float* recnet_global_outputs(const recnet_global_desc* d, void* workspace) {
   if (check_desc(d)) return nullptr;
   return by_prec<float*>(d->precision, nullptr, [&](auto t) { return rec::plan_global<decltype(t)>(*d, workspace).out; });
 }
+int recnet_plan_global_loops(const recnet_global_desc* d, int32_t* out) {
+  // layout of recnet_plan_persistent_loops at H = 0, coverage by the global rules (global_forward / global_backward launch these)
+  if (!out) return RECNET_ERR_BAD_SHAPE;
+  RN_TRY(check_desc(d));
+  for (int i = 0; i < 12; ++i) out[i] = 0;
+  if (d->precision != RECNET_PREC_BF16) return 0;
+  if (rec::persist_global_ok<bf16>(*d, false)) {
+    const int ks = rp::pick_ks(d->R, 0), res = rp::max_res_kb_fwd(d->R, 0, ks);
+    out[0] = 1; out[1] = ks; out[2] = d->R / rp::UNITS; out[3] = res; out[4] = rp::pick_stages_fwd(d->B, ks, res); out[5] = out[2] * ks;
+  }
+  if (rec::persist_global_ok<bf16>(*d, true)) {
+    const int ns = rp::pick_ns(d->R, 0), res = (4 * d->R / rp::BK + ns - 1) / ns;
+    out[6] = 1; out[7] = ns; out[8] = d->R / 128; out[9] = res; out[10] = rp::pick_stages_bwd(d->B, res); out[11] = out[8] * ns;
+  }
+  return 0;
+}
 
 // ---- regulariser -----------------------------------------------------------------------------------------------
 int recnet_param_norms_fwd(const int64_t* ptrs, const int64_t* sizes, int n, const int32_t* blk_tensor, const int32_t* blk_chunk,

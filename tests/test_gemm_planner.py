@@ -6,6 +6,7 @@ import pytest
 
 import recnet_b200  # noqa: F401
 from recnet_b200 import _lib as L
+from tests.test_gpu_loop_shapes import REC_CASES as LOOP_CASES
 
 B, T, E, H, A, V, Lr, R = 100, 28, 1536, 512, 128, 4188, 31, 1536
 LB, BT, SB, GR = Lr * B, B * T, 28 * B, 4 * R
@@ -90,6 +91,48 @@ def test_persistent_loop_layout_of_the_msvd_shape():
 def test_shapes_outside_the_persistent_loops_take_the_kernel_per_phase_path(kw):
     o = _loops(**kw)
     assert o[0] == 0 and o[6] == 0, (kw, o)
+
+
+def _global_loops(B, L_, R, H):
+    d = L.global_desc(B=B, L=L_, R=R, H=H, T=28, precision=L.PREC_BF16, train=1, p_drop=0.5, caption_max_len=30.0, cell=L.CELL_LSTM,
+                      dec_layers=1)
+    out = (C.c_int32 * 12)()
+    L.check(L.lib().recnet_plan_global_loops(C.byref(d), out), "recnet_plan_global_loops")
+    return list(out)
+
+
+@pytest.mark.parametrize("cid", sorted(LOOP_CASES))
+def test_loop_shape_cases_keep_the_layout_the_gpu_tests_expect(cid):
+    """tests/test_gpu_loop_shapes.py asserts on the GPU which loop each case runs and with how many CTAs; the planners decide that on the
+    host, so a planner change that moves a case fails here first."""
+    c = LOOP_CASES[cid]
+    if c.kind == "local":
+        o = _loops(B=c.B, S=c.S, R=c.R, H=c.H, A=128, L=c.L)
+    else:
+        o = _global_loops(c.B, c.L, c.R, c.H)
+    assert (bool(o[0]), bool(o[6])) == (c.fwd is not None, c.bwd is not None), (cid, o)
+    if c.fwd:
+        assert (o[1], o[5]) == c.fwd and o[5] == o[2] * o[1] <= 148 and o[4] >= 2, (cid, o)
+    if c.bwd:
+        assert (o[7], o[11]) == c.bwd and o[11] == o[8] * o[7] <= 148 and o[10] >= 2, (cid, o)
+
+
+def test_loop_shape_cases_reach_the_edges_they_are_named_for():
+    R3, R4, R5, G2 = (LOOP_CASES[k] for k in ("R3", "R4", "R5", "G2"))
+    assert _loops(B=R3.B, R=R3.R, H=R3.H)[4] == 2                                   # 2-stage ring at B > 112
+    assert R4.B == 128 and R4.L == 32
+    assert R5.B == R5.fwd[1] and _loops(B=R5.B + 1, R=R5.R, H=R5.H)[0] == 0        # B = UG x KS is the local forward's last batch
+    assert G2.B > G2.fwd[1] and _loops(B=G2.B, R=G2.R, H=0, L=G2.L)[0] == 0       # only global mode runs B > UG x KS
+    assert _global_loops(129, 31, 1536, 512)[0] == 0 and _global_loops(129, 31, 1536, 512)[6] == 0
+
+
+def test_global_loop_probe_rejects_bad_descriptors():
+    out = (C.c_int32 * 12)()
+    assert L.lib().recnet_plan_global_loops(None, out) < 0
+    d = L.global_desc(B=8, L=4, R=512, H=128, T=4, precision=7, train=0, p_drop=0.0, caption_max_len=30.0, cell=L.CELL_LSTM, dec_layers=1)
+    assert L.lib().recnet_plan_global_loops(C.byref(d), out) == -4                 # RECNET_ERR_UNSUPPORTED
+    d.precision = L.PREC_FP32
+    assert L.lib().recnet_plan_global_loops(C.byref(d), out) == 0 and list(out) == [0] * 12
 
 
 def test_smaller_batches_and_widths_stay_covered():
