@@ -336,7 +336,7 @@ int64_t recnet_greedy_workspace_bytes(const recnet_decoder_desc* d) {
   RN_TRY(split_desc(d, &dd));
   return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
     using T = decltype(t);
-    const int64_t a = (int64_t)dec::plan_greedy<T>(dd, nullptr, 64).bytes;
+    const int64_t a = (int64_t)dec::plan_decode<T>(dd, nullptr, dec::DecodeMode::GREEDY, 64).bytes;
     if constexpr (std::is_same<T, bf16>::value) {      // room for either bf16 driver: recnet_decoder_greedy picks one per call
       const int64_t b = dec::greedy_pf_ok(dd) ? (int64_t)dec::plan_greedy_pf<bf16>(dd, nullptr, 64).bytes : 0;
       return a > b ? a : b;
@@ -348,17 +348,18 @@ int recnet_decoder_greedy(const recnet_decoder_desc* d, const recnet_decoder_ten
                           void* workspace, int64_t workspace_bytes, int64_t* ids_out, int32_t* n_steps_out, void* stream) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
-  if (max_steps < 1 || max_steps > 64) return RECNET_ERR_BAD_SHAPE;
+  RN_TRY(dec::check_decode(&dd, dec::DecodeMode::GREEDY, 1, max_steps, 1.f, nullptr, nullptr));
   long long* ids = reinterpret_cast<long long*>(ids_out);
   return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
     using T = decltype(t);
     if constexpr (std::is_same<T, bf16>::value) {
       DecDesc d1 = dd; d1.L = 1; d1.train = 0;
-      // softmax decoders keep dec::greedy: moving them onto greedy_pf changes their launches and needs its own measurement
+      // softmax decoders keep dec::decode: moving them onto greedy_pf changes their launches and needs its own measurement
       if (dec::greedy_pf_ok(d1) && !dd.softmax)      // projected-feature kernels, 4 launches per step
         return dec::greedy_pf(dd, *w, feats, max_steps, workspace, workspace_bytes, ids, n_steps_out, ST(stream));
     }
-    return dec::greedy<T>(dd, *w, feats, max_steps, workspace, workspace_bytes, ids, n_steps_out, ST(stream));
+    return dec::decode<T>(dd, *w, feats, dec::DecodeMode::GREEDY, 1, max_steps, 1.f, 0, nullptr, nullptr, workspace, workspace_bytes,
+                          ids, nullptr, nullptr, n_steps_out, ST(stream));
   });
 }
 
@@ -387,28 +388,31 @@ int64_t recnet_global_error_offset(const recnet_global_desc* d) {
 int64_t recnet_beam_workspace_bytes(const recnet_decoder_desc* d, int beam_width, int max_steps) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
-  if (beam_width < 1 || beam_width > dec::BEAM_MAX_K || max_steps < 1 || max_steps > 64) return RECNET_ERR_BAD_SHAPE;
-  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED,
-                          [&](auto t) { return (int64_t)dec::plan_beam<decltype(t)>(dd, nullptr, beam_width, max_steps).bytes; });
+  RN_TRY(dec::check_decode(nullptr, dec::DecodeMode::BEAM, beam_width, max_steps, 1.f, nullptr, nullptr));
+  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    return (int64_t)dec::plan_decode<decltype(t)>(dd, nullptr, dec::DecodeMode::BEAM, max_steps).bytes;
+  });
 }
 int recnet_decoder_beam(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats_tiled, int beam_width, int max_steps,
                         int64_t eos_id, void* workspace, int64_t workspace_bytes, int64_t* seq_out, int32_t* n_steps_out, void* stream) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
+  RN_TRY(dec::check_decode(&dd, dec::DecodeMode::BEAM, beam_width, max_steps, 1.f, nullptr, nullptr));
   return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
-    return dec::beam<decltype(t)>(dd, *w, feats_tiled, beam_width, max_steps, (long long)eos_id, workspace, workspace_bytes,
-                                  reinterpret_cast<long long*>(seq_out), n_steps_out, ST(stream));
+    return dec::decode<decltype(t)>(dd, *w, feats_tiled, dec::DecodeMode::BEAM, beam_width, max_steps, 1.f, (long long)eos_id, nullptr,
+                                    nullptr, workspace, workspace_bytes, reinterpret_cast<long long*>(seq_out), nullptr, nullptr,
+                                    n_steps_out, ST(stream));
   });
 }
 
 int64_t recnet_sample_workspace_bytes(const recnet_decoder_desc* d, int max_steps) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
-  DecDesc d1 = dd; d1.L = 1;
-  RN_TRY(dec::check(d1));
-  if (max_steps < 1 || max_steps > 64) return RECNET_ERR_BAD_SHAPE;
-  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED,
-                          [&](auto t) { return (int64_t)dec::plan_sample<decltype(t)>(dd, nullptr, max_steps).bytes; });
+  const unsigned long long pair[2] = {0, 0};      // a query has no temperature, Gumbel pair or dropout pair: checked as valid ones
+  RN_TRY(dec::check_decode(&dd, dec::DecodeMode::SAMPLE, 1, max_steps, 1.f, pair, pair));
+  return by_prec<int64_t>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
+    return (int64_t)dec::plan_decode<decltype(t)>(dd, nullptr, dec::DecodeMode::SAMPLE, max_steps).bytes;
+  });
 }
 int recnet_decoder_sample(const recnet_decoder_desc* d, const recnet_decoder_tensors* w, const float* feats, int max_steps,
                           float temperature, int64_t eos_id, const unsigned long long* rng, const unsigned long long* noise,
@@ -416,9 +420,11 @@ int recnet_decoder_sample(const recnet_decoder_desc* d, const recnet_decoder_ten
                           int32_t* n_steps_out, void* stream) {
   DecDesc dd;
   RN_TRY(split_desc(d, &dd));
+  RN_TRY(dec::check_decode(&dd, dec::DecodeMode::SAMPLE, 1, max_steps, temperature, noise, rng));
   return by_prec<int>(dd.precision, RECNET_ERR_UNSUPPORTED, [&](auto t) {
-    return dec::sample<decltype(t)>(dd, *w, feats, max_steps, temperature, (long long)eos_id, rng, noise, workspace, workspace_bytes,
-                                    reinterpret_cast<long long*>(ids_out), logp_out, lengths_out, n_steps_out, ST(stream));
+    return dec::decode<decltype(t)>(dd, *w, feats, dec::DecodeMode::SAMPLE, 1, max_steps, temperature, (long long)eos_id, rng, noise,
+                                    workspace, workspace_bytes, reinterpret_cast<long long*>(ids_out), logp_out, lengths_out,
+                                    n_steps_out, ST(stream));
   });
 }
 

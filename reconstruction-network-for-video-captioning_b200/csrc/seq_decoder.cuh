@@ -409,8 +409,17 @@ static int backward(const DecDesc& d, const recnet_decoder_tensors& p, const flo
   return 0;
 }
 
-// ---- greedy decoding (eval.py:19-33) ---------------------------------------------------------------------------
-// argmax over the vocabulary (lowest index wins ties, like topk(1)), feeds the id back as next token, all on device.
+// ---- decoding: greedy, beam search and sampling as device loops ------------------------------------------------------------------
+// One butterfly step (lane distance o) of a warp's arg-max over (value, index) pairs: the larger value wins, the lower index on ties
+// (like topk(1)).  *carry, if given, moves with the winning pair.
+__device__ __forceinline__ void argmax_shfl(float& best, int& bi, int o, float* carry = nullptr) {
+  const float ob = __shfl_xor_sync(0xffffffffu, best, o);
+  const float oc = carry ? __shfl_xor_sync(0xffffffffu, *carry, o) : 0.f;
+  const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+  if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; if (carry) *carry = oc; }
+}
+
+// greedy (eval.py:19-33): argmax over the vocabulary (lowest index wins ties), fed back as the next token.
 __global__ void argmax_feedback_kernel(const float* __restrict__ logits, long long ld, int V, long long* __restrict__ ids_out,
                                        long long* __restrict__ next_tok, int* __restrict__ nonpad_count) {
   __shared__ float sv[32];
@@ -422,21 +431,13 @@ __global__ void argmax_feedback_kernel(const float* __restrict__ logits, long lo
     const float x = z[v];
     if (x > best || (x == best && v < bi)) { best = x; bi = v; }
   }
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-    if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-  }
+  for (int o = 16; o > 0; o >>= 1) argmax_shfl(best, bi, o);
   const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5, nw = blockDim.x >> 5;
   if (lane == 0) { sv[wp] = best; si[wp] = bi; }
   __syncthreads();
   if (wp == 0) {
     best = lane < nw ? sv[lane] : -INFINITY; bi = lane < nw ? si[lane] : 0x7fffffff;
-    for (int o = 16; o > 0; o >>= 1) {
-      const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-      const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-      if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-    }
+    for (int o = 16; o > 0; o >>= 1) argmax_shfl(best, bi, o);
     if (lane == 0) {
       ids_out[b] = bi; next_tok[b] = bi;
       if (bi != 0) atomicAdd(nonpad_count, 1);
@@ -454,77 +455,7 @@ __global__ void fill_tokens_kernel(long long* tok, int n, long long v) {
   if (i < n) tok[i] = v;
 }
 
-template <typename T>
-struct GreedyWs { Ws<T> w; long long* tok; int* nonpad; float* h_scratch; size_t bytes; };
-
-template <typename T>
-static GreedyWs<T> plan_greedy(const recnet_decoder_desc& d, void* base, int max_steps) {
-  GreedyWs<T> g;
-  recnet_decoder_desc d1 = d; d1.L = 1;
-  g.w = plan<T>(d1, base);
-  Bump m(base); m.off = g.w.bytes;
-  g.tok = m.take<long long>(d.B);
-  g.nonpad = m.take<int>(max_steps);
-  g.h_scratch = m.take<float>((size_t)d.B * d.H);
-  g.bytes = m.off + 256;
-  return g;
-}
-
-// zero initial state of the decode loops: both blocks of X and c, and of every X_x / c_x in a stack
-template <typename T>
-static int zero_decode_state(const DecDesc& d, Ws<T>& w, cudaStream_t st) {
-  const int B = d.B, H = d.H;
-  RN_CUDA_OK(cudaMemsetAsync(w.X, 0, (size_t)2 * B * w.KX * sizeof(T), st));
-  RN_CUDA_OK(cudaMemsetAsync(w.c, 0, (size_t)2 * B * H * sizeof(float), st));
-  for (int l = 1; l < w.NL; ++l) {
-    RN_CUDA_OK(cudaMemsetAsync(w.X_x[l - 1], 0, (size_t)2 * B * 2 * H * sizeof(T), st));
-    RN_CUDA_OK(cudaMemsetAsync(w.c_x[l - 1], 0, (size_t)2 * B * H * sizeof(float), st));
-  }
-  return 0;
-}
-
-template <typename T>
-static int greedy(const DecDesc& d0, const recnet_decoder_tensors& p, const float* feats, int max_steps, void* ws,
-                  long long ws_bytes, long long* ids_out, int* n_steps_out, cudaStream_t st) {
-  DecDesc d = d0; d.L = 1; d.train = 0;
-  RN_TRY(check(d));
-  GreedyWs<T> g = plan_greedy<T>(d0, ws, max_steps);
-  if ((long long)g.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
-  Ws<T>& w = g.w;
-  const int B = d.B, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, NL = w.NL;
-  RN_TRY(prepare<T>(d, p, feats, w, st));
-  RN_TRY(gemm_full<T>(w.feats, E, 0, w.U, E, 0, w.Uv, A, nullptr, B * Tn, A, E, 0, w.splitk, st));
-  RN_TRY(zero_decode_state<T>(d, w, st));
-  RN_CUDA_OK(cudaMemsetAsync(g.nonpad, 0, (size_t)max_steps * sizeof(int), st));
-  fill_tokens_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(g.tok, B, 1 /* <SOS> */);
-  RN_LAUNCH_OK();
-  // ping-pong the two blocks of every X / c buffer of the L=1 plan: step t reads block t & 1 and writes block (t + 1) & 1.  The top
-  // layer's h (attention query, vocabulary projection) sits at the same place in either block (top_h).
-  long long ldq;
-  const T* Htop = top_h(d, w, &ldq);
-  for (int t = 0; t < max_steps; ++t) {
-    const int rd = t & 1, wr = (t + 1) & 1;
-    T* x_t = w.X + (size_t)rd * B * w.KX;
-    T* x_n = w.X + (size_t)wr * B * w.KX;
-    float* c_p = w.c + (size_t)rd * B * H;
-    float* c_n = w.c + (size_t)wr * B * H;
-    misc::embed_gather_kernel<T><<<B, 128, 0, st>>>(p.embedding, g.tok, w.Xe, w.EMBp, B, d.EMB, w.EMBp, V, d.embedding_scale, 0.f,
-                                                    nullptr, SITE_EMB);
-    RN_LAUNCH_OK();
-    RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
-    // GRU keeps its fp32 state h in the c ping-pong rows (h_prev = c_p, h' -> c_n)
-    RN_TRY(step<T>(d, p, w, t, Htop + (size_t)rd * B * ldq, ldq, w.Gx, x_t, x_n, nullptr, nullptr, nullptr, c_p, c_n,
-                   d.cell == RECNET_CELL_GRU ? c_n : g.h_scratch, st, NL > 1 ? w.X_x[0] + (size_t)rd * B * 2 * H : nullptr));
-    RN_TRY(upper_layers<T>(d, p, w, t, rd, wr, nullptr, 0.f, nullptr, st));
-    RN_TRY(gemm_full<T>(Htop + (size_t)wr * B * ldq, ldq, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
-    argmax_feedback_kernel<<<B, 256, 0, st>>>(w.logits, w.Vld, V, ids_out + (size_t)t * B, g.tok, g.nonpad + t);
-    RN_LAUNCH_OK();
-  }
-  greedy_finalize_kernel<<<1, 1, 0, st>>>(g.nonpad, max_steps, n_steps_out);
-  RN_LAUNCH_OK();
-  return 0;
-}
-// ---- beam search (eval.beam_search, eval.py:36-120) as a device loop: zero host syncs ------------------------------------------
+// ---- beam search (eval.beam_search, eval.py:36-120) -----------------------------------------------------------------------------
 // Rows of every per-step tensor are (beam k, sample b) -> k * B0 + b; the caller passes the features tiled K times.  Per step: the
 // decoder step on all K * B0 rows (same kernels as greedy), then ONE selection kernel per sample -- scores log(sigmoid(logit)) +
 // cum / len^0.7 (eval.py:53-61: the running score is divided by the length at EVERY step; len = position of the last <EOS> + 1 once
@@ -564,20 +495,12 @@ __global__ void beam_select_kernel(const float* __restrict__ logits, long long l
       const float sc = logf(1.f / (1.f + expf(-x))) + base[i];
       if (sc > best || (sc == best && f < bi)) { best = sc; bi = f; }
     }
-    for (int o = 16; o > 0; o >>= 1) {
-      const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-      const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-      if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-    }
+    for (int o = 16; o > 0; o >>= 1) argmax_shfl(best, bi, o);
     if (lane == 0) { sv[warp] = best; si[warp] = bi; }
     __syncthreads();
     if (warp == 0) {
       best = lane < BEAM_THREADS / 32 ? sv[lane] : -INFINITY; bi = lane < BEAM_THREADS / 32 ? si[lane] : 0x7fffffff;
-      for (int o = 16; o > 0; o >>= 1) {
-        const float ob = __shfl_xor_sync(0xffffffffu, best, o);
-        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-        if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; }
-      }
+      for (int o = 16; o > 0; o >>= 1) argmax_shfl(best, bi, o);
       if (lane == 0) {
         chosen[k] = bi;
         const int i = bi / V, v = bi - i * V;
@@ -599,20 +522,9 @@ __global__ void beam_select_kernel(const float* __restrict__ logits, long long l
   if (tid == 0 && n_nonpad) atomicAdd(nonpad + t, n_nonpad);
 }
 
-// recurrent state of row (k, b) <- state of row (src[b][k], b): h operand rows (ld elements apart) and the fp32 state rows
-template <typename T>
-__global__ void beam_gather_kernel(const T* __restrict__ h_src, T* __restrict__ h_dst, long long ld, const float* __restrict__ c_src,
-                                   float* __restrict__ c_dst, int H, int B0, int K, const int* __restrict__ src, const int* __restrict__ nonpad, int t) {
-  if (t > 0 && nonpad[t - 1] == 0) return;                  // frozen (see beam_select_kernel)
-  const int row = blockIdx.x, k = row / B0, b = row - k * B0;
-  const int srow = src[b * K + k] * B0 + b;
-  for (int j = threadIdx.x; j < H; j += blockDim.x) {
-    h_dst[(long long)row * ld + j] = h_src[(long long)srow * ld + j];
-    c_dst[(long long)row * H + j] = c_src[(long long)srow * H + j];
-  }
-}
-// the same for every layer of a stack in one launch: layer 0's h rows (ld KX) and c, layer l's h (second half of the X_x[l-1] rows,
-// ld 2H) and c_x[l-1].  The input-slot halves need no gather: every step rewrites them before it reads them.
+// recurrent state of row (k, b) <- state of row (src[b][k], b), every layer in one launch: layer 0's h rows (ld KX) and c, layer l's
+// h (second half of the X_x[l-1] rows, ld 2H) and c_x[l-1].  The input-slot halves need no gather: every step rewrites them before it
+// reads them.
 template <typename T>
 struct BeamStateRows {
   const T* h_src[RECNET_MAX_LAYERS]; T* h_dst[RECNET_MAX_LAYERS]; long long ld[RECNET_MAX_LAYERS];
@@ -650,85 +562,7 @@ __global__ void beam_init_kernel(float* cum, int* eos, int n) {
   if (i < n) { cum[i] = 0.f; eos[i] = -1; }                  // log(1.) ; no <EOS> yet
 }
 
-template <typename T>
-struct BeamWs { GreedyWs<T> g; float* cum[2]; int* eos[2]; int* seq[2]; int* src; size_t bytes; };
-template <typename T>
-static BeamWs<T> plan_beam(const recnet_decoder_desc& d, void* base, int K, int max_steps) {
-  BeamWs<T> w;
-  w.g = plan_greedy<T>(d, base, max_steps);
-  Bump m(base); m.off = w.g.bytes;
-  const int B0 = d.B / (K > 0 ? K : 1);
-  for (int i = 0; i < 2; ++i) {
-    w.cum[i] = m.take<float>((size_t)d.B);
-    w.eos[i] = m.take<int>((size_t)d.B);
-    w.seq[i] = m.take<int>((size_t)d.B * max_steps);
-  }
-  w.src = m.take<int>((size_t)d.B);
-  (void)B0;
-  w.bytes = m.off + 256;
-  return w;
-}
-
-// d0.B = K * B0 rows; feats [K * B0, T, E] = the B0 samples tiled K times; seq_out [B0, max_steps] int64 (-1 beyond n_steps)
-template <typename T>
-static int beam(const DecDesc& d0, const recnet_decoder_tensors& p, const float* feats, int K, int max_steps, long long eos,
-                void* ws, long long ws_bytes, long long* seq_out, int* n_steps_out, cudaStream_t st) {
-  DecDesc d = d0; d.L = 1; d.train = 0;
-  RN_TRY(check(d));
-  if (K < 1 || K > BEAM_MAX_K || d.B % K || max_steps < 1 || max_steps > 64 || K > d.V) return RECNET_ERR_BAD_SHAPE;
-  BeamWs<T> bw = plan_beam<T>(d0, ws, K, max_steps);
-  if ((long long)bw.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
-  GreedyWs<T>& g = bw.g;
-  Ws<T>& w = g.w;
-  const int B = d.B, B0 = B / K, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, NL = w.NL;
-  RN_TRY(prepare<T>(d, p, feats, w, st));
-  RN_TRY(gemm_full<T>(w.feats, E, 0, w.U, E, 0, w.Uv, A, nullptr, B * Tn, A, E, 0, w.splitk, st));
-  RN_TRY(zero_decode_state<T>(d, w, st));
-  RN_CUDA_OK(cudaMemsetAsync(g.nonpad, 0, (size_t)max_steps * sizeof(int), st));
-  fill_tokens_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(g.tok, B, 1 /* <SOS> */);
-  RN_LAUNCH_OK();
-  beam_init_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(bw.cum[0], bw.eos[0], B);
-  RN_LAUNCH_OK();
-  // state buffers: step reads block 0 of every X / c buffer (x0, c0, ...) and writes block 1 (x1, c1, ...); the gather moves the
-  // selected beams' state back into block 0
-  T* x0 = w.X; T* x1 = w.X + (size_t)B * w.KX;
-  float* c0 = w.c; float* c1 = w.c + (size_t)B * H;
-  long long ldq;
-  const T* Htop = top_h(d, w, &ldq);
-  BeamStateRows<T> rows{};                 // a stack's gather: h (own recurrent slot) and c of every layer
-  rows.n = NL;
-  for (int l = 0; l < NL; ++l) {
-    T* h = l == 0 ? w.X + E : w.X_x[l - 1] + H;
-    float* c = l == 0 ? w.c : w.c_x[l - 1];
-    rows.ld[l] = l == 0 ? w.KX : 2 * H;
-    rows.h_dst[l] = h; rows.h_src[l] = h + (size_t)B * rows.ld[l];
-    rows.c_dst[l] = c; rows.c_src[l] = c + (size_t)B * H;
-  }
-  for (int t = 0; t < max_steps; ++t) {
-    misc::embed_gather_kernel<T><<<B, 128, 0, st>>>(p.embedding, g.tok, w.Xe, w.EMBp, B, d.EMB, w.EMBp, V, d.embedding_scale, 0.f,
-                                                    nullptr, SITE_EMB);
-    RN_LAUNCH_OK();
-    RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
-    RN_TRY(step<T>(d, p, w, t, Htop, ldq, w.Gx, x0, x1, nullptr, nullptr, nullptr, c0, c1, d.cell == RECNET_CELL_GRU ? c1 : g.h_scratch,
-                   st, NL > 1 ? w.X_x[0] : nullptr));
-    RN_TRY(upper_layers<T>(d, p, w, t, 0, 1, nullptr, 0.f, nullptr, st));
-    RN_TRY(gemm_full<T>(Htop + (size_t)B * ldq, ldq, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
-    const int in = t & 1, out = (t + 1) & 1;
-    beam_select_kernel<<<B0, BEAM_THREADS, 0, st>>>(w.logits, w.Vld, V, B0, K, t, max_steps, eos, bw.cum[in], bw.cum[out], bw.eos[in], bw.eos[out],
-                                                    bw.seq[in], bw.seq[out], g.tok, bw.src, g.nonpad);
-    RN_LAUNCH_OK();
-    if (NL == 1)
-      beam_gather_kernel<T><<<B, 128, 0, st>>>(x1 + E, x0 + E, w.KX, c1, c0, H, B0, K, bw.src, g.nonpad, t);
-    else
-      beam_gather_layers_kernel<T><<<B, 128, 0, st>>>(rows, H, B0, K, bw.src, g.nonpad, t);
-    RN_LAUNCH_OK();
-  }
-  beam_finalize_kernel<<<1, 256, 0, st>>>(g.nonpad, max_steps, B0, K, bw.seq[0], bw.seq[1], seq_out, n_steps_out);
-  RN_LAUNCH_OK();
-  return 0;
-}
-
-// ---- sampling (Gumbel-max) as a device loop: stochastic decoding and the sampling half of self-critical training ----------------
+// ---- sampling (Gumbel-max): stochastic decoding and the sampling half of self-critical training ---------------------------------
 // Per step: the decoder step on all rows (the kernels of greedy, plus the training-mode dropout masks when desc.train is set), then
 // ONE selection kernel that draws a token per row from softmax(z' / tau) by Gumbel-max, z' = the logits after their dropout.  Every
 // dropout mask is drawn at the element index the sequence forward (dec::forward) uses for row t * B + row, so a teacher-forced pass
@@ -751,9 +585,7 @@ __device__ __forceinline__ void lse_merge(float& m, float& s, float om, float os
   m = M;
 }
 __device__ __forceinline__ void sample_reduce_step(float& best, int& bi, float& bx, float& m, float& s, int o) {
-  const float ob = __shfl_xor_sync(0xffffffffu, best, o), ox = __shfl_xor_sync(0xffffffffu, bx, o);
-  const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-  if (ob > best || (ob == best && oi < bi)) { best = ob; bi = oi; bx = ox; }
+  argmax_shfl(best, bi, o, &bx);
   const float om = __shfl_xor_sync(0xffffffffu, m, o), os = __shfl_xor_sync(0xffffffffu, s, o);
   lse_merge(m, s, om, os);
 }
@@ -822,46 +654,128 @@ __global__ void sample_init_kernel(long long* tok, int* finished, int* lengths, 
   if (i < n) { tok[i] = 1; finished[i] = 0; lengths[i] = max_steps; }    // <SOS>; a row that never finishes has max_steps tokens
 }
 
+// ---- the decode loop ------------------------------------------------------------------------------------------------------------
+enum class DecodeMode { GREEDY, BEAM, SAMPLE };
+
+// Workspace of a decode call: the sequence plan at L = 1 (X and c hold the two state blocks a step reads and writes), then the fed-back
+// tokens, the per-step counts of non-<PAD> tokens (of unfinished rows when sampling) and the h rows nobody reads; beam search adds its
+// scores, <EOS> positions and sequences (two of each: step t reads t & 1, writes (t + 1) & 1) and the source beams, sampling the
+// rows' finished flags.
 template <typename T>
-struct SampleWs { GreedyWs<T> g; int* finished; size_t bytes; };
+struct DecodeWs {
+  Ws<T> w; long long* tok; int* nonpad; float* h_scratch;
+  float* cum[2]; int* eos[2]; int* seq[2]; int* src;       // beam search
+  int* finished;                                            // sampling
+  size_t bytes;
+};
 template <typename T>
-static SampleWs<T> plan_sample(const recnet_decoder_desc& d, void* base, int max_steps) {
-  SampleWs<T> s;
-  s.g = plan_greedy<T>(d, base, max_steps);
-  Bump m(base); m.off = s.g.bytes;
-  s.finished = m.take<int>((size_t)d.B);
-  s.bytes = m.off + 256;
-  return s;
+static DecodeWs<T> plan_decode(const recnet_decoder_desc& d, void* base, DecodeMode mode, int max_steps) {
+  DecodeWs<T> g{};
+  recnet_decoder_desc d1 = d; d1.L = 1;
+  g.w = plan<T>(d1, base);
+  Bump m(base); m.off = g.w.bytes;
+  g.tok = m.take<long long>(d.B);
+  g.nonpad = m.take<int>(max_steps);
+  g.h_scratch = m.take<float>((size_t)d.B * d.H);
+  if (mode != DecodeMode::GREEDY) m.off += 256;            // 256 bytes of slack after the greedy buffers, as after the sequence plan
+  if (mode == DecodeMode::BEAM) {
+    for (int i = 0; i < 2; ++i) {
+      g.cum[i] = m.take<float>((size_t)d.B);
+      g.eos[i] = m.take<int>((size_t)d.B);
+      g.seq[i] = m.take<int>((size_t)d.B * max_steps);
+    }
+    g.src = m.take<int>((size_t)d.B);
+  } else if (mode == DecodeMode::SAMPLE) {
+    g.finished = m.take<int>((size_t)d.B);
+  }
+  g.bytes = m.off + 256;
+  return g;
 }
 
-// ids_out / logp_out [max_steps, B], lengths_out [B] = sampled tokens of the row, the finishing one included; n_steps_out = the step at
-// which the last row finished + 1 (max_steps if a row never finishes).  rng = the dropout pair (read when d0.train is set),
-// noise = the Gumbel pair.  Always the general step path: greedy_pf hoists the embedding projection and could not drop the embedding.
+// The argument checks of the decode entry points and their workspace queries, all before anything is launched.  Greedy checks max_steps
+// before the descriptor, beam search and sampling after it.  d = nullptr leaves out every check that reads the descriptor: the greedy
+// and beam workspace queries answer for any descriptor.  A decode call ignores the descriptor's L.
+static inline int check_decode(const DecDesc* d, DecodeMode mode, int K, int max_steps, float tau, const unsigned long long* noise,
+                               const unsigned long long* rng) {
+  const bool steps_ok = max_steps >= 1 && max_steps <= 64;
+  if (mode == DecodeMode::GREEDY && !steps_ok) return RECNET_ERR_BAD_SHAPE;
+  if (d) {
+    DecDesc d1 = *d; d1.L = 1;
+    RN_TRY(check(d1));
+  }
+  if (!steps_ok) return RECNET_ERR_BAD_SHAPE;
+  if (mode == DecodeMode::BEAM && (K < 1 || K > BEAM_MAX_K || (d && (d->B % K || K > d->V)))) return RECNET_ERR_BAD_SHAPE;
+  if (mode == DecodeMode::SAMPLE && (!(tau > 0.f) || !noise || (d && d->train && !rng))) return RECNET_ERR_BAD_SHAPE;
+  return 0;
+}
+
+// zero initial state of the decode loops: both blocks of X and c, and of every X_x / c_x in a stack
 template <typename T>
-static int sample(const DecDesc& d0, const recnet_decoder_tensors& p, const float* feats, int max_steps, float tau, long long eos,
-                  const unsigned long long* rng, const unsigned long long* noise, void* ws, long long ws_bytes, long long* ids_out,
-                  float* logp_out, int* lengths_out, int* n_steps_out, cudaStream_t st) {
+static int zero_decode_state(const DecDesc& d, Ws<T>& w, cudaStream_t st) {
+  const int B = d.B, H = d.H;
+  RN_CUDA_OK(cudaMemsetAsync(w.X, 0, (size_t)2 * B * w.KX * sizeof(T), st));
+  RN_CUDA_OK(cudaMemsetAsync(w.c, 0, (size_t)2 * B * H * sizeof(float), st));
+  for (int l = 1; l < w.NL; ++l) {
+    RN_CUDA_OK(cudaMemsetAsync(w.X_x[l - 1], 0, (size_t)2 * B * 2 * H * sizeof(T), st));
+    RN_CUDA_OK(cudaMemsetAsync(w.c_x[l - 1], 0, (size_t)2 * B * H * sizeof(float), st));
+  }
+  return 0;
+}
+
+// One decode call on the general step path, the whole loop on the device with no host sync; the arguments passed check_decode.
+//   GREEDY: ids_out [max_steps, B]; n_steps_out = the first step (1-based) after which every fed-back token was <PAD> (eval.py:30),
+//           else max_steps.
+//   BEAM:   d0.B = K * B0 rows, feats [K * B0, T, E] = the B0 samples tiled K times; ids_out [B0, max_steps] = the top-1 sequences
+//           (-1 beyond n_steps), n_steps_out as for greedy.
+//   SAMPLE: ids_out / logp_out [max_steps, B], lengths_out [B] = sampled tokens of the row, the finishing one included; n_steps_out =
+//           the step at which the last row finished + 1 (max_steps if a row never finishes).  In train mode (d0.train) every dropout
+//           mask is drawn from the pair rng; noise = the Gumbel pair.
+// Greedy and beam search decode in eval mode.  Sampling always runs here: greedy_pf hoists the embedding projection and could not drop
+// the embedding.
+template <typename T>
+static int decode(const DecDesc& d0, const recnet_decoder_tensors& p, const float* feats, DecodeMode mode, int K, int max_steps,
+                  float tau, long long eos, const unsigned long long* rng, const unsigned long long* noise, void* ws, long long ws_bytes,
+                  long long* ids_out, float* logp_out, int* lengths_out, int* n_steps_out, cudaStream_t st) {
   DecDesc d = d0; d.L = 1;
-  RN_TRY(check(d));
-  if (max_steps < 1 || max_steps > 64 || !(tau > 0.f) || !noise || (d.train && !rng)) return RECNET_ERR_BAD_SHAPE;
-  SampleWs<T> sw = plan_sample<T>(d0, ws, max_steps);
-  if ((long long)sw.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
-  GreedyWs<T>& g = sw.g;
+  if (mode != DecodeMode::SAMPLE) d.train = 0;
+  DecodeWs<T> g = plan_decode<T>(d0, ws, mode, max_steps);
+  if ((long long)g.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
   Ws<T>& w = g.w;
-  const int B = d.B, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, NL = w.NL;
+  const bool beam = mode == DecodeMode::BEAM;
+  const int B = d.B, B0 = B / K, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, NL = w.NL;
   const float p_emb = d.train ? d.p_emb_drop : 0.f, p_out = d.train ? d.p_out_drop : 0.f, p_lay = d.train ? d.p_layer_drop : 0.f;
   RN_TRY(prepare<T>(d, p, feats, w, st));
   RN_TRY(gemm_full<T>(w.feats, E, 0, w.U, E, 0, w.Uv, A, nullptr, B * Tn, A, E, 0, w.splitk, st));
   RN_TRY(zero_decode_state<T>(d, w, st));
-  RN_CUDA_OK(cudaMemsetAsync(g.nonpad, 0, (size_t)max_steps * sizeof(int), st));        // live rows per step
-  RN_CUDA_OK(cudaMemsetAsync(ids_out, 0, (size_t)max_steps * B * sizeof(long long), st));
-  RN_CUDA_OK(cudaMemsetAsync(logp_out, 0, (size_t)max_steps * B * sizeof(float), st));
-  sample_init_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(g.tok, sw.finished, lengths_out, B, max_steps);
+  RN_CUDA_OK(cudaMemsetAsync(g.nonpad, 0, (size_t)max_steps * sizeof(int), st));
+  if (mode == DecodeMode::SAMPLE) {
+    RN_CUDA_OK(cudaMemsetAsync(ids_out, 0, (size_t)max_steps * B * sizeof(long long), st));
+    RN_CUDA_OK(cudaMemsetAsync(logp_out, 0, (size_t)max_steps * B * sizeof(float), st));
+    sample_init_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(g.tok, g.finished, lengths_out, B, max_steps);
+  } else {
+    fill_tokens_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(g.tok, B, 1 /* <SOS> */);
+  }
   RN_LAUNCH_OK();
+  if (beam) {
+    beam_init_kernel<<<rn_cdiv(B, 128), 128, 0, st>>>(g.cum[0], g.eos[0], B);
+    RN_LAUNCH_OK();
+  }
   long long ldq;
   const T* Htop = top_h(d, w, &ldq);
-  for (int t = 0; t < max_steps; ++t) {                      // the ping-pong of greedy
-    const int rd = t & 1, wr = (t + 1) & 1;
+  BeamStateRows<T> rows{};                 // beam search: h (own recurrent slot) and c of every layer, block 1 -> block 0
+  rows.n = NL;
+  for (int l = 0; l < NL; ++l) {
+    T* h = l == 0 ? w.X + E : w.X_x[l - 1] + H;
+    float* c = l == 0 ? w.c : w.c_x[l - 1];
+    rows.ld[l] = l == 0 ? w.KX : 2 * H;
+    rows.h_dst[l] = h; rows.h_src[l] = h + (size_t)B * rows.ld[l];
+    rows.c_dst[l] = c; rows.c_src[l] = c + (size_t)B * H;
+  }
+  for (int t = 0; t < max_steps; ++t) {
+    // Greedy and sampling ping-pong the two blocks of every X / c buffer: step t reads block t & 1 and writes block (t + 1) & 1.  Beam
+    // search reads block 0 and writes block 1, and its gather moves the selected beams' state back into block 0.  The top layer's h
+    // (attention query, vocabulary projection) sits at the same place in either block (top_h).
+    const int rd = beam ? 0 : t & 1, wr = beam ? 1 : (t + 1) & 1;
     T* x_t = w.X + (size_t)rd * B * w.KX;
     T* x_n = w.X + (size_t)wr * B * w.KX;
     float* c_p = w.c + (size_t)rd * B * H;
@@ -870,15 +784,29 @@ static int sample(const DecDesc& d0, const recnet_decoder_tensors& p, const floa
                                                     rng, SITE_EMB, (long long)t * B);
     RN_LAUNCH_OK();
     RN_TRY(gemm_full<T>(w.Xe, w.EMBp, 0, w.Wemb, w.EMBp, 0, w.Gx, w.G * H, p.b_ih, B, w.G * H, w.EMBp, 0, w.splitk, st));
+    // GRU keeps its fp32 state h in the c rows (h_prev = c_p, h' -> c_n)
     RN_TRY(step<T>(d, p, w, t, Htop + (size_t)rd * B * ldq, ldq, w.Gx, x_t, x_n, nullptr, nullptr, nullptr, c_p, c_n,
                    d.cell == RECNET_CELL_GRU ? c_n : g.h_scratch, st, NL > 1 ? w.X_x[0] + (size_t)rd * B * 2 * H : nullptr, rng));
     RN_TRY(upper_layers<T>(d, p, w, t, rd, wr, nullptr, p_lay, rng, st));
     RN_TRY(gemm_full<T>(Htop + (size_t)wr * B * ldq, ldq, 0, w.Wout, H, 0, w.logits, w.Vld, p.out_b, B, V, H, 0, w.splitk, st));
-    sample_select_kernel<<<B, SAMPLE_THREADS, 0, st>>>(w.logits, w.Vld, V, B, t, tau, eos, p_out, rng, noise, ids_out + (size_t)t * B,
-                                                       logp_out + (size_t)t * B, g.tok, sw.finished, lengths_out, g.nonpad);
+    if (mode == DecodeMode::GREEDY) {
+      argmax_feedback_kernel<<<B, 256, 0, st>>>(w.logits, w.Vld, V, ids_out + (size_t)t * B, g.tok, g.nonpad + t);
+    } else if (mode == DecodeMode::SAMPLE) {
+      sample_select_kernel<<<B, SAMPLE_THREADS, 0, st>>>(w.logits, w.Vld, V, B, t, tau, eos, p_out, rng, noise, ids_out + (size_t)t * B,
+                                                         logp_out + (size_t)t * B, g.tok, g.finished, lengths_out, g.nonpad);
+    } else {
+      const int in = t & 1, out = (t + 1) & 1;
+      beam_select_kernel<<<B0, BEAM_THREADS, 0, st>>>(w.logits, w.Vld, V, B0, K, t, max_steps, eos, g.cum[in], g.cum[out], g.eos[in],
+                                                      g.eos[out], g.seq[in], g.seq[out], g.tok, g.src, g.nonpad);
+      RN_LAUNCH_OK();
+      beam_gather_layers_kernel<T><<<B, 128, 0, st>>>(rows, H, B0, K, g.src, g.nonpad, t);
+    }
     RN_LAUNCH_OK();
   }
-  greedy_finalize_kernel<<<1, 1, 0, st>>>(g.nonpad, max_steps, n_steps_out);   // first step with no live row, + 1
+  if (beam)
+    beam_finalize_kernel<<<1, 256, 0, st>>>(g.nonpad, max_steps, B0, K, g.seq[0], g.seq[1], ids_out, n_steps_out);
+  else
+    greedy_finalize_kernel<<<1, 1, 0, st>>>(g.nonpad, max_steps, n_steps_out);
   RN_LAUNCH_OK();
   return 0;
 }

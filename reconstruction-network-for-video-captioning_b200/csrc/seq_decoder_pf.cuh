@@ -296,7 +296,8 @@ static int backward_pf(const DecDesc& d, const recnet_decoder_tensors& p, const 
 // 4 launches per step instead of 8: the embedding half of the gate projection is a GATHER from EW = Embedding . W_emb^T + b_ih
 // (one [V x 4H x EMB] GEMM per call; eval mode has no dropout), the context half is the hoisted VW (as in training), so a step is
 //   h_{t-1} [W_a ; W_hh]^T  ->  pf_fwd_kernel (scores, context, cell; Gx row = fed-back token)  ->  vocabulary projection  ->  argmax feedback.
-// The fp32 build keeps the general path (seq_decoder.cuh:greedy): its summation order is the one the bit-exact id tests pin.
+// The fp32 build keeps the general path (seq_decoder.cuh:decode): its summation order is the one the bit-exact id tests pin.
+// The arguments passed check_decode; the <SOS> fill, the arg-max feedback and the stop step are those of decode.
 template <typename T>
 struct GreedyPfWs {
   int EMBp, Vld, NP;
@@ -344,7 +345,6 @@ static int greedy_pf(const DecDesc& d0, const recnet_decoder_tensors& p, const f
                      long long ws_bytes, long long* ids_out, int* n_steps_out, cudaStream_t st) {
   typedef bf16 T;
   DecDesc d = d0; d.L = 1; d.train = 0;
-  RN_TRY(check(d));
   GreedyPfWs<T> w = plan_greedy_pf<T>(d, ws, max_steps);
   if ((long long)w.bytes > ws_bytes) return RECNET_ERR_WORKSPACE;
   const int B = d.B, H = d.H, E = d.E, A = d.A, V = d.V, Tn = d.T, EMB = d.EMB;

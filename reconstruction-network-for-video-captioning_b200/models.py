@@ -224,24 +224,13 @@ class Decoder(nn.Module, _RngMixin):
     def greedy(self, encoder_outputs, max_steps):
         """eval.greedy_search (eval.py:19-33) on device: returns (ids (max_steps,B) int64 on device, n).  One C call for the decoders
         with a fused driver (LSTM with 1-4 layers, single-layer GRU); the others step through ``forward``."""
-        import ctypes as C
         if not self.uses_fused_sequence:
             return self._greedy_stepwise(encoder_outputs, max_steps)
-        lib = L.lib()
         feats = Fn._f32c(encoder_outputs, "encoder_outputs")
-        B, T, E = feats.shape
-        meta = self._meta()
-        d = L.decoder_desc(B=B, T=T, E=E, H=meta["H"], A=meta["A"], EMB=meta["EMB"], V=meta["V"], L=1,
-                           precision=meta["precision"], train=0, embedding_scale=float(meta["embedding_scale"]),
-                           p_emb_drop=0.0, p_out_drop=0.0, cell=meta["cell"], n_layers=self.n_layers)
-        nbytes = lib.recnet_greedy_workspace_bytes(C.byref(d))
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=feats.device)
+        B = feats.shape[0]
         ids = torch.empty(max_steps, B, dtype=torch.int64, device=feats.device)
         n = torch.zeros(1, dtype=torch.int32, device=feats.device)
-        params = tuple(Fn._f32c(p, "param") for p in self._params())
-        w = Fn._pack(L.decoder_tensors, params)
-        L.check(lib.recnet_decoder_greedy(C.byref(d), C.byref(w), feats.data_ptr(), max_steps, ws.data_ptr(), nbytes,
-                                          ids.data_ptr(), n.data_ptr(), Fn._stream()), "recnet_decoder_greedy")
+        self._decode("greedy", feats, False, (), (max_steps,), (ids, n))
         return ids, n
 
     @torch.no_grad()
@@ -271,26 +260,13 @@ class Decoder(nn.Module, _RngMixin):
     def beam(self, encoder_outputs, beam_width, max_steps, eos_id=2):
         """eval.beam_search (eval.py:36-120) as ONE C call: the whole loop, top-k and state gather included, runs on the device.
         Returns (seqs (B, max_steps) int64 on device: top-1 beam per sample, -1 beyond n; n device int32)."""
-        import ctypes as C
-        lib = L.lib()
         feats = Fn._f32c(encoder_outputs, "encoder_outputs")
-        B0, T, E = feats.shape
+        B0 = feats.shape[0]
         K = int(beam_width)
         tiled = feats.repeat(K, 1, 1).contiguous()                 # row k * B0 + b = beam k of sample b
-        meta = self._meta()
-        d = L.decoder_desc(B=B0 * K, T=T, E=E, H=meta["H"], A=meta["A"], EMB=meta["EMB"], V=meta["V"], L=1,
-                           precision=meta["precision"], train=0, embedding_scale=float(meta["embedding_scale"]),
-                           p_emb_drop=0.0, p_out_drop=0.0, cell=meta["cell"], n_layers=self.n_layers)
-        nbytes = lib.recnet_beam_workspace_bytes(C.byref(d), K, max_steps)
-        if nbytes < 0:
-            L.check(int(nbytes), "recnet_beam_workspace_bytes")
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=feats.device)
         seqs = torch.empty(B0, max_steps, dtype=torch.int64, device=feats.device)
         n = torch.zeros(1, dtype=torch.int32, device=feats.device)
-        params = tuple(Fn._f32c(p, "param") for p in self._params())
-        w = Fn._pack(L.decoder_tensors, params)
-        L.check(lib.recnet_decoder_beam(C.byref(d), C.byref(w), tiled.data_ptr(), K, max_steps, int(eos_id), ws.data_ptr(), nbytes,
-                                        seqs.data_ptr(), n.data_ptr(), Fn._stream()), "recnet_decoder_beam")
+        self._decode("beam", tiled, False, (K, max_steps), (K, max_steps, int(eos_id)), (seqs, n))
         return seqs, n
 
     @torch.no_grad()
@@ -316,30 +292,38 @@ class Decoder(nn.Module, _RngMixin):
 
     def _sample(self, feats, max_steps, temperature, eos_id, noise):
         """``sample`` on rows that are already tiled, with the Gumbel (seed, offset) pair `noise` given as a device int64 (2,) tensor."""
-        import ctypes as C
-        lib = L.lib()
-        N, T, E = feats.shape
-        meta = self._meta()
-        d = L.decoder_desc(B=N, T=T, E=E, H=meta["H"], A=meta["A"], EMB=meta["EMB"], V=meta["V"], L=1,
-                           precision=meta["precision"], train=int(self.training), embedding_scale=float(meta["embedding_scale"]),
-                           p_emb_drop=float(meta["p_emb"]), p_out_drop=float(meta["p_out"]), cell=meta["cell"], n_layers=self.n_layers,
-                           p_layer_drop=float(meta["p_layer"]))
-        nbytes = lib.recnet_sample_workspace_bytes(C.byref(d), int(max_steps))
-        if nbytes < 0:
-            L.check(int(nbytes), "recnet_sample_workspace_bytes")
+        N = feats.shape[0]
         dev = feats.device
-        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
         ids = torch.empty(max_steps, N, dtype=torch.int64, device=dev)
         logp = torch.empty(max_steps, N, dtype=torch.float32, device=dev)
         lengths = torch.empty(N, dtype=torch.int32, device=dev)
         n = torch.zeros(1, dtype=torch.int32, device=dev)
         rng = self._next_rng() if self.training else None
+        self._decode("sample", feats, self.training, (int(max_steps),),
+                     (int(max_steps), float(temperature), int(eos_id), Fn._ptr(rng), noise.data_ptr()), (ids, logp, lengths, n))
+        return ids, logp, lengths, n
+
+    def _decode(self, kind, feats, train, query_args, args, outs):
+        """One device decode call on the rows of ``feats`` (kind: greedy, beam or sample): the descriptor (L = 1, train mode only when
+        ``train``), a workspace sized by recnet_<kind>_workspace_bytes(desc, *query_args), the packed parameters, then
+        recnet_decoder_<kind>(desc, params, feats, *args, workspace, its size, *outs, stream)."""
+        import ctypes as C
+        lib = L.lib()
+        N, T, E = feats.shape
+        meta = self._meta()
+        d = L.decoder_desc(B=N, T=T, E=E, H=meta["H"], A=meta["A"], EMB=meta["EMB"], V=meta["V"], L=1,
+                           precision=meta["precision"], train=int(train), embedding_scale=float(meta["embedding_scale"]),
+                           p_emb_drop=float(meta["p_emb"]), p_out_drop=float(meta["p_out"]), cell=meta["cell"], n_layers=self.n_layers,
+                           p_layer_drop=float(meta["p_layer"]))
+        query = f"recnet_{kind}_workspace_bytes"
+        nbytes = getattr(lib, query)(C.byref(d), *query_args)
+        if nbytes < 0:
+            L.check(int(nbytes), query)
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=feats.device)
         params = tuple(Fn._f32c(p, "param") for p in self._params())
         w = Fn._pack(L.decoder_tensors, params)
-        L.check(lib.recnet_decoder_sample(C.byref(d), C.byref(w), feats.data_ptr(), int(max_steps), float(temperature), int(eos_id),
-                                          Fn._ptr(rng), noise.data_ptr(), ws.data_ptr(), nbytes, ids.data_ptr(), logp.data_ptr(),
-                                          lengths.data_ptr(), n.data_ptr(), Fn._stream()), "recnet_decoder_sample")
-        return ids, logp, lengths, n
+        L.check(getattr(lib, f"recnet_decoder_{kind}")(C.byref(d), C.byref(w), feats.data_ptr(), *args, ws.data_ptr(), nbytes,
+                                                      *(t.data_ptr() for t in outs), Fn._stream()), f"recnet_decoder_{kind}")
 
     # ---- single timestep (reference API) ----
     def forward(self, input, hidden, encoder_outputs):
